@@ -15,6 +15,7 @@ with an in-run parity check against the oracle on every line.
 
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
   python bench.py --impl reference ...                    # CPU restatement of the reference (oracle/)
+  python bench.py ... --dump-outputs DIR                  # + the last timed step's index and hits as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -164,6 +165,74 @@ def sample_index_masses(g, n_entries: int, chunks: int = 64, chunk: int = 2048) 
         c = min(chunk, n_entries - b)
         out.append(g.fetch(b, c, with_ids=False)["mass"])
     return np.concatenate(out)
+
+
+DUMP_BYTES = 64_000_000  # --dump-outputs: every file together
+DUMP_SEED = 20240603
+
+
+def dump_outputs(out_dir: str, g, cnt, n_entries: int):
+    """--dump-outputs: what the last timed step computed, read from the handle after the timed region.
+
+    counts.npy         n_emitted, n_unique, n_entries of the index, n_hits of the query batch
+    index_mass.npy     the masses at 64 x 2048 fixed positions of the index
+    query.npy          a seeded sample of the batch's queries (ascending): the longest prefix of one fixed
+                       permutation whose hits fit in DUMP_BYTES
+    query_hits.npy     the number of hits of each sampled query
+    hit_*.npy          every hit of the sampled queries, one row per hit (the run-grouped answer expanded):
+                       query, mass, first_prot, first_off, len, modpat, flanks [n, 6], the peptide residues
+                       (hit_seq, CSR hit_seq_off) and the protein ids (hit_prot_ids, CSR hit_prot_list_off)
+    The hits of one query are in canonical order (query, mass, first_prot, first_off, len, modpat): ties in
+    mass have no contractual order, so two correct builds may deliver them differently.  Integers are
+    stored as float64 (exact), residue and flank bytes as float32."""
+    from dbindex_b200.capi import HIT_FIELDS, DbiHitBuffers, _expand_csr, expand_hits
+    raw, bufs = {}, DbiHitBuffers()
+    for name, (dt, size) in HIT_FIELDS.items():
+        raw[name] = np.empty(int(size(cnt)), dtype=dt)
+        setattr(bufs, name, raw[name].ctypes.data)
+    g.query_hits_read(bufs)
+    st = g.stats()
+    out = {"counts": np.array([st["n_emitted"], st["n_unique"], n_entries, cnt.n_hits], np.float64),
+           "index_mass": sample_index_masses(g, n_entries)}
+
+    ho, po, pho = (raw[k].astype(np.int64) for k in ("hit_off", "pep_off", "pep_hit_off"))
+    nq = len(ho) - 1
+    run_hits = np.diff(pho)
+    # bytes one query adds to the dump: 8 x (query, mass, first_prot, first_off, len, modpat, seq_off,
+    # prot_list_off) + 4 x 6 flanks per hit, 4 per residue, 8 per protein id, 16 in query / query_hits
+    run_bytes = run_hits * (8 * 8 + 4 * 6 + 4 * np.diff(raw["seq_off"].astype(np.int64)) +
+                            8 * np.diff(raw["prot_list_off"].astype(np.int64)))
+    cum = np.concatenate(([0], np.cumsum(run_bytes)))
+    q_bytes = cum[po[1:]] - cum[po[:-1]] + 16
+    perm = np.random.default_rng(DUMP_SEED).permutation(nq)
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 2 * 8 - 4096  # CSR terminators, .npy headers
+    k = int(np.searchsorted(np.cumsum(q_bytes[perm]), room, side="right"))
+    sel = np.sort(perm[:k])
+
+    # the run-grouped answer restricted to the sampled queries, then one record per hit
+    _, runs = _expand_csr(po, np.arange(len(run_hits), dtype=np.int64), sel)
+    sub = {"mass": raw["mass"][runs], "first_prot": raw["first_prot"][runs], "first_off": raw["first_off"][runs],
+           "len": raw["len"][runs], "flanks": raw["flanks"].reshape(-1, 6)[runs].reshape(-1)}
+    sub["pep_hit_off"], sub["modpat"] = _expand_csr(pho, raw["modpat"], runs)
+    sub["seq_off"], sub["seq"] = _expand_csr(raw["seq_off"], raw["seq"], runs)
+    sub["prot_list_off"], sub["prot_ids"] = _expand_csr(raw["prot_list_off"], raw["prot_ids"], runs)
+    h = expand_hits(sub)
+    n_q = np.diff(ho)[sel]
+    query = np.repeat(sel, n_q)
+    order = np.lexsort((h["modpat"], h["len"], h["first_off"], h["first_prot"],
+                        np.ascontiguousarray(h["mass"]).view(np.uint64), query))
+    seq_off, seq = _expand_csr(h["seq_off"], h["seq"], order)
+    prot_off, prot_ids = _expand_csr(h["prot_list_off"], h["prot_ids"], order)
+    out.update({"query": sel, "query_hits": n_q, "hit_query": query[order], "hit_mass": h["mass"][order],
+                "hit_first_prot": h["first_prot"][order], "hit_first_off": h["first_off"][order],
+                "hit_len": h["len"][order], "hit_modpat": h["modpat"][order],
+                "hit_flanks": h["flanks"].reshape(-1, 6)[order], "hit_seq": seq, "hit_seq_off": seq_off,
+                "hit_prot_ids": prot_ids, "hit_prot_list_off": prot_off})
+    out = {name: a.astype(np.float32 if name in ("hit_flanks", "hit_seq") else np.float64) for name, a in out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "queries": int(k), "hits": int(len(order)), "bytes": int(sum(a.nbytes for a in out.values()))}
 
 
 class PinnedHits:
@@ -432,6 +501,7 @@ def run_ours(args, rank: int, local_rank: int, world: int):
                                                      args.warmup, flush)
     clk = clocks.stop()
     n_entries = head["entries"]
+    dumped = dump_outputs(args.dump_outputs, g, cnt, n_entries) if args.dump_outputs else None
     parity = index_properties(g, n_entries, lo, hi, np.random.default_rng(1))
 
     # ---- e2e: the user-facing call sequence with HOST buffers, every copy inside the timed region ----
@@ -506,6 +576,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
                 "runs_per_step": int(cnt.n_peps)},
         "gpu_launches": head["gpu_launches"], "clocks": clk, "configs": configs,
     }
+    if dumped:
+        line["outputs"] = dumped
     try:
         line["fasta_ingest"] = fasta_ingest_rate(args.proteins)
     except Exception as e:  # a side measurement must never cost the bench line
@@ -807,10 +879,16 @@ def main():
     ap.add_argument("--sweep-queries", type=int, default=1000000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg1 / cfg3 / cfg5 sub-results")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the hits of the single-GPU path (--impl ours, one process)")
     if args.impl == "reference":
         run_reference(args, rank, world)
     else:
