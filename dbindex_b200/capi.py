@@ -105,6 +105,23 @@ class DbiHitBuffers(C.Structure):
                                           "len", "flanks", "seq_off", "seq", "prot_list_off", "prot_ids")]
 
 
+class DbiLookupCounts(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("n_found", C.c_uint64), ("n_prot_ids", C.c_uint64)]
+
+
+class DbiLookupBuffers(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("status", "mass", "entry", "first_prot", "first_off", "prot_list_off",
+                                          "prot_ids")]
+
+
+LOOKUP_ABSENT, LOOKUP_FOUND, LOOKUP_MALFORMED = 0, 1, 2
+LOOKUP_FIELDS = {  # dbi_lookup_buffers: name -> (dtype, size as a function of the counts)
+    "status": (np.uint8, lambda c: c.n), "mass": (np.float64, lambda c: c.n), "entry": (np.uint64, lambda c: c.n),
+    "first_prot": (np.uint32, lambda c: c.n), "first_off": (np.uint32, lambda c: c.n),
+    "prot_list_off": (np.uint64, lambda c: c.n + 1), "prot_ids": (np.uint32, lambda c: c.n_prot_ids),
+}
+
+
 # dbi_hit_buffers: the hits of a batch grouped in RUNS (consecutive hits of one query that are variants of one
 # peptide with one mass); per-run arrays have n_peps rows, only the mod pattern is per hit
 HIT_FIELDS = {  # name -> (dtype, size as a function of the counts)
@@ -195,6 +212,8 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "dbi_query_hits": (C.c_int, [vp, vp, vp, C.c_uint64, C.POINTER(DbiHitCounts)]),
         "dbi_query_hits_device": (C.c_int, [vp, vp, vp, C.c_uint64, C.POINTER(DbiHitCounts)]),
         "dbi_query_hits_read": (C.c_int, [vp, C.POINTER(DbiHitBuffers)]),
+        "dbi_lookup_peptides": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.POINTER(DbiLookupCounts)]),
+        "dbi_lookup_peptides_read": (C.c_int, [vp, C.POINTER(DbiLookupBuffers)]),
         "dbi_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(vp)]),
         "dbi_host_free": (C.c_int, [vp]),
         "dbi_get_protein": (C.c_int, [vp, C.c_uint32, C.POINTER(vp), u64p]),
@@ -233,7 +252,7 @@ ABI_SYMBOLS = [
     "dbi_default_params", "dbi_params_add_static_mod", "dbi_params_set_enzyme", "dbi_params_add_diff_mod",
     "dbi_create", "dbi_set_stream", "dbi_add_proteins", "dbi_upload", "dbi_reset_index", "dbi_build",
     "dbi_stats_get", "dbi_save", "dbi_load", "dbi_query", "dbi_query_device", "dbi_fetch", "dbi_query_hits", "dbi_query_hits_device", "dbi_query_hits_read",
-    "dbi_host_alloc", "dbi_host_free", "dbi_get_protein", "dbi_calculate_mass",
+    "dbi_lookup_peptides", "dbi_lookup_peptides_read", "dbi_host_alloc", "dbi_host_free", "dbi_get_protein", "dbi_calculate_mass",
     "dbi_entry_keys", "dbi_debug_emitted", "dbi_build_from_records", "dbi_debug_radix_sort", "dbi_destroy",
     "dbi_abi_sizes", "dbi_release_cached_memory",
     "dbi_last_error", "dbi_kernel_launches",
@@ -310,6 +329,18 @@ def parse_fasta(path: str, threads: int = 0, raw_deflines: bool = False):
     raw = dbuf.tobytes()
     deflines = [raw[int(doff[i]):int(doff[i + 1])].decode("latin-1") for i in range(n.value)]
     return deflines, residues, offsets
+
+
+def pack_peptides(seqs):
+    """Peptides -> the packed (residues uint8[R], offsets uint64[n + 1]) layout of the C ABI: a list of str / bytes,
+    or such a pair already."""
+    if isinstance(seqs, tuple) and len(seqs) == 2 and isinstance(seqs[0], np.ndarray):
+        return np.ascontiguousarray(seqs[0], dtype=np.uint8), np.ascontiguousarray(seqs[1], dtype=np.uint64)
+    bs = [s.encode("latin-1") if isinstance(s, str) else bytes(s) for s in seqs]
+    offsets = np.zeros(len(bs) + 1, dtype=np.uint64)
+    if bs:
+        np.cumsum(np.fromiter((len(b) for b in bs), dtype=np.uint64, count=len(bs)), out=offsets[1:])
+    return np.frombuffer(b"".join(bs), dtype=np.uint8), offsets
 
 
 class GpuIndex:
@@ -463,6 +494,32 @@ class GpuIndex:
             setattr(bufs, name, a.ctypes.data)
         self._check(self.lib.dbi_query_hits_read(self._h, C.byref(bufs)))
         return expand_hits(out) if per_hit else out
+
+    def lookup_peptides_begin(self, seqs, modpat=None) -> DbiLookupCounts:
+        """dbi_lookup_peptides alone: the answer stays in HBM until lookup_peptides_read / the next call."""
+        residues, offsets = pack_peptides(seqs)
+        pat = None if modpat is None else np.ascontiguousarray(modpat, dtype=np.uint32)
+        if pat is not None and len(pat) != len(offsets) - 1:
+            raise ValueError(f"{len(pat)} mod patterns for {len(offsets) - 1} peptides")
+        cnt = DbiLookupCounts()
+        self._check(self.lib.dbi_lookup_peptides(self._h, _ptr(residues), _ptr(offsets), _ptr(pat), len(offsets) - 1,
+                                                 C.byref(cnt)))
+        return cnt
+
+    def lookup_peptides_read(self, cnt: DbiLookupCounts) -> dict:
+        out, bufs = {"counts": cnt}, DbiLookupBuffers()
+        for name, (dt, size) in LOOKUP_FIELDS.items():
+            out[name] = a = np.empty(int(size(cnt)), dtype=dt)
+            setattr(bufs, name, a.ctypes.data)
+        self._check(self.lib.dbi_lookup_peptides_read(self._h, C.byref(bufs)))
+        return out
+
+    def lookup_peptides(self, seqs, modpat=None) -> dict:
+        """dbi_lookup_peptides + dbi_lookup_peptides_read: for every peptide (str / bytes, or a packed
+        (residues, offsets) pair) and mod pattern (byte k = position + 1 of the k-th modified residue; None = all
+        unmodified) whether the index holds it (status: LOOKUP_ABSENT / _FOUND / _MALFORMED), its mass, index entry,
+        first occurrence and protein ids (CSR prot_list_off / prot_ids), as numpy arrays."""
+        return self.lookup_peptides_read(self.lookup_peptides_begin(seqs, modpat))
 
     def entry_keys(self) -> np.ndarray:
         n = C.c_uint64(0)

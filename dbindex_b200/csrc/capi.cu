@@ -237,6 +237,17 @@ struct dbi_handle {
     }
   } hits;
 
+  // pending result of dbi_lookup_peptides, read by dbi_lookup_peptides_read
+  struct LookupResult {
+    bool valid = false;
+    dbi_lookup_counts n{};
+    DevBuf status, mass, entry, prot, off, plo, ids;
+    void drop() {
+      valid = false;
+      status.release(); mass.release(); entry.release(); prot.release(); off.release(); plo.release(); ids.release();
+    }
+  } lookup;
+
   DigestCfg cfg{};
   dbi_stats st{};
   // profiling (params.profile): event pairs recorded on the stream without any extra
@@ -406,6 +417,7 @@ void free_index(dbi_handle* h) {
   }
   h->built = false;
   h->hits.drop();
+  h->lookup.drop();
   h->d_res.release();
   h->d_pstart.release();
   h->u_mass.release(); h->u_gpos.release(); h->u_prot.release(); h->u_len.release();
@@ -1610,6 +1622,131 @@ int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out) {
   d2h(out->prot_ids, r.ids, r.n.n_prot_ids * 4);
   DBI_CUDA(cudaStreamSynchronize(s));
   r.drop();
+  return DBI_OK;
+  DBI_API_END
+}
+
+int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* offsets, const uint32_t* modpat,
+                        uint64_t n, dbi_lookup_counts* counts) {
+  DBI_API_BEGIN(h)
+  if (!h->built) {
+    set_error("Indexer is not initialized");
+    return DBI_ENOTINIT;
+  }
+  if (!counts || (n && !offsets)) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  for (uint64_t i = 0; i < n; ++i)
+    if (offsets[i + 1] < offsets[i]) {
+      set_error("offsets must be non-decreasing (row %llu)", (unsigned long long)i);
+      return DBI_EINVAL;
+    }
+  const uint64_t R = n ? offsets[n] - offsets[0] : 0;
+  if (R && !residues) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  const UniqView uv = uniq_view(h);
+  for (int r = 0; r < uv.world; ++r)
+    if (uv.uoff[r + 1] > uv.uoff[r] && !uv.len[r]) {
+      set_error("rank %d's unique-peptide window is not mapped on this handle: its peptides cannot be compared", r);
+      return DBI_EINVAL;
+    }
+  cudaStream_t s = h->stream;
+  dbi_handle::LookupResult& L = h->lookup;
+  L.drop();
+  std::memset(counts, 0, sizeof(*counts));
+  counts->n = n;
+  L.status.alloc(std::max<uint64_t>(n, 1), h->arena);
+  L.mass.alloc(std::max<uint64_t>(n, 1) * 8, h->arena);
+  L.entry.alloc(std::max<uint64_t>(n, 1) * 8, h->arena);
+  L.prot.alloc(std::max<uint64_t>(n, 1) * 4, h->arena);
+  L.off.alloc(std::max<uint64_t>(n, 1) * 4, h->arena);
+  L.plo.alloc((n + 1) * 8, h->arena);
+  if (n == 0) {
+    DBI_CUDA(cudaMemsetAsync(L.plo.p, 0, 8, s));
+    DBI_CUDA(cudaStreamSynchronize(s));
+    L.n = *counts;
+    L.valid = true;
+    return DBI_OK;
+  }
+  // input: residues | offsets | patterns | found counter
+  const uint64_t res_bytes = (R + 7) & ~7ull, pat_bytes = modpat ? (n * 4 + 7) & ~7ull : 0;
+  DevBuf in, np32, stmp;
+  in.alloc(res_bytes + (n + 1) * 8 + pat_bytes + 8, h->arena);
+  uint8_t* d_q = in.as<uint8_t>();
+  uint64_t* d_off = (uint64_t*)(d_q + res_bytes);
+  uint32_t* d_pat = modpat ? (uint32_t*)(d_off + n + 1) : nullptr;
+  unsigned long long* d_found = (unsigned long long*)((uint8_t*)(d_off + n + 1) + pat_bytes);
+  if (R) DBI_CUDA(cudaMemcpyAsync(d_q, residues + offsets[0], R, cudaMemcpyHostToDevice, s));
+  DBI_CUDA(cudaMemcpyAsync(d_off, offsets, (n + 1) * 8, cudaMemcpyHostToDevice, s));
+  if (modpat) DBI_CUDA(cudaMemcpyAsync(d_pat, modpat, n * 4, cudaMemcpyHostToDevice, s));
+  DBI_CUDA(cudaMemsetAsync(d_found, 0, 8, s));
+  np32.alloc(n * 4, h->arena);
+  stmp.alloc(full_scan_tmp_bytes(n), h->arena);
+  uint64_t n_found = 0, PI = 0;
+  {
+    Stage sg(h, DBI_STAGE_QUERY);
+    launch_lookup_match(h->d_res.as<uint8_t>(), h->entry_mass(), h->n_entries, h->entry_base(), h->ent_base_off,
+                        h->entry_pat(), uv, h->d_tables.as<DevTables>(), h->cfg.init_mass, h->cfg.max_mods, d_q, d_off,
+                        d_pat, n, L.status.as<uint8_t>(), L.mass.as<double>(), L.entry.as<uint64_t>(),
+                        np32.as<uint32_t>(), d_found, s);
+    int rounds = 1;  // the last one probes <= 32 consecutive entries
+    for (uint64_t w = h->n_entries; w > 32; w = w / 33 + 1) ++rounds;
+    // rows read (residues, offset, pattern), 32 eight-byte probes per search round, the row's residues compared
+    // once with its candidate, status + mass + entry + list length written
+    h->st.algo_bytes[DBI_STAGE_QUERY] += 2 * R + n * (12 + 256ull * rounds + 21);
+  }
+  {
+    Stage sg(h, DBI_STAGE_FETCH);
+    launch_full_scan_u32_to_u64(np32.as<uint32_t>(), n, L.plo.as<uint64_t>(), stmp.p, s);
+    DBI_CUDA(cudaMemcpyAsync(&PI, L.plo.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, s));
+    DBI_CUDA(cudaMemcpyAsync(&n_found, d_found, 8, cudaMemcpyDeviceToHost, s));
+    DBI_CUDA(cudaStreamSynchronize(s));
+    L.ids.alloc(std::max<uint64_t>(PI, 1) * 4, h->arena);
+    launch_lookup_gather(L.status.as<uint8_t>(), L.entry.as<uint64_t>(), h->entry_base(), h->ent_base_off, uv,
+                         h->d_pstart.as<uint32_t>(), L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(),
+                         L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
+    // list lengths scanned (4 read, 8 written); per row status + list offset read, first occurrence written;
+    // per found row entry, base id, peptide tables (4 + 4 + 16) and protein start read; ids copied
+    h->st.algo_bytes[DBI_STAGE_FETCH] += n * (12 + 9 + 8) + n_found * (8 + 4 + 24 + 4) + 8 * PI;
+  }
+  DBI_CUDA(cudaStreamSynchronize(s));
+  resolve_spans(h);
+  counts->n_found = n_found;
+  counts->n_prot_ids = PI;
+  L.n = *counts;
+  L.valid = true;
+  return DBI_OK;
+  DBI_API_END
+}
+
+int dbi_lookup_peptides_read(dbi_handle* h, const dbi_lookup_buffers* out) {
+  DBI_API_BEGIN(h)
+  dbi_handle::LookupResult& L = h->lookup;
+  if (!L.valid) {
+    set_error("no pending dbi_lookup_peptides result on this handle");
+    return DBI_ENOTINIT;
+  }
+  if (!out) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  cudaStream_t s = h->stream;
+  const uint64_t n = L.n.n;
+  auto d2h = [&](void* dst, const DevBuf& src, uint64_t bytes) {
+    if (dst && bytes) DBI_CUDA(cudaMemcpyAsync(dst, src.p, bytes, cudaMemcpyDeviceToHost, s));
+  };
+  d2h(out->status, L.status, n);
+  d2h(out->mass, L.mass, n * 8);
+  d2h(out->entry, L.entry, n * 8);
+  d2h(out->first_prot, L.prot, n * 4);
+  d2h(out->first_off, L.off, n * 4);
+  d2h(out->prot_list_off, L.plo, (n + 1) * 8);
+  d2h(out->prot_ids, L.ids, L.n.n_prot_ids * 4);
+  DBI_CUDA(cudaStreamSynchronize(s));
+  L.drop();
   return DBI_OK;
   DBI_API_END
 }

@@ -196,6 +196,18 @@ void launch_fetch_gather(const double* e_mass, const uint32_t* e_base, uint64_t 
                          const uint32_t* sizes, const uint64_t* tile_offs, double* o_mass, uint32_t* o_prot,
                          uint32_t* o_off, uint16_t* o_len, uint32_t* o_pat, uint64_t* o_list_off, uint32_t* o_ids,
                          cudaStream_t s);
+// K11 batched peptide lookup (dbi_lookup_peptides).  Row i = q_res[q_off[i] - q_off[0], q_off[i+1] - q_off[0])
+// with mod pattern q_pat[i] (nullptr = all unmodified).  K11a: status (0 absent, 1 found, 2 malformed), mass,
+// entry (UINT64_MAX unless found), protein-list length o_np, and *n_found += found rows.
+void launch_lookup_match(const uint8_t* d_res, const double* e_mass, uint64_t n_entries, const uint32_t* e_base,
+                         uint64_t ent_off, const uint32_t* e_pat, const UniqView& uv, const DevTables* d_tb,
+                         double init_mass, int max_mods, const uint8_t* q_res, const uint64_t* q_off,
+                         const uint32_t* q_pat, uint64_t n, uint8_t* o_status, double* o_mass, uint64_t* o_entry,
+                         uint32_t* o_np, unsigned long long* n_found, cudaStream_t s);
+// K11b: first occurrence + protein ids of the found rows (plo = scan of o_np); 0xffffffff for the others
+void launch_lookup_gather(const uint8_t* status, const uint64_t* entry, const uint32_t* e_base, uint64_t ent_off,
+                          const UniqView& uv, const uint32_t* pstart, const uint64_t* plo, uint64_t n,
+                          uint32_t* o_prot, uint32_t* o_off, uint32_t* o_ids, cudaStream_t s);
 // distinct (int)(mass*factor) keys: flags + compaction
 void launch_key_flags(const double* e_mass, uint64_t n, double factor, uint8_t* flags, uint32_t* tile_counts,
                       cudaStream_t s);

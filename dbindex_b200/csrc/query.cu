@@ -1,9 +1,11 @@
-// query.cu -- K9 batched lower/upper bound, K10 hit gather, entry-key listing.
+// query.cu -- K9 batched lower/upper bound, K10 hit gather, K11 peptide lookup, entry-key listing.
 //
 // Replaces DBIndexStoreSQLiteByteIndexMerge.getSequences (Merge:146-217): the
 // `SELECT ... WHERE precursor_mass_key BETWEEN minKey AND maxKey` plus the exact
 // double filter of parseAddPeptideInfo (Merge:415-419) become one lower_bound and
 // one upper_bound on the totally ordered mass array; both ends inclusive (Q5).
+#include <cassert>
+
 #include "kernels.cuh"
 
 namespace dbi {
@@ -187,6 +189,21 @@ __device__ __forceinline__ uint32_t ld_res4(const uint8_t* __restrict__ res, uin
   return __funnelshift_r(a, __ldg(w + 1), sh);
 }
 
+// What parseAddPeptideInfo takes from the peptide itself (K10c per run, K11b per found lookup row): the first
+// occurrence's protein and offset inside it (Merge:678-687), and every occurrence's protein id in insertion
+// order (Merge:449-475) into ids[0 ..).  Row `row` of rank r, whose tables are mapped; any output may be nullptr.
+__device__ __forceinline__ void peptide_occurrences(const UniqView& uv, int r, uint64_t row,
+                                                    const uint32_t* __restrict__ pstart, uint32_t* o_prot,
+                                                    uint32_t* o_off, uint32_t* ids) {
+  const uint32_t gp = uv.gpos[r][row], pr = uv.prot[r][row];
+  if (o_prot) *o_prot = pr;
+  if (o_off) *o_off = gp - pstart[pr];  // sequenceOffset inside the first protein
+  if (ids) {
+    const uint64_t src = uv.plo[r][row], n = uv.plo[r][row + 1] - src;
+    for (uint64_t k = 0; k < n; ++k) ids[k] = uv.plist[r][src + k];
+  }
+}
+
 __global__ void __launch_bounds__(Q_THREADS)
     peps_gather_kernel(const uint8_t* __restrict__ res, const uint32_t* __restrict__ pstart,
                        const uint32_t* __restrict__ e_base, uint64_t ent_off, const __grid_constant__ UniqView uv,
@@ -217,10 +234,8 @@ __global__ void __launch_bounds__(Q_THREADS)
       s_gpos[t] = 0;
       for (int k = 0; k < 6; ++k) f[k] = '-';
     } else {
-      const uint32_t gp = uv.gpos[r][row], pr = uv.prot[r][row], len = uv.len[r][row];
+      const uint32_t gp = uv.gpos[r][row], len = uv.len[r][row];
       s_gpos[t] = gp;
-      if (o_prot) o_prot[h] = pr;
-      if (o_off) o_off[h] = gp - pstart[pr];  // sequenceOffset inside the first protein
       if (o_len) o_len[h] = (uint16_t)len;
       // Util.getResidues (Util.java:130-162): up to 3 residues on the left, '-' padded on the left; on
       // the right min(3, protLen - end - 1) residues -- the reference's off-by-one drops the last
@@ -237,10 +252,8 @@ __global__ void __launch_bounds__(Q_THREADS)
       while (remaining < 4 && (rr[remaining] = ld_res(res, endp + remaining)) != 0) ++remaining;
       const uint32_t rl = remaining > 0 ? min(3u, remaining - 1u) : 0u;
       for (uint32_t k = 0; k < 3; ++k) f[3 + k] = k < rl ? rr[k] : (uint8_t)'-';
-      if (o_ids) {  // every occurrence's protein id, insertion order (Merge:449-475)
-        const uint64_t src = uv.plo[r][row], n = uv.plo[r][row + 1] - src, dst = plo_out[h];
-        for (uint64_t k = 0; k < n; ++k) o_ids[dst + k] = uv.plist[r][src + k];
-      }
+      peptide_occurrences(uv, r, row, pstart, o_prot ? o_prot + h : nullptr, o_off ? o_off + h : nullptr,
+                          o_ids ? o_ids + plo_out[h] : nullptr);
     }
   }
   __syncthreads();
@@ -362,6 +375,151 @@ __global__ void __launch_bounds__(Q_THREADS)
   }
 }
 
+// ---- K11 batched peptide lookup: getProteins(String) (DBIndexer.java:925-947) for a whole list ----------------
+constexpr uint8_t kLookupAbsent = 0, kLookupFound = 1, kLookupMalformed = 2;
+constexpr unsigned kFull = 0xffffffffu;
+
+// K11a: one warp per row.
+//  1. The row's mass in the index's own summation order: init_mass, the residues left to right (digest.cu), then
+//     the shift of every pattern position left to right (mods.cu, mods_grp.cu), so that it equals the indexed
+//     mass bit for bit.  It is ONE sequential FP64 chain; the lanes load the residue masses side by side and
+//     every lane runs the same chain over the shuffled values, so the whole warp holds the mass and the
+//     validation verdict without a broadcast.
+//  2. A 32-ary search for the first entry with mass >= the row's: each round the lanes probe 32 evenly spaced
+//     pivots of the interval (independent loads) and a ballot narrows it 33-fold, ~log33(V) dependent rounds.
+//  3. A walk over the run of equal mass bits, 32 entries per step.  A candidate has the row's mod pattern and
+//     length; the warp compares its residues with the row's (lane j: positions j, j + 32, ...).  Unique
+//     peptides are distinct strings and a (peptide, pattern) pair is indexed once, so the first full match is
+//     the answer (a build with -DDBI_DEBUG walks the rest of the run and asserts that no second one exists).
+__global__ void __launch_bounds__(Q_THREADS)
+    lookup_match_kernel(const uint8_t* __restrict__ res, const double* __restrict__ e_mass, uint64_t n_entries,
+                        const uint32_t* __restrict__ e_base, uint64_t ent_off, const uint32_t* __restrict__ e_pat,
+                        const __grid_constant__ UniqView uv, const DevTables* __restrict__ tb, double init_mass,
+                        int max_mods, const uint8_t* __restrict__ q_res, const uint64_t* __restrict__ q_off,
+                        const uint32_t* __restrict__ q_pat, uint64_t n, uint8_t* __restrict__ o_status,
+                        double* __restrict__ o_mass, uint64_t* __restrict__ o_entry, uint32_t* __restrict__ o_np,
+                        unsigned long long* __restrict__ n_found) {
+  const uint64_t i = (uint64_t)blockIdx.x * HX_WARPS + (threadIdx.x >> 5);
+  if (i >= n) return;  // warp-uniform
+  const unsigned lane = lane_id();
+  const uint8_t* q = q_res + (q_off[i] - q_off[0]);
+  const uint64_t len = q_off[i + 1] - q_off[i];
+  const uint32_t pat = q_pat ? q_pat[i] : 0u;
+  bool ok = len >= 1 && len <= DBI_MAX_PEP_LEN;
+  double m = init_mass;
+  if (ok) {
+    for (uint32_t c = 0; c < len; c += 32) {
+      const uint32_t p = c + lane;
+      const double rm = p < len ? __ldg(&tb->mass[q[p]]) : 0.0;
+      const uint32_t k_end = min(32u, (uint32_t)len - c);
+      for (uint32_t k = 0; k < k_end; ++k) m = __dadd_rn(m, __shfl_sync(kFull, rm, k));
+    }
+    // mod pattern: byte k = position + 1 of the k-th modified residue, strictly ascending, zeros only at the end
+    uint32_t prev = 0, n_mods = 0;
+    bool ended = false;
+    for (int k = 0; k < DBI_MAX_MODS_PER_PEP && ok; ++k) {
+      const uint32_t b = (pat >> (8 * k)) & 0xFFu;
+      if (b == 0) {
+        ended = true;
+        continue;
+      }
+      const uint32_t pos = b - 1;
+      ok = !ended && b > prev && pos < len && pos <= DBI_MAX_MOD_POS && (int)++n_mods <= max_mods;
+      if (!ok) break;
+      const uint8_t c = q[pos];
+      ok = (__ldg(&tb->flags[c]) & kFlagDiffMod) != 0;
+      m = __dadd_rn(m, __ldg(&tb->diff[c]));
+      prev = b;
+    }
+  }
+  if (!ok) {
+    if (lane == 0) {
+      o_status[i] = kLookupMalformed;
+      o_mass[i] = 0.0;
+      o_entry[i] = UINT64_MAX;
+      o_np[i] = 0;
+    }
+    return;
+  }
+
+  // first entry with mass >= m lies in [lo, hi]
+  uint64_t lo = 0, hi = n_entries;
+  while (hi - lo > 32) {
+    const uint64_t w = hi - lo;
+    const unsigned below = __ballot_sync(kFull, __ldg(e_mass + lo + (lane + 1) * w / 33) < m);
+    const uint64_t k = (uint64_t)__popc(below);  // pivots 0 .. k-1 lie below m
+    hi = k < 32 ? lo + (k + 1) * w / 33 : hi;
+    lo = k > 0 ? lo + k * w / 33 + 1 : lo;
+  }
+  const unsigned below = __ballot_sync(kFull, lo + lane < hi && __ldg(e_mass + lo + lane) < m);
+  const uint64_t first = lo + (uint64_t)__popc(below);
+
+  const unsigned long long mb = (unsigned long long)__double_as_longlong(m);
+  const unsigned long long* e_bits = reinterpret_cast<const unsigned long long*>(e_mass);
+  uint64_t hit = UINT64_MAX;
+  uint32_t hit_np = 0;
+  for (uint64_t e0 = first; e0 < n_entries; e0 += 32) {
+    const uint64_t e = e0 + lane;
+    const bool eq = e < n_entries && __ldg(e_bits + e) == mb;
+    bool cand = eq && (e_pat ? __ldg(e_pat + e) : 0u) == pat;
+    int r = 0;
+    uint64_t row = 0;
+    if (cand) {
+      r = uniq_owner(uv, e_base ? (uint64_t)__ldg(e_base + e) : ent_off + e, &row);
+      cand = uv.len[r][row] == len;
+    }
+    for (unsigned cm = __ballot_sync(kFull, cand); cm; cm &= cm - 1) {
+      const int src = __ffs(cm) - 1;
+      const int cr = __shfl_sync(kFull, r, src);
+      const uint64_t crow = __shfl_sync(kFull, row, src);
+      const uint32_t gp = uv.gpos[cr][crow];
+      bool same = true;
+      for (uint32_t p = lane; p < len; p += 32) same &= q[p] == ld_res(res, gp + p);
+      if (__all_sync(kFull, same)) {
+#ifdef DBI_DEBUG
+        assert(hit == UINT64_MAX);
+#endif
+        hit = e0 + src;
+        hit_np = (uint32_t)(uv.plo[cr][crow + 1] - uv.plo[cr][crow]);
+#ifndef DBI_DEBUG
+        break;
+#endif
+      }
+    }
+#ifndef DBI_DEBUG
+    if (hit != UINT64_MAX) break;
+#endif
+    if (__ballot_sync(kFull, eq) != kFull) break;  // the run of equal mass bits ends in this step
+  }
+  if (lane == 0) {
+    o_status[i] = hit != UINT64_MAX ? kLookupFound : kLookupAbsent;
+    o_mass[i] = m;
+    o_entry[i] = hit;
+    o_np[i] = hit_np;
+    if (hit != UINT64_MAX) atomicAdd(n_found, 1ull);
+  }
+}
+
+// K11b: one thread per row; found rows get their first occurrence and protein ids (prot_list_off = scan of the
+// list lengths K11a wrote), the others first_prot = first_off = 0xffffffff.
+__global__ void __launch_bounds__(Q_THREADS)
+    lookup_gather_kernel(const uint8_t* __restrict__ status, const uint64_t* __restrict__ entry,
+                         const uint32_t* __restrict__ e_base, uint64_t ent_off, const __grid_constant__ UniqView uv,
+                         const uint32_t* __restrict__ pstart, const uint64_t* __restrict__ plo, uint64_t n,
+                         uint32_t* __restrict__ o_prot, uint32_t* __restrict__ o_off, uint32_t* __restrict__ o_ids) {
+  const uint64_t i = (uint64_t)blockIdx.x * Q_THREADS + threadIdx.x;
+  if (i >= n) return;
+  if (status[i] != kLookupFound) {
+    o_prot[i] = 0xffffffffu;
+    o_off[i] = 0xffffffffu;
+    return;
+  }
+  const uint64_t e = entry[i];
+  uint64_t row;
+  const int r = uniq_owner(uv, e_base ? (uint64_t)e_base[e] : ent_off + e, &row);
+  peptide_occurrences(uv, r, row, pstart, o_prot + i, o_off + i, o_ids + plo[i]);
+}
+
 __device__ __forceinline__ int32_t row_key(double m, double factor) { return (int32_t)(m * factor); }
 
 __global__ void __launch_bounds__(Q_THREADS)
@@ -470,6 +628,26 @@ void launch_fetch_gather(const double* e_mass, const uint32_t* e_base, uint64_t 
   const unsigned tiles = (unsigned)((count + kScanTile - 1) / kScanTile);
   DBI_LAUNCH(fetch_gather_kernel, tiles, Q_THREADS, 0, s, e_mass, e_base, base_off, uv, e_pat, pstart, begin, count,
              sizes, tile_offs, o_mass, o_prot, o_off, o_len, o_pat, o_list_off, o_ids);
+}
+
+void launch_lookup_match(const uint8_t* d_res, const double* e_mass, uint64_t n_entries, const uint32_t* e_base,
+                         uint64_t ent_off, const uint32_t* e_pat, const UniqView& uv, const DevTables* d_tb,
+                         double init_mass, int max_mods, const uint8_t* q_res, const uint64_t* q_off,
+                         const uint32_t* q_pat, uint64_t n, uint8_t* o_status, double* o_mass, uint64_t* o_entry,
+                         uint32_t* o_np, unsigned long long* n_found, cudaStream_t s) {
+  if (n == 0) return;
+  const unsigned grid = (unsigned)((n + HX_WARPS - 1) / HX_WARPS);
+  DBI_LAUNCH(lookup_match_kernel, grid, Q_THREADS, 0, s, d_res, e_mass, n_entries, e_base, ent_off, e_pat, uv, d_tb,
+             init_mass, max_mods, q_res, q_off, q_pat, n, o_status, o_mass, o_entry, o_np, n_found);
+}
+
+void launch_lookup_gather(const uint8_t* status, const uint64_t* entry, const uint32_t* e_base, uint64_t ent_off,
+                          const UniqView& uv, const uint32_t* pstart, const uint64_t* plo, uint64_t n,
+                          uint32_t* o_prot, uint32_t* o_off, uint32_t* o_ids, cudaStream_t s) {
+  if (n == 0) return;
+  const unsigned grid = (unsigned)((n + Q_THREADS - 1) / Q_THREADS);
+  DBI_LAUNCH(lookup_gather_kernel, grid, Q_THREADS, 0, s, status, entry, e_base, ent_off, uv, pstart, plo, n, o_prot,
+             o_off, o_ids);
 }
 
 void launch_key_flags(const double* e_mass, uint64_t n, double factor, uint8_t* flags, uint32_t* tile_counts,

@@ -425,17 +425,35 @@ class DBIndexer:
             out.extend(lst)
         return out
 
+    def _protein(self, pid: int) -> IndexedProtein:
+        return IndexedProtein(self.deflines[pid] if pid < len(self.deflines) else "", pid)
+
     def getProteins(self, seq) -> Set[IndexedProtein] | List[IndexedProtein]:
         """getProteins(String) (DBIndexer.java:925-947) / getProteins(IndexedSequence) (:882)."""
         self._require()
         if isinstance(seq, IndexedSequence):
-            return [IndexedProtein(self.deflines[i] if i < len(self.deflines) else "", i) for i in seq.proteinIds]
-        mass = self.index.calculate_mass(seq.encode("latin-1"))  # IndexUtil.calculateMass
-        ret: Set[IndexedProtein] = set()
-        for s in self.getSequencesUsingDaltonTolerance(mass, 0.0):
-            if s.sequence == seq and not s.modPositions:
-                ret.update(self.getProteins(s))
-        return ret
+            return [self._protein(i) for i in seq.proteinIds]
+        return self.getProteinsBatch([seq])[0]
+
+    def getProteinsBatch(self, seqs: Sequence[str]) -> List[Set[IndexedProtein]]:
+        """getProteins(String) for a whole list in one device call (dbi_lookup_peptides): the unmodified entry
+        whose peptide equals the string, found by its mass computed the way the index computes it
+        (IndexUtil.calculateMass) -- the zero-tolerance getSequences + `s.sequence.equals(seq)` filter of the
+        reference.  A mass whose bucket lies beyond MAX_MASS gives the empty set, as that query does."""
+        self._require()
+        try:
+            r = self.index.lookup_peptides(list(seqs))
+        except DbiError as e:
+            raise DBIndexStoreException(str(e)) from e
+        plo = r["prot_list_off"].astype(np.int64)
+        out: List[Set[IndexedProtein]] = []
+        for i in range(len(seqs)):
+            m = float(r["mass"][i])
+            if r["status"][i] != 1 or self._out_of_buckets(m, m):
+                out.append(set())
+            else:
+                out.append({self._protein(p) for p in r["prot_ids"][plo[i]:plo[i + 1]].tolist()})
+        return out
 
     def getNumberSequences(self) -> int:
         self._require()
@@ -488,11 +506,17 @@ class DBIndexImpl:
         return self.indexer.getSequences(list(args[0]))
 
     def getProteins(self, seq):
-        if isinstance(seq, str):  # DBIndexImpl.java:222-237, memoised
-            if seq not in self._proteins_by_seq:
-                self._proteins_by_seq[seq] = self.indexer.getProteins(seq)
-            return self._proteins_by_seq[seq]
-        return self.indexer.getProteins(seq)  # DBIndexImpl.java:208
+        """getProteins(String) (DBIndexImpl.java:222-237, memoised), getProteins(IndexedSequence) (:208), or for a
+        list of strings the list of their protein sets: the strings not memoised yet go to the device in one call."""
+        if isinstance(seq, str):
+            return self.getProteins([seq])[0]
+        if isinstance(seq, IndexedSequence):
+            return self.indexer.getProteins(seq)
+        seqs = list(seq)
+        todo = list(dict.fromkeys(s for s in seqs if s not in self._proteins_by_seq))
+        if todo:
+            self._proteins_by_seq.update(zip(todo, self.indexer.getProteinsBatch(todo)))
+        return [self._proteins_by_seq[s] for s in seqs]
 
     def getIndexedProteinById(self, pid: int) -> IndexedProtein:
         return IndexedProtein(self.indexer.deflines[pid], pid)  # DBIndexImpl.java:501-504

@@ -547,3 +547,43 @@ def split_masses(index, world: int) -> np.ndarray:
     out = np.zeros(max(n - 1, 0), dtype=np.float64)
     index._check(lib.dbi_mg_split_masses(index._h, out.ctypes.data if n > 1 else None))
     return out
+
+
+def lookup_local(handles, seqs, modpat=None) -> dict:
+    """dbi_lookup_peptides on a sharded index whose handles all live in this process: every rank gets the whole
+    batch (the mass that decides ownership is computed on the device) and the answers are merged.  A row is found
+    on at most one rank, the owner of the slice holding its mass; anything else raises.  Returns the arrays of
+    GpuIndex.lookup_peptides, `entry` being an entry of rank `rank` (-1 where nothing was found)."""
+    from .capi import LOOKUP_FOUND, pack_peptides
+    packed = pack_peptides(seqs)
+    world = len(handles)
+    split = split_masses(handles[0], world)
+    parts = [g.lookup_peptides(packed, modpat) for g in handles]
+    n = len(packed[1]) - 1
+    rank = np.full(n, -1, dtype=np.int32)
+    for r, p in enumerate(parts):
+        found = p["status"] == LOOKUP_FOUND
+        if np.any(found & (rank >= 0)):
+            raise RuntimeError(f"rows {np.nonzero(found & (rank >= 0))[0][:8].tolist()} found on two ranks")
+        if not np.all(owned_mask(p["mass"][found], split, r, world)):
+            raise RuntimeError(f"rank {r} found rows whose mass lies outside its slices")
+        rank[found] = r
+    first = parts[0]
+    for p in parts[1:]:
+        if not (np.array_equal(p["status"] == 2, first["status"] == 2) and np.array_equal(p["mass"], first["mass"])):
+            raise RuntimeError("the ranks disagree on the masses or the malformed rows of the batch")
+    out = {k: first[k].copy() for k in ("status", "mass", "entry", "first_prot", "first_off")}
+    sizes = np.zeros(n, dtype=np.int64)
+    ids = [np.zeros(0, np.uint32)] * n
+    for r, p in enumerate(parts):
+        sel = np.nonzero(rank == r)[0]
+        plo = p["prot_list_off"].astype(np.int64)
+        for k in ("status", "entry", "first_prot", "first_off"):
+            out[k][sel] = p[k][sel]
+        sizes[sel] = plo[sel + 1] - plo[sel]
+        for i in sel:
+            ids[i] = p["prot_ids"][plo[i]:plo[i + 1]]
+    out["rank"] = rank
+    out["prot_list_off"] = np.concatenate(([0], np.cumsum(sizes))).astype(np.uint64)
+    out["prot_ids"] = np.concatenate(ids) if n else np.zeros(0, np.uint32)
+    return out

@@ -285,6 +285,46 @@ int dbi_query_hits(dbi_handle* h, const double* lo, const double* hi, uint64_t n
 int dbi_query_hits_device(dbi_handle* h, const double* d_lo, const double* d_hi, uint64_t nq, dbi_hit_counts* counts);
 int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out);
 
+/* Batched DBIndexer.getProteins(String) (DBIndexer.java:925-947, DBIndexImpl.java:222-237): which index entry,
+ * and so which proteins, every peptide of a list is.  Peptide i is residues[offsets[i], offsets[i+1]) (the packed
+ * layout of dbi_add_proteins; offsets non-decreasing) with mod pattern modpat[i] in the index's own encoding
+ * (byte k = position + 1 of the k-th modified residue, ascending, zero bytes only after the last mod; modpat =
+ * NULL: every row unmodified).  A row is FOUND iff the index holds an entry whose peptide is byte-equal to the
+ * row and whose mod pattern equals modpat[i] -- the reference's `s.sequence.equals(seq)` filter at zero
+ * tolerance.  Its mass is computed on the device the way the index computes it (h2o_proton if added, cterm,
+ * nterm, the residues left to right, then the shift of every pattern position left to right) and matched bit
+ * for bit; a row matches at most one entry.
+ *
+ * A row is MALFORMED (status 2; the rest of the batch is answered) when its length is 0 or above
+ * DBI_MAX_PEP_LEN, its pattern is not strictly ascending or has a nonzero byte after a zero byte, names a position
+ * >= its length or above DBI_MAX_MOD_POS, a residue without a differential shift, or more mods than
+ * max_mods_per_peptide (any mod at all on an index without differential mods).  A well-formed row the index does
+ * not hold (e.g. a variant whose shifted mass is outside [min_mass, max_mass]) is status 0.
+ *
+ *   dbi_lookup_peptides(h, ..., &n)        device: mass, search, protein lists (results stay in HBM)
+ *   dbi_lookup_peptides_read(h, &out)      D2H into the caller's buffers; any pointer may be NULL
+ *
+ * A sharded handle answers for its own mass slice (the owner of the slice holding a row's mass finds it) and
+ * compares residues through the other ranks' mapped window 2; a handle on which a rank's window 2 is not mapped
+ * refuses the call (DBI_EINVAL).  The pending lookup result of a handle is separate from that of
+ * dbi_query_hits and is dropped by the next dbi_lookup_peptides, a successful read, dbi_reset_index or
+ * dbi_destroy. */
+typedef struct dbi_lookup_counts {
+  uint64_t n, n_found, n_prot_ids;
+} dbi_lookup_counts;
+typedef struct dbi_lookup_buffers {
+  uint8_t* status;         /* n           0 = not in the index, 1 = found, 2 = malformed row                */
+  double* mass;            /* n           calculateMass (+ shifts) as the index computes it; 0 if malformed  */
+  uint64_t* entry;         /* n           index entry of this handle (for dbi_fetch); UINT64_MAX unless found */
+  uint32_t* first_prot;    /* n           first occurrence (Merge:678-687); 0xffffffff unless found          */
+  uint32_t* first_off;     /* n                                                                              */
+  uint64_t* prot_list_off; /* n + 1       CSR over prot_ids; empty list unless found                         */
+  uint32_t* prot_ids;      /* n_prot_ids  every occurrence, insertion order, duplicates kept (Q6)            */
+} dbi_lookup_buffers;
+int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* offsets, const uint32_t* modpat,
+                        uint64_t n, dbi_lookup_counts* counts);
+int dbi_lookup_peptides_read(dbi_handle* h, const dbi_lookup_buffers* out);
+
 /* Page-locked host memory for the buffers above (cudaHostAlloc / cudaFreeHost); a JVM cannot pin
  * its own allocations.  Pageable memory works too, at staging-copy speed. */
 int dbi_host_alloc(uint64_t bytes, void** out);
@@ -296,9 +336,9 @@ int dbi_host_free(void* p);
 int dbi_get_protein(dbi_handle* h, uint32_t id, const uint8_t** residues, uint64_t* len);
 
 /* IndexUtil.calculateMass(seq) (util/IndexUtil.java:197-208): same summation
- * order as the digestion, so a zero-tolerance lookup finds the peptide
- * (DBIndexer.getProteins(String), DBIndexer.java:925-947).  Pure host arithmetic
- * on the handle's parameter table. */
+ * order as the digestion, so a zero-tolerance lookup finds the peptide.  Pure host
+ * arithmetic on the handle's parameter table (dbi_lookup_peptides computes the
+ * same mass on the device for a whole list). */
 int dbi_calculate_mass(dbi_handle* h, const uint8_t* seq, uint64_t len, double* mass);
 
 /* DBIndexStore.getEntryKeys(): distinct (int)(mass*factor) row keys in ascending

@@ -22,7 +22,7 @@ import static java.lang.foreign.ValueLayout.JAVA_LONG;
  * NOT COMPILED IN THIS REPOSITORY: the build image has no JDK and the reference's core dependency
  * (edu.scripps.yates:utilities:1.6-SNAPSHOT) is not vendored. The same calls are exercised from Python
  * (dbindex_b200/capi.py); this file is what a dbIndex maintainer drops next to DBIndexStoreSQLiteMult.
- * tests/test_java_layout.py parses the three layouts below and checks every field offset against
+ * tests/test_java_layout.py and tests/test_peptide_lookup.py parse the layouts below and checks every field offset against
  * offsetof() of the compiled C structs, so a drift fails in CI without a JDK.
  */
 public final class DbiNative {
@@ -61,6 +61,15 @@ public final class DbiNative {
 			ADDRESS.withName("len"), ADDRESS.withName("flanks"), ADDRESS.withName("seq_off"), ADDRESS.withName("seq"),
 			ADDRESS.withName("prot_list_off"), ADDRESS.withName("prot_ids"));
 
+	/** struct dbi_lookup_counts */
+	static final StructLayout LOOKUP_COUNTS = MemoryLayout.structLayout(JAVA_LONG.withName("n"),
+			JAVA_LONG.withName("n_found"), JAVA_LONG.withName("n_prot_ids"));
+
+	/** struct dbi_lookup_buffers: seven caller-owned output pointers (one row per looked-up peptide) */
+	static final StructLayout LOOKUP_BUFFERS = MemoryLayout.structLayout(ADDRESS.withName("status"),
+			ADDRESS.withName("mass"), ADDRESS.withName("entry"), ADDRESS.withName("first_prot"),
+			ADDRESS.withName("first_off"), ADDRESS.withName("prot_list_off"), ADDRESS.withName("prot_ids"));
+
 	private static final Linker LINKER = Linker.nativeLinker();
 	private static final SymbolLookup LIB = SymbolLookup
 			.libraryLookup(System.getProperty("dbindex.gpu.lib", "libdbindex_gpu.so"), Arena.global());
@@ -85,6 +94,11 @@ public final class DbiNative {
 	static final MethodHandle dbi_query_hits = h("dbi_query_hits",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
 	static final MethodHandle dbi_query_hits_read = h("dbi_query_hits_read",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
+	// batched getProteins(String): which entry (and so which proteins) every peptide of a list is
+	static final MethodHandle dbi_lookup_peptides = h("dbi_lookup_peptides",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
+	static final MethodHandle dbi_lookup_peptides_read = h("dbi_lookup_peptides_read",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_host_alloc = h("dbi_host_alloc", FunctionDescriptor.of(JAVA_INT, JAVA_LONG, ADDRESS));
 	static final MethodHandle dbi_host_free = h("dbi_host_free", FunctionDescriptor.of(JAVA_INT, ADDRESS));

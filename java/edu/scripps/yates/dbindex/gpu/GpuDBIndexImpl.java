@@ -1,6 +1,7 @@
 package edu.scripps.yates.dbindex.gpu;
 
 import java.io.File;
+import java.util.Collection;
 import java.util.List;
 import java.util.Map;
 import java.util.Set;
@@ -70,8 +71,14 @@ public class GpuDBIndexImpl extends DBIndexImpl {
 		return super.getProteins(seq);
 	}
 
+	/** Memoised as in the reference; a miss reaches GpuDBIndexer.getProteins(String), one dbi_lookup_peptides. */
 	@Override
 	public Set<IndexedProtein> getProteins(String seq) throws DBIndexStoreException {
 		return super.getProteins(seq);
+	}
+
+	/** getProteins(String) for a whole collection (e.g. every distinct identified peptide) in one device call. */
+	public Map<String, Set<IndexedProtein>> getProteins(Collection<String> seqs) throws DBIndexStoreException {
+		return ((GpuDBIndexer) indexer).getProteins(seqs);
 	}
 }

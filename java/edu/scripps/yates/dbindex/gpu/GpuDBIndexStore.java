@@ -381,6 +381,66 @@ public class GpuDBIndexStore implements DBIndexStore {
 		return sb.toString();
 	}
 
+	/**
+	 * getProteins(String) (DBIndexer.java:925-947) for a whole list in one dbi_lookup_peptides + _read per GPU: the
+	 * proteins of the unmodified entry whose peptide equals each string (its mass computed on the device the way
+	 * the index computes it), an empty set when there is none or when that mass has no bucket (Mult:333-338). A
+	 * sharded index asks every GPU: a row is found at most once, by the owner of the slice holding its mass.
+	 */
+	public List<java.util.Set<IndexedProtein>> lookupPeptides(List<String> peptides) throws DBIndexStoreException {
+		requireInit();
+		final int n = peptides.size();
+		final List<java.util.Set<IndexedProtein>> ret = new ArrayList<>(n);
+		for (int i = 0; i < n; ++i)
+			ret.add(new java.util.HashSet<>());
+		final int bucketRange = MAX_MASS / sparam.getIndexFactor();
+		try (Arena a = Arena.ofConfined()) {
+			final java.io.ByteArrayOutputStream packed = new java.io.ByteArrayOutputStream();
+			final MemorySegment off = a.allocate(JAVA_LONG, n + 1L);
+			for (int i = 0; i < n; ++i) {
+				final byte[] b = peptides.get(i).getBytes(java.nio.charset.StandardCharsets.ISO_8859_1);
+				packed.write(b, 0, b.length);
+				off.setAtIndex(JAVA_LONG, i + 1, packed.size());
+			}
+			final byte[] res = packed.toByteArray();
+			final MemorySegment r = a.allocate(Math.max(1, res.length));
+			MemorySegment.copy(res, 0, r, JAVA_BYTE, 0, res.length);
+			final boolean[] found = new boolean[n];
+			for (final MemorySegment h : handles) {
+				final MemorySegment cnt = a.allocate(DbiNative.LOOKUP_COUNTS);
+				check((int) DbiNative.dbi_lookup_peptides.invoke(h, r, off, MemorySegment.NULL, (long) n, cnt));
+				final long nIds = cnt.get(JAVA_LONG, 16);
+				final MemorySegment status = a.allocate(Math.max(1, n)), mass = a.allocate(JAVA_DOUBLE, Math.max(1, n));
+				final MemorySegment plo = a.allocate(JAVA_LONG, n + 1L), ids = a.allocate(JAVA_INT, Math.max(1, nIds));
+				final MemorySegment bufs = a.allocate(DbiNative.LOOKUP_BUFFERS);
+				final MemorySegment[] order = { status, mass, MemorySegment.NULL /* entry */, MemorySegment.NULL /* first_prot */,
+						MemorySegment.NULL /* first_off */, plo, ids };
+				for (int k = 0; k < order.length; ++k)
+					bufs.setAtIndex(ADDRESS, k, order[k]);
+				check((int) DbiNative.dbi_lookup_peptides_read.invoke(h, bufs));
+				for (int i = 0; i < n; ++i) {
+					if (status.get(JAVA_BYTE, i) != 1)
+						continue;
+					if (found[i])
+						throw new DBIndexStoreException("peptide " + peptides.get(i) + " found on two GPUs");
+					found[i] = true;
+					final double m = mass.getAtIndex(JAVA_DOUBLE, i);
+					if ((int) m / bucketRange > sparam.getIndexFactor() - 1)
+						continue; // the zero-tolerance query of the reference returns nothing there
+					for (long k = plo.getAtIndex(JAVA_LONG, i); k < plo.getAtIndex(JAVA_LONG, i + 1); ++k) {
+						final int id = ids.getAtIndex(JAVA_INT, k);
+						ret.get(i).add(new IndexedProtein(proteinCache.getProteinDef(id), id));
+					}
+				}
+			}
+		} catch (final DBIndexStoreException e) {
+			throw e;
+		} catch (final Throwable t) {
+			throw new DBIndexStoreException("Error looking peptides up ", t);
+		}
+		return ret;
+	}
+
 	@Override
 	public Iterator<IndexedSequence> getSequencesIterator(List<MassRange> ranges) throws DBIndexStoreException {
 		return getSequences(ranges).iterator(); // Mult:634-636

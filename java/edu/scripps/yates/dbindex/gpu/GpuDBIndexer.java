@@ -1,10 +1,18 @@
 package edu.scripps.yates.dbindex.gpu;
 
 import java.io.IOException;
+import java.util.ArrayList;
+import java.util.Collection;
+import java.util.LinkedHashMap;
+import java.util.LinkedHashSet;
+import java.util.List;
+import java.util.Map;
+import java.util.Set;
 
 import edu.scripps.yates.dbindex.DBIndexer;
 import edu.scripps.yates.utilities.fasta.dbindex.DBIndexSearchParams;
 import edu.scripps.yates.utilities.fasta.dbindex.DBIndexStoreException;
+import edu.scripps.yates.utilities.fasta.dbindex.IndexedProtein;
 
 /**
  * DBIndexer with the digestion moved to the GPU: run() still streams the FASTA and fills the
@@ -25,5 +33,21 @@ public class GpuDBIndexer extends DBIndexer {
 		} catch (final DBIndexStoreException e) {
 			throw new IOException(e);
 		}
+	}
+
+	/** getProteins(String) (DBIndexer.java:925-947) through the batched device lookup (dbi_lookup_peptides). */
+	@Override
+	public Set<IndexedProtein> getProteins(String sequence) throws DBIndexStoreException {
+		return getProteins(List.of(sequence)).get(sequence);
+	}
+
+	/** getProteins(String) for every distinct string of the collection, in one device call per GPU. */
+	public Map<String, Set<IndexedProtein>> getProteins(Collection<String> sequences) throws DBIndexStoreException {
+		final List<String> distinct = new ArrayList<>(new LinkedHashSet<>(sequences));
+		final List<Set<IndexedProtein>> sets = ((GpuDBIndexStore) indexStore).lookupPeptides(distinct);
+		final Map<String, Set<IndexedProtein>> ret = new LinkedHashMap<>();
+		for (int i = 0; i < distinct.size(); ++i)
+			ret.put(distinct.get(i), sets.get(i));
+		return ret;
 	}
 }
