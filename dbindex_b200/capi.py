@@ -165,10 +165,17 @@ def expand_hits(raw: dict) -> dict:
     return out
 
 
+DBI_ERANGE = -7
+
+
 class DbiError(RuntimeError):
-    def __init__(self, code: int, msg: str):
+    """A non-zero status.  n_candidates: the candidate records of a dbi_search_unindexed that failed (DBI_ERANGE
+    when they exceed the cap), else None."""
+
+    def __init__(self, code: int, msg: str, n_candidates: Optional[int] = None):
         super().__init__(f"{ERR_NAMES.get(code, code)}: {msg}")
         self.code = code
+        self.n_candidates = n_candidates
 
 
 _lib = None
@@ -212,6 +219,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "dbi_query_hits": (C.c_int, [vp, vp, vp, C.c_uint64, C.POINTER(DbiHitCounts)]),
         "dbi_query_hits_device": (C.c_int, [vp, vp, vp, C.c_uint64, C.POINTER(DbiHitCounts)]),
         "dbi_query_hits_read": (C.c_int, [vp, C.POINTER(DbiHitBuffers)]),
+        "dbi_search_unindexed": (C.c_int, [vp, vp, vp, C.c_uint64, C.c_uint64, C.POINTER(DbiHitCounts), u64p]),
         "dbi_lookup_peptides": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.POINTER(DbiLookupCounts)]),
         "dbi_lookup_peptides_read": (C.c_int, [vp, C.POINTER(DbiLookupBuffers)]),
         "dbi_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(vp)]),
@@ -252,6 +260,7 @@ ABI_SYMBOLS = [
     "dbi_default_params", "dbi_params_add_static_mod", "dbi_params_set_enzyme", "dbi_params_add_diff_mod",
     "dbi_create", "dbi_set_stream", "dbi_add_proteins", "dbi_upload", "dbi_reset_index", "dbi_build",
     "dbi_stats_get", "dbi_save", "dbi_load", "dbi_query", "dbi_query_device", "dbi_fetch", "dbi_query_hits", "dbi_query_hits_device", "dbi_query_hits_read",
+    "dbi_search_unindexed",
     "dbi_lookup_peptides", "dbi_lookup_peptides_read", "dbi_host_alloc", "dbi_host_free", "dbi_get_protein", "dbi_calculate_mass",
     "dbi_entry_keys", "dbi_debug_emitted", "dbi_build_from_records", "dbi_debug_radix_sort", "dbi_destroy",
     "dbi_abi_sizes", "dbi_release_cached_memory",
@@ -480,6 +489,31 @@ class GpuIndex:
         hi = np.ascontiguousarray(hi, dtype=np.float64)
         cnt = DbiHitCounts()
         self._check(self.lib.dbi_query_hits(self._h, _ptr(lo), _ptr(hi), len(lo), C.byref(cnt)))
+        return self._read_hits(cnt, fields, alloc, per_hit)
+
+    def search_unindexed_begin(self, lo: np.ndarray, hi: np.ndarray, max_candidates: int = 0) -> DbiHitCounts:
+        """dbi_search_unindexed alone: the hits stay in HBM until query_hits_read / the next call.  Raises DbiError
+        (code DBI_ERANGE, n_candidates set) when the candidate records exceed max_candidates (0 = no cap)."""
+        lo = np.ascontiguousarray(lo, dtype=np.float64)
+        hi = np.ascontiguousarray(hi, dtype=np.float64)
+        if len(lo) != len(hi):
+            raise ValueError(f"{len(lo)} lower and {len(hi)} upper bounds")
+        cnt, n_cand = DbiHitCounts(), C.c_uint64(0)
+        rc = self.lib.dbi_search_unindexed(self._h, _ptr(lo), _ptr(hi), len(lo), int(max_candidates), C.byref(cnt),
+                                           C.byref(n_cand))
+        self.last_candidates = n_cand.value
+        if rc != 0:
+            raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
+        return cnt
+
+    def search_unindexed(self, lo: np.ndarray, hi: np.ndarray, max_candidates: int = 0, fields=None, alloc=None,
+                         per_hit: bool = True) -> dict:
+        """dbi_search_unindexed + dbi_query_hits_read: what query_hits returns for these ranges, answered from the
+        proteins added so far without a built index (the handle stays unbuilt).  The candidate records of the
+        call are in self.last_candidates."""
+        return self._read_hits(self.search_unindexed_begin(lo, hi, max_candidates), fields, alloc, per_hit)
+
+    def _read_hits(self, cnt: DbiHitCounts, fields, alloc, per_hit: bool) -> dict:
         out, bufs = {"counts": cnt}, DbiHitBuffers()
         want = None if fields is None else set(fields)
         if want is not None and per_hit:

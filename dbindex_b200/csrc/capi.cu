@@ -182,6 +182,7 @@ struct dbi_handle {
   bool built = false;
   DevBuf d_tables, d_err;
   DevBuf d_res, d_pstart;
+  uint64_t packed_prot = UINT64_MAX;  // proteins d_res / d_pstart hold (K1 ran on them)
   uint32_t res_end = 0;
   uint64_t res_alloc = 0;  // bytes readable at d_res (multiple of 16: tiles are staged with bulk copies)
   uint64_t n_emitted = 0, n_unique = 0, n_entries = 0;
@@ -206,6 +207,7 @@ struct dbi_handle {
     uint64_t peer_cap[kMaxRanks] = {};
   };
   int mg_rank = 0, mg_world = 1;
+  bool mg_begun = false;  // dbi_mg_begin was called
   MgWindow win[3];
   uint64_t prot_off[kMaxRanks + 1] = {};  // global id of every rank's first protein
   uint64_t pos_off[kMaxRanks + 1] = {};   // buffer position of every rank's first separator
@@ -249,6 +251,7 @@ struct dbi_handle {
   } lookup;
 
   DigestCfg cfg{};
+  MassWindows shifts{};  // the shift intervals of an unindexed search (no windows yet)
   dbi_stats st{};
   // profiling (params.profile): event pairs recorded on the stream without any extra
   // synchronisation and resolved after the final sync of the call
@@ -410,22 +413,34 @@ uint64_t read_u64(dbi_handle* h, const uint64_t* d) {
   return v;
 }
 
-void free_index(dbi_handle* h) {
-  if (h->pull_pending) {  // peer copies into d_res still in flight
-    cudaStreamSynchronize(h->side_stream);
-    h->pull_pending = false;
-  }
-  h->built = false;
-  h->hits.drop();
-  h->lookup.drop();
-  h->d_res.release();
-  h->d_pstart.release();
+// The tables an index build derives from the packed residues: unique peptides, protein lists, entries.
+void free_tables(dbi_handle* h) {
   h->u_mass.release(); h->u_gpos.release(); h->u_prot.release(); h->u_len.release();
   h->u_plo.release(); h->plist.release();
   h->e_mass.release(); h->e_base.release(); h->e_pat.release();
   h->u_cmask.release(); h->d_nlong.release();
   h->cmask_n = UINT64_MAX;
   h->k_mass.release(); h->k_gpos.release(); h->k_prot.release(); h->k_len.release();
+  h->n_emitted = h->n_unique = h->n_entries = 0;
+}
+
+// The pending results of dbi_query_hits / dbi_search_unindexed and dbi_lookup_peptides.
+void drop_results(dbi_handle* h) {
+  h->hits.drop();
+  h->lookup.drop();
+}
+
+void free_index(dbi_handle* h) {
+  if (h->pull_pending) {  // peer copies into d_res still in flight
+    cudaStreamSynchronize(h->side_stream);
+    h->pull_pending = false;
+  }
+  h->built = false;
+  drop_results(h);
+  h->d_res.release();
+  h->d_pstart.release();
+  h->packed_prot = UINT64_MAX;
+  free_tables(h);
   h->mg_mass.release(); h->mg_gpos.release(); h->mg_prot.release(); h->mg_len.release();
   h->mg_nmod.release();
   h->mg_vkey.release(); h->mg_vpay.release();
@@ -434,7 +449,6 @@ void free_index(dbi_handle* h) {
   h->mg_layout = false;
   h->ent_base_off = 0;
   std::memset(h->uoff, 0, sizeof(h->uoff));
-  h->n_emitted = h->n_unique = h->n_entries = 0;
   h->spans.clear();
   h->ev_used = 0;
   const uint64_t np = h->st.n_proteins, nr = h->st.n_residues;
@@ -495,6 +509,7 @@ void upload_tables(dbi_handle* h) {
     h->cfg.n_seq = g <= 32 ? (int)g : 0;
     if (std::getenv("DBI_NO_GROUPS")) h->cfg.n_seq = 0;  // diagnostic: force the per-variant path
   }
+  shift_intervals(t, h->cfg, &h->shifts);
   h->d_tables.alloc(sizeof(DevTables), h->arena);
   DBI_CUDA(cudaMemcpyAsync(h->d_tables.p, &t, sizeof(t), cudaMemcpyHostToDevice, h->stream));
   DBI_CUDA(cudaStreamSynchronize(h->stream));  // `t` is on this stack frame
@@ -540,6 +555,7 @@ void pack_residues(dbi_handle* h) {
   DBI_CUDA(cudaMemsetAsync((uint8_t*)h->d_res.p + res_end, 0, padded - res_end, h->stream));
   launch_pack(h->d_raw.as<uint8_t>(), h->d_off.as<uint64_t>(), n_prot, n_res, h->d_res.as<uint8_t>(),
               h->d_pstart.as<uint32_t>(), 0u, h->d_err.as<uint32_t>(), h->stream);
+  h->packed_prot = n_prot;
   h->st.algo_bytes[DBI_STAGE_PACK] += 2 * n_res + (uint64_t)n_prot * 12;
 }
 
@@ -1623,6 +1639,132 @@ int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out) {
   DBI_CUDA(cudaStreamSynchronize(s));
   r.drop();
   return DBI_OK;
+  DBI_API_END
+}
+
+int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, uint64_t max_candidates,
+                         dbi_hit_counts* counts, uint64_t* n_candidates) {
+  DBI_API_BEGIN(h)
+  if (h->built) {
+    set_error("the index is built: query it with dbi_query_hits");
+    return DBI_EALREADY;
+  }
+  if (h->mg_begun) {
+    set_error("an unindexed search runs on one GPU; this handle is part of a sharded build");
+    return DBI_EINVAL;
+  }
+  if (!counts || (nq && (!lo || !hi))) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  cudaStream_t s = h->stream;
+  drop_results(h);
+  if (n_candidates) *n_candidates = 0;
+  if (nq >= (1ull << 32)) {
+    set_error("%llu windows in one batch (< 2^32)", (unsigned long long)nq);
+    return DBI_ERANGE;
+  }
+  // this search's candidate pipeline replaces the stats of the previous one
+  h->spans.clear();
+  h->ev_used = 0;
+  {
+    const uint64_t np = h->st.n_proteins, nr = h->st.n_residues;
+    std::memset(&h->st, 0, sizeof(h->st));
+    h->st.n_proteins = np;
+    h->st.n_residues = nr;
+  }
+  ensure_uploaded(h);
+  const uint32_t zero = 0;
+  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, s));
+  const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
+  if (h->packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
+
+  // K12: the batch's windows, sorted by lo, with the prefix maximum of hi
+  DevBuf io;  // lo | hi (the caller's order, for the materialisation) | sorted lo | prefix max of hi
+  io.alloc(std::max<uint64_t>(nq, 1) * 32, h->arena);
+  double* d_lo = io.as<double>();
+  double* d_hi = d_lo + nq;
+  double* w_lo = d_hi + nq;
+  double* w_pmax = w_lo + nq;
+  MassWindows win = h->shifts;
+  win.lo = w_lo;
+  win.pmax = w_pmax;
+  win.n = (uint32_t)nq;
+  if (nq) {
+    DBI_CUDA(cudaMemcpyAsync(d_lo, lo, nq * 8, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, cudaMemcpyHostToDevice, s));
+    Stage sg(h, DBI_STAGE_OTHER);
+    DevBuf wk[2], wv[2], wtmp;
+    for (int i = 0; i < 2; ++i) {
+      wk[i].alloc(nq * 8, h->arena);
+      wv[i].alloc(nq * 8, h->arena);
+    }
+    wtmp.alloc(radix_sort_tmp_bytes(nq), h->arena);
+    launch_win_keys(d_lo, d_hi, nq, h->p.min_mass, h->p.max_mass, wk[0].as<uint64_t>(), wv[0].as<uint64_t>(), s);
+    uint64_t* kk[2] = {wk[0].as<uint64_t>(), wk[1].as<uint64_t>()};
+    uint64_t* vv[2] = {wv[0].as<uint64_t>(), wv[1].as<uint64_t>()};
+    const int nbits = bit_length(win_drop_key(h->p.min_mass, h->p.max_mass));
+    const int r = radix_sort_pairs<uint64_t, uint64_t>(kk, vv, nq, 0, nbits, wtmp.p, s, nullptr);
+    launch_win_pmax(kk[r], vv[r], nq, h->p.min_mass, h->p.max_mass, w_lo, w_pmax, s);
+    h->st.algo_bytes[DBI_STAGE_OTHER] += nq * (16 + 16) + nq * 32ull * ((nbits + 7) / 8) + nq * 32;
+  }
+
+  // K2u: the records that can land in a window, counted before anything is allocated
+  const uint64_t tiles = nq ? ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile : 0;
+  DevBuf tile_counts, tile_offs, start_cnt;
+  tile_counts.alloc(std::max<uint64_t>(tiles, 1) * 4, h->arena);
+  tile_offs.alloc((tiles + 1) * 8, h->arena);
+  start_cnt.alloc(std::max<uint64_t>(tiles, 1) * kDigestTile, h->arena);
+  const DigestRange whole{0u, h->res_end, 0u, n_prot};
+  uint64_t N = 0;
+  if (tiles) {
+    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
+    launch_digest_count(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
+                        (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), s,
+                        &win);
+    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
+    N = read_u64(h, tile_offs.as<uint64_t>() + tiles);
+    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2ull * h->res_end + tiles * 16;
+  }
+  if (int rc = check_err_bits(read_err(h))) return rc;
+  if (n_candidates) *n_candidates = N;
+  h->st.n_emitted = N;
+  if ((max_candidates && N > max_candidates) || N >= (1ull << 32)) {
+    set_error("%llu candidate records exceed the cap of %llu (and 2^32): split the batch", (unsigned long long)N,
+              (unsigned long long)(max_candidates ? max_candidates : (1ull << 32) - 1));
+    resolve_spans(h);
+    return DBI_ERANGE;
+  }
+  DevBuf r_mass, r_gpos, r_prot, r_len;
+  r_mass.alloc(std::max<uint64_t>(N, 1) * 8, h->arena);
+  r_gpos.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
+  r_prot.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
+  r_len.alloc(std::max<uint64_t>(N, 1) * 2, h->arena);
+  if (N) {  // K4u
+    Stage sg(h, DBI_STAGE_DIGEST_EMIT);
+    launch_digest_emit(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
+                       (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
+                       r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>(),
+                       nullptr, h->d_err.as<uint32_t>(), s, &win);
+    h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2ull * h->res_end + N * 18;
+  }
+  tile_counts.release();
+  tile_offs.release();
+  start_cnt.release();
+
+  // the candidate index lives for this call only; the pending result does not depend on it
+  struct DropCandidates {
+    dbi_handle* h;
+    ~DropCandidates() {
+      free_tables(h);
+      h->built = false;
+    }
+  } drop_candidates{h};
+  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
+  if (int rc = index_records(h, rv, N, h->p.min_mass, h->p.max_mass)) return rc;
+  if (int rc = check_err_bits(read_err(h))) return rc;
+  r_mass.release(); r_gpos.release(); r_prot.release(); r_len.release();
+  return query_hits_impl(h, d_lo, d_hi, nq, counts);
   DBI_API_END
 }
 

@@ -127,11 +127,12 @@ __device__ __forceinline__ void at_pos(const TileCtx& cx, uint32_t pos, uint8_t*
 }
 
 // The body of the reference's `for start` iteration (DBIndexer.java:256-395) for the
-// start at buffer position g.  F is called as emit(mass, len) for every record.
+// start at buffer position g.  F is called as emit(mass, len, n_mod) for every record that keep(mass, n_mod)
+// accepts; a rejected record is neither emitted nor counted, and the walk goes on.
 // FILTERS = false compiles the two peptide filters (SURVEY 8 f4) out of the loop.
-template <bool FILTERS, typename F>
+template <bool FILTERS, typename Keep, typename F>
 __device__ __forceinline__ uint32_t walk_start(const TileCtx& cx, uint32_t g, const DigestCfg& cfg, uint32_t* err,
-                                               F&& emit) {
+                                               const Keep& keep, F&& emit) {
   uint8_t inf;
   double m;
   at_pos(cx, g, &inf, &m);
@@ -169,8 +170,10 @@ __device__ __forceinline__ uint32_t walk_start(const TileCtx& cx, uint32_t g, co
             atomicOr(err, kErrPepTooLong);
             break;
           }
-          emit(mass, len, n_mod);
-          ++count;
+          if (keep(mass, n_mod)) {
+            emit(mass, len, n_mod);
+            ++count;
+          }
         }
       }
     }
@@ -209,15 +212,21 @@ __device__ __forceinline__ void stage_tile(TileSmem& s, const uint8_t* __restric
   __syncthreads();
 }
 
+// every record of the walk (the index build)
+struct AllRecords {
+  __device__ __forceinline__ bool operator()(double, uint32_t) const { return true; }
+};
+
 // ---- K2 -----------------------------------------------------------------------------
 // Warp-cooperative cleavage-site scan: the CTA compacts the live starts of its tile (for trypsin
 // ~11 % of the residues can start a peptide), one lane walks each, and the per-start counts go
-// back to HBM for K4.
-template <bool FILTERS>
+// back to HBM for K4.  Keep = AllRecords: the index build; InWindows: K2u of an unindexed search.
+template <bool FILTERS, typename Keep>
 __global__ void __launch_bounds__(DG_THREADS)
     digest_count_kernel(const uint8_t* __restrict__ res, DigestRange rg, uint64_t res_alloc,
                         const DevTables* __restrict__ tb, DigestCfg cfg, uint32_t tile0,
-                        uint8_t* __restrict__ start_cnt, uint32_t* __restrict__ tile_counts, uint32_t* err) {
+                        uint8_t* __restrict__ start_cnt, uint32_t* __restrict__ tile_counts, uint32_t* err,
+                        const Keep keep) {
   __shared__ TileSmem s;
   const int t = threadIdx.x;
   const uint32_t w0 = (tile0 + blockIdx.x) * (uint32_t)kDigestTile;  // start l of the tile sits at w0 + 1 + l
@@ -245,7 +254,7 @@ __global__ void __launch_bounds__(DG_THREADS)
   uint32_t cnt = 0;
   for (uint32_t i = t; i < total; i += DG_THREADS) {
     const uint32_t l = s.list[i];
-    const uint32_t c = walk_start<FILTERS>(cx, w0 + 1 + l, cfg, err, [](double, uint32_t, uint32_t) {});
+    const uint32_t c = walk_start<FILTERS>(cx, w0 + 1 + l, cfg, err, keep, [](double, uint32_t, uint32_t) {});
     s.cnt8[l] = (uint8_t)(c < 255u ? c : 255u);
     cnt += c;
   }
@@ -256,14 +265,15 @@ __global__ void __launch_bounds__(DG_THREADS)
 }
 
 // ---- K4 -----------------------------------------------------------------------------
-template <bool FILTERS>
+// (K4u: the same with the Keep of K2u, so that counts and recounts agree)
+template <bool FILTERS, typename Keep>
 __global__ void __launch_bounds__(DG_THREADS)
     digest_emit_kernel(const uint8_t* __restrict__ res, DigestRange rg, uint64_t res_alloc,
                        const DevTables* __restrict__ tb, DigestCfg cfg, uint32_t tile0,
                        const uint8_t* __restrict__ start_cnt, const uint64_t* __restrict__ tile_offs,
                        const uint32_t* __restrict__ pstart, uint64_t* __restrict__ o_mass,
                        uint32_t* __restrict__ o_gpos, uint32_t* __restrict__ o_prot, uint16_t* __restrict__ o_len,
-                       uint8_t* __restrict__ o_nmod, uint32_t* err) {
+                       uint8_t* __restrict__ o_nmod, uint32_t* err, const Keep keep) {
   __shared__ TileSmem s;
   __shared__ uint32_t s_off[kDigestTile];   // first record of each emitting start (tile-local)
   __shared__ uint16_t s_zero[kDigestTile];  // separators between the tile's first start and this one
@@ -296,7 +306,8 @@ __global__ void __launch_bounds__(DG_THREADS)
 #pragma unroll
     for (int k = 0; k < DG_SPT; ++k) {
       c[k] = ((k < 4 ? packed.x : packed.y) >> (8 * (k & 3))) & 0xffu;
-      if (c[k] == 255u) c[k] = walk_start<FILTERS>(cx, w0 + 1 + t * DG_SPT + k, cfg, err, [](double, uint32_t, uint32_t) {});
+      if (c[k] == 255u)
+        c[k] = walk_start<FILTERS>(cx, w0 + 1 + t * DG_SPT + k, cfg, err, keep, [](double, uint32_t, uint32_t) {});
       n_emit += c[k] ? 1u : 0u;
       sum += c[k];
       if ((s.info[1 + t * DG_SPT + k] & I_SEP) && w0 + 1 + t * DG_SPT + k >= rg.start_lo) {
@@ -325,7 +336,7 @@ __global__ void __launch_bounds__(DG_THREADS)
     // protein of this start = separators at positions <= g, minus one
     const uint32_t prot = zbase + s_zero[i] - 1u;
     uint64_t o = tile_off + s_off[i];
-    walk_start<FILTERS>(cx, g, cfg, err, [&](double m, uint32_t len, uint32_t n_mod) {
+    walk_start<FILTERS>(cx, g, cfg, err, keep, [&](double m, uint32_t len, uint32_t n_mod) {
       o_mass[o] = (uint64_t)__double_as_longlong(m);
       o_gpos[o] = g;
       o_prot[o] = prot;
@@ -397,16 +408,36 @@ void launch_pack(const uint8_t* d_raw, const uint64_t* d_off, uint32_t n_prot, u
   DBI_LAUNCH(pack_kernel, grid, PK_THREADS, 0, s, d_raw, d_off, n_prot, n_res, d_res, d_pstart, pos_base, d_err);
 }
 
+namespace {
+template <typename Keep>
+void digest_count(const uint8_t* d_res, const DigestRange& rg, uint64_t res_alloc, const DevTables* d_tb,
+                  const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, uint8_t* d_start_cnt, uint32_t* d_tile_counts,
+                  uint32_t* d_err, cudaStream_t s, const Keep& keep) {
+  // FILTERS = true only when a peptide filter is on
+  const auto kern = (cfg.mand_on || cfg.filt_max >= 0) ? digest_count_kernel<true, Keep> : digest_count_kernel<false, Keep>;
+  DBI_LAUNCH(kern, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc,
+             d_tb, cfg, tile0, d_start_cnt, d_tile_counts, d_err, keep);
+}
+template <typename Keep>
+void digest_emit(const uint8_t* d_res, const DigestRange& rg, uint64_t res_alloc, const DevTables* d_tb,
+                 const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, const uint8_t* d_start_cnt,
+                 const uint64_t* d_tile_offs, const uint32_t* d_pstart, uint64_t* o_mass, uint32_t* o_gpos,
+                 uint32_t* o_prot, uint16_t* o_len, uint8_t* o_nmod, uint32_t* d_err, cudaStream_t s, const Keep& keep) {
+  // FILTERS = true only when a peptide filter is on
+  const auto kern = (cfg.mand_on || cfg.filt_max >= 0) ? digest_emit_kernel<true, Keep> : digest_emit_kernel<false, Keep>;
+  DBI_LAUNCH(kern, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc,
+             d_tb, cfg, tile0, d_start_cnt, d_tile_offs, d_pstart, o_mass, o_gpos, o_prot, o_len, o_nmod, d_err, keep);
+}
+}  // namespace
+
 void launch_digest_count(const uint8_t* d_res, const DigestRange& rg, uint64_t res_alloc, const DevTables* d_tb,
                          const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, uint8_t* d_start_cnt,
-                         uint32_t* d_tile_counts, uint32_t* d_err, cudaStream_t s) {
+                         uint32_t* d_tile_counts, uint32_t* d_err, cudaStream_t s, const MassWindows* windows) {
   if (ntiles == 0) return;
-  if (cfg.mand_on || cfg.filt_max >= 0)
-    DBI_LAUNCH(digest_count_kernel<true>, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc, d_tb, cfg, tile0,
-               d_start_cnt, d_tile_counts, d_err);
+  if (windows)
+    digest_count(d_res, rg, res_alloc, d_tb, cfg, tile0, ntiles, d_start_cnt, d_tile_counts, d_err, s, InWindows{*windows});
   else
-    DBI_LAUNCH(digest_count_kernel<false>, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc, d_tb, cfg, tile0,
-               d_start_cnt, d_tile_counts, d_err);
+    digest_count(d_res, rg, res_alloc, d_tb, cfg, tile0, ntiles, d_start_cnt, d_tile_counts, d_err, s, AllRecords{});
 }
 
 void launch_scan_u32_to_u64(const uint32_t* d_in, uint64_t n, uint64_t* d_offs, cudaStream_t s) {
@@ -417,14 +448,14 @@ void launch_digest_emit(const uint8_t* d_res, const DigestRange& rg, uint64_t re
                         const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, const uint8_t* d_start_cnt,
                         const uint64_t* d_tile_offs, const uint32_t* d_pstart, uint64_t* o_mass,
                         uint32_t* o_gpos, uint32_t* o_prot, uint16_t* o_len, uint8_t* o_nmod, uint32_t* d_err,
-                        cudaStream_t s) {
+                        cudaStream_t s, const MassWindows* windows) {
   if (ntiles == 0) return;
-  if (cfg.mand_on || cfg.filt_max >= 0)
-    DBI_LAUNCH(digest_emit_kernel<true>, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc, d_tb, cfg, tile0,
-               d_start_cnt, d_tile_offs, d_pstart, o_mass, o_gpos, o_prot, o_len, o_nmod, d_err);
+  if (windows)
+    digest_emit(d_res, rg, res_alloc, d_tb, cfg, tile0, ntiles, d_start_cnt, d_tile_offs, d_pstart, o_mass, o_gpos,
+                o_prot, o_len, o_nmod, d_err, s, InWindows{*windows});
   else
-    DBI_LAUNCH(digest_emit_kernel<false>, ntiles, DG_THREADS, 0, s, d_res, rg, res_alloc, d_tb, cfg, tile0,
-               d_start_cnt, d_tile_offs, d_pstart, o_mass, o_gpos, o_prot, o_len, o_nmod, d_err);
+    digest_emit(d_res, rg, res_alloc, d_tb, cfg, tile0, ntiles, d_start_cnt, d_tile_offs, d_pstart, o_mass, o_gpos,
+                o_prot, o_len, o_nmod, d_err, s, AllRecords{});
 }
 
 }  // namespace dbi

@@ -51,9 +51,53 @@ void launch_pack(const uint8_t* d_raw, const uint64_t* d_off, uint32_t n_prot, u
 struct DigestRange {
   uint32_t start_lo, start_hi, prot_lo, prot_hi;
 };
+
+// Unindexed search (dbi_search_unindexed): the mass windows of a query batch and the mass shifts a peptide's
+// variants can add.  K2u / K4u keep a record of base mass m with n_mod modifiable sites iff for some
+// k <= min(max_mods, n_mod) and some shift interval [s_lo, s_hi] of k mods, [m + s_lo, m + s_hi] meets the
+// union of the windows.  Windows are sorted by lo; pmax[i] = max(hi[0..i]); a mass interval [a, b] meets the
+// union iff the last window with lo <= b has pmax >= a.  Dropped windows (inverted, NaN, outside
+// [min_mass, max_mass]) sort last with lo = +inf.  Passed by value: a kernel parameter.
+constexpr int kMaxShiftIv = 64;
+struct MassWindows {
+  const double* lo;
+  const double* pmax;
+  uint32_t n;
+  int32_t kmax;                               // max_mods (0 without differential mods)
+  uint8_t k_end[DBI_MAX_MODS_PER_PEP + 1];    // intervals of <= k mods: [0, k_end[k])
+  double s_lo[kMaxShiftIv], s_hi[kMaxShiftIv];
+};
+#ifdef __CUDACC__
+__device__ __forceinline__ bool windows_meet(const MassWindows& w, double a, double b) {
+  uint32_t lo = 0, hi = w.n;  // upper_bound(lo[], b)
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (__ldg(w.lo + mid) <= b) lo = mid + 1; else hi = mid;
+  }
+  return lo > 0 && __ldg(w.pmax + lo - 1) >= a;
+}
+// the record filter of K2u / K4u
+struct InWindows {
+  MassWindows w;
+  __device__ __forceinline__ bool operator()(double m, uint32_t n_mod) const {
+    const uint32_t k = n_mod < (uint32_t)w.kmax ? n_mod : (uint32_t)w.kmax;
+    const int end = w.k_end[k];
+    for (int j = 0; j < end; ++j)
+      if (windows_meet(w, __dadd_rn(m, w.s_lo[j]), __dadd_rn(m, w.s_hi[j]))) return true;
+    return false;
+  }
+};
+#endif
+// host: the shift intervals of p's differential mods (distinct sums of k class shifts +- eps for k = 0, 1, ...;
+// a k whose sums do not fit any more gets the band [k mod_lo - eps, k mod_hi + eps])
+constexpr double kShiftEps = 1e-9;
+void shift_intervals(const DevTables& t, const DigestCfg& cfg, MassWindows* w);
+
+// windows: K2 / K4 emit only the records InWindows keeps (nullptr = every record)
 void launch_digest_count(const uint8_t* d_res, const DigestRange& rg, uint64_t res_alloc, const DevTables* d_tb,
                          const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, uint8_t* d_start_cnt,
-                         uint32_t* d_tile_counts, uint32_t* d_err, cudaStream_t s);
+                         uint32_t* d_tile_counts, uint32_t* d_err, cudaStream_t s,
+                         const MassWindows* windows = nullptr);
 
 // K3: exclusive scan of u32 tile counts into u64 offsets; offs[n] = total.
 void launch_scan_u32_to_u64(const uint32_t* d_in, uint64_t n, uint64_t* d_offs, cudaStream_t s);
@@ -66,7 +110,16 @@ void launch_digest_emit(const uint8_t* d_res, const DigestRange& rg, uint64_t re
                         const DigestCfg& cfg, uint32_t tile0, uint32_t ntiles, const uint8_t* d_start_cnt,
                         const uint64_t* d_tile_offs, const uint32_t* d_pstart, uint64_t* o_mass,
                         uint32_t* o_gpos, uint32_t* o_prot, uint16_t* o_len, uint8_t* o_nmod, uint32_t* d_err,
-                        cudaStream_t s);
+                        cudaStream_t s, const MassWindows* windows = nullptr);
+
+// K12 (window.cu): the windows of a batch for InWindows.  K12a: sort records key = bits(clipped lo) - bits(min_mass)
+// (dropped windows: drop_key), value = bits(clipped hi); *nbits = key width.  K12b (after the K7 sort): lo and the
+// inclusive prefix max of hi in sorted order.
+void launch_win_keys(const double* lo, const double* hi, uint64_t n, double min_mass, double max_mass, uint64_t* key,
+                     uint64_t* val, cudaStream_t s);
+uint64_t win_drop_key(double min_mass, double max_mass);
+void launch_win_pmax(const uint64_t* key, const uint64_t* val, uint64_t n, double min_mass, double max_mass,
+                     double* w_lo, double* w_pmax, cudaStream_t s);
 
 // ---- sort helpers / K8 dedup -------------------------------------------------
 // hash[i] = seeded hash of the residues of record i (u32, or u64 when wide); idx[i] = i.

@@ -21,7 +21,7 @@ from typing import List, Optional, Sequence, Set, Tuple
 
 import numpy as np
 
-from .capi import DbiError, DbiParams, GpuIndex, parse_fasta
+from .capi import DBI_ERANGE, DbiError, DbiHitCounts, DbiParams, GpuIndex, _expand_csr, parse_fasta
 
 MAX_INDEX_RESIDUE_LEN = 3      # Constants.java:44
 MAX_PRECURSOR_MASS = 8000      # Constants.java:20
@@ -243,17 +243,85 @@ def createFullIndexFileName(sparam: "DBIndexSearchParams") -> str:
 
 INDEX_FILE_SUFFIX = ".gpuidx"  # the reference's directory is <name>.idx (DBIndexer.java:63,429-431)
 
+# Unindexed search (useIndex = false): candidate records one dbi_search_unindexed may index.  A candidate of a
+# 3-mod parameter set expands to ~26 entries of ~40 bytes while it is indexed, so 2^25 candidates stay well inside
+# one GPU's memory and below 2^32 entries.
+UNINDEXED_MAX_CANDIDATES = 1 << 25
+
+
+def _merge_hits(parts, nq: int) -> dict:
+    """The per-hit answers of several batches of queries (part = (query ids, query_hits-style dict)) as one answer
+    for queries 0 .. nq-1 in that order; a query's hits keep their order."""
+    qid = np.concatenate([np.repeat(ids, np.diff(h["hit_off"].astype(np.int64))) for ids, h in parts] +
+                         [np.zeros(0, np.int64)]).astype(np.int64)
+    perm = np.argsort(qid, kind="stable")
+
+    def cat(k, dt):
+        return np.concatenate([h[k] for _, h in parts] + [np.zeros(0, dt)])
+
+    def cat_csr(off_key, data_key, dt):
+        offs, base = [], 0
+        for _, h in parts:
+            offs.append(h[off_key][:-1].astype(np.int64) + base)
+            base += int(h[off_key][-1])
+        return np.append(np.concatenate(offs + [np.zeros(0, np.int64)]), base), cat(data_key, dt)
+
+    out = {k: cat(k, dt)[perm] for k, dt in (("modpat", np.uint32), ("mass", np.float64), ("first_prot", np.uint32),
+                                             ("first_off", np.uint32), ("len", np.uint16))}
+    run_base = np.cumsum([0] + [int(h["counts"].n_peps) for _, h in parts])
+    out["hit_pep"] = np.concatenate([h["hit_pep"] + run_base[i] for i, (_, h) in enumerate(parts)] +
+                                    [np.zeros(0, np.int64)])[perm]
+    out["flanks"] = np.ascontiguousarray(cat("flanks", np.uint8).reshape(-1, 6)[perm]).reshape(-1)
+    out["seq_off"], out["seq"] = _expand_csr(*cat_csr("seq_off", "seq", np.uint8), perm)
+    out["prot_list_off"], out["prot_ids"] = _expand_csr(*cat_csr("prot_list_off", "prot_ids", np.uint32), perm)
+    out["hit_off"] = np.concatenate(([0], np.cumsum(np.bincount(qid, minlength=nq)))).astype(np.uint64)
+    out["counts"] = DbiHitCounts(nq, len(perm), int(run_base[-1]), len(out["seq"]), len(out["prot_ids"]))
+    return out
+
+
+def search_unindexed_chunked(index: GpuIndex, lo, hi, max_candidates: int) -> dict:
+    """query_hits-style answer (one record per hit) of the ranges [lo[i], hi[i]] on an unbuilt handle, through
+    dbi_search_unindexed calls of at most max_candidates candidate records each (0 = one call, no cap).  The
+    ranges go to the device sorted by mass; a batch whose N_c candidates exceed the cap is split into
+    ceil(N_c / cap) + 1 contiguous chunks of the sorted order (again if a chunk still exceeds it), and the answer
+    comes back in the caller's order."""
+    lo = np.ascontiguousarray(lo, dtype=np.float64)
+    hi = np.ascontiguousarray(hi, dtype=np.float64)
+    parts = []
+
+    def run(ids):
+        try:
+            parts.append((ids, index.search_unindexed(lo[ids], hi[ids], max_candidates)))
+        except DbiError as e:
+            n_c = e.n_candidates or 0
+            if e.code != DBI_ERANGE or not max_candidates or n_c <= max_candidates or len(ids) < 2:
+                raise
+            for chunk in np.array_split(ids, min(len(ids), -(-n_c // max_candidates) + 1)):
+                run(chunk)
+
+    run(np.argsort(lo, kind="stable"))
+    return _merge_hits(parts, len(lo))
+
 
 class DBIndexer:
     """DBIndexer.java: the indexer / orchestrator, GPU store behind it."""
 
-    def __init__(self, params: DbiParams, index_factor: int = 8, index_path: Optional[str] = None):
+    def __init__(self, params: DbiParams, index_factor: int = 8, index_path: Optional[str] = None,
+                 use_index: bool = True):
         """index_path: where the finished index lives on disk (None = in-memory index only).  run() skips
         indexing when the file exists ("Found existing index, skipping indexing", DBIndexer.java:522-531)
-        and writes it after a fresh build."""
+        and writes it after a fresh build.
+
+        use_index = False is the reference's SEARCH_UNINDEXED mode (DBIndexer.java:58-61, MassRangeFilteringIndex):
+        run() only adds the proteins, and every getSequences* digests them again for its batch of ranges on the
+        GPU (dbi_search_unindexed), max_candidates candidate records per device call.  No index file is read or
+        written.  getNumberSequences, getParentMasses and export_reference_index need an index and raise
+        DBIndexStoreException in this mode."""
         self.sparam = params
         self.index_factor = index_factor  # dbindex.properties:6; only shapes the ">= MAX_MASS" query rule
         self.index_path = index_path
+        self.use_index = use_index
+        self.max_candidates = UNINDEXED_MAX_CANDIDATES
         self.loaded_from_disk = False
         self.inited = False
         self.index: Optional[GpuIndex] = None
@@ -273,7 +341,7 @@ class DBIndexer:
         DBIndexStoreSQLiteByteIndexMerge.java:696-716) -- so that an unmodified reference finds an existing index
         there (SURVEY.md 8 f3).  Differential-mod variants have no counterpart in that format and are left out."""
         from .sqlite_export import export_sqlite
-        self._require()
+        self._require_index()
         n = self.index.stats()["n_entries"]
         return export_sqlite(lambda b, c: self.index.fetch(b, c), n, database_id, index_factor=self.index_factor,
                              mass_group_factor=self.sparam.mass_group_factor)
@@ -281,6 +349,11 @@ class DBIndexer:
     def _require(self):
         if not self.inited or self.index is None:
             raise DBIndexStoreException("Indexer is not initialized")  # DBIndexStoreSQLiteMult.java:153
+
+    def _require_index(self):
+        self._require()
+        if not self.use_index:
+            raise DBIndexStoreException("not available in unindexed search mode (useIndex = false): there is no index")
 
     def add_proteins(self, deflines: Sequence[str], residues: np.ndarray, offsets: np.ndarray):
         """protCache.addProtein for a packed batch (DBIndexer.java:605)."""
@@ -291,7 +364,7 @@ class DBIndexer:
     def run(self, fasta: Optional[str] = None, proteins: Optional[Tuple[Sequence[str], Sequence[str]]] = None):
         """DBIndexer.run(): stream the FASTA, cut every protein, close the store."""
         self._require()
-        if self.index_path is not None and os.path.exists(self.index_path):
+        if self.use_index and self.index_path is not None and os.path.exists(self.index_path):
             # indexStore.indexExists() -> "Found existing index, skipping indexing" (DBIndexer.java:522-531)
             try:
                 self.index.load(self.index_path)
@@ -313,6 +386,8 @@ class DBIndexer:
             offsets = np.zeros(len(seqs) + 1, dtype=np.uint64)
             np.cumsum([len(s) for s in seqs], out=offsets[1:])
             self.add_proteins(deflines, residues, offsets)
+        if not self.use_index:  # SEARCH_UNINDEXED: the proteins are all the store keeps
+            return
         try:
             self.index.build()  # cutSeq per protein + stopAddSeq (DBIndexer.java:616,666)
             if self.index_path is not None:
@@ -342,14 +417,21 @@ class DBIndexer:
         nb = self.index_factor
         return int(lo) // bucket_range > nb - 1 or int(hi) // bucket_range > nb - 1
 
-    def _materialise(self, lo: np.ndarray, hi: np.ndarray, keep: Optional[np.ndarray] = None) -> List[List[IndexedSequence]]:
-        """getSequences for a batch of ranges in ONE device pass (dbi_query_hits): the objects
-        parseAddPeptideInfo builds (DBIndexStoreSQLiteByteIndexMerge.java:452-462) -- sequence, flanks,
-        mass and protein ids all come back from the GPU; only the Python objects are made here."""
+    def _hits(self, lo: np.ndarray, hi: np.ndarray) -> dict:
+        """The hit source of every getSequences*: one record per hit of every [lo[i], hi[i]] (query_hits), from
+        the index, or in unindexed mode from the proteins (chunked dbi_search_unindexed)."""
         try:
-            h = self.index.query_hits(lo, hi)
+            if self.use_index:
+                return self.index.query_hits(lo, hi)
+            return search_unindexed_chunked(self.index, lo, hi, self.max_candidates)
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
+
+    def _materialise(self, lo: np.ndarray, hi: np.ndarray, keep: Optional[np.ndarray] = None) -> List[List[IndexedSequence]]:
+        """getSequences for a batch of ranges in ONE device pass (dbi_query_hits, or dbi_search_unindexed): the
+        objects parseAddPeptideInfo builds (DBIndexStoreSQLiteByteIndexMerge.java:452-462) -- sequence, flanks,
+        mass and protein ids all come back from the GPU; only the Python objects are made here."""
+        h = self._hits(lo, hi)
         ho, so, po = (h[k].astype(np.int64) for k in ("hit_off", "seq_off", "prot_list_off"))
         seq, flanks = h["seq"].tobytes().decode("latin-1"), h["flanks"].tobytes().decode("latin-1")
         out = []
@@ -439,8 +521,14 @@ class DBIndexer:
         """getProteins(String) for a whole list in one device call (dbi_lookup_peptides): the unmodified entry
         whose peptide equals the string, found by its mass computed the way the index computes it
         (IndexUtil.calculateMass) -- the zero-tolerance getSequences + `s.sequence.equals(seq)` filter of the
-        reference.  A mass whose bucket lies beyond MAX_MASS gives the empty set, as that query does."""
+        reference.  A mass whose bucket lies beyond MAX_MASS gives the empty set, as that query does.
+
+        Unindexed mode takes the reference's own route (DBIndexer.java:925-947): masses by IndexUtil.calculateMass
+        (dbi_calculate_mass), one search with zero-width windows, and the unmodified hit whose sequence equals
+        the string."""
         self._require()
+        if not self.use_index:
+            return self._proteins_unindexed(seqs)
         try:
             r = self.index.lookup_peptides(list(seqs))
         except DbiError as e:
@@ -455,13 +543,30 @@ class DBIndexer:
                 out.append({self._protein(p) for p in r["prot_ids"][plo[i]:plo[i + 1]].tolist()})
         return out
 
+    def _proteins_unindexed(self, seqs: Sequence[str]) -> List[Set[IndexedProtein]]:
+        bs = [s.encode("latin-1") for s in seqs]
+        m = np.array([self.index.calculate_mass(b) for b in bs], dtype=np.float64)
+        h = self._hits(m, m)
+        ho, so, po = (h[k].astype(np.int64) for k in ("hit_off", "seq_off", "prot_list_off"))
+        seq = h["seq"].tobytes()
+        out: List[Set[IndexedProtein]] = []
+        for i, b in enumerate(bs):
+            prots: Set[IndexedProtein] = set()
+            if not self._out_of_buckets(m[i], m[i]):
+                for j in range(ho[i], ho[i + 1]):
+                    if h["modpat"][j] == 0 and seq[so[j]:so[j + 1]] == b:
+                        prots = {self._protein(p) for p in h["prot_ids"][po[j]:po[j + 1]].tolist()}
+                        break
+            out.append(prots)
+        return out
+
     def getNumberSequences(self) -> int:
-        self._require()
+        self._require_index()
         return int(self.index.stats()["n_entries"])
 
     def getParentMasses(self) -> List[float]:
         """DBIndexer.java:984-992: entry keys divided back by massGroupFactor."""
-        self._require()
+        self._require_index()
         f = float(self.sparam.mass_group_factor)
         return [k / f for k in self.index.entry_keys().tolist()]
 
@@ -482,10 +587,11 @@ class DBIndexImpl:
             index_factor = self.sparam.indexFactor
             params = self.sparam.params
         index_path = None
-        if self.sparam is not None and not self.sparam.inMemoryIndex:
+        use_index = self.sparam.useIndex if self.sparam is not None else True
+        if self.sparam is not None and use_index and not self.sparam.inMemoryIndex:
             # an on-disk index, named like the reference's (DBIndexer.java:429 createFullIndexFileName)
             index_path = createFullIndexFileName(self.sparam) + INDEX_FILE_SUFFIX
-        self.indexer = DBIndexer(params, index_factor, index_path=index_path)
+        self.indexer = DBIndexer(params, index_factor, index_path=index_path, use_index=use_index)
         self.indexer.init()
         self.indexer.run(fasta=fasta, proteins=proteins)
         self._proteins_by_seq: dict = {}  # DBIndexImpl.java:33

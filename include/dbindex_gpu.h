@@ -261,7 +261,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
  *
  * seq_off / prot_list_off [n_peps + 1] are CSRs over seq[] and prot_ids[]; flanks holds 6 bytes per run
  * (3 left, 3 right).  The pending result of a handle is dropped by the next dbi_query_hits,
- * dbi_reset_index or dbi_destroy. */
+ * dbi_search_unindexed, a successful read, dbi_reset_index or dbi_destroy. */
 typedef struct dbi_hit_counts {
   uint64_t nq, n_hits, n_peps, n_seq_bytes, n_prot_ids;
 } dbi_hit_counts;
@@ -284,6 +284,32 @@ int dbi_query_hits(dbi_handle* h, const double* lo, const double* hi, uint64_t n
 /* same with the bounds already in device memory of the handle's GPU */
 int dbi_query_hits_device(dbi_handle* h, const double* d_lo, const double* d_hi, uint64_t nq, dbi_hit_counts* counts);
 int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out);
+
+/* DBIndexer in SEARCH_UNINDEXED mode (DBIndexer.java:58-61; MassRangeFilteringIndex.java:90-108): the hits of a
+ * batch of ranges, straight from the proteins added so far, with no index built or kept -- the way to search a
+ * proteome whose index does not fit one GPU.  lo / hi are host pointers with the inclusive semantics of
+ * dbi_query_hits.  The proteins are digested once per call, keeping only the records that can land in a window
+ * (K2u / K4u: base mass + some sum of <= min(max_mods, mod sites) shifts meets the union of the windows); those
+ * CANDIDATES are indexed as dbi_build indexes a proteome, the hits materialised, and the candidate index freed.
+ * For every query the hits equal what dbi_build followed by dbi_query_hits would return on this handle (the
+ * multiset of mass bits, first occurrence, length, residues, flanks, mod pattern and protein list, grouped in
+ * maximal runs; ties inside a query have no contractual order).
+ *
+ * The result is the handle's pending hit result: read it with dbi_query_hits_read (same buffers, same runs).
+ * The call drops any earlier pending result.  It needs a handle that is not built (built: DBI_EALREADY) and
+ * not part of a sharded build (after dbi_mg_begin: DBI_EINVAL).  The handle stays unbuilt: dbi_add_proteins
+ * still works and later searches see the added proteins, dbi_build still builds the normal index, and
+ * dbi_query_hits / dbi_lookup_peptides still return DBI_ENOTINIT.  The packed residues (K1) are kept between
+ * calls and packed again only when proteins were added since.
+ *
+ * max_candidates (0 = no cap) bounds the candidate records, N_c, which the count pass knows before anything is
+ * allocated.  N_c > max_candidates or N_c >= 2^32: DBI_ERANGE and no pending result, so that the host can split
+ * the batch.  *n_candidates (may be NULL) receives N_c in both cases.  The < 2^32 hits rule of dbi_query_hits
+ * applies unchanged.  dbi_stats_get afterwards reports this search's candidate pipeline: n_emitted = N_c,
+ * n_unique and n_entries of the candidate index, and with params.profile the stage times (K12 windows under
+ * DBI_STAGE_OTHER). */
+int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, uint64_t max_candidates,
+                         dbi_hit_counts* counts, uint64_t* n_candidates);
 
 /* Batched DBIndexer.getProteins(String) (DBIndexer.java:925-947, DBIndexImpl.java:222-237): which index entry,
  * and so which proteins, every peptide of a list is.  Peptide i is residues[offsets[i], offsets[i+1]) (the packed

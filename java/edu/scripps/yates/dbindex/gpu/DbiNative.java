@@ -95,6 +95,9 @@ public final class DbiNative {
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
 	static final MethodHandle dbi_query_hits_read = h("dbi_query_hits_read",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
+	// SEARCH_UNINDEXED: the hits of a batch from the proteins, no index kept; read with dbi_query_hits_read
+	static final MethodHandle dbi_search_unindexed = h("dbi_search_unindexed",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS));
 	// batched getProteins(String): which entry (and so which proteins) every peptide of a list is
 	static final MethodHandle dbi_lookup_peptides = h("dbi_lookup_peptides",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));

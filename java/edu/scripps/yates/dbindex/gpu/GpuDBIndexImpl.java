@@ -38,11 +38,15 @@ public class GpuDBIndexImpl extends DBIndexImpl {
 		this(getDefaultDBIndexParams(fastaFile));
 	}
 
-	/** Same sequence as DBIndexImpl(DBIndexSearchParams) (DBIndexImpl.java:117-145): indexer, init(), run(). */
+	/**
+	 * Same sequence as DBIndexImpl(DBIndexSearchParams) (DBIndexImpl.java:117-145): indexer, init(), run().
+	 * useIndex = false (default_use_index, dbindex.properties) selects SEARCH_UNINDEXED (DBIndexer.java:58-61): the
+	 * proteins are uploaded and every query digests them again on the GPU (dbi_search_unindexed).
+	 */
 	public GpuDBIndexImpl(DBIndexSearchParams sParam) {
 		super(); // the no-arg constructor builds nothing (DBIndexImpl.java:51-53)
 		try {
-			indexer = new GpuDBIndexer(sParam, IndexerMode.INDEX);
+			indexer = new GpuDBIndexer(sParam, sParam.isUseIndex() ? IndexerMode.INDEX : IndexerMode.SEARCH_UNINDEXED);
 			indexer.init();
 			indexer.run(); // FASTA streaming as in the reference; cutSeq only hands proteins to the GPU store
 			synchronized (GpuDBIndexImpl.class) {

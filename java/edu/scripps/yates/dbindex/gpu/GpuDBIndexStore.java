@@ -44,14 +44,19 @@ public class GpuDBIndexStore implements DBIndexStore {
 	private MemorySegment[] handles = new MemorySegment[0];
 	private double[] splitMass = new double[0]; // masses at which the slices of the sharded index are cut
 	private boolean inited = false, built = false;
+	// SEARCH_UNINDEXED (DBIndexer.java:58-61, MassRangeFilteringIndex.java:90-108): no index, every query digests
+	// the proteins again for its ranges (dbi_search_unindexed), at most maxCandidates candidate records per call
+	private final boolean unindexed;
+	private final long maxCandidates = Long.getLong("dbindex.gpu.maxCandidates", 1L << 25);
 	private ProteinCache proteinCache;
 	private String indexFile; // null = in-memory index only
 	// proteins gathered by addProteinDef until stopAddSeq() (subsystem 1: packed residue buffer)
 	private final java.io.ByteArrayOutputStream residues = new java.io.ByteArrayOutputStream();
 	private final List<Long> offsets = new ArrayList<>(List.of(0L));
 
-	public GpuDBIndexStore(DBIndexSearchParams sparam) {
+	public GpuDBIndexStore(DBIndexSearchParams sparam, boolean unindexed) {
 		this.sparam = sparam;
+		this.unindexed = unindexed;
 	}
 
 	private static void check(int rc) throws DBIndexStoreException {
@@ -128,6 +133,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 	public void init(String databaseID) throws DBIndexStoreException {
 		if (inited)
 			throw new DBIndexStoreException("Already intialized"); // DBIndexStoreSQLiteMult.java:97-99
+		if (unindexed && nDevices > 1)
+			throw new DBIndexStoreException("an unindexed search (useIndex = false) runs on one GPU: -Ddbindex.gpu.devices=1");
 		try {
 			handles = new MemorySegment[nDevices];
 			for (int d = 0; d < nDevices; ++d) {
@@ -140,7 +147,7 @@ public class GpuDBIndexStore implements DBIndexStore {
 			handle = handles[0];
 			// on-disk index (in_memory_index = false): <fasta>_<md5(params)> like the reference (IndexUtil.java:270-324);
 			// if the file is there the index is loaded and DBIndexer.run() skips indexing (DBIndexer.java:522-531)
-			if (!sparam.isInMemoryIndex() && nDevices == 1) { // a sharded index is rebuilt (dbi_save holds one GPU's index)
+			if (!sparam.isInMemoryIndex() && nDevices == 1 && !unindexed) { // a sharded index is rebuilt (dbi_save holds one GPU's index)
 				indexFile = sparam.getFullIndexFileName(null, null, false, null, false, null) + ".gpuidx";
 				if (new java.io.File(indexFile).exists()) {
 					check((int) DbiNative.dbi_load.invoke(handle, arena.allocateFrom(indexFile)));
@@ -202,6 +209,10 @@ public class GpuDBIndexStore implements DBIndexStore {
 			final MemorySegment o = a.allocate(JAVA_LONG, offsets.size());
 			for (int i = 0; i < offsets.size(); ++i)
 				o.setAtIndex(JAVA_LONG, i, offsets.get(i));
+			if (unindexed) { // the proteins are all there is: every query digests them (dbi_search_unindexed)
+				check((int) DbiNative.dbi_add_proteins.invoke(handle, r, o, offsets.size() - 1));
+				return;
+			}
 			if (nDevices == 1) {
 				check((int) DbiNative.dbi_add_proteins.invoke(handle, r, o, offsets.size() - 1));
 				check((int) DbiNative.dbi_build.invoke(handle));
@@ -284,6 +295,15 @@ public class GpuDBIndexStore implements DBIndexStore {
 		for (int i = 0; i < lo.length; ++i) // "Cannot query, unsupported precursor mass" -> empty (Mult:333-338)
 			if ((int) lo[i] / bucketRange > sparam.getIndexFactor() - 1 || (int) hi[i] / bucketRange > sparam.getIndexFactor() - 1)
 				return ret;
+		if (unindexed) {
+			// one range, or the merged intervals of getSequences(List<MassRange>), which are sorted by mass already: the
+			// chunks of the mass-sorted batch come back in the caller's order
+			searchUnindexed(lo, hi, (q, pep, resLeft, resRight, mass, off, pids, patterns) -> {
+				for (final int mp : patterns)
+					ret.add(sequence(pep, resLeft, resRight, mass, off, pids, mp));
+			});
+			return ret;
+		}
 		if (nDevices > 1) {
 			// Mult.getSequences walks the buckets a range touches (:333-343); here: the GPUs owning the slices it
 			// touches.  Slice s = [splitMass[s-1], splitMass[s]) lives on GPU s < N ? s : slices - 1 - s.
@@ -323,10 +343,85 @@ public class GpuDBIndexStore implements DBIndexStore {
 			MemorySegment.copy(hi, 0, dhi, JAVA_DOUBLE, 0, nq);
 			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS);
 			check((int) DbiNative.dbi_query_hits.invoke(handle, dlo, dhi, (long) nq, cnt));
+			readHits(handle, a, cnt, null, (q, pep, resLeft, resRight, mass, off, pids, patterns) -> {
+				for (final int mp : patterns)
+					ret.add(sequence(pep, resLeft, resRight, mass, off, pids, mp));
+			});
+		} catch (final DBIndexStoreException e) {
+			throw e;
+		} catch (final Throwable t) {
+			throw new DBIndexStoreException("Error getting peptides ", t);
+		}
+	}
+
+	/** IndexedSequence as parseAddPeptideInfo builds it (Merge:452-462), the mod pattern as a mod sequence */
+	private static IndexedSequence sequence(String pep, String resLeft, String resRight, double mass, int off,
+			List<Integer> pids, int modPattern) {
+		final IndexedSequence s = new IndexedSequence(0, mass, pep, resLeft, resRight);
+		s.setProteinIds(pids);
+		s.setSequenceOffset(off); // SURVEY Q10: the offset is known, hand it over
+		if (modPattern != 0)
+			s.setModSequence(modNotation(pep, modPattern));
+		return s;
+	}
+
+	/** what readHits hands over per run: the caller's query number, the peptide, and the mod pattern of every hit */
+	private interface RunSink {
+		void run(int query, String pep, String resLeft, String resRight, double mass, int off, List<Integer> pids,
+				int[] patterns) throws DBIndexStoreException;
+	}
+
+	/**
+	 * SEARCH_UNINDEXED: the ranges sorted by mass go to dbi_search_unindexed; a batch whose candidate records exceed
+	 * maxCandidates (DBI_ERANGE, N_c reported) is split into ceil(N_c / cap) + 1 contiguous chunks, again if needed.
+	 * The sink sees the runs of every query, chunk by chunk in mass order, with the caller's query numbers.
+	 */
+	private void searchUnindexed(double[] lo, double[] hi, RunSink sink) throws DBIndexStoreException {
+		final Integer[] order = new Integer[lo.length];
+		for (int i = 0; i < order.length; ++i)
+			order[i] = i;
+		java.util.Arrays.sort(order, (x, y) -> Double.compare(lo[x], lo[y]));
+		final int[] ids = new int[order.length];
+		for (int i = 0; i < ids.length; ++i)
+			ids[i] = order[i];
+		searchChunk(lo, hi, ids, sink);
+	}
+
+	private void searchChunk(double[] lo, double[] hi, int[] ids, RunSink sink) throws DBIndexStoreException {
+		try (Arena a = Arena.ofConfined()) {
+			final int nq = ids.length;
+			final MemorySegment dlo = a.allocate(JAVA_DOUBLE, Math.max(1, nq)), dhi = a.allocate(JAVA_DOUBLE, Math.max(1, nq));
+			for (int i = 0; i < nq; ++i) {
+				dlo.setAtIndex(JAVA_DOUBLE, i, lo[ids[i]]);
+				dhi.setAtIndex(JAVA_DOUBLE, i, hi[ids[i]]);
+			}
+			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS), nCand = a.allocate(JAVA_LONG);
+			final int rc = (int) DbiNative.dbi_search_unindexed.invoke(handle, dlo, dhi, (long) nq, maxCandidates, cnt, nCand);
+			final long nc = nCand.get(JAVA_LONG, 0);
+			if (rc == DbiNative.DBI_ERANGE && nc > maxCandidates && nq > 1) {
+				final int chunks = (int) Math.min(nq, (nc + maxCandidates - 1) / maxCandidates + 1);
+				for (int c = 0; c < chunks; ++c)
+					searchChunk(lo, hi, java.util.Arrays.copyOfRange(ids, (int) ((long) nq * c / chunks),
+							(int) ((long) nq * (c + 1) / chunks)), sink);
+				return;
+			}
+			check(rc);
+			readHits(handle, a, cnt, ids, sink);
+		} catch (final DBIndexStoreException e) {
+			throw e;
+		} catch (final Throwable t) {
+			throw new DBIndexStoreException("Error getting peptides ", t);
+		}
+	}
+
+	/** dbi_query_hits_read of the pending result; queryIds: the caller's number of every query (null = itself) */
+	private void readHits(MemorySegment handle, Arena a, MemorySegment cnt, int[] queryIds, RunSink sink)
+			throws Throwable {
+		{
 			// the answer comes back grouped in RUNS (consecutive hits that are variants of one peptide with one
 			// mass): peptide string, flanks, first occurrence and protein list once per run, the mod pattern per hit
-			final long nHits = cnt.get(JAVA_LONG, 8), nPeps = cnt.get(JAVA_LONG, 16), nSeq = cnt.get(JAVA_LONG, 24),
-					nIds = cnt.get(JAVA_LONG, 32);
+			final long nq = cnt.get(JAVA_LONG, 0), nHits = cnt.get(JAVA_LONG, 8), nPeps = cnt.get(JAVA_LONG, 16),
+					nSeq = cnt.get(JAVA_LONG, 24), nIds = cnt.get(JAVA_LONG, 32);
 			final MemorySegment pat = a.allocate(JAVA_INT, Math.max(1, nHits));
 			final MemorySegment pepHitOff = a.allocate(JAVA_LONG, nPeps + 1);
 			final MemorySegment mass = a.allocate(JAVA_DOUBLE, Math.max(1, nPeps));
@@ -335,15 +430,19 @@ public class GpuDBIndexStore implements DBIndexStore {
 			final MemorySegment flanks = a.allocate(Math.max(1, 6 * nPeps));
 			final MemorySegment seqOff = a.allocate(JAVA_LONG, nPeps + 1), seq = a.allocate(Math.max(1, nSeq));
 			final MemorySegment plo = a.allocate(JAVA_LONG, nPeps + 1), ids = a.allocate(JAVA_INT, Math.max(1, nIds));
+			final MemorySegment pepOff = a.allocate(JAVA_LONG, nq + 1);
 			final MemorySegment bufs = a.allocate(DbiNative.HIT_BUFFERS);
-			final MemorySegment[] order = { MemorySegment.NULL /* hit_off: the union is returned as one list */,
-					MemorySegment.NULL /* pep_off */, pat, pepHitOff, mass, prot, off, len, flanks, seqOff, seq, plo, ids };
+			final MemorySegment[] order = { MemorySegment.NULL /* hit_off */, pepOff, pat, pepHitOff, mass, prot, off, len,
+					flanks, seqOff, seq, plo, ids };
 			for (int k = 0; k < order.length; ++k)
 				bufs.setAtIndex(ADDRESS, k, order[k]);
 			check((int) DbiNative.dbi_query_hits_read.invoke(handle, bufs));
 			final byte[] seqBytes = seq.asSlice(0, nSeq).toArray(JAVA_BYTE);
 			final byte[] flankBytes = flanks.asSlice(0, 6 * nPeps).toArray(JAVA_BYTE);
+			int q = 0;
 			for (long p = 0; p < nPeps; ++p) {
+				while (pepOff.getAtIndex(JAVA_LONG, q + 1) <= p) // the query this run belongs to
+					++q;
 				final int s0 = (int) seqOff.getAtIndex(JAVA_LONG, p), s1 = (int) seqOff.getAtIndex(JAVA_LONG, p + 1);
 				final String pep = new String(seqBytes, s0, s1 - s0, java.nio.charset.StandardCharsets.ISO_8859_1);
 				final String resLeft = new String(flankBytes, (int) (6 * p), 3, java.nio.charset.StandardCharsets.ISO_8859_1);
@@ -351,20 +450,13 @@ public class GpuDBIndexStore implements DBIndexStore {
 				final List<Integer> pids = new ArrayList<>();
 				for (long k = plo.getAtIndex(JAVA_LONG, p); k < plo.getAtIndex(JAVA_LONG, p + 1); ++k)
 					pids.add(ids.getAtIndex(JAVA_INT, k));
-				for (long i = pepHitOff.getAtIndex(JAVA_LONG, p); i < pepHitOff.getAtIndex(JAVA_LONG, p + 1); ++i) {
-					final IndexedSequence s = new IndexedSequence(0, mass.getAtIndex(JAVA_DOUBLE, p), pep, resLeft, resRight);
-					s.setProteinIds(pids);
-					s.setSequenceOffset(off.getAtIndex(JAVA_INT, p)); // SURVEY Q10: the offset is known, hand it over
-					final int mp = pat.getAtIndex(JAVA_INT, i);
-					if (mp != 0)
-						s.setModSequence(modNotation(pep, mp));
-					ret.add(s);
-				}
+				final long h0 = pepHitOff.getAtIndex(JAVA_LONG, p), h1 = pepHitOff.getAtIndex(JAVA_LONG, p + 1);
+				final int[] patterns = new int[(int) (h1 - h0)];
+				for (long i = h0; i < h1; ++i)
+					patterns[(int) (i - h0)] = pat.getAtIndex(JAVA_INT, i);
+				sink.run(queryIds == null ? q : queryIds[q], pep, resLeft, resRight, mass.getAtIndex(JAVA_DOUBLE, p),
+						off.getAtIndex(JAVA_INT, p), pids, patterns);
 			}
-		} catch (final DBIndexStoreException e) {
-			throw e;
-		} catch (final Throwable t) {
-			throw new DBIndexStoreException("Error getting peptides ", t);
 		}
 	}
 
@@ -394,6 +486,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 		for (int i = 0; i < n; ++i)
 			ret.add(new java.util.HashSet<>());
 		final int bucketRange = MAX_MASS / sparam.getIndexFactor();
+		if (unindexed)
+			return lookupUnindexed(peptides, ret, bucketRange);
 		try (Arena a = Arena.ofConfined()) {
 			final java.io.ByteArrayOutputStream packed = new java.io.ByteArrayOutputStream();
 			final MemorySegment off = a.allocate(JAVA_LONG, n + 1L);
@@ -441,6 +535,40 @@ public class GpuDBIndexStore implements DBIndexStore {
 		return ret;
 	}
 
+	/**
+	 * SEARCH_UNINDEXED getProteins(String): the reference's own route (DBIndexer.java:925-947) -- the mass by
+	 * IndexUtil.calculateMass (dbi_calculate_mass), one search with zero-width windows, and the proteins of the
+	 * unmodified hit whose peptide equals the string.
+	 */
+	private List<java.util.Set<IndexedProtein>> lookupUnindexed(List<String> peptides, List<java.util.Set<IndexedProtein>> ret,
+			int bucketRange) throws DBIndexStoreException {
+		final int n = peptides.size();
+		final double[] m = new double[n];
+		try (Arena a = Arena.ofConfined()) {
+			final MemorySegment out = a.allocate(JAVA_DOUBLE);
+			for (int i = 0; i < n; ++i) {
+				final byte[] b = peptides.get(i).getBytes(java.nio.charset.StandardCharsets.ISO_8859_1);
+				final MemorySegment seg = a.allocate(Math.max(1, b.length));
+				MemorySegment.copy(b, 0, seg, JAVA_BYTE, 0, b.length);
+				check((int) DbiNative.dbi_calculate_mass.invoke(handle, seg, (long) b.length, out));
+				m[i] = out.get(JAVA_DOUBLE, 0);
+			}
+		} catch (final DBIndexStoreException e) {
+			throw e;
+		} catch (final Throwable t) {
+			throw new DBIndexStoreException("dbi_calculate_mass failed", t);
+		}
+		searchUnindexed(m, m, (q, pep, resLeft, resRight, mass, off, pids, patterns) -> {
+			if ((int) m[q] / bucketRange > sparam.getIndexFactor() - 1 || !pep.equals(peptides.get(q)))
+				return;
+			for (final int mp : patterns)
+				if (mp == 0)
+					for (final int id : pids)
+						ret.get(q).add(new IndexedProtein(proteinCache.getProteinDef(id), id));
+		});
+		return ret;
+	}
+
 	@Override
 	public Iterator<IndexedSequence> getSequencesIterator(List<MassRange> ranges) throws DBIndexStoreException {
 		return getSequences(ranges).iterator(); // Mult:634-636
@@ -467,6 +595,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 	@Override
 	public long getNumberSequences() throws DBIndexStoreException {
 		requireInit();
+		if (unindexed)
+			throw new DBIndexStoreException("not available in unindexed search mode (useIndex = false): there is no index");
 		try (Arena a = Arena.ofConfined()) {
 			long total = 0;
 			for (final MemorySegment h : handles) {
@@ -494,6 +624,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 	@Override
 	public List<Integer> getEntryKeys() throws DBIndexStoreException {
 		requireInit();
+		if (unindexed)
+			throw new DBIndexStoreException("not available in unindexed search mode (useIndex = false): there is no index");
 		try (Arena a = Arena.ofConfined()) {
 			final List<Integer> ret = new ArrayList<>();
 			for (final MemorySegment h : handles) { // Mult.getEntryKeys concatenates its buckets the same way (:196-201)

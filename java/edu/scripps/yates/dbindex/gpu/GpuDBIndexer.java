@@ -18,12 +18,13 @@ import edu.scripps.yates.utilities.fasta.dbindex.IndexedProtein;
  * DBIndexer with the digestion moved to the GPU: run() still streams the FASTA and fills the
  * ProteinCache (DBIndexer.java:600-616), but cutSeq only hands the protein to the store; the windows,
  * masses and gates of DBIndexer.java:256-394 are computed by digest_count/emit_kernel when
- * stopAddSeq() calls dbi_build. Uses the reference's own plugin constructor (DBIndexer.java:143).
+ * stopAddSeq() calls dbi_build (in SEARCH_UNINDEXED mode: when a query calls dbi_search_unindexed). Uses the
+ * reference's own plugin constructor (DBIndexer.java:143).
  * NOT COMPILED HERE (no JDK, see DbiNative).
  */
 public class GpuDBIndexer extends DBIndexer {
 	public GpuDBIndexer(DBIndexSearchParams sparam, IndexerMode mode) {
-		super(sparam, mode, new GpuDBIndexStore(sparam));
+		super(sparam, mode, new GpuDBIndexStore(sparam, mode == IndexerMode.SEARCH_UNINDEXED));
 	}
 
 	@Override
