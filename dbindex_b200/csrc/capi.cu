@@ -590,6 +590,10 @@ struct UniqLayout {
   }
 };
 
+// Test hook: DBI_GROUP_RADIX sends the single-GPU group path through the K7 sort of the sharded build
+// (peptide-major records) instead of K6g's sorted lists + the K7m merge; the results are identical.
+bool group_radix(const dbi_handle*) { return std::getenv("DBI_GROUP_RADIX") != nullptr; }
+
 // K7 + K8: sort N records by (mass, sequence hash, arrival order), merge equal peptides into
 // the handle's unique tables (u_*, plist).
 int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) {
@@ -654,7 +658,9 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
         r1 = radix_sort_pairs<uint32_t, uint32_t>(hk, ix, N, 0, 32, tmp.p, s, nullptr);
       }
       DomProbe base_probe(h);
-      const bool base_is_dominant = h->p.profile && h->cfg.max_mods == 0;
+      // the largest K7 sort of the build: the base sort, unless the variant groups go through K7 too
+      const bool base_is_dominant =
+          h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->mg_world <= 1 && !group_radix(h)));
       if (base_is_dominant) {  // a retry re-runs the sort: count only the final attempt
         h->spans.erase(std::remove_if(h->spans.begin(), h->spans.end(),
                                       [](const dbi_handle::Span& sp) { return sp.kind == kSpanDominant; }),
@@ -840,40 +846,64 @@ void ensure_site_masks(dbi_handle* h) {
   h->st.algo_bytes[DBI_STAGE_MOD_COUNT] += h->n_unique * (4 + 2 + 12 + 8ull * h->cfg.n_classes);
 }
 
+// lists != nullptr (single GPU): K6g writes one sorted list per class sequence, described in *lists (the
+// input of K7m); nullptr (sharded build): peptide-major records, sorted after the exchange by K7.
 int emit_groups(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& ks, DevBuf& gkey, DevBuf& gpay,
-                uint64_t* NG_out, uint64_t* V_out) {
+                uint64_t* NG_out, uint64_t* V_out, GroupLists* lists = nullptr) {
   cudaStream_t s = h->stream;
   const uint64_t n_unique = h->n_unique;
+  const int S = h->cfg.n_seq;
   *NG_out = 0;
   *V_out = 0;
+  if (lists) {
+    std::memset(lists, 0, sizeof(*lists));
+    lists->n_lists = S;
+  }
   if (ntiles == 0 || n_unique == 0) {
     gkey.alloc(8, h->arena);
     gpay.alloc(8, h->arena);
     return DBI_OK;
   }
   ensure_site_masks(h);
-  DevBuf ng, tg, tv, goffs, voffs;
-  ng.alloc(n_unique, h->arena);  // indexed by global peptide id
+  DevBuf mask, tg, tv, goffs, voffs, vt, vtmp;
+  mask.alloc(n_unique * 4, h->arena);  // indexed by global peptide id
   tg.alloc((uint64_t)ntiles * 4, h->arena);
   tv.alloc((uint64_t)ntiles * 4, h->arena);
-  goffs.alloc(((uint64_t)ntiles + 1) * 8, h->arena);
   voffs.alloc(((uint64_t)ntiles + 1) * 8, h->arena);
+  const uint64_t n_vt = (uint64_t)S * ntiles;  // list layout: (class sequence, tile) counts, v-major
+  if (lists) {
+    vt.alloc(n_vt * 4, h->arena);
+    goffs.alloc((n_vt + 1) * 8, h->arena);
+    vtmp.alloc(full_scan_tmp_bytes(n_vt), h->arena);
+  } else {
+    goffs.alloc(((uint64_t)ntiles + 1) * 8, h->arena);
+  }
   const uint64_t n_in_tiles = std::min<uint64_t>((uint64_t)ntiles * kModTile, n_unique - (uint64_t)tile0 * kModTile);
-  const uint64_t per_pep = 8 + 4 + 2 + 1 + 8ull * h->cfg.n_classes;
+  const uint64_t per_pep = 8 + 4 + 2 + 4 + 8ull * h->cfg.n_classes;
   uint64_t NG = 0, V = 0;
   {
     Stage sg(h, DBI_STAGE_MOD_COUNT);
     launch_grp_count(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
                      h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->u_cmask.as<uint64_t>(), n_unique, tile0,
-                     ntiles, ng.as<uint8_t>(), tg.as<uint32_t>(), tv.as<uint32_t>(), h->d_err.as<uint32_t>(), s);
-    launch_scan_u32_to_u64(tg.as<uint32_t>(), ntiles, goffs.as<uint64_t>(), s);
+                     ntiles, mask.as<uint32_t>(), tg.as<uint32_t>(), tv.as<uint32_t>(),
+                     lists ? vt.as<uint32_t>() : nullptr, h->d_err.as<uint32_t>(), s);
+    if (lists) launch_full_scan_u32_to_u64(vt.as<uint32_t>(), n_vt, goffs.as<uint64_t>(), vtmp.p, s);
+    else launch_scan_u32_to_u64(tg.as<uint32_t>(), ntiles, goffs.as<uint64_t>(), s);
     launch_scan_u32_to_u64(tv.as<uint32_t>(), ntiles, voffs.as<uint64_t>(), s);
     uint32_t e = 0;
-    DBI_CUDA(cudaMemcpyAsync(&NG, goffs.as<uint64_t>() + ntiles, 8, cudaMemcpyDeviceToHost, s));
+    if (lists)  // list v starts at goffs[v * ntiles]; goffs[S * ntiles] = NG
+      DBI_CUDA(cudaMemcpy2DAsync(lists->start, 8, goffs.p, (size_t)ntiles * 8, 8, (size_t)S + 1,
+                                 cudaMemcpyDeviceToHost, s));
+    else
+      DBI_CUDA(cudaMemcpyAsync(&NG, goffs.as<uint64_t>() + ntiles, 8, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaMemcpyAsync(&V, voffs.as<uint64_t>() + ntiles, 8, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaMemcpyAsync(&e, h->d_err.p, 4, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
-    h->st.algo_bytes[DBI_STAGE_MOD_COUNT] += n_in_tiles * per_pep;
+    if (lists) {
+      NG = lists->start[S];
+      group_lists_plan(lists);
+    }
+    h->st.algo_bytes[DBI_STAGE_MOD_COUNT] += n_in_tiles * per_pep + (lists ? n_vt * (4 + 8) : 0);
     if (int rc = check_err_bits(e)) return rc;
   }
   TR("ir_modcount+sync");
@@ -884,8 +914,8 @@ int emit_groups(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& 
     Stage sg(h, DBI_STAGE_MOD_EMIT);
     launch_grp_emit(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
                     h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->u_cmask.as<uint64_t>(), n_unique, tile0,
-                    ntiles, ng.as<uint8_t>(), goffs.as<uint64_t>(), ks.base_bits, h->ent_base_off,
-                    gkey.as<uint64_t>(), gpay.as<uint64_t>(), h->d_err.as<uint32_t>(), s);
+                    ntiles, mask.as<uint32_t>(), goffs.as<uint64_t>(), lists != nullptr, ks.base_bits,
+                    h->ent_base_off, gkey.as<uint64_t>(), gpay.as<uint64_t>(), h->d_err.as<uint32_t>(), s);
     h->st.algo_bytes[DBI_STAGE_MOD_EMIT] += n_in_tiles * per_pep + NG * 16;
   }
   TR("ir_modemit");
@@ -902,8 +932,9 @@ struct GroupSide {
   const uint32_t* gid = nullptr;     // [row]
   const UniqView* uv = nullptr;      // where the peptides' (gpos, len) live: only peptides longer than 64 residues need it
 };
+// lists (single GPU, K6g's list layout): K7m merges the lists instead of the sort.
 int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64_t NG, const KeySpace& ks,
-                       const GroupSide* side = nullptr) {
+                       const GroupSide* side = nullptr, const GroupLists* lists = nullptr) {
   cudaStream_t s = h->stream;
   if (NG >= (1ull << 32)) {
     set_error("more than 2^32 variant groups on one GPU (%llu)", (unsigned long long)NG);
@@ -917,14 +948,24 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
   }
   const bool sharded = side != nullptr;
   if (!sharded) ensure_site_masks(h);
-  DevBuf key2, pay2, vtmp;
+  DevBuf key2, pay2, vtmp, cnt;
   key2.alloc(NG * 8, h->arena);
   pay2.alloc(NG * 8, h->arena);
-  vtmp.alloc(radix_sort_tmp_bytes(NG), h->arena);
+  cnt.alloc(NG * 4, h->arena);
   uint64_t* vk[2] = {key_in, key2.as<uint64_t>()};
   uint64_t* vp[2] = {pay_in, pay2.as<uint64_t>()};
   int r = 0;
-  {
+  if (lists) {
+    vtmp.alloc(group_merge_tmp_bytes(*lists), h->arena);
+    Stage sg(h, DBI_STAGE_SORT_VAR);
+    launch_group_merge(*lists, key_in, pay_in, vk[1], vp[1], cnt.as<uint32_t>(), vtmp.p, h->d_err.as<uint32_t>(), s);
+    r = 1;
+    h->st.sort_bits_var = 0;
+    // records read once, written once with their count; samples gathered, ranked and searched in L2
+    const uint64_t ns = lists->soff[lists->n_lists];
+    h->st.algo_bytes[DBI_STAGE_SORT_VAR] += NG * (16 + 20) + ns * 16 * 2;
+  } else {
+    vtmp.alloc(radix_sort_tmp_bytes(NG), h->arena);
     Stage sg(h, DBI_STAGE_SORT_VAR);
     DomProbe var_probe(h);
     if (h->p.profile) {
@@ -936,20 +977,26 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
     h->st.algo_bytes[DBI_STAGE_SORT_VAR] += NG * 8 + NG * 32ull * ((ks.nbits + 7) / 8);
   }
   TR("ir_sortvar");
-  DevBuf cnt, eoff, stmp, tfirst, llist, lcount;
-  cnt.alloc(NG * 4, h->arena);
+  DevBuf eoff, stmp, tfirst, llist, lcount;
   eoff.alloc((NG + 1) * 8, h->arena);
   stmp.alloc(full_scan_tmp_bytes(NG), h->arena);
   lcount.alloc(16, h->arena);
   uint64_t V = 0, n_long = 0;
   {
     Stage sg(h, DBI_STAGE_GATHER_VAR);
-    launch_grp_extract_cnt(vp[r], NG, cnt.as<uint32_t>(), s);
+    if (!lists) launch_grp_extract_cnt(vp[r], NG, cnt.as<uint32_t>(), s);  // K7m wrote the counts
     launch_full_scan_u32_to_u64(cnt.as<uint32_t>(), NG, eoff.as<uint64_t>(), stmp.p, s);
     DBI_CUDA(cudaMemsetAsync(lcount.p, 0, 16, s));
     DBI_CUDA(cudaMemcpyAsync(&V, eoff.as<uint64_t>() + NG, 8, cudaMemcpyDeviceToHost, s));
     if (!sharded) DBI_CUDA(cudaMemcpyAsync(&n_long, h->d_nlong.p, 8, cudaMemcpyDeviceToHost, s));
+    uint32_t e = 0;
+    DBI_CUDA(cudaMemcpyAsync(&e, h->d_err.p, 4, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
+    if (e & kErrMergeCap) {
+      set_error("a tile of the group merge exceeds its capacity of %d records",
+                (kGmSplit + kGrpMaxLists) * kGmStride);
+      return DBI_ERANGE;
+    }
     if (sharded) n_long = NG;  // unknown here: any received group may belong to a long peptide
     if (V >= (1ull << 32)) {
       set_error("more than 2^32 index entries on one GPU (%llu)", (unsigned long long)V);
@@ -985,7 +1032,8 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
       // per entry: mass + peptide + pattern written
       h->st.exp_bytes_per_launch = NG * (8 + 8 + 8 + 8ull * h->cfg.max_mods) + V * 16;
     }
-    h->st.algo_bytes[DBI_STAGE_GATHER_VAR] += NG * (8 + 4 + 8 + 8 + 8 + 8ull * h->cfg.max_mods) + V * 16;
+    h->st.algo_bytes[DBI_STAGE_GATHER_VAR] +=
+        NG * ((lists ? 0 : 8 + 4) + 8 + 8 + 8 + 8ull * h->cfg.max_mods) + V * 16;
   }
   TR("ir_expand");
   h->n_entries = V;
@@ -1010,9 +1058,11 @@ int index_records(dbi_handle* h, const RecView& r, uint64_t N, double lo_mass, d
   const uint32_t utiles = (uint32_t)((h->n_unique + kModTile - 1) / kModTile);
   DevBuf vkey, vpay;
   uint64_t V = 0, NG = 0;
-  if (h->cfg.n_seq > 0) {  // group path: sort one record per (peptide, class sequence)
-    if (int rc = emit_groups(h, 0, utiles, ks, vkey, vpay, &NG, &V)) return rc;
-    if (int rc = sort_expand_groups(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), NG, ks)) return rc;
+  if (h->cfg.n_seq > 0) {  // group path: one record per (peptide, class sequence), merged from sorted lists
+    GroupLists lists;
+    GroupLists* gl = group_radix(h) ? nullptr : &lists;
+    if (int rc = emit_groups(h, 0, utiles, ks, vkey, vpay, &NG, &V, gl)) return rc;
+    if (int rc = sort_expand_groups(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), NG, ks, nullptr, gl)) return rc;
   } else {  // many shift classes: one record per variant
     if (int rc = emit_variants(h, 0, utiles, ks, vkey, vpay, &V)) return rc;
     if (int rc = sort_variants(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), V, ks)) return rc;

@@ -53,6 +53,7 @@ constexpr uint32_t kErrZeroResidue = 1;   // residue byte 0 in the input
 constexpr uint32_t kErrPepTooLong = 2;    // window longer than DBI_MAX_PEP_LEN
 constexpr uint32_t kErrModPos = 4;        // modified residue beyond DBI_MAX_MOD_POS
 constexpr uint32_t kErrHashCollision = 8; // equal (mass, hash) but different sequence
+constexpr uint32_t kErrMergeCap = 16;     // a tile of the group merge over its shared-memory capacity
 
 #ifdef __CUDACC__
 

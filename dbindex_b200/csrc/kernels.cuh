@@ -185,15 +185,38 @@ void launch_site_masks(const uint8_t* d_res, const DevTables* d_tb, const Digest
                        cudaStream_t s);
 // *n_long += peptides longer than 64 residues in a length table
 void launch_count_long(const uint16_t* len, uint64_t n, unsigned long long* n_long, cudaStream_t s);
+// K5g: mask[u] (global id) = the class sequences whose group exists (bit 0 always); tile_groups / tile_vars
+// per tile; vt_cnt (nullptr = not wanted) [v * ntiles + tile] = groups of class sequence v in the tile.
 void launch_grp_count(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg, const double* u_mass,
                       const uint32_t* u_gpos, const uint16_t* u_len, const uint64_t* cmask, uint64_t n_unique,
-                      uint32_t tile0, uint32_t ntiles, uint8_t* ng, uint32_t* tile_groups, uint32_t* tile_vars,
-                      uint32_t* d_err, cudaStream_t s);
+                      uint32_t tile0, uint32_t ntiles, uint32_t* mask, uint32_t* tile_groups, uint32_t* tile_vars,
+                      uint32_t* vt_cnt, uint32_t* d_err, cudaStream_t s);
+// K6g: lists = false: peptide-major, goffs[tile] = first group of the tile (scan of tile_groups);
+// lists = true: one list per class sequence, goffs[v * ntiles + tile] = v-major scan of vt_cnt.
 void launch_grp_emit(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg, const double* u_mass,
                      const uint32_t* u_gpos, const uint16_t* u_len, const uint64_t* cmask, uint64_t n_unique,
-                     uint32_t tile0, uint32_t ntiles, const uint8_t* ng, const uint64_t* tile_goffs,
+                     uint32_t tile0, uint32_t ntiles, const uint32_t* mask, const uint64_t* goffs, bool lists,
                      uint64_t base_bits, uint64_t id_off, uint64_t* g_key, uint64_t* g_pay, uint32_t* d_err,
                      cudaStream_t s);
+// K7m (merge.cu): the S sorted group lists of K6g's list layout merged by (key, payload) in one pass.
+// Every kGmStride-th record of each list is a sample; the samples whose rank among all samples is a multiple
+// of kGmSplit cut the output into tiles of at most (kGmSplit + S) * kGmStride records, each merged in
+// shared memory.  The output order is that of a stable key sort of the peptide-major layout.
+constexpr int kGrpMaxLists = 32;
+constexpr int kGmStride = 32;
+constexpr int kGmSplit = 64;
+struct GroupLists {
+  uint64_t start[kGrpMaxLists + 1];  // list v = records [start[v], start[v + 1])
+  uint64_t soff[kGrpMaxLists + 1];   // samples of list v = [soff[v], soff[v + 1]) (group_lists_plan)
+  int n_lists;
+};
+// fills soff from start / n_lists
+void group_lists_plan(GroupLists* gl);
+size_t group_merge_tmp_bytes(const GroupLists& gl);
+// o_cnt[i] = variant count of merged record i (payload & (2^27 - 1)).  A tile over its capacity raises
+// kErrMergeCap (cannot happen by construction; checked anyway).
+void launch_group_merge(const GroupLists& gl, const uint64_t* key, const uint64_t* pay, uint64_t* o_key,
+                        uint64_t* o_pay, uint32_t* o_cnt, void* tmp, uint32_t* d_err, cudaStream_t s);
 void launch_grp_extract_cnt(const uint64_t* pay, uint64_t n, uint32_t* cnt, cudaStream_t s);
 // first[t] = group holding entry t * kExpTile, t in [0, tiles]; first[tiles] = n_groups - 1
 void launch_grp_tile_first(const uint64_t* eoff, uint64_t n_groups, uint64_t n_entries, uint32_t* first,

@@ -10,7 +10,8 @@
 //   K5m site_masks : per peptide and shift class, the 64-bit mask of its sites        (thread/peptide)
 //   K5g grp_count  : groups and variants per peptide: subsequence-count DP over sites (thread/peptide)
 //   K6g grp_emit   : {key = mass bits - base, payload = peptide << 32 | sequence << 27 | count}
-//   (K7 sorts the records, K3 scans the counts into entry offsets)
+//   (single GPU: K6g writes one sorted list per class sequence and K7m (merge.cu) merges them; sharded
+//   build: K7 sorts the records after the exchange.  K3 scans the counts into entry offsets)
 //   K6t grp_tile_first : first group of every tile of kExpTile consecutive ENTRIES
 //   K6x grp_expand_tab : one thread per ENTRY: un-rank the entry inside its group in constant
 //                    time (product-set blocks, per-group block tables in shared memory) and write
@@ -18,7 +19,7 @@
 //   K6l grp_expand_long : groups of peptides longer than 64 residues (no masks): one warp each
 //
 // HBM-bound byte/integer work; no tensor cores.  Algorithmic bytes: K5m 14 + len per peptide read,
-// 8 C written; K5g/K6g 22 + 8 C per peptide, 16 per group written; K6x 24 per group + 8 C per
+// 8 C written; K5g/K6g 25 + 8 C per peptide, 16 per group written; K6x 24 per group + 8 C per
 // group (random 32-B sectors) read, 16 per entry written.
 #include <cstring>
 
@@ -158,27 +159,32 @@ __global__ void __launch_bounds__(MD_THREADS)
 }
 
 // ---- K5g ------------------------------------------------------------------------------
+// mask_out[u]: bit v set iff group (u, v) exists (v = 0 always).  vt_cnt (optional, list layout of K6g):
+// vt_cnt[v * vt_stride + tile] = groups of class sequence v in the tile.
 __global__ void __launch_bounds__(MD_THREADS)
     grp_count_kernel(const uint8_t* __restrict__ res, const DevTables* __restrict__ tb, DigestCfg cfg,
                      const double* __restrict__ u_mass, const uint32_t* __restrict__ u_gpos,
                      const uint16_t* __restrict__ u_len, const uint64_t* __restrict__ cmask, uint64_t n_unique,
-                     uint32_t tile0, uint8_t* __restrict__ ng_out, uint32_t* __restrict__ tile_groups,
-                     uint32_t* __restrict__ tile_vars, uint32_t* err) {
+                     uint32_t tile0, uint32_t* __restrict__ mask_out, uint32_t* __restrict__ tile_groups,
+                     uint32_t* __restrict__ tile_vars, uint32_t* __restrict__ vt_cnt, uint32_t vt_stride,
+                     uint32_t* err) {
   extern __shared__ uint32_t s_cnt[];  // [n_seq][MD_THREADS]
   __shared__ ModTables mt;
   __shared__ uint32_t scratch[MD_WARPS + 1];
+  __shared__ uint32_t s_vc[32];  // groups of every class sequence in the tile
+  if (threadIdx.x < 32) s_vc[threadIdx.x] = 0;
   load_mod_tables(mt, tb);
   __syncthreads();
   const int C = cfg.n_classes;
   const int n_par = (cfg.n_seq - 1) / C;
   const uint64_t u = (uint64_t)(tile0 + blockIdx.x) * kModTile + threadIdx.x;
-  uint32_t ng = 0, nv = 0;
+  uint32_t mask = 0, nv = 0;
   if (u < n_unique) {
     SeqCounts sc{s_cnt + threadIdx.x};
     const double bm = u_mass[u];
     peptide_dp(sc, res, cmask, mt, cfg, u, u_gpos[u], u_len[u], n_par, err);
     const bool gated = gate_reachable(bm, cfg);
-    ng = 1;
+    mask = 1;
     nv = 1;  // the unmodified peptide is always present
     for (int v = 1; v < cfg.n_seq; ++v) {
       const uint32_t c = sc.get(v);
@@ -188,13 +194,19 @@ __global__ void __launch_bounds__(MD_THREADS)
         if (!(m >= cfg.min_mass && m <= cfg.max_mass)) continue;
       }
       if (c > kGrpCntMask) atomicOr(err, kErrModPos);  // > 2^27 variants in one group
-      ++ng;
+      mask |= 1u << v;
       nv += c;
     }
-    ng_out[u] = (uint8_t)ng;
+    mask_out[u] = mask;
   }
+  if (vt_cnt)
+    for (int v = 0; v < cfg.n_seq; ++v) {
+      const unsigned b = __ballot_sync(0xffffffffu, (mask >> v) & 1u);
+      if (lane_id() == 0 && b) atomicAdd(&s_vc[v], (uint32_t)__popc(b));
+    }
   uint32_t tot_g;
-  block_exclusive_sum<uint32_t, MD_THREADS>(ng, scratch, &tot_g);
+  block_exclusive_sum<uint32_t, MD_THREADS>((uint32_t)__popc(mask), scratch, &tot_g);  // syncs: s_vc is complete
+  if (vt_cnt && (int)threadIdx.x < cfg.n_seq) vt_cnt[(uint64_t)threadIdx.x * vt_stride + blockIdx.x] = s_vc[threadIdx.x];
   // the variant total of a tile is informational (the entry count comes from the 64-bit scan of the sorted
   // groups); summed in 64 bits and saturated so that a wrap can never look like a small number
   __shared__ unsigned long long scratch64[MD_WARPS + 1];
@@ -207,13 +219,19 @@ __global__ void __launch_bounds__(MD_THREADS)
 }
 
 // ---- K6g ------------------------------------------------------------------------------
+// Peptide-major layout (kLists = false, the sharded build): the groups of a tile from tile_goffs[tile] on,
+// peptide by peptide, v ascending.  List layout (kLists = true): the groups of class sequence v form list v,
+// in peptide order; group (u, v) goes to goffs[v * vt_stride + tile] + (earlier peptides of the tile with v).
+// Either way every list v is strictly increasing in (key, payload): u_mass grows with u, and the rounded
+// additions of f_v(base) are monotone in the base.
+template <bool kLists>
 __global__ void __launch_bounds__(MD_THREADS)
     grp_emit_kernel(const uint8_t* __restrict__ res, const DevTables* __restrict__ tb, DigestCfg cfg,
                     const double* __restrict__ u_mass, const uint32_t* __restrict__ u_gpos,
                     const uint16_t* __restrict__ u_len, const uint64_t* __restrict__ cmask, uint64_t n_unique,
-                    uint32_t tile0, const uint8_t* __restrict__ ng_in, const uint64_t* __restrict__ tile_goffs,
-                    uint64_t base_bits, uint64_t id_off, uint64_t* __restrict__ g_key, uint64_t* __restrict__ g_pay,
-                    uint32_t* err) {
+                    uint32_t tile0, const uint32_t* __restrict__ mask_in, const uint64_t* __restrict__ goffs,
+                    uint32_t vt_stride, uint64_t base_bits, uint64_t id_off, uint64_t* __restrict__ g_key,
+                    uint64_t* __restrict__ g_pay, uint32_t* err) {
   extern __shared__ uint32_t s_cnt[];  // [n_seq][MD_THREADS]
   __shared__ ModTables mt;
   __shared__ uint32_t scratch[MD_WARPS + 1];
@@ -223,28 +241,56 @@ __global__ void __launch_bounds__(MD_THREADS)
   const int n_par = (cfg.n_seq - 1) / C;
   const uint64_t u = (uint64_t)(tile0 + blockIdx.x) * kModTile + threadIdx.x;
   const bool valid = u < n_unique;
-  const uint32_t ng = valid ? ng_in[u] : 0u;
-  uint32_t tot;
-  const uint32_t ex = block_exclusive_sum<uint32_t, MD_THREADS>(ng, scratch, &tot);
-  if (!valid) return;
-  uint64_t o = tile_goffs[blockIdx.x] + ex;
+  const uint32_t mask = valid ? mask_in[u] : 0u;
+  const int w = threadIdx.x >> 5;
+  // list layout: ballot of every class sequence per warp, and where each warp's groups of it start
+  __shared__ uint32_t s_bal[kLists ? 32 * MD_WARPS : 1];
+  __shared__ uint64_t s_wbase[kLists ? 32 * MD_WARPS : 1];
+  uint64_t o = 0;
+  if constexpr (kLists) {
+    for (int v = 0; v < cfg.n_seq; ++v) {
+      const unsigned b = __ballot_sync(0xffffffffu, (mask >> v) & 1u);
+      if (lane_id() == 0) s_bal[v * MD_WARPS + w] = b;
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < cfg.n_seq) {
+      uint64_t run = goffs[(uint64_t)threadIdx.x * vt_stride + blockIdx.x];
+      for (int x = 0; x < MD_WARPS; ++x) {
+        s_wbase[threadIdx.x * MD_WARPS + x] = run;
+        run += (uint32_t)__popc(s_bal[threadIdx.x * MD_WARPS + x]);
+      }
+    }
+    __syncthreads();
+    if (!valid) return;
+  } else {
+    uint32_t tot;
+    const uint32_t ex = block_exclusive_sum<uint32_t, MD_THREADS>((uint32_t)__popc(mask), scratch, &tot);
+    if (!valid) return;
+    o = goffs[blockIdx.x] + ex;
+  }
+  auto slot = [&](int v) -> uint64_t {
+    if constexpr (kLists)
+      return s_wbase[v * MD_WARPS + w] + (uint32_t)__popc(s_bal[v * MD_WARPS + w] & lanemask_lt());
+    else
+      return o++;
+  };
   const double bm = u_mass[u];
-  g_key[o] = (uint64_t)__double_as_longlong(bm) - base_bits;
   const uint64_t gid = (id_off + u) << 32;  // global id of the peptide (id_off = 0 on a single GPU)
-  g_pay[o] = gid | 1u;
-  ++o;
-  if (ng == 1) return;  // no sites, or every modified mass is gated out
+  {
+    const uint64_t x = slot(0);
+    g_key[x] = (uint64_t)__double_as_longlong(bm) - base_bits;
+    g_pay[x] = gid | 1u;
+  }
+  if (mask == 1u) return;  // no sites, or every modified mass is gated out
   SeqCounts sc{s_cnt + threadIdx.x};
   peptide_dp(sc, res, cmask, mt, cfg, u, u_gpos[u], u_len[u], n_par, err);
-  const bool gated = gate_reachable(bm, cfg);
   for (int v = 1; v < cfg.n_seq; ++v) {
+    if (!((mask >> v) & 1u)) continue;  // no variant, or gated out (K5g)
     const uint32_t c = sc.get(v);
-    if (c == 0) continue;
     const double m = seq_mass((uint32_t)v, C, bm, mt.cls_delta);
-    if (gated && !(m >= cfg.min_mass && m <= cfg.max_mass)) continue;
-    g_key[o] = (uint64_t)__double_as_longlong(m) - base_bits;
-    g_pay[o] = gid | ((uint64_t)v << kGrpCntBits) | (uint64_t)(c & kGrpCntMask);
-    ++o;
+    const uint64_t x = slot(v);
+    g_key[x] = (uint64_t)__double_as_longlong(m) - base_bits;
+    g_pay[x] = gid | ((uint64_t)v << kGrpCntBits) | (uint64_t)(c & kGrpCntMask);
   }
 }
 
@@ -681,23 +727,27 @@ void launch_count_long(const uint16_t* len, uint64_t n, unsigned long long* n_lo
 
 void launch_grp_count(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg, const double* u_mass,
                       const uint32_t* u_gpos, const uint16_t* u_len, const uint64_t* cmask, uint64_t n_unique,
-                      uint32_t tile0, uint32_t ntiles, uint8_t* ng, uint32_t* tile_groups, uint32_t* tile_vars,
-                      uint32_t* d_err, cudaStream_t s) {
+                      uint32_t tile0, uint32_t ntiles, uint32_t* mask, uint32_t* tile_groups, uint32_t* tile_vars,
+                      uint32_t* vt_cnt, uint32_t* d_err, cudaStream_t s) {
   if (n_unique == 0 || ntiles == 0) return;
   const size_t smem = (size_t)cfg.n_seq * MD_THREADS * 4;
   DBI_LAUNCH(grp_count_kernel, ntiles, MD_THREADS, smem, s, d_res, d_tb, cfg, u_mass, u_gpos, u_len, cmask, n_unique,
-             tile0, ng, tile_groups, tile_vars, d_err);
+             tile0, mask, tile_groups, tile_vars, vt_cnt, ntiles, d_err);
 }
 
 void launch_grp_emit(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg, const double* u_mass,
                      const uint32_t* u_gpos, const uint16_t* u_len, const uint64_t* cmask, uint64_t n_unique,
-                     uint32_t tile0, uint32_t ntiles, const uint8_t* ng, const uint64_t* tile_goffs,
+                     uint32_t tile0, uint32_t ntiles, const uint32_t* mask, const uint64_t* goffs, bool lists,
                      uint64_t base_bits, uint64_t id_off, uint64_t* g_key, uint64_t* g_pay, uint32_t* d_err,
                      cudaStream_t s) {
   if (n_unique == 0 || ntiles == 0) return;
   const size_t smem = (size_t)cfg.n_seq * MD_THREADS * 4;
-  DBI_LAUNCH(grp_emit_kernel, ntiles, MD_THREADS, smem, s, d_res, d_tb, cfg, u_mass, u_gpos, u_len, cmask, n_unique,
-             tile0, ng, tile_goffs, base_bits, id_off, g_key, g_pay, d_err);
+  if (lists)
+    DBI_LAUNCH(grp_emit_kernel<true>, ntiles, MD_THREADS, smem, s, d_res, d_tb, cfg, u_mass, u_gpos, u_len, cmask,
+               n_unique, tile0, mask, goffs, ntiles, base_bits, id_off, g_key, g_pay, d_err);
+  else
+    DBI_LAUNCH(grp_emit_kernel<false>, ntiles, MD_THREADS, smem, s, d_res, d_tb, cfg, u_mass, u_gpos, u_len, cmask,
+               n_unique, tile0, mask, goffs, ntiles, base_bits, id_off, g_key, g_pay, d_err);
 }
 
 void launch_grp_extract_cnt(const uint64_t* pay, uint64_t n, uint32_t* cnt, cudaStream_t s) {
