@@ -271,6 +271,7 @@ ABI_SYMBOLS = [
     "dbi_mg_side_classes", "dbi_mg_pull_proteome", "dbi_mg_digest", "dbi_mg_hist", "dbi_mg_plan", "dbi_mg_default_cost", "dbi_mg_count", "dbi_mg_scatter",
     "dbi_mg_index_base", "dbi_mg_unique_count", "dbi_mg_set_unique", "dbi_mg_groups", "dbi_mg_index_variants",
     "dbi_mg_finish", "dbi_mg_split_masses", "dbi_mg_slices", "dbi_mg_plan_matrix", "dbi_mg_build_local",
+    "dbi_mg_search_unindexed_local",
 ]
 
 

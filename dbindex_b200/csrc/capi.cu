@@ -215,6 +215,9 @@ struct dbi_handle {
   cudaStream_t side_stream = nullptr;     // carries the peer pulls of the proteome next to the digest
   cudaEvent_t pull_done = nullptr;
   bool pull_pending = false;
+  // world of the sharded unindexed search whose layout window 0 still holds (0 = none): the next search of the
+  // same handles with the same shards reuses it (dbi_mg_search_unindexed_local)
+  int mg_search_world = 0;
   uint64_t ent_base_off = 0;  // global id of this rank's first unique peptide (0 on a single GPU)
   uint64_t uoff[kMaxRanks + 1] = {};      // global id of every rank's first unique peptide
   uint64_t uniq_cap[kMaxRanks] = {};      // layout capacity of every rank's window 2
@@ -430,25 +433,31 @@ void drop_results(dbi_handle* h) {
   h->lookup.drop();
 }
 
-void free_index(dbi_handle* h) {
-  if (h->pull_pending) {  // peer copies into d_res still in flight
-    cudaStreamSynchronize(h->side_stream);
-    h->pull_pending = false;
-  }
+// The index tables and the sharded state between the stages of a build; the packed residues stay.
+void free_sharded_tables(dbi_handle* h) {
   h->built = false;
-  drop_results(h);
-  h->d_res.release();
-  h->d_pstart.release();
-  h->packed_prot = UINT64_MAX;
   free_tables(h);
   h->mg_mass.release(); h->mg_gpos.release(); h->mg_prot.release(); h->mg_len.release();
   h->mg_nmod.release();
   h->mg_vkey.release(); h->mg_vpay.release();
   h->mg_n = h->mg_v = 0;
   h->mg_recv[0] = h->mg_recv[1] = 0;
-  h->mg_layout = false;
   h->ent_base_off = 0;
   std::memset(h->uoff, 0, sizeof(h->uoff));
+}
+
+void free_index(dbi_handle* h) {
+  if (h->pull_pending) {  // peer copies into d_res still in flight
+    cudaStreamSynchronize(h->side_stream);
+    h->pull_pending = false;
+  }
+  drop_results(h);
+  h->d_res.release();
+  h->d_pstart.release();
+  h->packed_prot = UINT64_MAX;
+  free_sharded_tables(h);
+  h->mg_layout = false;
+  h->mg_search_world = 0;
   h->spans.clear();
   h->ev_used = 0;
   const uint64_t np = h->st.n_proteins, nr = h->st.n_residues;
@@ -1618,6 +1627,52 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
   r.valid = true;
   return DBI_OK;
 }
+
+// The start of an unindexed search on one handle: its candidate pipeline replaces the stats of the previous one.
+void search_begin(dbi_handle* h) {
+  h->spans.clear();
+  h->ev_used = 0;
+  const uint64_t np = h->st.n_proteins, nr = h->st.n_residues;
+  std::memset(&h->st, 0, sizeof(h->st));
+  h->st.n_proteins = np;
+  h->st.n_residues = nr;
+  ensure_uploaded(h);
+  const uint32_t zero = 0;
+  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, h->stream));
+}
+
+// K12: a batch's windows on the handle's GPU, sorted by lo, with the prefix maximum of hi.  io = lo | hi (the
+// caller's order, for the materialisation) | sorted lo | prefix max of hi; *win = the handle's shift intervals
+// over those windows.
+void upload_windows(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, DevBuf& io, MassWindows* win) {
+  cudaStream_t s = h->stream;
+  io.alloc(std::max<uint64_t>(nq, 1) * 32, h->arena);
+  double* d_lo = io.as<double>();
+  double* d_hi = d_lo + nq;
+  double* w_lo = d_hi + nq;
+  double* w_pmax = w_lo + nq;
+  *win = h->shifts;
+  win->lo = w_lo;
+  win->pmax = w_pmax;
+  win->n = (uint32_t)nq;
+  if (!nq) return;
+  DBI_CUDA(cudaMemcpyAsync(d_lo, lo, nq * 8, cudaMemcpyHostToDevice, s));
+  DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, cudaMemcpyHostToDevice, s));
+  Stage sg(h, DBI_STAGE_OTHER);
+  DevBuf wk[2], wv[2], wtmp;
+  for (int i = 0; i < 2; ++i) {
+    wk[i].alloc(nq * 8, h->arena);
+    wv[i].alloc(nq * 8, h->arena);
+  }
+  wtmp.alloc(radix_sort_tmp_bytes(nq), h->arena);
+  launch_win_keys(d_lo, d_hi, nq, h->p.min_mass, h->p.max_mass, wk[0].as<uint64_t>(), wv[0].as<uint64_t>(), s);
+  uint64_t* kk[2] = {wk[0].as<uint64_t>(), wk[1].as<uint64_t>()};
+  uint64_t* vv[2] = {wv[0].as<uint64_t>(), wv[1].as<uint64_t>()};
+  const int nbits = bit_length(win_drop_key(h->p.min_mass, h->p.max_mass));
+  const int r = radix_sort_pairs<uint64_t, uint64_t>(kk, vv, nq, 0, nbits, wtmp.p, s, nullptr);
+  launch_win_pmax(kk[r], vv[r], nq, h->p.min_mass, h->p.max_mass, w_lo, w_pmax, s);
+  h->st.algo_bytes[DBI_STAGE_OTHER] += nq * (16 + 16) + nq * 32ull * ((nbits + 7) / 8) + nq * 32;
+}
 }  // namespace
 
 extern "C" {
@@ -1714,50 +1769,15 @@ int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint
     set_error("%llu windows in one batch (< 2^32)", (unsigned long long)nq);
     return DBI_ERANGE;
   }
-  // this search's candidate pipeline replaces the stats of the previous one
-  h->spans.clear();
-  h->ev_used = 0;
-  {
-    const uint64_t np = h->st.n_proteins, nr = h->st.n_residues;
-    std::memset(&h->st, 0, sizeof(h->st));
-    h->st.n_proteins = np;
-    h->st.n_residues = nr;
-  }
-  ensure_uploaded(h);
-  const uint32_t zero = 0;
-  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, s));
+  search_begin(h);
   const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
   if (h->packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
 
-  // K12: the batch's windows, sorted by lo, with the prefix maximum of hi
-  DevBuf io;  // lo | hi (the caller's order, for the materialisation) | sorted lo | prefix max of hi
-  io.alloc(std::max<uint64_t>(nq, 1) * 32, h->arena);
-  double* d_lo = io.as<double>();
-  double* d_hi = d_lo + nq;
-  double* w_lo = d_hi + nq;
-  double* w_pmax = w_lo + nq;
-  MassWindows win = h->shifts;
-  win.lo = w_lo;
-  win.pmax = w_pmax;
-  win.n = (uint32_t)nq;
-  if (nq) {
-    DBI_CUDA(cudaMemcpyAsync(d_lo, lo, nq * 8, cudaMemcpyHostToDevice, s));
-    DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, cudaMemcpyHostToDevice, s));
-    Stage sg(h, DBI_STAGE_OTHER);
-    DevBuf wk[2], wv[2], wtmp;
-    for (int i = 0; i < 2; ++i) {
-      wk[i].alloc(nq * 8, h->arena);
-      wv[i].alloc(nq * 8, h->arena);
-    }
-    wtmp.alloc(radix_sort_tmp_bytes(nq), h->arena);
-    launch_win_keys(d_lo, d_hi, nq, h->p.min_mass, h->p.max_mass, wk[0].as<uint64_t>(), wv[0].as<uint64_t>(), s);
-    uint64_t* kk[2] = {wk[0].as<uint64_t>(), wk[1].as<uint64_t>()};
-    uint64_t* vv[2] = {wv[0].as<uint64_t>(), wv[1].as<uint64_t>()};
-    const int nbits = bit_length(win_drop_key(h->p.min_mass, h->p.max_mass));
-    const int r = radix_sort_pairs<uint64_t, uint64_t>(kk, vv, nq, 0, nbits, wtmp.p, s, nullptr);
-    launch_win_pmax(kk[r], vv[r], nq, h->p.min_mass, h->p.max_mass, w_lo, w_pmax, s);
-    h->st.algo_bytes[DBI_STAGE_OTHER] += nq * (16 + 16) + nq * 32ull * ((nbits + 7) / 8) + nq * 32;
-  }
+  DevBuf io;
+  MassWindows win;
+  upload_windows(h, lo, hi, nq, io, &win);
+  const double* d_lo = io.as<double>();
+  const double* d_hi = d_lo + nq;
 
   // K2u: the records that can land in a window, counted before anything is allocated
   const uint64_t tiles = nq ? ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile : 0;

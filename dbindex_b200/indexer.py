@@ -280,7 +280,8 @@ def _merge_hits(parts, nq: int) -> dict:
 
 
 def search_unindexed_chunked(index: GpuIndex, lo, hi, max_candidates: int) -> dict:
-    """query_hits-style answer (one record per hit) of the ranges [lo[i], hi[i]] on an unbuilt handle, through
+    """query_hits-style answer (one record per hit) of the ranges [lo[i], hi[i]] on an unbuilt handle (or on the
+    handles of a sharded proteome: multigpu.ShardedSearcher, whose N_c is the largest per-rank count), through
     dbi_search_unindexed calls of at most max_candidates candidate records each (0 = one call, no cap).  The
     ranges go to the device sorted by mass; a batch whose N_c candidates exceed the cap is split into
     ceil(N_c / cap) + 1 contiguous chunks of the sorted order (again if a chunk still exceeds it), and the answer
@@ -307,7 +308,7 @@ class DBIndexer:
     """DBIndexer.java: the indexer / orchestrator, GPU store behind it."""
 
     def __init__(self, params: DbiParams, index_factor: int = 8, index_path: Optional[str] = None,
-                 use_index: bool = True):
+                 use_index: bool = True, devices: Optional[Sequence[int]] = None):
         """index_path: where the finished index lives on disk (None = in-memory index only).  run() skips
         indexing when the file exists ("Found existing index, skipping indexing", DBIndexer.java:522-531)
         and writes it after a fresh build.
@@ -316,11 +317,20 @@ class DBIndexer:
         run() only adds the proteins, and every getSequences* digests them again for its batch of ranges on the
         GPU (dbi_search_unindexed), max_candidates candidate records per device call.  No index file is read or
         written.  getNumberSequences, getParentMasses and export_reference_index need an index and raise
-        DBIndexStoreException in this mode."""
+        DBIndexStoreException in this mode.
+
+        devices (unindexed mode only; what -Ddbindex.gpu.devices is to the Java shim): one handle per entry, on that
+        CUDA device (a device may repeat).  The proteome is cut into residue-balanced shards in file order, proteins
+        added later go to the last shard, and every search runs over all of them (dbi_mg_search_unindexed_local)."""
+        if devices is not None and use_index:
+            raise DBIndexerException("a sharded index is not available here: devices needs use_index = False")
         self.sparam = params
         self.index_factor = index_factor  # dbindex.properties:6; only shapes the ">= MAX_MASS" query rule
         self.index_path = index_path
         self.use_index = use_index
+        self.devices = None if devices is None else list(devices)
+        self.shards: List[GpuIndex] = []  # the handles of a sharded proteome, rank order
+        self._shard_first = [0]           # global id of every shard's first protein, then the total
         self.max_candidates = UNINDEXED_MAX_CANDIDATES
         self.loaded_from_disk = False
         self.inited = False
@@ -332,7 +342,17 @@ class DBIndexer:
     def init(self):
         if self.inited:
             raise DBIndexerException("Already inited")  # DBIndexer.java:413-415
-        self.index = GpuIndex(self.sparam)
+        if self.devices is None:
+            self.index = GpuIndex(self.sparam)
+            self._searcher = self.index
+        else:
+            from .multigpu import ShardedSearcher
+            for d in self.devices:
+                p = self.sparam.copy()
+                p.device = int(d)
+                self.shards.append(GpuIndex(p))
+            self.index = self.shards[0]  # the masses (calculate_mass) are every shard's
+            self._searcher = ShardedSearcher(self.shards)
         self.inited = True
 
     def export_reference_index(self, database_id: str) -> dict:
@@ -359,7 +379,22 @@ class DBIndexer:
         """protCache.addProtein for a packed batch (DBIndexer.java:605)."""
         self._require()
         self.deflines.extend(d.replace("\t", " ") for d in deflines)  # ProteinCache.java:87-89
-        self.index.add_proteins(residues, offsets)
+        if not self.shards:
+            self.index.add_proteins(residues, offsets)
+            return
+        from .multigpu import shard_proteins
+        offsets = np.asarray(offsets, dtype=np.uint64)
+        n = len(offsets) - 1
+        if self._shard_first[-1] == 0:  # the first proteins are cut the way the Java shim cuts them
+            first = []
+            for r, g in enumerate(self.shards):
+                res, off, p0 = shard_proteins(residues, offsets, r, len(self.shards))
+                g.add_proteins(res, off)
+                first.append(p0)
+            self._shard_first = first + [n]
+        else:  # later ones go to the last shard, so that ids stay in insertion order
+            self.shards[-1].add_proteins(residues, offsets)
+            self._shard_first[-1] += n
 
     def run(self, fasta: Optional[str] = None, proteins: Optional[Tuple[Sequence[str], Sequence[str]]] = None):
         """DBIndexer.run(): stream the FASTA, cut every protein, close the store."""
@@ -396,16 +431,21 @@ class DBIndexer:
             raise DBIndexerException(str(e)) from e
 
     def close(self):
-        if self.index is not None:
-            self.index.close()
-            self.index = None
+        for g in self.shards or ([self.index] if self.index is not None else []):
+            g.close()
+        self.index = None
+        self.shards = []
         self.inited = False
 
     # -- helpers ---------------------------------------------------------------------------
     def getProteinSequence(self, pid: int) -> str:
         s = self._seq_cache.get(pid)
         if s is None:
-            s = self.index.get_protein(pid).decode("latin-1")
+            if self.shards:
+                r = min(int(np.searchsorted(self._shard_first, pid, side="right")) - 1, len(self.shards) - 1)
+                s = self.shards[r].get_protein(pid - self._shard_first[r]).decode("latin-1")
+            else:
+                s = self.index.get_protein(pid).decode("latin-1")
             if len(self._seq_cache) < 100000:
                 self._seq_cache[pid] = s
         return s
@@ -423,7 +463,7 @@ class DBIndexer:
         try:
             if self.use_index:
                 return self.index.query_hits(lo, hi)
-            return search_unindexed_chunked(self.index, lo, hi, self.max_candidates)
+            return search_unindexed_chunked(self._searcher, lo, hi, self.max_candidates)
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
 
@@ -577,9 +617,10 @@ class DBIndexImpl:
     _by_param_key: dict = {}  # DBIndexImpl.java:35 dbIndexByParamKey
 
     def __init__(self, params, fasta: Optional[str] = None,
-                 proteins: Optional[Tuple[Sequence[str], Sequence[str]]] = None, index_factor: int = 8):
+                 proteins: Optional[Tuple[Sequence[str], Sequence[str]]] = None, index_factor: int = 8,
+                 devices: Optional[Sequence[int]] = None):
         """params: dbi_params, or a DBIndexSearchParams (then the FASTA is its dataBaseName, as in
-        DBIndexImpl(DBIndexSearchParams), DBIndexImpl.java:117-145)."""
+        DBIndexImpl(DBIndexSearchParams), DBIndexImpl.java:117-145).  devices: DBIndexer's (unindexed mode)."""
         self.sparam = params if isinstance(params, DBIndexSearchParams) else None
         if self.sparam is not None:
             if fasta is None and proteins is None:
@@ -591,7 +632,7 @@ class DBIndexImpl:
         if self.sparam is not None and use_index and not self.sparam.inMemoryIndex:
             # an on-disk index, named like the reference's (DBIndexer.java:429 createFullIndexFileName)
             index_path = createFullIndexFileName(self.sparam) + INDEX_FILE_SUFFIX
-        self.indexer = DBIndexer(params, index_factor, index_path=index_path, use_index=use_index)
+        self.indexer = DBIndexer(params, index_factor, index_path=index_path, use_index=use_index, devices=devices)
         self.indexer.init()
         self.indexer.run(fasta=fasta, proteins=proteins)
         self._proteins_by_seq: dict = {}  # DBIndexImpl.java:33

@@ -587,3 +587,48 @@ def lookup_local(handles, seqs, modpat=None) -> dict:
     out["prot_list_off"] = np.concatenate(([0], np.cumsum(sizes))).astype(np.uint64)
     out["prot_ids"] = np.concatenate(ids) if n else np.zeros(0, np.uint32)
     return out
+
+
+def search_unindexed_local(handles, lo, hi, max_candidates: int = 0) -> dict:
+    """dbi_mg_search_unindexed_local: dbi_search_unindexed over a proteome sharded over `handles` of this process
+    (`handles[r]` was given shard r, as for build_local).  Returns one query_hits-style answer (one record per hit)
+    for the ranges [lo[i], hi[i]], the ranks' hits of every query concatenated, and under "n_candidates" the
+    candidate records every rank indexed.  DBI_ERANGE (a rank over max_candidates, 0 = no cap) raises DbiError with
+    n_candidates = the largest per-rank count and the per-rank counts in its `rank_candidates`."""
+    import ctypes as C
+    from .capi import DbiError, DbiHitCounts
+    from .indexer import _merge_hits
+    lib = handles[0].lib
+    lib.dbi_mg_search_unindexed_local.restype = C.c_int
+    lib.dbi_mg_search_unindexed_local.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_uint64,
+                                                  C.c_uint64, C.POINTER(DbiHitCounts), C.c_void_p]
+    lo = np.ascontiguousarray(lo, dtype=np.float64)
+    hi = np.ascontiguousarray(hi, dtype=np.float64)
+    if len(lo) != len(hi):
+        raise ValueError(f"{len(lo)} lower and {len(hi)} upper bounds")
+    n = len(handles)
+    arr = (C.c_void_p * n)(*[g._h for g in handles])
+    counts = (DbiHitCounts * n)()
+    n_cand = np.zeros(n, dtype=np.uint64)
+    rc = lib.dbi_mg_search_unindexed_local(arr, n, lo.ctypes.data, hi.ctypes.data, len(lo), int(max_candidates),
+                                           counts, n_cand.ctypes.data)
+    if rc != 0:
+        err = DbiError(rc, (lib.dbi_last_error() or b"").decode(errors="replace"), int(n_cand.max()))
+        err.rank_candidates = n_cand
+        raise err
+    q = np.arange(len(lo), dtype=np.int64)
+    out = _merge_hits([(q, g._read_hits(counts[r], None, None, True)) for r, g in enumerate(handles)], len(lo))
+    out["n_candidates"] = n_cand
+    return out
+
+
+class ShardedSearcher:
+    """The handles of a sharded proteome in this process as one unindexed searcher.  search_unindexed has the
+    signature of GpuIndex.search_unindexed, so indexer.search_unindexed_chunked splits sharded batches unchanged:
+    its ceil(N_c / cap) + 1 rule acts on the largest per-rank count, and every call plans its cuts again."""
+
+    def __init__(self, handles):
+        self.handles = list(handles)
+
+    def search_unindexed(self, lo, hi, max_candidates: int = 0) -> dict:
+        return search_unindexed_local(self.handles, lo, hi, max_candidates)

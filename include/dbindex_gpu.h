@@ -501,6 +501,32 @@ int dbi_mg_slices(dbi_handle* h); /* slices of the built sharded index (world or
 int dbi_mg_split_masses(dbi_handle* h, double* split_mass); /* [dbi_mg_slices - 1] */
 int dbi_mg_build_local(dbi_handle** handles, int n);
 
+/* dbi_search_unindexed over a proteome spread over n handles of this process, prepared as for dbi_mg_build_local
+ * (handles[r] is rank r and was given shard r with dbi_add_proteins, shards in rank order).  Every rank digests
+ * only the start positions of its own shard, keeping the records that can land in a window (K2u / K4u); exchange 0
+ * moves them to the owners of their mass slices, with cuts planned from the candidates' histograms; every rank
+ * indexes its slices (with mods: exchange 1 and the variant index) and materialises its hits through the other
+ * ranks' window 2.  Afterwards every rank's candidate index is dropped, once all ranks are idle.
+ *
+ * Every rank ends with a pending hit result for all nq windows in the caller's order (counts[r].nq == nq), read with
+ * dbi_query_hits_read on handles[r]: rank r's hits of a window are those inside the mass slices it owns in this
+ * call.  For every query the union over the ranks equals what dbi_search_unindexed returns on one handle holding the
+ * whole proteome (first occurrences and protein lists are global; order inside a query is not a contract).  lo / hi
+ * are host pointers with the semantics of dbi_query_hits; the < 2^32 hits rule applies per rank.
+ *
+ * The handles stay unbuilt (a built one: DBI_EALREADY): dbi_query_hits still returns DBI_ENOTINIT and
+ * dbi_mg_build_local still builds the normal sharded index.  The packed proteome (window 0) is kept between calls
+ * and packed and pulled again only when a handle received proteins, or the handles are not the ones of the last
+ * call.  n_candidates[r] (may be NULL) = candidate records rank r would index after the exchange, known before any
+ * arena grows: one above max_candidates (0 = no cap) or at >= 2^32, or an own shard digesting to >= 2^32 records,
+ * gives DBI_ERANGE with the counts filled in.  No handle has a pending result after any failure.  dbi_stats_get on
+ * handles[r] reports rank r's candidate pipeline: n_emitted = candidates digested from its shard, n_unique /
+ * n_entries of its slices, the stage times with params.profile; n_emitted and n_entries summed over the ranks equal
+ * the single-GPU call's.  Null or repeated handles, handles created with other parameters (the device aside) and n
+ * outside 1..DBI_MG_MAX_RANKS are DBI_EINVAL.  n = 1 is dbi_search_unindexed on handles[0]. */
+int dbi_mg_search_unindexed_local(dbi_handle** handles, int n, const double* lo, const double* hi, uint64_t nq,
+                                  uint64_t max_candidates, dbi_hit_counts* counts, uint64_t* n_candidates);
+
 /* Test hook for K7: stable radix sort of n host (key, value) pairs on key bits
  * [begin_bit, end_bit), in place, on the handle's GPU. */
 int dbi_debug_radix_sort(dbi_handle* h, uint64_t* keys, uint64_t* vals, uint64_t n, int begin_bit, int end_bit);

@@ -123,6 +123,10 @@ public final class DbiNative {
 	// two multisplit / peer-memory scatter kernels) is one call; afterwards every handle answers for its mass slice
 	// and reads base peptides owned by another GPU through the mapped window of that GPU
 	static final MethodHandle dbi_mg_build_local = h("dbi_mg_build_local", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));
+	// SEARCH_UNINDEXED over those handles: every GPU digests its shard, indexes its mass slices for this batch only and
+	// keeps its hits pending (dbi_query_hits_read on each handle)
+	static final MethodHandle dbi_mg_search_unindexed_local = h("dbi_mg_search_unindexed_local", FunctionDescriptor.of(
+			JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_mg_slices = h("dbi_mg_slices", FunctionDescriptor.of(JAVA_INT, ADDRESS));
 	static final MethodHandle dbi_mg_split_masses = h("dbi_mg_split_masses", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_destroy = h("dbi_destroy", FunctionDescriptor.ofVoid(ADDRESS));

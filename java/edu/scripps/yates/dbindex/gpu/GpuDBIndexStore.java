@@ -45,7 +45,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 	private double[] splitMass = new double[0]; // masses at which the slices of the sharded index are cut
 	private boolean inited = false, built = false;
 	// SEARCH_UNINDEXED (DBIndexer.java:58-61, MassRangeFilteringIndex.java:90-108): no index, every query digests
-	// the proteins again for its ranges (dbi_search_unindexed), at most maxCandidates candidate records per call
+	// the proteins again for its ranges (dbi_search_unindexed; with -Ddbindex.gpu.devices=N every GPU its shard,
+	// dbi_mg_search_unindexed_local), at most maxCandidates candidate records per call (and GPU)
 	private final boolean unindexed;
 	private final long maxCandidates = Long.getLong("dbindex.gpu.maxCandidates", 1L << 25);
 	private ProteinCache proteinCache;
@@ -133,8 +134,6 @@ public class GpuDBIndexStore implements DBIndexStore {
 	public void init(String databaseID) throws DBIndexStoreException {
 		if (inited)
 			throw new DBIndexStoreException("Already intialized"); // DBIndexStoreSQLiteMult.java:97-99
-		if (unindexed && nDevices > 1)
-			throw new DBIndexStoreException("an unindexed search (useIndex = false) runs on one GPU: -Ddbindex.gpu.devices=1");
 		try {
 			handles = new MemorySegment[nDevices];
 			for (int d = 0; d < nDevices; ++d) {
@@ -209,12 +208,10 @@ public class GpuDBIndexStore implements DBIndexStore {
 			final MemorySegment o = a.allocate(JAVA_LONG, offsets.size());
 			for (int i = 0; i < offsets.size(); ++i)
 				o.setAtIndex(JAVA_LONG, i, offsets.get(i));
-			if (unindexed) { // the proteins are all there is: every query digests them (dbi_search_unindexed)
-				check((int) DbiNative.dbi_add_proteins.invoke(handle, r, o, offsets.size() - 1));
-				return;
-			}
 			if (nDevices == 1) {
 				check((int) DbiNative.dbi_add_proteins.invoke(handle, r, o, offsets.size() - 1));
+				if (unindexed) // the proteins are all there is: every query digests them (dbi_search_unindexed)
+					return;
 				check((int) DbiNative.dbi_build.invoke(handle));
 			} else {
 				// contiguous shards of about equal residue count, in protein order (ids stay global and in file order);
@@ -232,6 +229,8 @@ public class GpuDBIndexStore implements DBIndexStore {
 					check((int) DbiNative.dbi_add_proteins.invoke(handles[d], r, o.asSlice(8L * first), last - first));
 					first = last;
 				}
+				if (unindexed) // every query digests the shards (dbi_mg_search_unindexed_local)
+					return;
 				// the whole exchange in one call: shard packing, NVLink pulls, own-shard digest, the two multisplit /
 				// peer-memory scatter kernels into folded mass slices, per-GPU sort + merge + expansion
 				final MemorySegment hs = a.allocate(ADDRESS, nDevices);
@@ -372,8 +371,9 @@ public class GpuDBIndexStore implements DBIndexStore {
 	}
 
 	/**
-	 * SEARCH_UNINDEXED: the ranges sorted by mass go to dbi_search_unindexed; a batch whose candidate records exceed
-	 * maxCandidates (DBI_ERANGE, N_c reported) is split into ceil(N_c / cap) + 1 contiguous chunks, again if needed.
+	 * SEARCH_UNINDEXED: the ranges sorted by mass go to dbi_search_unindexed (sharded: dbi_mg_search_unindexed_local,
+	 * N_c = the largest per-GPU count); a batch whose candidate records exceed maxCandidates (DBI_ERANGE, N_c
+	 * reported) is split into ceil(N_c / cap) + 1 contiguous chunks, again if needed.
 	 * The sink sees the runs of every query, chunk by chunk in mass order, with the caller's query numbers.
 	 */
 	private void searchUnindexed(double[] lo, double[] hi, RunSink sink) throws DBIndexStoreException {
@@ -395,9 +395,20 @@ public class GpuDBIndexStore implements DBIndexStore {
 				dlo.setAtIndex(JAVA_DOUBLE, i, lo[ids[i]]);
 				dhi.setAtIndex(JAVA_DOUBLE, i, hi[ids[i]]);
 			}
-			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS), nCand = a.allocate(JAVA_LONG);
-			final int rc = (int) DbiNative.dbi_search_unindexed.invoke(handle, dlo, dhi, (long) nq, maxCandidates, cnt, nCand);
-			final long nc = nCand.get(JAVA_LONG, 0);
+			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS, nDevices), nCand = a.allocate(JAVA_LONG, nDevices);
+			final int rc;
+			if (nDevices == 1) {
+				rc = (int) DbiNative.dbi_search_unindexed.invoke(handle, dlo, dhi, (long) nq, maxCandidates, cnt, nCand);
+			} else {
+				final MemorySegment hs = a.allocate(ADDRESS, nDevices);
+				for (int d = 0; d < nDevices; ++d)
+					hs.setAtIndex(ADDRESS, d, handles[d]);
+				rc = (int) DbiNative.dbi_mg_search_unindexed_local.invoke(hs, nDevices, dlo, dhi, (long) nq, maxCandidates,
+						cnt, nCand);
+			}
+			long nc = 0;
+			for (int d = 0; d < nDevices; ++d)
+				nc = Math.max(nc, nCand.getAtIndex(JAVA_LONG, d));
 			if (rc == DbiNative.DBI_ERANGE && nc > maxCandidates && nq > 1) {
 				final int chunks = (int) Math.min(nq, (nc + maxCandidates - 1) / maxCandidates + 1);
 				for (int c = 0; c < chunks; ++c)
@@ -406,7 +417,9 @@ public class GpuDBIndexStore implements DBIndexStore {
 				return;
 			}
 			check(rc);
-			readHits(handle, a, cnt, ids, sink);
+			final long cb = DbiNative.HIT_COUNTS.byteSize();
+			for (int d = 0; d < nDevices; ++d) // every GPU answers for the mass slices it owns in this call
+				readHits(handles[d], a, cnt.asSlice(d * cb, cb), ids, sink);
 		} catch (final DBIndexStoreException e) {
 			throw e;
 		} catch (final Throwable t) {
