@@ -166,6 +166,34 @@ def expand_hits(raw: dict) -> dict:
 
 
 DBI_ERANGE = -7
+DBI_TOL_DA = 0   # dbi_query_spectra: spectrum s = ranges [range_off[s], range_off[s+1]) of (mass, tol in Da)
+DBI_TOL_PPM = 1  # dbi_query_spectra: spectrum s = mass[s] at tol[s] ppm
+
+
+def spectra_arrays(mass, tol, range_off, tol_mode: int):
+    """The contiguous arrays of a dbi_query_spectra batch and its number of spectra (range_off None: PPM only)."""
+    mass = np.ascontiguousarray(mass, dtype=np.float64)
+    tol = np.ascontiguousarray(tol, dtype=np.float64)
+    if len(mass) != len(tol):
+        raise ValueError(f"{len(mass)} masses and {len(tol)} tolerances")
+    if range_off is None:
+        if tol_mode == DBI_TOL_DA:
+            raise ValueError("DBI_TOL_DA needs range_off")
+        return mass, tol, None, len(mass)
+    range_off = np.ascontiguousarray(range_off, dtype=np.uint64)
+    if len(range_off) == 0 or (tol_mode == DBI_TOL_DA and int(range_off[-1]) > len(mass)):
+        raise ValueError(f"range_off of {len(range_off)} offsets over {len(mass)} ranges")
+    return mass, tol, range_off, len(range_off) - 1
+
+
+def ppm_probe_bound(mass: float, ppm: float) -> float:
+    """The upper end of the candidate window dbi_search_unindexed_spectra digests for one PPM spectrum: an upper
+    bound of every probe u the walk of getSequencesUsingPPMTolerance admits (u - tol(u) < mass), computed as
+    K13b computes it (spec_ppm_window_kernel)."""
+    p1 = ppm / 1e6 + 1.0
+    hi = mass + mass * (1 - 1 / p1)
+    ext = (mass * p1) * (1.0 + 2.0 ** -40) if mass > 0.0 and p1 > 0.0 else float("inf")
+    return max(ext, hi)
 
 
 class DbiError(RuntimeError):
@@ -220,6 +248,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "dbi_query_hits_device": (C.c_int, [vp, vp, vp, C.c_uint64, C.POINTER(DbiHitCounts)]),
         "dbi_query_hits_read": (C.c_int, [vp, C.POINTER(DbiHitBuffers)]),
         "dbi_search_unindexed": (C.c_int, [vp, vp, vp, C.c_uint64, C.c_uint64, C.POINTER(DbiHitCounts), u64p]),
+        "dbi_query_spectra": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_int, C.c_int, C.POINTER(DbiHitCounts)]),
+        "dbi_search_unindexed_spectra": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_int, C.c_int, C.c_uint64,
+                                                   C.POINTER(DbiHitCounts), u64p]),
         "dbi_lookup_peptides": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.POINTER(DbiLookupCounts)]),
         "dbi_lookup_peptides_read": (C.c_int, [vp, C.POINTER(DbiLookupBuffers)]),
         "dbi_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(vp)]),
@@ -260,7 +291,7 @@ ABI_SYMBOLS = [
     "dbi_default_params", "dbi_params_add_static_mod", "dbi_params_set_enzyme", "dbi_params_add_diff_mod",
     "dbi_create", "dbi_set_stream", "dbi_add_proteins", "dbi_upload", "dbi_reset_index", "dbi_build",
     "dbi_stats_get", "dbi_save", "dbi_load", "dbi_query", "dbi_query_device", "dbi_fetch", "dbi_query_hits", "dbi_query_hits_device", "dbi_query_hits_read",
-    "dbi_search_unindexed",
+    "dbi_search_unindexed", "dbi_query_spectra", "dbi_search_unindexed_spectra",
     "dbi_lookup_peptides", "dbi_lookup_peptides_read", "dbi_host_alloc", "dbi_host_free", "dbi_get_protein", "dbi_calculate_mass",
     "dbi_entry_keys", "dbi_debug_emitted", "dbi_build_from_records", "dbi_debug_radix_sort", "dbi_destroy",
     "dbi_abi_sizes", "dbi_release_cached_memory",
@@ -513,6 +544,33 @@ class GpuIndex:
         proteins added so far without a built index (the handle stays unbuilt).  The candidate records of the
         call are in self.last_candidates."""
         return self._read_hits(self.search_unindexed_begin(lo, hi, max_candidates), fields, alloc, per_hit)
+
+    def query_spectra(self, mass, tol, range_off=None, tol_mode: int = DBI_TOL_DA, index_factor: int = 0,
+                      fields=None, alloc=None, per_hit: bool = True) -> dict:
+        """dbi_query_spectra + dbi_query_hits_read: the answer of every spectrum of a batch as one query of a
+        query_hits-style dict.  DBI_TOL_DA: spectrum s = the (mass, tol in Da) ranges [range_off[s], range_off[s+1])
+        answered as getSequences(List<MassRange>); DBI_TOL_PPM (range_off None): mass[s] at tol[s] ppm answered as
+        getSequencesUsingPPMTolerance.  index_factor: the bucket rule of the reference (0 = off)."""
+        mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
+        cnt = DbiHitCounts()
+        self._check(self.lib.dbi_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
+                                               int(index_factor), C.byref(cnt)))
+        return self._read_hits(cnt, fields, alloc, per_hit)
+
+    def search_unindexed_spectra(self, mass, tol, range_off=None, tol_mode: int = DBI_TOL_DA, index_factor: int = 0,
+                                 max_candidates: int = 0, fields=None, alloc=None, per_hit: bool = True) -> dict:
+        """dbi_search_unindexed_spectra + dbi_query_hits_read: query_spectra answered from the proteins added so far
+        without a built index.  DbiError (DBI_ERANGE, n_candidates set) above max_candidates (0 = no cap); the
+        candidate records of the call are in self.last_candidates."""
+        mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
+        cnt, n_cand = DbiHitCounts(), C.c_uint64(0)
+        rc = self.lib.dbi_search_unindexed_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
+                                                   int(index_factor), int(max_candidates), C.byref(cnt),
+                                                   C.byref(n_cand))
+        self.last_candidates = n_cand.value
+        if rc != 0:
+            raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
+        return self._read_hits(cnt, fields, alloc, per_hit)
 
     def _read_hits(self, cnt: DbiHitCounts, fields, alloc, per_hit: bool) -> dict:
         out, bufs = {"counts": cnt}, DbiHitBuffers()

@@ -3,6 +3,7 @@
 // hand-written kernels of this directory; there is no CPU fallback.
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -1643,8 +1644,9 @@ void search_begin(dbi_handle* h) {
 
 // K12: a batch's windows on the handle's GPU, sorted by lo, with the prefix maximum of hi.  io = lo | hi (the
 // caller's order, for the materialisation) | sorted lo | prefix max of hi; *win = the handle's shift intervals
-// over those windows.
-void upload_windows(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, DevBuf& io, MassWindows* win) {
+// over those windows.  lo / hi are host pointers, or device pointers with kind = cudaMemcpyDeviceToDevice.
+void upload_windows(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, DevBuf& io, MassWindows* win,
+                    cudaMemcpyKind kind = cudaMemcpyHostToDevice) {
   cudaStream_t s = h->stream;
   io.alloc(std::max<uint64_t>(nq, 1) * 32, h->arena);
   double* d_lo = io.as<double>();
@@ -1656,8 +1658,8 @@ void upload_windows(dbi_handle* h, const double* lo, const double* hi, uint64_t 
   win->pmax = w_pmax;
   win->n = (uint32_t)nq;
   if (!nq) return;
-  DBI_CUDA(cudaMemcpyAsync(d_lo, lo, nq * 8, cudaMemcpyHostToDevice, s));
-  DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, cudaMemcpyHostToDevice, s));
+  DBI_CUDA(cudaMemcpyAsync(d_lo, lo, nq * 8, kind, s));
+  DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, kind, s));
   Stage sg(h, DBI_STAGE_OTHER);
   DevBuf wk[2], wv[2], wtmp;
   for (int i = 0; i < 2; ++i) {
@@ -1672,6 +1674,230 @@ void upload_windows(dbi_handle* h, const double* lo, const double* hi, uint64_t 
   const int r = radix_sort_pairs<uint64_t, uint64_t>(kk, vv, nq, 0, nbits, wtmp.p, s, nullptr);
   launch_win_pmax(kk[r], vv[r], nq, h->p.min_mass, h->p.max_mass, w_lo, w_pmax, s);
   h->st.algo_bytes[DBI_STAGE_OTHER] += nq * (16 + 16) + nq * 32ull * ((nbits + 7) / 8) + nq * 32;
+}
+
+// An unindexed search needs an unbuilt handle that is not part of a sharded build.
+int check_unindexed(dbi_handle* h) {
+  if (h->built) {
+    set_error("the index is built: query it with dbi_query_hits");
+    return DBI_EALREADY;
+  }
+  if (h->mg_begun) {
+    set_error("an unindexed search runs on one GPU; this handle is part of a sharded build");
+    return DBI_EINVAL;
+  }
+  return DBI_OK;
+}
+
+// The candidate index of an unindexed search lives for one call only; the pending result does not depend on it.
+struct DropCandidates {
+  dbi_handle* h;
+  bool armed = true;
+  ~DropCandidates() {
+    if (!armed) return;
+    free_tables(h);
+    h->built = false;
+  }
+};
+
+// K12 windows, K2u / K4u candidates, and their index on the handle (h->built until the caller's DropCandidates
+// drops it) for the windows [lo[i], hi[i]] (kind: where lo / hi live).  io = upload_windows' buffer, whose first
+// 2 nq doubles are lo | hi on the device.  N_c over max_candidates (or at 2^32): DBI_ERANGE with *n_candidates set.
+int index_candidates(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, cudaMemcpyKind kind,
+                     uint64_t max_candidates, uint64_t* n_candidates, DevBuf& io) {
+  cudaStream_t s = h->stream;
+  if (nq >= (1ull << 32)) {
+    set_error("%llu windows in one batch (< 2^32)", (unsigned long long)nq);
+    return DBI_ERANGE;
+  }
+  search_begin(h);
+  const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
+  if (h->packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
+
+  MassWindows win;
+  upload_windows(h, lo, hi, nq, io, &win, kind);
+  // K2u: the records that can land in a window, counted before anything is allocated
+  const uint64_t tiles = nq ? ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile : 0;
+  DevBuf tile_counts, tile_offs, start_cnt;
+  tile_counts.alloc(std::max<uint64_t>(tiles, 1) * 4, h->arena);
+  tile_offs.alloc((tiles + 1) * 8, h->arena);
+  start_cnt.alloc(std::max<uint64_t>(tiles, 1) * kDigestTile, h->arena);
+  const DigestRange whole{0u, h->res_end, 0u, n_prot};
+  uint64_t N = 0;
+  if (tiles) {
+    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
+    launch_digest_count(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
+                        (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), s,
+                        &win);
+    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
+    N = read_u64(h, tile_offs.as<uint64_t>() + tiles);
+    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2ull * h->res_end + tiles * 16;
+  }
+  if (int rc = check_err_bits(read_err(h))) return rc;
+  if (n_candidates) *n_candidates = N;
+  h->st.n_emitted = N;
+  if ((max_candidates && N > max_candidates) || N >= (1ull << 32)) {
+    set_error("%llu candidate records exceed the cap of %llu (and 2^32): split the batch", (unsigned long long)N,
+              (unsigned long long)(max_candidates ? max_candidates : (1ull << 32) - 1));
+    resolve_spans(h);
+    return DBI_ERANGE;
+  }
+  DevBuf r_mass, r_gpos, r_prot, r_len;
+  r_mass.alloc(std::max<uint64_t>(N, 1) * 8, h->arena);
+  r_gpos.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
+  r_prot.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
+  r_len.alloc(std::max<uint64_t>(N, 1) * 2, h->arena);
+  if (N) {  // K4u
+    Stage sg(h, DBI_STAGE_DIGEST_EMIT);
+    launch_digest_emit(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
+                       (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
+                       r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>(),
+                       nullptr, h->d_err.as<uint32_t>(), s, &win);
+    h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2ull * h->res_end + N * 18;
+  }
+  tile_counts.release();
+  tile_offs.release();
+  start_cnt.release();
+
+  DropCandidates drop_candidates{h};
+  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
+  if (int rc = index_records(h, rv, N, h->p.min_mass, h->p.max_mass)) return rc;
+  if (int rc = check_err_bits(read_err(h))) return rc;
+  r_mass.release(); r_gpos.release(); r_prot.release(); r_len.release();
+  drop_candidates.armed = false;
+  return DBI_OK;
+}
+
+// ---- batches of spectra (dbi_query_spectra, dbi_search_unindexed_spectra; K13 / K14 in spectra.cu) ----
+int check_spectra(const double* mass, const double* tol, const uint64_t* range_off, uint64_t n, int tol_mode,
+                  int index_factor, const dbi_hit_counts* counts) {
+  if (tol_mode != DBI_TOL_DA && tol_mode != DBI_TOL_PPM) {
+    set_error("tol_mode %d is neither DBI_TOL_DA nor DBI_TOL_PPM", tol_mode);
+    return DBI_EINVAL;
+  }
+  if (tol_mode == DBI_TOL_PPM && range_off) {
+    set_error("DBI_TOL_PPM takes one mass per spectrum: range_off must be NULL");
+    return DBI_EINVAL;
+  }
+  if (index_factor < 0 || index_factor > 8000) {
+    set_error("index_factor %d outside 0..8000", index_factor);
+    return DBI_EINVAL;
+  }
+  if (!counts || (n && (!mass || !tol || (tol_mode == DBI_TOL_DA && !range_off)))) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  for (uint64_t sp = 0; sp < n; ++sp) {
+    const uint64_t r0 = tol_mode == DBI_TOL_DA ? range_off[sp] : sp;
+    const uint64_t r1 = tol_mode == DBI_TOL_DA ? range_off[sp + 1] : sp + 1;
+    if (r1 < r0) {
+      set_error("spectrum %llu: range_off decreases (%llu -> %llu)", (unsigned long long)sp, (unsigned long long)r0,
+                (unsigned long long)r1);
+      return DBI_EINVAL;
+    }
+    for (uint64_t r = r0; r < r1; ++r)
+      if (!std::isfinite(mass[r]) || !std::isfinite(tol[r])) {
+        set_error("spectrum %llu: non-finite mass or tolerance (%g, %g)", (unsigned long long)sp, mass[r], tol[r]);
+        return DBI_EINVAL;
+      }
+  }
+  return DBI_OK;
+}
+
+// A batch of spectra on the device.  in = mass | tol (| range_off for Dalton lists).  Dalton: K13a merges every
+// list, iv = the kept intervals of all spectra, spectrum s owning [ioff[s], ioff[s+1]).  PPM: K13b writes win =
+// window lo | hi (| candidate lo | hi), and spectra_probe (K14, on the handle's entries) makes iv and ioff.
+struct SpectraBatch {
+  uint64_t n = 0, n_ranges = 0, n_iv = 0;
+  int mode = DBI_TOL_DA, factor = 0;
+  DevBuf in, win, cnt, ioff, stmp, iv;
+  const double* mass() const { return in.as<double>(); }
+  const double* tol() const { return in.as<double>() + n_ranges; }
+  const uint64_t* range_off() const { return (const uint64_t*)(in.as<double>() + 2 * n_ranges); }
+  const double* iv_lo() const { return iv.as<double>(); }
+  const double* iv_hi() const { return iv.as<double>() + n_iv; }
+};
+
+// scan of cnt into ioff, then iv sized for the intervals
+void spectra_offsets(dbi_handle* h, SpectraBatch& b) {
+  b.ioff.alloc((b.n + 1) * 8, h->arena);
+  b.stmp.alloc(full_scan_tmp_bytes(b.n), h->arena);
+  launch_full_scan_u32_to_u64(b.cnt.as<uint32_t>(), b.n, b.ioff.as<uint64_t>(), b.stmp.p, h->stream);
+  b.n_iv = read_u64(h, b.ioff.as<uint64_t>() + b.n);
+  b.iv.alloc(std::max<uint64_t>(b.n_iv, 1) * 16, h->arena);
+}
+
+// upload and K13; with `candidates` (PPM) also the candidate windows of an unindexed search
+void spectra_prepare(dbi_handle* h, SpectraBatch& b, const double* mass, const double* tol, const uint64_t* range_off,
+                     uint64_t n, int mode, int factor, bool candidates) {
+  cudaStream_t s = h->stream;
+  b.n = n;
+  b.mode = mode;
+  b.factor = factor;
+  b.n_ranges = mode == DBI_TOL_DA ? (n ? range_off[n] : 0) : n;
+  const uint64_t R = b.n_ranges;
+  b.in.alloc(std::max<uint64_t>(2 * R + (mode == DBI_TOL_DA ? n + 1 : 0), 1) * 8, h->arena);
+  if (R) {
+    DBI_CUDA(cudaMemcpyAsync(b.in.p, mass, R * 8, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(b.in.as<double>() + R, tol, R * 8, cudaMemcpyHostToDevice, s));
+  }
+  b.cnt.alloc(std::max<uint64_t>(n, 1) * 4, h->arena);
+  Stage sg(h, DBI_STAGE_QUERY);
+  if (mode == DBI_TOL_DA) {
+    if (n) DBI_CUDA(cudaMemcpyAsync((void*)b.range_off(), range_off, (n + 1) * 8, cudaMemcpyHostToDevice, s));
+    b.win.alloc(std::max<uint64_t>(R, 1) * 16, h->arena);
+    double* s_lo = b.win.as<double>();
+    double* s_hi = s_lo + R;
+    launch_spec_intervals(b.mass(), b.tol(), b.range_off(), n, factor, s_lo, s_hi, b.cnt.as<uint32_t>(), s);
+    spectra_offsets(h, b);
+    launch_spec_compact(b.range_off(), b.ioff.as<uint64_t>(), n, s_lo, s_hi, b.iv.as<double>(),
+                        b.iv.as<double>() + b.n_iv, s);
+    // per range: (mass, tol) read, slot written, interval packed (16 + 16 + 32); per spectrum: offsets and count
+    h->st.algo_bytes[DBI_STAGE_QUERY] += R * 64 + n * (16 + 4 + 16);
+  } else {
+    b.win.alloc(std::max<uint64_t>(n, 1) * (candidates ? 32 : 16), h->arena);
+    double* w = b.win.as<double>();
+    launch_spec_ppm_window(b.mass(), b.tol(), n, w, w + n, candidates ? w + 2 * n : nullptr,
+                           candidates ? w + 3 * n : nullptr, s);
+    h->st.algo_bytes[DBI_STAGE_QUERY] += n * (16 + (candidates ? 32 : 16));
+  }
+}
+
+// K14: the window and the continuing probes of every PPM spectrum, over the handle's (or candidate) index
+void spectra_probe(dbi_handle* h, SpectraBatch& b) {
+  cudaStream_t s = h->stream;
+  Stage sg(h, DBI_STAGE_QUERY);
+  const double* w_lo = b.win.as<double>();
+  const double* w_hi = w_lo + b.n;
+  launch_spec_probe_count(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor,
+                          b.cnt.as<uint32_t>(), s);
+  spectra_offsets(h, b);
+  launch_spec_probe_emit(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor,
+                         b.ioff.as<uint64_t>(), b.iv.as<double>(), b.iv.as<double>() + b.n_iv, s);
+  // both passes: (mass, ppm, window) read, one lower bound per probe (~1 per spectrum); count, offsets, interval
+  const uint64_t probe = 32 + 8ull * (uint64_t)bit_length(h->n_entries);
+  h->st.algo_bytes[DBI_STAGE_QUERY] += 2 * b.n * (32 + probe) + b.n * (4 + 8) + b.n_iv * 16;
+}
+
+// K9 / K10 over the intervals, then the per-interval offsets of the pending result collapsed to per-spectrum ones
+int spectra_answer(dbi_handle* h, SpectraBatch& b, dbi_hit_counts* counts) {
+  if (b.n_iv >= (1ull << 32)) {
+    set_error("%llu intervals in one batch (< 2^32): split the batch", (unsigned long long)b.n_iv);
+    return DBI_ERANGE;
+  }
+  if (int rc = query_hits_impl(h, b.iv_lo(), b.iv_hi(), b.n_iv, counts)) return rc;
+  dbi_handle::HitResult& r = h->hits;
+  DevBuf hit_off, pep_off;
+  hit_off.alloc((b.n + 1) * 8, h->arena);
+  pep_off.alloc((b.n + 1) * 8, h->arena);
+  launch_spec_collapse(b.ioff.as<uint64_t>(), b.n, r.hit_off.as<uint64_t>(), r.pep_off.as<uint64_t>(),
+                       hit_off.as<uint64_t>(), pep_off.as<uint64_t>(), h->stream);
+  DBI_CUDA(cudaStreamSynchronize(h->stream));
+  r.hit_off.swap(hit_off);
+  r.pep_off.swap(pep_off);
+  counts->nq = b.n;
+  r.n.nq = b.n;
+  return DBI_OK;
 }
 }  // namespace
 
@@ -1750,91 +1976,58 @@ int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out) {
 int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, uint64_t max_candidates,
                          dbi_hit_counts* counts, uint64_t* n_candidates) {
   DBI_API_BEGIN(h)
-  if (h->built) {
-    set_error("the index is built: query it with dbi_query_hits");
-    return DBI_EALREADY;
-  }
-  if (h->mg_begun) {
-    set_error("an unindexed search runs on one GPU; this handle is part of a sharded build");
-    return DBI_EINVAL;
-  }
+  if (int rc = check_unindexed(h)) return rc;
   if (!counts || (nq && (!lo || !hi))) {
     set_error("null argument");
     return DBI_EINVAL;
   }
-  cudaStream_t s = h->stream;
   drop_results(h);
   if (n_candidates) *n_candidates = 0;
-  if (nq >= (1ull << 32)) {
-    set_error("%llu windows in one batch (< 2^32)", (unsigned long long)nq);
-    return DBI_ERANGE;
-  }
-  search_begin(h);
-  const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
-  if (h->packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
-
   DevBuf io;
-  MassWindows win;
-  upload_windows(h, lo, hi, nq, io, &win);
-  const double* d_lo = io.as<double>();
-  const double* d_hi = d_lo + nq;
+  if (int rc = index_candidates(h, lo, hi, nq, cudaMemcpyHostToDevice, max_candidates, n_candidates, io)) return rc;
+  DropCandidates drop_candidates{h};
+  return query_hits_impl(h, io.as<double>(), io.as<double>() + nq, nq, counts);
+  DBI_API_END
+}
 
-  // K2u: the records that can land in a window, counted before anything is allocated
-  const uint64_t tiles = nq ? ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile : 0;
-  DevBuf tile_counts, tile_offs, start_cnt;
-  tile_counts.alloc(std::max<uint64_t>(tiles, 1) * 4, h->arena);
-  tile_offs.alloc((tiles + 1) * 8, h->arena);
-  start_cnt.alloc(std::max<uint64_t>(tiles, 1) * kDigestTile, h->arena);
-  const DigestRange whole{0u, h->res_end, 0u, n_prot};
-  uint64_t N = 0;
-  if (tiles) {
-    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
-    launch_digest_count(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                        (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), s,
-                        &win);
-    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
-    N = read_u64(h, tile_offs.as<uint64_t>() + tiles);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2ull * h->res_end + tiles * 16;
+int dbi_query_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
+                      uint64_t n_spectra, int tol_mode, int index_factor, dbi_hit_counts* counts) {
+  DBI_API_BEGIN(h)
+  if (!h->built) {
+    set_error("Indexer is not initialized");
+    return DBI_ENOTINIT;
   }
-  if (int rc = check_err_bits(read_err(h))) return rc;
-  if (n_candidates) *n_candidates = N;
-  h->st.n_emitted = N;
-  if ((max_candidates && N > max_candidates) || N >= (1ull << 32)) {
-    set_error("%llu candidate records exceed the cap of %llu (and 2^32): split the batch", (unsigned long long)N,
-              (unsigned long long)(max_candidates ? max_candidates : (1ull << 32) - 1));
-    resolve_spans(h);
-    return DBI_ERANGE;
-  }
-  DevBuf r_mass, r_gpos, r_prot, r_len;
-  r_mass.alloc(std::max<uint64_t>(N, 1) * 8, h->arena);
-  r_gpos.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
-  r_prot.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
-  r_len.alloc(std::max<uint64_t>(N, 1) * 2, h->arena);
-  if (N) {  // K4u
-    Stage sg(h, DBI_STAGE_DIGEST_EMIT);
-    launch_digest_emit(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                       (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
-                       r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>(),
-                       nullptr, h->d_err.as<uint32_t>(), s, &win);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2ull * h->res_end + N * 18;
-  }
-  tile_counts.release();
-  tile_offs.release();
-  start_cnt.release();
+  if (int rc = check_spectra(mass, tol, range_off, n_spectra, tol_mode, index_factor, counts)) return rc;
+  h->hits.drop();
+  SpectraBatch b;
+  spectra_prepare(h, b, mass, tol, range_off, n_spectra, tol_mode, index_factor, false);
+  if (tol_mode == DBI_TOL_PPM) spectra_probe(h, b);
+  return spectra_answer(h, b, counts);
+  DBI_API_END
+}
 
-  // the candidate index lives for this call only; the pending result does not depend on it
-  struct DropCandidates {
-    dbi_handle* h;
-    ~DropCandidates() {
-      free_tables(h);
-      h->built = false;
-    }
-  } drop_candidates{h};
-  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
-  if (int rc = index_records(h, rv, N, h->p.min_mass, h->p.max_mass)) return rc;
-  if (int rc = check_err_bits(read_err(h))) return rc;
-  r_mass.release(); r_gpos.release(); r_prot.release(); r_len.release();
-  return query_hits_impl(h, d_lo, d_hi, nq, counts);
+int dbi_search_unindexed_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
+                                 uint64_t n_spectra, int tol_mode, int index_factor, uint64_t max_candidates,
+                                 dbi_hit_counts* counts, uint64_t* n_candidates) {
+  DBI_API_BEGIN(h)
+  if (int rc = check_unindexed(h)) return rc;
+  if (int rc = check_spectra(mass, tol, range_off, n_spectra, tol_mode, index_factor, counts)) return rc;
+  drop_results(h);
+  if (n_candidates) *n_candidates = 0;
+  SpectraBatch b;
+  spectra_prepare(h, b, mass, tol, range_off, n_spectra, tol_mode, index_factor, true);
+  // the candidate windows: the merged intervals, or [min(lo, u_0), bound of the probes] of every PPM spectrum
+  const bool da = tol_mode == DBI_TOL_DA;
+  const uint64_t nw = da ? b.n_iv : n_spectra;
+  const double* c_lo = da ? b.iv_lo() : b.win.as<double>() + 2 * n_spectra;
+  const double* c_hi = da ? b.iv_hi() : b.win.as<double>() + 3 * n_spectra;
+  DevBuf io;
+  if (int rc = index_candidates(h, c_lo, c_hi, nw, cudaMemcpyDeviceToDevice, max_candidates, n_candidates, io))
+    return rc;
+  DropCandidates drop_candidates{h};
+  io.release();
+  if (!da) spectra_probe(h, b);
+  return spectra_answer(h, b, counts);
   DBI_API_END
 }
 

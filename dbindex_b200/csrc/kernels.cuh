@@ -238,6 +238,31 @@ void launch_grp_expand(const uint8_t* d_res, const DevTables* d_tb, const Digest
 void launch_query(const double* e_mass, uint64_t n_entries, const double* lo, const double* hi, uint64_t nq,
                   uint64_t* hit_begin, uint64_t* hit_count, uint32_t* cnt32, cudaStream_t s);
 
+// ---- K13/K14 spectra (spectra.cu) --------------------------------------------------
+// K13a: the Dalton range lists of n spectra (spectrum s = ranges [range_off[s], range_off[s+1])) clamped, sorted,
+// merged and checked against the bucket rule (index_factor 0: off); the merged intervals of s in its slots from
+// range_off[s] of o_lo / o_hi, cnt[s] = their number (0: the spectrum is empty).  launch_spec_compact packs them
+// at ioff = exclusive scan of cnt.
+void launch_spec_intervals(const double* mass, const double* tol, const uint64_t* range_off, uint64_t n,
+                           int index_factor, double* o_lo, double* o_hi, uint32_t* cnt, cudaStream_t s);
+void launch_spec_compact(const uint64_t* range_off, const uint64_t* ioff, uint64_t n, const double* s_lo,
+                         const double* s_hi, double* o_lo, double* o_hi, cudaStream_t s);
+// K13b: the window [max(0, m - tol), m + tol] of n PPM spectra; c_lo / c_hi (both NULL or neither): the candidate
+// window of an unindexed search, which also holds every probe the walk can make
+void launch_spec_ppm_window(const double* mass, const double* ppm, uint64_t n, double* w_lo, double* w_hi,
+                            double* c_lo, double* c_hi, cudaStream_t s);
+// K14: the exact-mass probe walk of every PPM spectrum over the sorted entry masses; count pass (window + probes per
+// spectrum), then the intervals at ioff = exclusive scan of the counts
+void launch_spec_probe_count(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
+                             const double* w_lo, const double* w_hi, uint64_t n, int index_factor, uint32_t* cnt,
+                             cudaStream_t s);
+void launch_spec_probe_emit(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
+                            const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* ioff,
+                            double* o_lo, double* o_hi, cudaStream_t s);
+// per-interval hit_off / pep_off (K10) -> per-spectrum: hit_off[s] = iv_hit_off[ioff[s]], s = 0..n
+void launch_spec_collapse(const uint64_t* ioff, uint64_t n, const uint64_t* iv_hit_off, const uint64_t* iv_pep_off,
+                          uint64_t* hit_off, uint64_t* pep_off, cudaStream_t s);
+
 // K10a-c: the hits of a query batch grouped in RUNS (consecutive hits of one query that are variants of
 // one peptide with one mass).  hit_off = exclusive scan of the hit counts; pep_off = runs before every
 // query; what parseAddPeptideInfo materialises

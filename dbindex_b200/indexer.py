@@ -21,7 +21,8 @@ from typing import List, Optional, Sequence, Set, Tuple
 
 import numpy as np
 
-from .capi import DBI_ERANGE, DbiError, DbiHitCounts, DbiParams, GpuIndex, _expand_csr, parse_fasta
+from .capi import (DBI_ERANGE, DBI_TOL_DA, DBI_TOL_PPM, DbiError, DbiHitCounts, DbiParams, GpuIndex, _expand_csr,
+                   parse_fasta)
 
 MAX_INDEX_RESIDUE_LEN = 3      # Constants.java:44
 MAX_PRECURSOR_MASS = 8000      # Constants.java:20
@@ -304,6 +305,48 @@ def search_unindexed_chunked(index: GpuIndex, lo, hi, max_candidates: int) -> di
     return _merge_hits(parts, len(lo))
 
 
+def search_unindexed_spectra_chunked(index: GpuIndex, mass, tol, range_off, tol_mode: int, index_factor: int,
+                                     max_candidates: int) -> dict:
+    """query_hits-style answer (one query per spectrum) of a dbi_search_unindexed_spectra batch on an unbuilt handle,
+    through calls of at most max_candidates candidate records each (0 = one call, no cap).  As in
+    search_unindexed_chunked, the spectra go to the device sorted by mass (a Dalton list by its first range) and a
+    batch over the cap is split into ceil(N_c / cap) + 1 contiguous chunks of that order, again if needed; a
+    spectrum is never split, and the answer comes back in the caller's order."""
+    mass = np.ascontiguousarray(mass, dtype=np.float64)
+    tol = np.ascontiguousarray(tol, dtype=np.float64)
+    if tol_mode == DBI_TOL_PPM:
+        n, key = len(mass), mass
+        lens = np.ones(n, dtype=np.int64)
+        first = np.arange(n, dtype=np.int64)
+    else:
+        ro = np.asarray(range_off, dtype=np.int64)
+        n = len(ro) - 1
+        lens, first = np.diff(ro), ro[:-1]
+        key = np.zeros(n)
+        key[lens > 0] = mass[first[lens > 0]]
+    parts = []
+
+    def run(ids):
+        if tol_mode == DBI_TOL_PPM:
+            args = (mass[ids], tol[ids], None)
+        else:
+            off = np.concatenate(([0], np.cumsum(lens[ids])))
+            rows = np.repeat(first[ids] - off[:-1], lens[ids]) + np.arange(off[-1], dtype=np.int64)
+            args = (mass[rows], tol[rows], off.astype(np.uint64))
+        try:
+            parts.append((ids, index.search_unindexed_spectra(*args, tol_mode=tol_mode, index_factor=index_factor,
+                                                              max_candidates=max_candidates)))
+        except DbiError as e:
+            n_c = e.n_candidates or 0
+            if e.code != DBI_ERANGE or not max_candidates or n_c <= max_candidates or len(ids) < 2:
+                raise
+            for chunk in np.array_split(ids, min(len(ids), -(-n_c // max_candidates) + 1)):
+                run(chunk)
+
+    run(np.argsort(key, kind="stable"))
+    return _merge_hits(parts, n)
+
+
 class DBIndexer:
     """DBIndexer.java: the indexer / orchestrator, GPU store behind it."""
 
@@ -467,15 +510,29 @@ class DBIndexer:
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
 
+    def _spectra_hits(self, mass, tol, range_off, tol_mode: int) -> dict:
+        """The hit source of the spectrum batches: one query per spectrum (dbi_query_spectra, or in unindexed mode
+        the chunked dbi_search_unindexed_spectra), the bucket rule of this index_factor applied on the device."""
+        try:
+            if self.use_index:
+                return self.index.query_spectra(mass, tol, range_off, tol_mode, self.index_factor)
+            return search_unindexed_spectra_chunked(self.index, mass, tol, range_off, tol_mode, self.index_factor,
+                                                    self.max_candidates)
+        except DbiError as e:
+            raise DBIndexStoreException(str(e)) from e
+
     def _materialise(self, lo: np.ndarray, hi: np.ndarray, keep: Optional[np.ndarray] = None) -> List[List[IndexedSequence]]:
-        """getSequences for a batch of ranges in ONE device pass (dbi_query_hits, or dbi_search_unindexed): the
-        objects parseAddPeptideInfo builds (DBIndexStoreSQLiteByteIndexMerge.java:452-462) -- sequence, flanks,
-        mass and protein ids all come back from the GPU; only the Python objects are made here."""
-        h = self._hits(lo, hi)
+        """getSequences for a batch of ranges in ONE device pass (dbi_query_hits, or dbi_search_unindexed)."""
+        return self._sequences(self._hits(lo, hi), len(lo), keep)
+
+    def _sequences(self, h: dict, nq: int, keep: Optional[np.ndarray] = None) -> List[List[IndexedSequence]]:
+        """The objects parseAddPeptideInfo builds (DBIndexStoreSQLiteByteIndexMerge.java:452-462) for every query of
+        a query_hits-style answer -- sequence, flanks, mass and protein ids all come back from the GPU; only the
+        Python objects are made here."""
         ho, so, po = (h[k].astype(np.int64) for k in ("hit_off", "seq_off", "prot_list_off"))
         seq, flanks = h["seq"].tobytes().decode("latin-1"), h["flanks"].tobytes().decode("latin-1")
         out = []
-        for q in range(len(lo)):
+        for q in range(nq):
             if keep is not None and not keep[q]:
                 out.append([])
                 continue
@@ -506,7 +563,24 @@ class DBIndexer:
 
     def getSequencesUsingPPMTolerance(self, precursorMass: float, massToleranceInPPM: float) -> List[IndexedSequence]:
         """DBIndexer.java:787-844: one Dalton query, then exact-mass probes above the upper
-        bound until one comes back empty."""
+        bound until one comes back empty (a batch of one spectrum on one GPU)."""
+        if not self.shards:
+            return self.getSequencesUsingPPMToleranceBatch([precursorMass], massToleranceInPPM)[0]
+        return self._ppm_probe_loop(precursorMass, massToleranceInPPM)
+
+    def getSequencesUsingPPMToleranceBatch(self, masses: Sequence[float], massToleranceInPPM) -> List[List[IndexedSequence]]:
+        """getSequencesUsingPPMTolerance for every mass in one device call (dbi_query_spectra, DBI_TOL_PPM; in
+        unindexed mode dbi_search_unindexed_spectra): the window and the probe walk of every spectrum run on the GPU.
+        massToleranceInPPM: one value, or one per mass.  A sharded proteome asks one mass at a time."""
+        self._require()
+        m = np.ascontiguousarray(masses, dtype=np.float64)
+        ppm = np.ascontiguousarray(np.broadcast_to(np.asarray(massToleranceInPPM, dtype=np.float64), m.shape))
+        if self.shards:
+            return [self._ppm_probe_loop(float(m[i]), float(ppm[i])) for i in range(len(m))]
+        return self._sequences(self._spectra_hits(m, ppm, None, DBI_TOL_PPM), len(m))
+
+    def _ppm_probe_loop(self, precursorMass: float, massToleranceInPPM: float) -> List[IndexedSequence]:
+        """The reference's probe loop on the host, one device call per probe."""
         tol = tolerance_in_dalton(precursorMass, massToleranceInPPM)
         sequences = self.getSequencesUsingDaltonTolerance(precursorMass, tol)
         have = {s.key() for s in sequences}
@@ -530,8 +604,11 @@ class DBIndexer:
         return sequences
 
     def getSequences(self, ranges: Sequence[MassRange]) -> List[IndexedSequence]:
-        """DBIndexer.java:855-871 -> Mult.getSequences(List<MassRange>) (Mult:353-430)."""
+        """DBIndexer.java:855-871 -> Mult.getSequences(List<MassRange>) (Mult:353-430): a batch of one spectrum on
+        one GPU; a sharded proteome merges the intervals here."""
         self._require()
+        if not self.shards:
+            return self.getSequencesForSpectra([ranges])[0]
         if len(ranges) == 1:
             return self.getSequencesUsingDaltonTolerance(ranges[0].precMass, ranges[0].tolerance)
         merged = merge_intervals(ranges)
@@ -546,6 +623,21 @@ class DBIndexer:
         for lst in self._materialise(lo, hi):
             out.extend(lst)
         return out
+
+    def getSequencesForSpectra(self, spectra: Sequence[Sequence[MassRange]]) -> List[List[IndexedSequence]]:
+        """getSequences(List<MassRange>) for every spectrum of a list in one device call (dbi_query_spectra,
+        DBI_TOL_DA; in unindexed mode dbi_search_unindexed_spectra): the intervals of every spectrum are clamped,
+        sorted, merged and checked against the bucket rule on the GPU.  A sharded proteome asks one spectrum at a
+        time."""
+        self._require()
+        if self.shards:
+            return [self.getSequences(list(sp)) for sp in spectra]
+        lists = [list(sp) for sp in spectra]
+        mass = np.array([r.precMass for sp in lists for r in sp], dtype=np.float64)
+        tol = np.array([r.tolerance for sp in lists for r in sp], dtype=np.float64)
+        range_off = np.zeros(len(lists) + 1, dtype=np.uint64)
+        np.cumsum([len(sp) for sp in lists], out=range_off[1:])
+        return self._sequences(self._spectra_hits(mass, tol, range_off, DBI_TOL_DA), len(lists))
 
     def _protein(self, pid: int) -> IndexedProtein:
         return IndexedProtein(self.deflines[pid] if pid < len(self.deflines) else "", pid)
@@ -651,6 +743,10 @@ class DBIndexImpl:
         if len(args) == 2:
             return self.indexer.getSequencesUsingDaltonTolerance(float(args[0]), float(args[1]))
         return self.indexer.getSequences(list(args[0]))
+
+    def getSequencesForSpectra(self, spectra) -> List[List[IndexedSequence]]:
+        """getSequences(List<MassRange>) for a list of spectra, one device call (DBIndexer.getSequencesForSpectra)."""
+        return self.indexer.getSequencesForSpectra(spectra)
 
     def getProteins(self, seq):
         """getProteins(String) (DBIndexImpl.java:222-237, memoised), getProteins(IndexedSequence) (:208), or for a

@@ -311,6 +311,37 @@ int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out);
 int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, uint64_t max_candidates,
                          dbi_hit_counts* counts, uint64_t* n_candidates);
 
+/* A batch of spectra, each answered as the reference answers one spectrum's precursor query, in one call.
+ *   DBI_TOL_DA:  spectrum s is the ranges [range_off[s], range_off[s+1]) of (mass, tol in Da), answered as
+ *                DBIndexer.getSequences(List<MassRange>) (DBIndexer.java:855-871, Mult:353-430): lo = max(0, m - t),
+ *                hi = m + t, stable sort by lo, merge while end >= next start (end = max), and an empty answer when
+ *                a merged interval fails the bucket rule; otherwise the hits of every merged interval in order.
+ *                No ranges: empty.  One range: the same rules (= getSequences(mass, tol)).
+ *   DBI_TOL_PPM: spectrum s is mass[s] at tol[s] ppm (range_off must be NULL), answered as
+ *                DBIndexer.getSequencesUsingPPMTolerance (DBIndexer.java:787-844): the window of
+ *                tol = m (1 - 1 / (ppm / 1e6 + 1)), then the hits of the exact-mass probes u_0 = m + tol,
+ *                u_{k+1} = u_k + 1e-6 while u_k - tol(u_k) < m and u_{k+1} != u_k, up to the first empty probe,
+ *                except those the window already holds.
+ * The bucket rule (DBIndexStoreSQLiteMult, Mult:55-56,333-338) empties a query whose bound b has
+ * (int)b / (8000 / index_factor) > index_factor - 1; index_factor 0 turns it off (1..8000 otherwise).
+ * Every double is computed as the host computes it.  Non-finite mass or tol, a decreasing range_off,
+ * range_off != NULL with DBI_TOL_PPM, or another tol_mode: DBI_EINVAL, the message naming the spectrum.
+ *
+ * The result is the handle's pending hit result with one query per spectrum: counts->nq = n_spectra, hit_off and
+ * pep_off per spectrum (no run straddles two spectra), read with dbi_query_hits_read; the < 2^32 hits rule applies.
+ * dbi_query_spectra needs a built handle (DBI_ENOTINIT).  dbi_search_unindexed_spectra is dbi_search_unindexed
+ * for spectra: same handle rules, candidate cap, *n_candidates, DBI_ERANGE without a pending result and stats; its
+ * candidate windows are the merged intervals, or per PPM spectrum its window up to a bound of every probe the walk
+ * can make, so every answer equals dbi_query_spectra on the built index.  An index sharded over several GPUs and
+ * the sharded unindexed search are not covered: ask those one spectrum at a time. */
+#define DBI_TOL_DA 0
+#define DBI_TOL_PPM 1
+int dbi_query_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
+                      uint64_t n_spectra, int tol_mode, int index_factor, dbi_hit_counts* counts);
+int dbi_search_unindexed_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
+                                 uint64_t n_spectra, int tol_mode, int index_factor, uint64_t max_candidates,
+                                 dbi_hit_counts* counts, uint64_t* n_candidates);
+
 /* Batched DBIndexer.getProteins(String) (DBIndexer.java:925-947, DBIndexImpl.java:222-237): which index entry,
  * and so which proteins, every peptide of a list is.  Peptide i is residues[offsets[i], offsets[i+1]) (the packed
  * layout of dbi_add_proteins; offsets non-decreasing) with mod pattern modpat[i] in the index's own encoding

@@ -99,6 +99,14 @@ public final class DbiNative {
 	static final MethodHandle dbi_search_unindexed = h("dbi_search_unindexed",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS));
 	// batched getProteins(String): which entry (and so which proteins) every peptide of a list is
+	// a batch of spectra (Dalton range lists or PPM masses) answered as getSequences(List<MassRange>) /
+	// getSequencesUsingPPMTolerance answer one; read with dbi_query_hits_read, one query per spectrum
+	static final int DBI_TOL_DA = 0, DBI_TOL_PPM = 1;
+	static final MethodHandle dbi_query_spectra = h("dbi_query_spectra",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, ADDRESS));
+	static final MethodHandle dbi_search_unindexed_spectra = h("dbi_search_unindexed_spectra",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, JAVA_LONG,
+					ADDRESS, ADDRESS));
 	static final MethodHandle dbi_lookup_peptides = h("dbi_lookup_peptides",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
 	static final MethodHandle dbi_lookup_peptides_read = h("dbi_lookup_peptides_read",

@@ -81,6 +81,14 @@ public class GpuDBIndexImpl extends DBIndexImpl {
 		return super.getProteins(seq);
 	}
 
+	/**
+	 * getSequences(List<MassRange>) for every spectrum of a run in one device call. Not an overload of
+	 * getSequences(List): both would erase to the same signature.
+	 */
+	public List<List<IndexedSequence>> getSequencesForSpectra(List<List<MassRange>> spectra) throws DBIndexStoreException {
+		return ((GpuDBIndexer) indexer).getSequencesForSpectra(spectra);
+	}
+
 	/** getProteins(String) for a whole collection (e.g. every distinct identified peptide) in one device call. */
 	public Map<String, Set<IndexedProtein>> getProteins(Collection<String> seqs) throws DBIndexStoreException {
 		return ((GpuDBIndexer) indexer).getProteins(seqs);

@@ -353,6 +353,95 @@ public class GpuDBIndexStore implements DBIndexStore {
 		}
 	}
 
+	/**
+	 * A batch of spectra in one device call per chunk: tolMode DBI_TOL_DA, spectrum s = the ranges
+	 * [rangeOff[s], rangeOff[s+1]) of (mass, tol in Da), answered as getSequences(List<MassRange>); DBI_TOL_PPM
+	 * (rangeOff null), mass[s] at tol[s] ppm, answered as DBIndexer.getSequencesUsingPPMTolerance. The bucket rule
+	 * of sparam.getIndexFactor() is applied on the device (dbi_query_spectra; SEARCH_UNINDEXED:
+	 * dbi_search_unindexed_spectra, spectra sorted by mass and split into chunks like searchUnindexed, never inside
+	 * a spectrum). Not available with -Ddbindex.gpu.devices=N > 1: the callers ask one spectrum at a time there.
+	 */
+	public List<List<IndexedSequence>> querySpectra(double[] mass, double[] tol, long[] rangeOff, int tolMode)
+			throws DBIndexStoreException {
+		requireInit();
+		if (nDevices > 1)
+			throw new DBIndexStoreException("spectrum batches run on one GPU");
+		final int n = rangeOff == null ? mass.length : rangeOff.length - 1;
+		final List<List<IndexedSequence>> ret = new ArrayList<>();
+		for (int i = 0; i < n; ++i)
+			ret.add(new ArrayList<>());
+		final RunSink sink = (q, pep, resLeft, resRight, m, off, pids, patterns) -> {
+			for (final int mp : patterns)
+				ret.get(q).add(sequence(pep, resLeft, resRight, m, off, pids, mp));
+		};
+		final Integer[] order = new Integer[n];
+		for (int i = 0; i < n; ++i)
+			order[i] = i;
+		if (unindexed) { // by mass (a range list by its first range), as searchUnindexed sorts its ranges
+			final double[] key = new double[n];
+			for (int i = 0; i < n; ++i)
+				key[i] = rangeOff == null ? mass[i] : rangeOff[i + 1] > rangeOff[i] ? mass[(int) rangeOff[i]] : 0;
+			java.util.Arrays.sort(order, (x, y) -> Double.compare(key[x], key[y]));
+		}
+		final int[] ids = new int[n];
+		for (int i = 0; i < n; ++i)
+			ids[i] = order[i];
+		spectraChunk(mass, tol, rangeOff, tolMode, ids, sink);
+		return ret;
+	}
+
+	private void spectraChunk(double[] mass, double[] tol, long[] rangeOff, int tolMode, int[] ids, RunSink sink)
+			throws DBIndexStoreException {
+		try (Arena a = Arena.ofConfined()) {
+			final int n = ids.length;
+			long nr = 0;
+			for (final int i : ids)
+				nr += rangeOff == null ? 1 : rangeOff[i + 1] - rangeOff[i];
+			final MemorySegment dm = a.allocate(JAVA_DOUBLE, Math.max(1, nr)), dt = a.allocate(JAVA_DOUBLE, Math.max(1, nr));
+			final MemorySegment dro = rangeOff == null ? MemorySegment.NULL : a.allocate(JAVA_LONG, n + 1);
+			long r = 0;
+			for (int k = 0; k < n; ++k) {
+				final long r0 = rangeOff == null ? ids[k] : rangeOff[ids[k]];
+				final long r1 = rangeOff == null ? ids[k] + 1 : rangeOff[ids[k] + 1];
+				if (rangeOff != null)
+					dro.setAtIndex(JAVA_LONG, k, r);
+				for (long j = r0; j < r1; ++j, ++r) {
+					dm.setAtIndex(JAVA_DOUBLE, r, mass[(int) j]);
+					dt.setAtIndex(JAVA_DOUBLE, r, tol[(int) j]);
+				}
+			}
+			if (rangeOff != null)
+				dro.setAtIndex(JAVA_LONG, n, r);
+			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS), nCand = a.allocate(JAVA_LONG);
+			final int factor = sparam.getIndexFactor();
+			if (!unindexed) {
+				check((int) DbiNative.dbi_query_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode, factor, cnt));
+			} else {
+				final int rc = (int) DbiNative.dbi_search_unindexed_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode,
+						factor, maxCandidates, cnt, nCand);
+				final long nc = nCand.get(JAVA_LONG, 0);
+				if (rc == DbiNative.DBI_ERANGE && nc > maxCandidates && n > 1) {
+					final int chunks = (int) Math.min(n, (nc + maxCandidates - 1) / maxCandidates + 1);
+					for (int c = 0; c < chunks; ++c)
+						spectraChunk(mass, tol, rangeOff, tolMode, java.util.Arrays.copyOfRange(ids,
+								(int) ((long) n * c / chunks), (int) ((long) n * (c + 1) / chunks)), sink);
+					return;
+				}
+				check(rc);
+			}
+			readHits(handle, a, cnt, ids, sink);
+		} catch (final DBIndexStoreException e) {
+			throw e;
+		} catch (final Throwable t) {
+			throw new DBIndexStoreException("Error getting peptides ", t);
+		}
+	}
+
+	/** with -Ddbindex.gpu.devices=N > 1 the spectrum batches are not available (one spectrum at a time) */
+	public boolean supportsSpectrumBatches() {
+		return nDevices == 1;
+	}
+
 	/** IndexedSequence as parseAddPeptideInfo builds it (Merge:452-462), the mod pattern as a mod sequence */
 	private static IndexedSequence sequence(String pep, String resLeft, String resRight, double mass, int off,
 			List<Integer> pids, int modPattern) {

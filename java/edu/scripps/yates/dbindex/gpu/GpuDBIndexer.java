@@ -13,6 +13,8 @@ import edu.scripps.yates.dbindex.DBIndexer;
 import edu.scripps.yates.utilities.fasta.dbindex.DBIndexSearchParams;
 import edu.scripps.yates.utilities.fasta.dbindex.DBIndexStoreException;
 import edu.scripps.yates.utilities.fasta.dbindex.IndexedProtein;
+import edu.scripps.yates.utilities.fasta.dbindex.IndexedSequence;
+import edu.scripps.yates.utilities.fasta.dbindex.MassRange;
 
 /**
  * DBIndexer with the digestion moved to the GPU: run() still streams the FASTA and fills the
@@ -34,6 +36,55 @@ public class GpuDBIndexer extends DBIndexer {
 		} catch (final DBIndexStoreException e) {
 			throw new IOException(e);
 		}
+	}
+
+	/**
+	 * getSequencesUsingPPMTolerance (DBIndexer.java:787-844) as a batch of one: the window and the exact-mass
+	 * probe walk run on the GPU in one call. With -Ddbindex.gpu.devices=N > 1: the reference's loop.
+	 */
+	@Override
+	public List<IndexedSequence> getSequencesUsingPPMTolerance(double precursorMass, double massToleranceInPPM)
+			throws DBIndexStoreException {
+		if (!((GpuDBIndexStore) indexStore).supportsSpectrumBatches())
+			return super.getSequencesUsingPPMTolerance(precursorMass, massToleranceInPPM);
+		return getSequencesUsingPPMTolerance(new double[] { precursorMass }, massToleranceInPPM).get(0);
+	}
+
+	/** getSequencesUsingPPMTolerance for every mass, one device call (dbi_query_spectra, DBI_TOL_PPM). */
+	public List<List<IndexedSequence>> getSequencesUsingPPMTolerance(double[] masses, double massToleranceInPPM)
+			throws DBIndexStoreException {
+		final GpuDBIndexStore store = (GpuDBIndexStore) indexStore;
+		if (!store.supportsSpectrumBatches()) {
+			final List<List<IndexedSequence>> ret = new ArrayList<>();
+			for (final double m : masses)
+				ret.add(super.getSequencesUsingPPMTolerance(m, massToleranceInPPM));
+			return ret;
+		}
+		final double[] ppm = new double[masses.length];
+		java.util.Arrays.fill(ppm, massToleranceInPPM);
+		return store.querySpectra(masses, ppm, null, DbiNative.DBI_TOL_PPM);
+	}
+
+	/** getSequences(List<MassRange>) for every spectrum, one device call (dbi_query_spectra, DBI_TOL_DA). */
+	public List<List<IndexedSequence>> getSequencesForSpectra(List<List<MassRange>> spectra) throws DBIndexStoreException {
+		final GpuDBIndexStore store = (GpuDBIndexStore) indexStore;
+		if (!store.supportsSpectrumBatches()) {
+			final List<List<IndexedSequence>> ret = new ArrayList<>();
+			for (final List<MassRange> sp : spectra)
+				ret.add(getSequences(sp));
+			return ret;
+		}
+		final long[] rangeOff = new long[spectra.size() + 1];
+		for (int s = 0; s < spectra.size(); ++s)
+			rangeOff[s + 1] = rangeOff[s] + spectra.get(s).size();
+		final double[] mass = new double[(int) rangeOff[spectra.size()]], tol = new double[mass.length];
+		int r = 0;
+		for (final List<MassRange> sp : spectra)
+			for (final MassRange m : sp) {
+				mass[r] = m.getPrecMass();
+				tol[r++] = m.getTolerance();
+			}
+		return store.querySpectra(mass, tol, rangeOff, DbiNative.DBI_TOL_DA);
 	}
 
 	/** getProteins(String) (DBIndexer.java:925-947) through the batched device lookup (dbi_lookup_peptides). */
