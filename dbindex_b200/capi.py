@@ -251,6 +251,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "dbi_query_spectra": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_int, C.c_int, C.POINTER(DbiHitCounts)]),
         "dbi_search_unindexed_spectra": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_int, C.c_int, C.c_uint64,
                                                    C.POINTER(DbiHitCounts), u64p]),
+        "dbi_mg_spectra_stops": (C.c_int, [vp, vp, vp, C.c_uint64, C.c_int, vp, C.c_int, C.c_int, C.c_int, vp]),
+        "dbi_mg_query_spectra": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.c_int, C.c_int, vp,
+                                           C.POINTER(DbiHitCounts)]),
         "dbi_lookup_peptides": (C.c_int, [vp, vp, vp, vp, C.c_uint64, C.POINTER(DbiLookupCounts)]),
         "dbi_lookup_peptides_read": (C.c_int, [vp, C.POINTER(DbiLookupBuffers)]),
         "dbi_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(vp)]),
@@ -302,7 +305,8 @@ ABI_SYMBOLS = [
     "dbi_mg_side_classes", "dbi_mg_pull_proteome", "dbi_mg_digest", "dbi_mg_hist", "dbi_mg_plan", "dbi_mg_default_cost", "dbi_mg_count", "dbi_mg_scatter",
     "dbi_mg_index_base", "dbi_mg_unique_count", "dbi_mg_set_unique", "dbi_mg_groups", "dbi_mg_index_variants",
     "dbi_mg_finish", "dbi_mg_split_masses", "dbi_mg_slices", "dbi_mg_plan_matrix", "dbi_mg_build_local",
-    "dbi_mg_search_unindexed_local",
+    "dbi_mg_search_unindexed_local", "dbi_mg_spectra_stops", "dbi_mg_query_spectra", "dbi_mg_query_spectra_local",
+    "dbi_mg_search_unindexed_spectra_local",
 ]
 
 
@@ -570,6 +574,28 @@ class GpuIndex:
         self.last_candidates = n_cand.value
         if rc != 0:
             raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
+        return self._read_hits(cnt, fields, alloc, per_hit)
+
+    def mg_spectra_stops(self, mass, ppm, split_mass, rank: int, world: int, index_factor: int = 0) -> np.ndarray:
+        """dbi_mg_spectra_stops: K_r of every PPM spectrum (mass[s] at ppm[s]) on this built handle as rank `rank` of
+        `world` under the cuts split_mass (world or 2 * world slices): the probe at which this rank's share of the
+        walk ends, UINT64_MAX where it cannot end here.  The walk ends at the minimum over the ranks."""
+        mass, ppm, _, n = spectra_arrays(mass, ppm, None, DBI_TOL_PPM)
+        split = np.ascontiguousarray(split_mass, dtype=np.float64)
+        stop = np.zeros(n, dtype=np.uint64)
+        self._check(self.lib.dbi_mg_spectra_stops(self._h, _ptr(mass), _ptr(ppm), n, int(index_factor), _ptr(split),
+                                                  len(split) + 1, int(rank), int(world), _ptr(stop)))
+        return stop
+
+    def mg_query_spectra(self, mass, tol, range_off=None, tol_mode: int = DBI_TOL_DA, index_factor: int = 0,
+                         stop=None, fields=None, alloc=None, per_hit: bool = True) -> dict:
+        """dbi_mg_query_spectra + dbi_query_hits_read: this rank's share of query_spectra on a sharded index;
+        DBI_TOL_PPM needs `stop`, the minimum over the ranks of mg_spectra_stops."""
+        mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
+        stop = None if stop is None else np.ascontiguousarray(stop, dtype=np.uint64)
+        cnt = DbiHitCounts()
+        self._check(self.lib.dbi_mg_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
+                                                  int(index_factor), _ptr(stop), C.byref(cnt)))
         return self._read_hits(cnt, fields, alloc, per_hit)
 
     def _read_hits(self, cnt: DbiHitCounts, fields, alloc, per_hit: bool) -> dict:

@@ -1863,20 +1863,45 @@ void spectra_prepare(dbi_handle* h, SpectraBatch& b, const double* mass, const d
   }
 }
 
-// K14: the window and the continuing probes of every PPM spectrum, over the handle's (or candidate) index
-void spectra_probe(dbi_handle* h, SpectraBatch& b) {
+// K14: the window and the continuing probes of every PPM spectrum, over the handle's (or candidate) index.
+// d_stop (device, n u64): the walks of a sharded index end at the given probes (the minimum of K14s over the ranks).
+void spectra_probe(dbi_handle* h, SpectraBatch& b, const uint64_t* d_stop = nullptr) {
   cudaStream_t s = h->stream;
   Stage sg(h, DBI_STAGE_QUERY);
   const double* w_lo = b.win.as<double>();
   const double* w_hi = w_lo + b.n;
-  launch_spec_probe_count(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor,
+  launch_spec_probe_count(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
                           b.cnt.as<uint32_t>(), s);
   spectra_offsets(h, b);
-  launch_spec_probe_emit(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor,
+  launch_spec_probe_emit(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
                          b.ioff.as<uint64_t>(), b.iv.as<double>(), b.iv.as<double>() + b.n_iv, s);
-  // both passes: (mass, ppm, window) read, one lower bound per probe (~1 per spectrum); count, offsets, interval
-  const uint64_t probe = 32 + 8ull * (uint64_t)bit_length(h->n_entries);
+  // both passes: (mass, ppm, window) read, one lower bound (or one stop) per spectrum; count, offsets, interval
+  const uint64_t probe = d_stop ? 8 : 32 + 8ull * (uint64_t)bit_length(h->n_entries);
   h->st.algo_bytes[DBI_STAGE_QUERY] += 2 * b.n * (32 + probe) + b.n * (4 + 8) + b.n_iv * 16;
+}
+
+// K14s on the handle's entries for the PPM batch b (K13b done): stop[s] = K_r of this rank, copied to the host
+void spectra_stops(dbi_handle* h, SpectraBatch& b, const SliceCuts& cuts, uint64_t* stop) {
+  cudaStream_t s = h->stream;
+  if (!b.n) return;
+  DevBuf d_stop;
+  d_stop.alloc(b.n * 8, h->arena);
+  {
+    Stage sg(h, DBI_STAGE_QUERY);
+    launch_spec_stops(h->entry_mass(), h->n_entries, b.mass(), b.tol(), b.win.as<double>() + b.n, b.n, b.factor, cuts,
+                      d_stop.as<uint64_t>(), s);
+    h->st.algo_bytes[DBI_STAGE_QUERY] += b.n * (24 + 32 + 8ull * (uint64_t)bit_length(h->n_entries) + 8);
+  }
+  DBI_CUDA(cudaMemcpyAsync(stop, d_stop.p, b.n * 8, cudaMemcpyDeviceToHost, s));
+  DBI_CUDA(cudaStreamSynchronize(s));
+}
+
+// spectra_probe with the host stops of every PPM spectrum
+void spectra_probe_stops(dbi_handle* h, SpectraBatch& b, const uint64_t* stop) {
+  DevBuf d_stop;
+  d_stop.alloc(std::max<uint64_t>(b.n, 1) * 8, h->arena);
+  if (b.n) DBI_CUDA(cudaMemcpyAsync(d_stop.p, stop, b.n * 8, cudaMemcpyHostToDevice, h->stream));
+  spectra_probe(h, b, d_stop.as<uint64_t>());
 }
 
 // K9 / K10 over the intervals, then the per-interval offsets of the pending result collapsed to per-spectrum ones

@@ -252,13 +252,25 @@ void launch_spec_compact(const uint64_t* range_off, const uint64_t* ioff, uint64
 void launch_spec_ppm_window(const double* mass, const double* ppm, uint64_t n, double* w_lo, double* w_hi,
                             double* c_lo, double* c_hi, cudaStream_t s);
 // K14: the exact-mass probe walk of every PPM spectrum over the sorted entry masses; count pass (window + probes per
-// spectrum), then the intervals at ioff = exclusive scan of the counts
+// spectrum), then the intervals at ioff = exclusive scan of the counts.  stop != NULL (a sharded index): the walk of
+// spectrum s ends at probe stop[s] (K14s, minimum over the ranks) instead of at the first probe without an entry.
 void launch_spec_probe_count(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
-                             const double* w_lo, const double* w_hi, uint64_t n, int index_factor, uint32_t* cnt,
-                             cudaStream_t s);
+                             const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* stop,
+                             uint32_t* cnt, cudaStream_t s);
 void launch_spec_probe_emit(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
-                            const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* ioff,
-                            double* o_lo, double* o_hi, cudaStream_t s);
+                            const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* stop,
+                            const uint64_t* ioff, double* o_lo, double* o_hi, cudaStream_t s);
+// The mass slices of a sharded index as one rank sees them: slice x = [cut[x-1], cut[x]) (cut[-1] = -inf,
+// cut[n_slices-1] = +inf); bit x of `mine` is set when the rank owns slice x.  Passed by value (~260 bytes).
+struct SliceCuts {
+  double cut[2 * kMaxRanks - 1];
+  int n_slices;
+  uint32_t mine;
+};
+// K14s: stop[s] = the probe at which this rank's share of spectrum s's walk ends (UINT64_MAX: not on this rank)
+void launch_spec_stops(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
+                       const double* w_hi, uint64_t n, int index_factor, const SliceCuts& cuts, uint64_t* stop,
+                       cudaStream_t s);
 // per-interval hit_off / pep_off (K10) -> per-spectrum: hit_off[s] = iv_hit_off[ioff[s]], s = 0..n
 void launch_spec_collapse(const uint64_t* ioff, uint64_t n, const uint64_t* iv_hit_off, const uint64_t* iv_pep_off,
                           uint64_t* hit_off, uint64_t* pep_off, cudaStream_t s);

@@ -193,15 +193,18 @@ __device__ __forceinline__ uint64_t lower_bound_d(const double* __restrict__ a, 
 // fails the bucket rule or when no entry has mass u_k.  The spectrum's intervals: its window unless that fails the
 // bucket rule, then every continuing probe with k >= 1, and u_0 too when the window does not already hold it
 // (inverted or dropped; the reference appends only hits it has not seen).  Count pass (o_lo == nullptr): cnt[s];
-// emit pass: the intervals at ioff[s].
+// emit pass: the intervals at ioff[s].  kGivenStops (a sharded index, whose probes are spread over the ranks): the
+// walk ends at probe stop[s] (K14s, reduced over the ranks) in place of the search for an entry of mass u_k.
+template <bool kGivenStops>
 __global__ void __launch_bounds__(SP_THREADS)
     spec_probe_kernel(const double* __restrict__ e_mass, uint64_t n_entries, const double* __restrict__ mass,
                       const double* __restrict__ ppm, const double* __restrict__ w_lo, const double* __restrict__ w_hi,
                       uint64_t n, int index_factor, uint32_t* __restrict__ cnt, const uint64_t* __restrict__ ioff,
-                      double* __restrict__ o_lo, double* __restrict__ o_hi) {
+                      double* __restrict__ o_lo, double* __restrict__ o_hi, const uint64_t* __restrict__ stop) {
   const uint64_t s = (uint64_t)blockIdx.x * SP_THREADS + threadIdx.x;
   if (s >= n) return;
   const double m = mass[s], p = ppm[s], lo = w_lo[s], hi = w_hi[s];
+  const uint64_t k_end = kGivenStops ? stop[s] : 0;
   const bool window = !out_of_buckets(lo, index_factor) && !out_of_buckets(hi, index_factor);
   const uint64_t o = o_lo ? ioff[s] : 0;
   uint32_t c = 0;
@@ -217,8 +220,12 @@ __global__ void __launch_bounds__(SP_THREADS)
   for (uint64_t k = 0;; ++k) {
     if (!(__dsub_rn(u, tol_in_dalton(u, p)) < m)) break;
     if (u < 0.0 || out_of_buckets(u, index_factor)) break;
-    const uint64_t b = lower_bound_d(e_mass, n_entries, u);
-    if (b >= n_entries || e_mass[b] != u) break;
+    if constexpr (kGivenStops) {
+      if (k >= k_end) break;
+    } else {
+      const uint64_t b = lower_bound_d(e_mass, n_entries, u);
+      if (b >= n_entries || e_mass[b] != u) break;
+    }
     if (k > 0 || probe0) {
       if (o_lo) {
         o_lo[o + c] = u;
@@ -231,6 +238,49 @@ __global__ void __launch_bounds__(SP_THREADS)
     u = nu;
   }
   if (!o_lo) cnt[s] = c;
+}
+
+// K14s: one thread per PPM spectrum: K_r, where this rank's share of the probe walk of K14 ends when the entries
+// are spread over the ranks by mass (slice of u = number of cuts <= u, owner(slice) holds every entry of mass u).
+// It ends on the walk's own end conditions, which every rank evaluates alike, and at a probe it owns whose mass
+// none of its entries has; a probe it does not own it steps over without a search.  The walk's end is the minimum
+// of K_r over the ranks.  Once no slice of this rank meets [u_k, bound] (bound = m (1 + p) (1 + 2^-40) >= every
+// probe the guard admits, as K13b computes it) the rank cannot end the walk: stop[s] = UINT64_MAX.
+__global__ void __launch_bounds__(SP_THREADS)
+    spec_stop_kernel(const double* __restrict__ e_mass, uint64_t n_entries, const double* __restrict__ mass,
+                     const double* __restrict__ ppm, const double* __restrict__ w_hi, uint64_t n, int index_factor,
+                     const SliceCuts cuts, uint64_t* __restrict__ stop) {
+  const uint64_t s = (uint64_t)blockIdx.x * SP_THREADS + threadIdx.x;
+  if (s >= n) return;
+  const double m = mass[s], p = ppm[s];
+  const double p1 = __dadd_rn(__ddiv_rn(p, 1e6), 1.0);
+  const double bound = m > 0.0 && p1 > 0.0 ? __dmul_rn(__dmul_rn(m, p1), 1.0 + 0x1p-40) : CUDART_INF;
+  double u = w_hi[s];
+  uint64_t k = 0;
+  for (;; ++k) {
+    if (!(__dsub_rn(u, tol_in_dalton(u, p)) < m)) break;
+    if (u < 0.0 || out_of_buckets(u, index_factor)) break;
+    uint32_t sl = 0;
+    for (int x = 0; x + 1 < cuts.n_slices; ++x) sl += cuts.cut[x] <= u ? 1u : 0u;
+    if ((cuts.mine >> sl) & 1u) {
+      const uint64_t b = lower_bound_d(e_mass, n_entries, u);
+      if (b >= n_entries || e_mass[b] != u) break;
+    } else {
+      // the next slice of this rank above u is slice sl + ffs(above); it starts at cut[sl + ffs(above) - 1]
+      const uint32_t above = sl + 1 < 32 ? cuts.mine >> (sl + 1) : 0u;
+      if (!above || cuts.cut[sl + __ffs(above) - 1] > bound) {
+        k = UINT64_MAX;
+        break;
+      }
+    }
+    const double nu = __dadd_rn(u, kPrecision);
+    if (nu == u) {
+      ++k;
+      break;
+    }
+    u = nu;
+  }
+  stop[s] = k;
 }
 
 // per-interval hit / run offsets (n_iv + 1) -> per-spectrum ones (n + 1): the value at the spectrum's first interval
@@ -270,19 +320,36 @@ void launch_spec_ppm_window(const double* mass, const double* ppm, uint64_t n, d
 }
 
 void launch_spec_probe_count(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
-                             const double* w_lo, const double* w_hi, uint64_t n, int index_factor, uint32_t* cnt,
-                             cudaStream_t s) {
+                             const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* stop,
+                             uint32_t* cnt, cudaStream_t s) {
   if (n == 0) return;
-  DBI_LAUNCH(spec_probe_kernel, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi, n,
-             index_factor, cnt, (const uint64_t*)nullptr, (double*)nullptr, (double*)nullptr);
+  if (stop)
+    DBI_LAUNCH(spec_probe_kernel<true>, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi,
+               n, index_factor, cnt, (const uint64_t*)nullptr, (double*)nullptr, (double*)nullptr, stop);
+  else
+    DBI_LAUNCH(spec_probe_kernel<false>, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi,
+               n, index_factor, cnt, (const uint64_t*)nullptr, (double*)nullptr, (double*)nullptr,
+               (const uint64_t*)nullptr);
 }
 
 void launch_spec_probe_emit(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
-                            const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* ioff,
-                            double* o_lo, double* o_hi, cudaStream_t s) {
+                            const double* w_lo, const double* w_hi, uint64_t n, int index_factor, const uint64_t* stop,
+                            const uint64_t* ioff, double* o_lo, double* o_hi, cudaStream_t s) {
   if (n == 0) return;
-  DBI_LAUNCH(spec_probe_kernel, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi, n,
-             index_factor, (uint32_t*)nullptr, ioff, o_lo, o_hi);
+  if (stop)
+    DBI_LAUNCH(spec_probe_kernel<true>, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi,
+               n, index_factor, (uint32_t*)nullptr, ioff, o_lo, o_hi, stop);
+  else
+    DBI_LAUNCH(spec_probe_kernel<false>, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_lo, w_hi,
+               n, index_factor, (uint32_t*)nullptr, ioff, o_lo, o_hi, (const uint64_t*)nullptr);
+}
+
+void launch_spec_stops(const double* e_mass, uint64_t n_entries, const double* mass, const double* ppm,
+                       const double* w_hi, uint64_t n, int index_factor, const SliceCuts& cuts, uint64_t* stop,
+                       cudaStream_t s) {
+  if (n == 0) return;
+  DBI_LAUNCH(spec_stop_kernel, grid_threads(n), SP_THREADS, 0, s, e_mass, n_entries, mass, ppm, w_hi, n, index_factor,
+             cuts, stop);
 }
 
 void launch_spec_collapse(const uint64_t* ioff, uint64_t n, const uint64_t* iv_hit_off, const uint64_t* iv_pep_off,

@@ -516,7 +516,7 @@ class DBIndexer:
         try:
             if self.use_index:
                 return self.index.query_spectra(mass, tol, range_off, tol_mode, self.index_factor)
-            return search_unindexed_spectra_chunked(self.index, mass, tol, range_off, tol_mode, self.index_factor,
+            return search_unindexed_spectra_chunked(self._searcher, mass, tol, range_off, tol_mode, self.index_factor,
                                                     self.max_candidates)
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
@@ -563,24 +563,21 @@ class DBIndexer:
 
     def getSequencesUsingPPMTolerance(self, precursorMass: float, massToleranceInPPM: float) -> List[IndexedSequence]:
         """DBIndexer.java:787-844: one Dalton query, then exact-mass probes above the upper
-        bound until one comes back empty (a batch of one spectrum on one GPU)."""
-        if not self.shards:
-            return self.getSequencesUsingPPMToleranceBatch([precursorMass], massToleranceInPPM)[0]
-        return self._ppm_probe_loop(precursorMass, massToleranceInPPM)
+        bound until one comes back empty (a batch of one spectrum)."""
+        return self.getSequencesUsingPPMToleranceBatch([precursorMass], massToleranceInPPM)[0]
 
     def getSequencesUsingPPMToleranceBatch(self, masses: Sequence[float], massToleranceInPPM) -> List[List[IndexedSequence]]:
         """getSequencesUsingPPMTolerance for every mass in one device call (dbi_query_spectra, DBI_TOL_PPM; in
         unindexed mode dbi_search_unindexed_spectra): the window and the probe walk of every spectrum run on the GPU.
-        massToleranceInPPM: one value, or one per mass.  A sharded proteome asks one mass at a time."""
+        massToleranceInPPM: one value, or one per mass.  A sharded proteome runs the walk over its ranks
+        (dbi_mg_search_unindexed_spectra_local)."""
         self._require()
         m = np.ascontiguousarray(masses, dtype=np.float64)
         ppm = np.ascontiguousarray(np.broadcast_to(np.asarray(massToleranceInPPM, dtype=np.float64), m.shape))
-        if self.shards:
-            return [self._ppm_probe_loop(float(m[i]), float(ppm[i])) for i in range(len(m))]
         return self._sequences(self._spectra_hits(m, ppm, None, DBI_TOL_PPM), len(m))
 
     def _ppm_probe_loop(self, precursorMass: float, massToleranceInPPM: float) -> List[IndexedSequence]:
-        """The reference's probe loop on the host, one device call per probe."""
+        """The reference's probe loop on the host, one device call per probe (kept as the reference of the batch)."""
         tol = tolerance_in_dalton(precursorMass, massToleranceInPPM)
         sequences = self.getSequencesUsingDaltonTolerance(precursorMass, tol)
         have = {s.key() for s in sequences}
@@ -604,34 +601,15 @@ class DBIndexer:
         return sequences
 
     def getSequences(self, ranges: Sequence[MassRange]) -> List[IndexedSequence]:
-        """DBIndexer.java:855-871 -> Mult.getSequences(List<MassRange>) (Mult:353-430): a batch of one spectrum on
-        one GPU; a sharded proteome merges the intervals here."""
+        """DBIndexer.java:855-871 -> Mult.getSequences(List<MassRange>) (Mult:353-430): a batch of one spectrum."""
         self._require()
-        if not self.shards:
-            return self.getSequencesForSpectra([ranges])[0]
-        if len(ranges) == 1:
-            return self.getSequencesUsingDaltonTolerance(ranges[0].precMass, ranges[0].tolerance)
-        merged = merge_intervals(ranges)
-        for lo, hi in merged:  # "Cannot query, unsupported precursor mass" -> empty list (Mult:383-387)
-            if self._out_of_buckets(lo, hi):
-                return []
-        if not merged:
-            return []
-        lo = np.array([m[0] for m in merged])
-        hi = np.array([m[1] for m in merged])
-        out: List[IndexedSequence] = []
-        for lst in self._materialise(lo, hi):
-            out.extend(lst)
-        return out
+        return self.getSequencesForSpectra([ranges])[0]
 
     def getSequencesForSpectra(self, spectra: Sequence[Sequence[MassRange]]) -> List[List[IndexedSequence]]:
         """getSequences(List<MassRange>) for every spectrum of a list in one device call (dbi_query_spectra,
         DBI_TOL_DA; in unindexed mode dbi_search_unindexed_spectra): the intervals of every spectrum are clamped,
-        sorted, merged and checked against the bucket rule on the GPU.  A sharded proteome asks one spectrum at a
-        time."""
+        sorted, merged and checked against the bucket rule on the GPU (on every rank of a sharded proteome)."""
         self._require()
-        if self.shards:
-            return [self.getSequences(list(sp)) for sp in spectra]
         lists = [list(sp) for sp in spectra]
         mass = np.array([r.precMass for sp in lists for r in sp], dtype=np.float64)
         tol = np.array([r.tolerance for sp in lists for r in sp], dtype=np.float64)

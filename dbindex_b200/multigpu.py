@@ -622,13 +622,78 @@ def search_unindexed_local(handles, lo, hi, max_candidates: int = 0) -> dict:
     return out
 
 
+def _handles_arg(handles):
+    import ctypes as C
+    return (C.c_void_p * max(len(handles), 1))(*[g._h for g in handles])
+
+
+def query_spectra_local(handles, mass, tol, range_off=None, tol_mode: int = 0, index_factor: int = 0) -> dict:
+    """dbi_mg_query_spectra_local: GpuIndex.query_spectra on a built sharded index whose handles all live in this
+    process (`handles[r]` is rank r, as build_local left them).  Returns one query_hits-style answer (one record per
+    hit, one query per spectrum), the ranks' hits of every spectrum concatenated."""
+    import ctypes as C
+    from .capi import DbiError, DbiHitCounts, _ptr, spectra_arrays
+    from .indexer import _merge_hits
+    lib = handles[0].lib
+    lib.dbi_mg_query_spectra_local.restype = C.c_int
+    lib.dbi_mg_query_spectra_local.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64,
+                                               C.c_int, C.c_int, C.POINTER(DbiHitCounts)]
+    mass, tol, range_off, ns = spectra_arrays(mass, tol, range_off, tol_mode)
+    n = len(handles)
+    counts = (DbiHitCounts * n)()
+    rc = lib.dbi_mg_query_spectra_local(_handles_arg(handles), n, _ptr(mass), _ptr(tol), _ptr(range_off), ns,
+                                        int(tol_mode), int(index_factor), counts)
+    if rc != 0:
+        raise DbiError(rc, (lib.dbi_last_error() or b"").decode(errors="replace"))
+    q = np.arange(ns, dtype=np.int64)
+    return _merge_hits([(q, g._read_hits(counts[r], None, None, True)) for r, g in enumerate(handles)], ns)
+
+
+def search_unindexed_spectra_local(handles, mass, tol, range_off=None, tol_mode: int = 0, index_factor: int = 0,
+                                   max_candidates: int = 0) -> dict:
+    """dbi_mg_search_unindexed_spectra_local: GpuIndex.search_unindexed_spectra over a proteome sharded over
+    `handles` of this process (as for search_unindexed_local).  Returns one query_hits-style answer (one query per
+    spectrum) and under "n_candidates" the candidate records of every rank.  DBI_ERANGE (a rank over max_candidates,
+    0 = no cap) raises DbiError with n_candidates = the largest per-rank count and the per-rank counts in its
+    `rank_candidates`."""
+    import ctypes as C
+    from .capi import DbiError, DbiHitCounts, _ptr, spectra_arrays
+    from .indexer import _merge_hits
+    lib = handles[0].lib
+    lib.dbi_mg_search_unindexed_spectra_local.restype = C.c_int
+    lib.dbi_mg_search_unindexed_spectra_local.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                          C.c_uint64, C.c_int, C.c_int, C.c_uint64,
+                                                          C.POINTER(DbiHitCounts), C.c_void_p]
+    mass, tol, range_off, ns = spectra_arrays(mass, tol, range_off, tol_mode)
+    n = len(handles)
+    counts = (DbiHitCounts * n)()
+    n_cand = np.zeros(n, dtype=np.uint64)
+    rc = lib.dbi_mg_search_unindexed_spectra_local(_handles_arg(handles), n, _ptr(mass), _ptr(tol), _ptr(range_off),
+                                                   ns, int(tol_mode), int(index_factor), int(max_candidates), counts,
+                                                   n_cand.ctypes.data)
+    if rc != 0:
+        err = DbiError(rc, (lib.dbi_last_error() or b"").decode(errors="replace"), int(n_cand.max()))
+        err.rank_candidates = n_cand
+        raise err
+    q = np.arange(ns, dtype=np.int64)
+    out = _merge_hits([(q, g._read_hits(counts[r], None, None, True)) for r, g in enumerate(handles)], ns)
+    out["n_candidates"] = n_cand
+    return out
+
+
 class ShardedSearcher:
-    """The handles of a sharded proteome in this process as one unindexed searcher.  search_unindexed has the
-    signature of GpuIndex.search_unindexed, so indexer.search_unindexed_chunked splits sharded batches unchanged:
-    its ceil(N_c / cap) + 1 rule acts on the largest per-rank count, and every call plans its cuts again."""
+    """The handles of a sharded proteome in this process as one unindexed searcher.  search_unindexed and
+    search_unindexed_spectra have the signatures of GpuIndex's, so indexer.search_unindexed_chunked and
+    search_unindexed_spectra_chunked split sharded batches unchanged: their ceil(N_c / cap) + 1 rule acts on the
+    largest per-rank count, and every call plans its cuts again."""
 
     def __init__(self, handles):
         self.handles = list(handles)
 
     def search_unindexed(self, lo, hi, max_candidates: int = 0) -> dict:
         return search_unindexed_local(self.handles, lo, hi, max_candidates)
+
+    def search_unindexed_spectra(self, mass, tol, range_off=None, tol_mode: int = 0, index_factor: int = 0,
+                                 max_candidates: int = 0) -> dict:
+        return search_unindexed_spectra_local(self.handles, mass, tol, range_off, tol_mode, index_factor,
+                                              max_candidates)

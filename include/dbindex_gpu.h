@@ -332,8 +332,10 @@ int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint
  * dbi_query_spectra needs a built handle (DBI_ENOTINIT).  dbi_search_unindexed_spectra is dbi_search_unindexed
  * for spectra: same handle rules, candidate cap, *n_candidates, DBI_ERANGE without a pending result and stats; its
  * candidate windows are the merged intervals, or per PPM spectrum its window up to a bound of every probe the walk
- * can make, so every answer equals dbi_query_spectra on the built index.  An index sharded over several GPUs and
- * the sharded unindexed search are not covered: ask those one spectrum at a time. */
+ * can make, so every answer equals dbi_query_spectra on the built index.  On one rank of a sharded index,
+ * dbi_query_spectra answers Dalton lists with that rank's share, but its PPM walk only sees the rank's own
+ * entries: ask a sharded index through dbi_mg_query_spectra_local (or dbi_mg_spectra_stops +
+ * dbi_mg_query_spectra), and a sharded unindexed search through dbi_mg_search_unindexed_spectra_local. */
 #define DBI_TOL_DA 0
 #define DBI_TOL_PPM 1
 int dbi_query_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
@@ -557,6 +559,47 @@ int dbi_mg_build_local(dbi_handle** handles, int n);
  * outside 1..DBI_MG_MAX_RANKS are DBI_EINVAL.  n = 1 is dbi_search_unindexed on handles[0]. */
 int dbi_mg_search_unindexed_local(dbi_handle** handles, int n, const double* lo, const double* hi, uint64_t nq,
                                   uint64_t max_candidates, dbi_hit_counts* counts, uint64_t* n_candidates);
+
+/* Batches of spectra (dbi_query_spectra) on a sharded index.  Every rank ends with a pending hit result with one
+ * query per spectrum (counts.nq = n_spectra), read with dbi_query_hits_read on that handle; for every spectrum the
+ * union over the ranks equals dbi_query_spectra on one handle holding the whole index (same bucket rule, same
+ * check_spectra errors; order inside a spectrum is not a contract).  Dalton lists need no exchange: every rank
+ * merges the same intervals and answers them over its own entries.  The PPM walk does: its probes u_k have one
+ * owner each (the owner of the slice holding u_k, a cut at u_k belonging to the upper slice), and only the owner
+ * knows whether a probe is empty.  Rank r computes K_r, the probe at which its share of the walk ends (the walk's
+ * own end conditions, or a probe it owns without an entry of that mass); the walk ends at K = min over r of K_r,
+ * and every rank then answers the window and the probes before K over its own entries.
+ *
+ * Rank level (one call per rank, with any transport between the ranks):
+ *   dbi_mg_spectra_stops    K_r of every PPM spectrum (mass, ppm) on the built handle h, as rank `rank` of
+ *                           `world` under the cuts split_mass[n_slices - 1] (dbi_mg_split_masses gives them for a
+ *                           sharded index; n_slices = world or 2 * world, owner(s) = s < world ? s : n_slices-1-s).
+ *                           stop[s] = UINT64_MAX when the walk cannot end on this rank.
+ *   dbi_mg_query_spectra    dbi_query_spectra on one rank; stop = the minimum over the ranks of their stops
+ *                           (DBI_TOL_PPM; NULL is DBI_EINVAL), NULL with DBI_TOL_DA.
+ * One process holds every rank:
+ *   dbi_mg_query_spectra_local             handles[r] must be rank r of one built sharded index of world n
+ *                                          (DBI_EINVAL otherwise, DBI_ENOTINIT for an unbuilt handle); n = 1 is
+ *                                          dbi_query_spectra.  counts[n].
+ *   dbi_mg_search_unindexed_spectra_local  dbi_mg_search_unindexed_local fed with the candidate windows of
+ *                                          dbi_search_unindexed_spectra, computed on every rank's GPU; the walk uses
+ *                                          that call's cuts.  Same handle rules, per-rank cap, DBI_ERANGE with
+ *                                          n_candidates[r], no pending result on any handle after a failure; every
+ *                                          candidate index is dropped once all ranks are idle.  n = 1 is
+ *                                          dbi_search_unindexed_spectra.
+ * Both _local calls drop every handle's earlier pending result; after a failure none holds one. */
+int dbi_mg_spectra_stops(dbi_handle* h, const double* mass, const double* ppm, uint64_t n_spectra, int index_factor,
+                         const double* split_mass, int n_slices, int rank, int world, uint64_t* stop);
+int dbi_mg_query_spectra(dbi_handle* h, const double* mass, const double* tol, const uint64_t* range_off,
+                         uint64_t n_spectra, int tol_mode, int index_factor, const uint64_t* stop,
+                         dbi_hit_counts* counts);
+int dbi_mg_query_spectra_local(dbi_handle** handles, int n, const double* mass, const double* tol,
+                               const uint64_t* range_off, uint64_t n_spectra, int tol_mode, int index_factor,
+                               dbi_hit_counts* counts);
+int dbi_mg_search_unindexed_spectra_local(dbi_handle** handles, int n, const double* mass, const double* tol,
+                                          const uint64_t* range_off, uint64_t n_spectra, int tol_mode,
+                                          int index_factor, uint64_t max_candidates, dbi_hit_counts* counts,
+                                          uint64_t* n_candidates);
 
 /* Test hook for K7: stable radix sort of n host (key, value) pairs on key bits
  * [begin_bit, end_bit), in place, on the handle's GPU. */

@@ -135,6 +135,13 @@ public final class DbiNative {
 	// keeps its hits pending (dbi_query_hits_read on each handle)
 	static final MethodHandle dbi_mg_search_unindexed_local = h("dbi_mg_search_unindexed_local", FunctionDescriptor.of(
 			JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS));
+	// spectrum batches over those handles (built index / SEARCH_UNINDEXED): every GPU keeps its share of every
+	// spectrum pending, the PPM probe walk ending where the GPU owning the first empty probe says
+	static final MethodHandle dbi_mg_query_spectra_local = h("dbi_mg_query_spectra_local", FunctionDescriptor.of(
+			JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, ADDRESS));
+	static final MethodHandle dbi_mg_search_unindexed_spectra_local = h("dbi_mg_search_unindexed_spectra_local",
+			FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT,
+					JAVA_LONG, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_mg_slices = h("dbi_mg_slices", FunctionDescriptor.of(JAVA_INT, ADDRESS));
 	static final MethodHandle dbi_mg_split_masses = h("dbi_mg_split_masses", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_destroy = h("dbi_destroy", FunctionDescriptor.ofVoid(ADDRESS));

@@ -359,13 +359,12 @@ public class GpuDBIndexStore implements DBIndexStore {
 	 * (rangeOff null), mass[s] at tol[s] ppm, answered as DBIndexer.getSequencesUsingPPMTolerance. The bucket rule
 	 * of sparam.getIndexFactor() is applied on the device (dbi_query_spectra; SEARCH_UNINDEXED:
 	 * dbi_search_unindexed_spectra, spectra sorted by mass and split into chunks like searchUnindexed, never inside
-	 * a spectrum). Not available with -Ddbindex.gpu.devices=N > 1: the callers ask one spectrum at a time there.
+	 * a spectrum). With -Ddbindex.gpu.devices=N > 1: dbi_mg_query_spectra_local (SEARCH_UNINDEXED:
+	 * dbi_mg_search_unindexed_spectra_local, chunked on the largest per-GPU N_c), then every GPU's share is read.
 	 */
 	public List<List<IndexedSequence>> querySpectra(double[] mass, double[] tol, long[] rangeOff, int tolMode)
 			throws DBIndexStoreException {
 		requireInit();
-		if (nDevices > 1)
-			throw new DBIndexStoreException("spectrum batches run on one GPU");
 		final int n = rangeOff == null ? mass.length : rangeOff.length - 1;
 		final List<List<IndexedSequence>> ret = new ArrayList<>();
 		for (int i = 0; i < n; ++i)
@@ -412,14 +411,28 @@ public class GpuDBIndexStore implements DBIndexStore {
 			}
 			if (rangeOff != null)
 				dro.setAtIndex(JAVA_LONG, n, r);
-			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS), nCand = a.allocate(JAVA_LONG);
+			final MemorySegment cnt = a.allocate(DbiNative.HIT_COUNTS, nDevices), nCand = a.allocate(JAVA_LONG, nDevices);
+			final MemorySegment hs = a.allocate(ADDRESS, nDevices);
+			for (int d = 0; d < nDevices; ++d)
+				hs.setAtIndex(ADDRESS, d, handles[d]);
 			final int factor = sparam.getIndexFactor();
 			if (!unindexed) {
-				check((int) DbiNative.dbi_query_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode, factor, cnt));
+				if (nDevices == 1)
+					check((int) DbiNative.dbi_query_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode, factor, cnt));
+				else
+					check((int) DbiNative.dbi_mg_query_spectra_local.invoke(hs, nDevices, dm, dt, dro, (long) n, tolMode,
+							factor, cnt));
 			} else {
-				final int rc = (int) DbiNative.dbi_search_unindexed_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode,
-						factor, maxCandidates, cnt, nCand);
-				final long nc = nCand.get(JAVA_LONG, 0);
+				final int rc;
+				if (nDevices == 1)
+					rc = (int) DbiNative.dbi_search_unindexed_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode, factor,
+							maxCandidates, cnt, nCand);
+				else
+					rc = (int) DbiNative.dbi_mg_search_unindexed_spectra_local.invoke(hs, nDevices, dm, dt, dro, (long) n,
+							tolMode, factor, maxCandidates, cnt, nCand);
+				long nc = 0;
+				for (int d = 0; d < nDevices; ++d)
+					nc = Math.max(nc, nCand.getAtIndex(JAVA_LONG, d));
 				if (rc == DbiNative.DBI_ERANGE && nc > maxCandidates && n > 1) {
 					final int chunks = (int) Math.min(n, (nc + maxCandidates - 1) / maxCandidates + 1);
 					for (int c = 0; c < chunks; ++c)
@@ -429,17 +442,14 @@ public class GpuDBIndexStore implements DBIndexStore {
 				}
 				check(rc);
 			}
-			readHits(handle, a, cnt, ids, sink);
+			final long cb = DbiNative.HIT_COUNTS.byteSize();
+			for (int d = 0; d < nDevices; ++d) // every GPU answers for the mass slices it owns
+				readHits(handles[d], a, cnt.asSlice(d * cb, cb), ids, sink);
 		} catch (final DBIndexStoreException e) {
 			throw e;
 		} catch (final Throwable t) {
 			throw new DBIndexStoreException("Error getting peptides ", t);
 		}
-	}
-
-	/** with -Ddbindex.gpu.devices=N > 1 the spectrum batches are not available (one spectrum at a time) */
-	public boolean supportsSpectrumBatches() {
-		return nDevices == 1;
 	}
 
 	/** IndexedSequence as parseAddPeptideInfo builds it (Merge:452-462), the mod pattern as a mod sequence */

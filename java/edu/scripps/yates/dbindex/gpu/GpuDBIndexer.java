@@ -40,13 +40,11 @@ public class GpuDBIndexer extends DBIndexer {
 
 	/**
 	 * getSequencesUsingPPMTolerance (DBIndexer.java:787-844) as a batch of one: the window and the exact-mass
-	 * probe walk run on the GPU in one call. With -Ddbindex.gpu.devices=N > 1: the reference's loop.
+	 * probe walk run on the GPU in one call (on every GPU of a sharded index).
 	 */
 	@Override
 	public List<IndexedSequence> getSequencesUsingPPMTolerance(double precursorMass, double massToleranceInPPM)
 			throws DBIndexStoreException {
-		if (!((GpuDBIndexStore) indexStore).supportsSpectrumBatches())
-			return super.getSequencesUsingPPMTolerance(precursorMass, massToleranceInPPM);
 		return getSequencesUsingPPMTolerance(new double[] { precursorMass }, massToleranceInPPM).get(0);
 	}
 
@@ -54,12 +52,6 @@ public class GpuDBIndexer extends DBIndexer {
 	public List<List<IndexedSequence>> getSequencesUsingPPMTolerance(double[] masses, double massToleranceInPPM)
 			throws DBIndexStoreException {
 		final GpuDBIndexStore store = (GpuDBIndexStore) indexStore;
-		if (!store.supportsSpectrumBatches()) {
-			final List<List<IndexedSequence>> ret = new ArrayList<>();
-			for (final double m : masses)
-				ret.add(super.getSequencesUsingPPMTolerance(m, massToleranceInPPM));
-			return ret;
-		}
 		final double[] ppm = new double[masses.length];
 		java.util.Arrays.fill(ppm, massToleranceInPPM);
 		return store.querySpectra(masses, ppm, null, DbiNative.DBI_TOL_PPM);
@@ -68,12 +60,6 @@ public class GpuDBIndexer extends DBIndexer {
 	/** getSequences(List<MassRange>) for every spectrum, one device call (dbi_query_spectra, DBI_TOL_DA). */
 	public List<List<IndexedSequence>> getSequencesForSpectra(List<List<MassRange>> spectra) throws DBIndexStoreException {
 		final GpuDBIndexStore store = (GpuDBIndexStore) indexStore;
-		if (!store.supportsSpectrumBatches()) {
-			final List<List<IndexedSequence>> ret = new ArrayList<>();
-			for (final List<MassRange> sp : spectra)
-				ret.add(getSequences(sp));
-			return ret;
-		}
 		final long[] rangeOff = new long[spectra.size() + 1];
 		for (int s = 0; s < spectra.size(); ++s)
 			rangeOff[s + 1] = rangeOff[s] + spectra.get(s).size();
