@@ -90,7 +90,7 @@ class DbiStats(C.Structure):
         ("dom_kernel", C.c_uint32),
         ("exp_launches", C.c_uint32),
         ("exp_ms", C.c_float),
-        ("_pad", C.c_uint32),
+        ("n_groups", C.c_uint32),
         ("exp_bytes_per_launch", C.c_uint64),
     ]
 
@@ -457,7 +457,7 @@ class GpuIndex:
         d = {k: getattr(st, k) for k in ("n_proteins", "n_residues", "n_emitted", "n_unique", "n_entries",
                                          "n_hash_retries", "device_bytes", "sort_bits_base", "sort_bits_var",
                                          "dom_ms", "dom_launches", "dom_bytes_per_launch", "dom_kernel",
-                                         "exp_ms", "exp_launches", "exp_bytes_per_launch")}
+                                         "exp_ms", "exp_launches", "exp_bytes_per_launch", "n_groups")}
         d["algo_bytes"] = dict(zip(STAGE_NAMES, list(st.algo_bytes)))
         d["stage_ms"] = dict(zip(STAGE_NAMES, [float(x) for x in st.stage_ms]))
         d["stage_launches"] = dict(zip(STAGE_NAMES, list(st.stage_launches)))

@@ -193,6 +193,11 @@ struct dbi_handle {
   // d_nlong = how many peptides are longer than 64 residues (they have no masks)
   DevBuf u_cmask, d_nlong;
   uint64_t cmask_n = UINT64_MAX;
+  // compact layout (single GPU, group path): the sorted groups instead of the entry arrays.  g_mass = group
+  // mass, g_pay = peptide << 32 | class sequence << 27 | variant count, g_eoff = entries before each group
+  // (n_groups + 1); n_groups = 0 when the entries are expanded.  n_long = peptides longer than 64 residues.
+  DevBuf g_mass, g_pay, g_eoff;
+  uint64_t n_groups = 0, n_long = 0;
   // kept raw records (params.keep_emitted)
   DevBuf k_mass, k_gpos, k_prot, k_len;
 
@@ -275,6 +280,9 @@ struct dbi_handle {
   const double* entry_mass() const { return e_mass.p ? e_mass.as<double>() : u_mass.as<double>(); }
   const uint32_t* entry_base() const { return e_base.as<uint32_t>(); }
   const uint32_t* entry_pat() const { return e_pat.as<uint32_t>(); }
+  // what K9 / K14 / the key listing search: the groups of a compact index, else the entries
+  const double* key_mass() const { return n_groups ? g_mass.as<double>() : entry_mass(); }
+  uint64_t n_keys() const { return n_groups ? n_groups : n_entries; }
 };
 
 namespace {
@@ -423,6 +431,8 @@ void free_tables(dbi_handle* h) {
   h->u_plo.release(); h->plist.release();
   h->e_mass.release(); h->e_base.release(); h->e_pat.release();
   h->u_cmask.release(); h->d_nlong.release();
+  h->g_mass.release(); h->g_pay.release(); h->g_eoff.release();
+  h->n_groups = h->n_long = 0;
   h->cmask_n = UINT64_MAX;
   h->k_mass.release(); h->k_gpos.release(); h->k_prot.release(); h->k_len.release();
   h->n_emitted = h->n_unique = h->n_entries = 0;
@@ -603,6 +613,9 @@ struct UniqLayout {
 // Test hook: DBI_GROUP_RADIX sends the single-GPU group path through the K7 sort of the sharded build
 // (peptide-major records) instead of K6g's sorted lists + the K7m merge; the results are identical.
 bool group_radix(const dbi_handle*) { return std::getenv("DBI_GROUP_RADIX") != nullptr; }
+// Test hook: DBI_COMPACT_VARIANTS keeps a single-GPU group-path index compact even below 2^32 entries, so that
+// tests and benchmarks can compare the two layouts on small proteomes
+bool compact_variants(const dbi_handle*) { return std::getenv("DBI_COMPACT_VARIANTS") != nullptr; }
 
 // K7 + K8: sort N records by (mass, sequence hash, arrival order), merge equal peptides into
 // the handle's unique tables (u_*, plist).
@@ -943,8 +956,10 @@ struct GroupSide {
   const UniqView* uv = nullptr;      // where the peptides' (gpos, len) live: only peptides longer than 64 residues need it
 };
 // lists (single GPU, K6g's list layout): K7m merges the lists instead of the sort.
+// in_bufs (single GPU): the buffers of key_in / pay_in, which a compact index keeps when they hold the result.
 int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64_t NG, const KeySpace& ks,
-                       const GroupSide* side = nullptr, const GroupLists* lists = nullptr) {
+                       const GroupSide* side = nullptr, const GroupLists* lists = nullptr,
+                       DevBuf* const* in_bufs = nullptr) {
   cudaStream_t s = h->stream;
   if (NG >= (1ull << 32)) {
     set_error("more than 2^32 variant groups on one GPU (%llu)", (unsigned long long)NG);
@@ -1008,6 +1023,21 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
       return DBI_ERANGE;
     }
     if (sharded) n_long = NG;  // unknown here: any received group may belong to a long peptide
+    if (!sharded && in_bufs && (V >= (1ull << 32) || compact_variants(h))) {
+      // compact layout: keep the sorted groups, their masses and entry offsets; queries expand what they return
+      launch_grp_key_mass(vk[r], NG, ks.base_bits, s);
+      h->g_mass.swap(r ? key2 : *in_bufs[0]);
+      h->g_pay.swap(r ? pay2 : *in_bufs[1]);
+      h->g_eoff.swap(eoff);
+      h->e_mass.release(); h->e_base.release(); h->e_pat.release();
+      h->n_groups = NG;
+      h->n_long = n_long;
+      h->st.n_groups = (uint32_t)NG;
+      h->st.algo_bytes[DBI_STAGE_GATHER_VAR] += NG * ((lists ? 0 : 8 + 4) + 16);
+      h->n_entries = V;
+      h->st.n_entries = V;
+      return DBI_OK;
+    }
     if (V >= (1ull << 32)) {
       set_error("more than 2^32 index entries on one GPU (%llu)", (unsigned long long)V);
       return DBI_ERANGE;
@@ -1057,6 +1087,7 @@ int index_records(dbi_handle* h, const RecView& r, uint64_t N, double lo_mass, d
   h->n_emitted = N;
   h->st.n_emitted = N;
   const KeySpace ks(lo_mass, hi_mass);
+  h->st.n_groups = 0;  // set again if the build keeps the compact layout
   if (int rc = sort_dedup(h, r, N, ks)) return rc;
   h->ent_base_off = 0;
   if (h->cfg.max_mods == 0 || h->n_unique == 0) {
@@ -1072,7 +1103,8 @@ int index_records(dbi_handle* h, const RecView& r, uint64_t N, double lo_mass, d
     GroupLists lists;
     GroupLists* gl = group_radix(h) ? nullptr : &lists;
     if (int rc = emit_groups(h, 0, utiles, ks, vkey, vpay, &NG, &V, gl)) return rc;
-    if (int rc = sort_expand_groups(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), NG, ks, nullptr, gl)) return rc;
+    DevBuf* in_bufs[2] = {&vkey, &vpay};
+    if (int rc = sort_expand_groups(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), NG, ks, nullptr, gl, in_bufs)) return rc;
   } else {  // many shift classes: one record per variant
     if (int rc = emit_variants(h, 0, utiles, ks, vkey, vpay, &V)) return rc;
     if (int rc = sort_variants(h, vkey.as<uint64_t>(), vpay.as<uint64_t>(), V, ks)) return rc;
@@ -1086,6 +1118,8 @@ void finish_stats(dbi_handle* h) {
   h->st.device_bytes = h->d_res.bytes + h->d_pstart.bytes + h->u_mass.bytes + h->u_gpos.bytes + h->u_prot.bytes +
                        h->u_len.bytes + h->u_plo.bytes + h->plist.bytes + h->e_mass.bytes + h->e_base.bytes +
                        h->e_pat.bytes;
+  if (h->n_groups)  // a compact index needs the site masks to expand its groups
+    h->st.device_bytes += h->g_mass.bytes + h->g_pay.bytes + h->g_eoff.bytes + h->u_cmask.bytes;
 }
 
 // The unique-peptide tables a fetch resolves base peptides through: this GPU's own, and in a
@@ -1118,6 +1152,59 @@ UniqView uniq_view(dbi_handle* h) {
   }
   uv.uoff[h->mg_world] = h->uoff[h->mg_world];
   return uv;
+}
+
+// K9 over the handle's masses: entry ranges [d_b, d_b + d_c).  On a compact index K9 finds group ranges,
+// which become entry ranges through g_eoff; cnt32 / ntile32 / over as in launch_grp_entry_ranges.
+void query_ranges(dbi_handle* h, const double* d_lo, const double* d_hi, uint64_t nq, uint64_t* d_b, uint64_t* d_c,
+                  uint32_t* cnt32, uint32_t* ntile32 = nullptr, uint32_t* over = nullptr) {
+  launch_query(h->key_mass(), h->n_keys(), d_lo, d_hi, nq, d_b, d_c, h->n_groups ? nullptr : cnt32, h->stream);
+  h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (32 + 2ull * 32 * (uint64_t)bit_length(h->n_keys()));
+  if (h->n_groups) {
+    launch_grp_entry_ranges(h->g_eoff.as<uint64_t>(), nq, d_b, d_c, cnt32, ntile32, over, h->stream);
+    h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (16 + 2 * 32 + 16 + (cnt32 ? 4 : 0) + (ntile32 ? 4 : 0));
+  }
+}
+
+// K6q and the windowed K6l: the entries of the ranges rg (n_tiles tiles, n_out entries) of a compact index into
+// x_mass / x_base / x_pat, in output order.  The groups of long peptides are listed per (group, tile); a
+// proteome without peptides over 64 residues reads nothing back.
+void expand_ranges(dbi_handle* h, const ExpRanges& rg, uint64_t n_tiles, uint64_t n_out, DevBuf& x_mass,
+                   DevBuf& x_base, DevBuf& x_pat) {
+  cudaStream_t s = h->stream;
+  x_mass.alloc(std::max<uint64_t>(n_out, 1) * 8, h->arena);
+  x_base.alloc(std::max<uint64_t>(n_out, 1) * 4, h->arena);
+  x_pat.alloc(std::max<uint64_t>(n_out, 1) * 4, h->arena);
+  Stage sg(h, DBI_STAGE_FETCH);
+  DevBuf lcount, llist;
+  lcount.alloc(16, h->arena);
+  // one (group, tile) pair per tile is the common case; a tile can hold up to kExpTile + 1 long groups (peptides
+  // over 64 residues with few sites), and then the list overflows and the tiles run again with room for all
+  uint64_t cap = h->n_long ? n_tiles + 1024 : 0;
+  for (;;) {
+    llist.alloc(std::max<uint64_t>(cap, 1) * 8, h->arena);
+    DBI_CUDA(cudaMemsetAsync(lcount.p, 0, 4, s));
+    launch_grp_expand_ranges(h->cfg, h->u_cmask.as<uint64_t>(), h->g_mass.as<double>(), h->g_pay.as<uint64_t>(),
+                             h->g_eoff.as<uint64_t>(), h->n_groups, rg, n_tiles, x_mass.as<double>(),
+                             x_base.as<uint32_t>(), x_pat.as<uint32_t>(), llist.as<uint32_t>(), lcount.as<uint32_t>(),
+                             (uint32_t)cap, h->d_err.as<uint32_t>(), s);
+    if (!h->n_long) break;
+    uint32_t n_listed = 0;
+    DBI_CUDA(cudaMemcpyAsync(&n_listed, lcount.p, 4, cudaMemcpyDeviceToHost, s));
+    DBI_CUDA(cudaStreamSynchronize(s));
+    if (n_listed <= cap) {
+      launch_grp_expand_ranges_long(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg,
+                                    h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->g_mass.as<double>(),
+                                    h->g_pay.as<uint64_t>(), h->g_eoff.as<uint64_t>(), rg, llist.as<uint32_t>(),
+                                    lcount.as<uint32_t>(), n_listed, x_mass.as<double>(), x_base.as<uint32_t>(),
+                                    x_pat.as<uint32_t>(), s);
+      break;
+    }
+    cap = n_listed;  // the list overflowed: run the tiles again with room for every pair
+  }
+  // per tile: the range and two searches of g_eoff; per entry 16 written.  The group records a tile reads (offset,
+  // mass, payload, site masks; between 1 and kExpTile + 1 of them) are not counted.
+  h->st.algo_bytes[DBI_STAGE_FETCH] += n_tiles * (28 + 16ull * (uint64_t)bit_length(h->n_groups)) + n_out * 16;
 }
 
 void mg_release(dbi_handle* h);  // capi_mg.inl
@@ -1409,8 +1496,7 @@ int dbi_query_device(dbi_handle* h, const double* d_lo, const double* d_hi, uint
     return DBI_ENOTINIT;
   }
   Stage sg(h, DBI_STAGE_QUERY);
-  launch_query(h->entry_mass(), h->n_entries, d_lo, d_hi, nq, d_hit_begin, d_hit_count, nullptr, h->stream);
-  h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (32 + 2ull * 32 * (uint64_t)bit_length(h->n_entries));
+  query_ranges(h, d_lo, d_hi, nq, d_hit_begin, d_hit_count, nullptr);
   return DBI_OK;
   DBI_API_END
 }
@@ -1438,8 +1524,7 @@ int dbi_query(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, ui
   DBI_CUDA(cudaMemcpyAsync(d_hi, hi, nq * 8, cudaMemcpyHostToDevice, s));
   {
     Stage sg(h, DBI_STAGE_QUERY);
-    launch_query(h->entry_mass(), h->n_entries, d_lo, d_hi, nq, d_b, d_c, nullptr, s);
-    h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (32 + 2ull * 32 * (uint64_t)bit_length(h->n_entries));
+    query_ranges(h, d_lo, d_hi, nq, d_b, d_c, nullptr);
   }
   DBI_CUDA(cudaMemcpyAsync(hit_begin, d_b, nq * 8, cudaMemcpyDeviceToHost, s));
   DBI_CUDA(cudaMemcpyAsync(hit_count, d_c, nq * 8, cudaMemcpyDeviceToHost, s));
@@ -1470,6 +1555,26 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   cudaStream_t s = h->stream;
   const uint64_t tiles = (count + kScanTile - 1) / kScanTile;
   const UniqView uv = uniq_view(h);
+  const double* em = h->entry_mass();
+  const uint32_t* eb = h->entry_base();
+  const uint32_t* ep = h->entry_pat();
+  uint64_t fb = begin;
+  DevBuf x_mass, x_base, x_pat, rng;
+  if (h->n_groups) {  // compact index: K6q expands the range first
+    const uint64_t NT = (count + kExpTile - 1) / kExpTile;
+    const uint64_t hr[5] = {begin, 0, count, 0, NT};  // begin | out_off | tile_off
+    rng.alloc(40 + NT * 4, h->arena);
+    uint64_t* d_r = rng.as<uint64_t>();
+    DBI_CUDA(cudaMemcpyAsync(d_r, hr, 40, cudaMemcpyHostToDevice, s));
+    uint32_t* tile_q = (uint32_t*)(d_r + 5);
+    DBI_CUDA(cudaMemsetAsync(tile_q, 0, NT * 4, s));
+    expand_ranges(h, ExpRanges{tile_q, d_r + 3, d_r, d_r + 1}, NT, count, x_mass, x_base, x_pat);
+    DBI_CUDA(cudaStreamSynchronize(s));  // hr leaves scope
+    em = x_mass.as<double>();
+    eb = x_base.as<uint32_t>();
+    ep = x_pat.as<uint32_t>();
+    fb = 0;
+  }
   DevBuf sizes, tcnt, toff;
   sizes.alloc(count * 4, h->arena);
   tcnt.alloc(tiles * 4, h->arena);
@@ -1477,7 +1582,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   uint64_t total_ids = 0;
   {
     Stage sg(h, DBI_STAGE_FETCH);
-    launch_fetch_sizes(h->entry_base(), h->ent_base_off, uv, begin, count, sizes.as<uint32_t>(), tcnt.as<uint32_t>(), s);
+    launch_fetch_sizes(eb, h->ent_base_off, uv, fb, count, sizes.as<uint32_t>(), tcnt.as<uint32_t>(), s);
     launch_scan_u32_to_u64(tcnt.as<uint32_t>(), tiles, toff.as<uint64_t>(), s);
     total_ids = read_u64(h, toff.as<uint64_t>() + tiles);
   }
@@ -1497,8 +1602,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   if (want_ids) o_ids.alloc(total_ids * 4, h->arena);
   {
     Stage sg(h, DBI_STAGE_FETCH);
-    launch_fetch_gather(h->entry_mass(), h->entry_base(), h->ent_base_off, uv, h->entry_pat(),
-                        h->d_pstart.as<uint32_t>(), begin, count, sizes.as<uint32_t>(), toff.as<uint64_t>(),
+    launch_fetch_gather(em, eb, h->ent_base_off, uv, ep, h->d_pstart.as<uint32_t>(), fb, count, sizes.as<uint32_t>(), toff.as<uint64_t>(),
                         o_mass.as<double>(), o_prot.as<uint32_t>(), o_off.as<uint32_t>(), o_len.as<uint16_t>(),
                         o_pat.as<uint32_t>(), o_lo.as<uint64_t>(), o_ids.as<uint32_t>(), s);
     h->st.algo_bytes[DBI_STAGE_FETCH] += count * (20 + 8 + 26) + total_ids * 8;
@@ -1535,18 +1639,30 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     r.valid = true;
     return DBI_OK;
   }
-  DevBuf io, cnt32, stmp, len32, np32, stmp2, nseg32, seg_off;
-  io.alloc(nq * 16, h->arena);  // begin | count
+  DevBuf io, cnt32, stmp, len32, np32, stmp2, nseg32, seg_off, ntile32, tile_off;
+  io.alloc(nq * 16 + 8, h->arena);  // begin | count | over
   uint64_t* d_b = io.as<uint64_t>();
   uint64_t* d_c = d_b + nq;
+  uint32_t* d_over = (uint32_t*)(d_c + nq);
   cnt32.alloc(nq * 4, h->arena);
   stmp.alloc(full_scan_tmp_bytes(nq), h->arena);
-  uint64_t H = 0, NS = 0;
+  const bool compact = h->n_groups > 0;
+  uint64_t H = 0, NS = 0, NT = 0;
+  uint32_t over = 0;
   {
     Stage sg(h, DBI_STAGE_QUERY);
-    launch_query(h->entry_mass(), h->n_entries, d_lo, d_hi, nq, d_b, d_c, cnt32.as<uint32_t>(), s);
+    if (compact) {  // and the K6q tiles of every query
+      ntile32.alloc(nq * 4, h->arena);
+      tile_off.alloc((nq + 1) * 8, h->arena);
+      DBI_CUDA(cudaMemsetAsync(d_over, 0, 4, s));
+    }
+    query_ranges(h, d_lo, d_hi, nq, d_b, d_c, cnt32.as<uint32_t>(), ntile32.as<uint32_t>(), d_over);
     launch_full_scan_u32_to_u64(cnt32.as<uint32_t>(), nq, r.hit_off.as<uint64_t>(), stmp.p, s);
-    h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (32 + 2ull * 32 * (uint64_t)bit_length(h->n_entries));
+    if (compact) {
+      launch_full_scan_u32_to_u64(ntile32.as<uint32_t>(), nq, tile_off.as<uint64_t>(), stmp.p, s);
+      DBI_CUDA(cudaMemcpyAsync(&NT, tile_off.as<uint64_t>() + nq, 8, cudaMemcpyDeviceToHost, s));
+      DBI_CUDA(cudaMemcpyAsync(&over, d_over, 4, cudaMemcpyDeviceToHost, s));
+    }
     // the hits of a query are materialised in segments of 256 (one warp each)
     nseg32.alloc(nq * 4, h->arena);
     seg_off.alloc((nq + 1) * 8, h->arena);
@@ -1556,12 +1672,32 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     DBI_CUDA(cudaMemcpyAsync(&NS, seg_off.as<uint64_t>() + nq, 8, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
   }
-  if (H >= (1ull << 32)) {
-    set_error("%llu hits in one batch: split the batch (< 2^32 hits per call)", (unsigned long long)H);
+  if (H >= (1ull << 32) || over) {
+    set_error("%s hits in one batch: split the batch (< 2^32 hits per call)",
+              over ? "2^32 or more" : std::to_string(H).c_str());
     r.drop();
     return DBI_ERANGE;
   }
   const UniqView uv = uniq_view(h);
+  // where K10 reads the hits: the index's entries, or on a compact index the hits expanded by K6q (hit h of
+  // the batch at position h: the queries' hits begin at hit_off)
+  const double* em = h->entry_mass();
+  const uint32_t* eb = h->entry_base();
+  const uint32_t* ep = h->entry_pat();
+  const uint64_t* hb = d_b;
+  uint64_t eo = h->ent_base_off;
+  DevBuf x_mass, x_base, x_pat, tile_q;
+  if (compact && H) {
+    tile_q.alloc(NT * 4, h->arena);
+    launch_hits_seg_fill(tile_off.as<uint64_t>(), nq, tile_q.as<uint32_t>(), s);
+    const ExpRanges rg{tile_q.as<uint32_t>(), tile_off.as<uint64_t>(), d_b, r.hit_off.as<uint64_t>()};
+    expand_ranges(h, rg, NT, H, x_mass, x_base, x_pat);
+    em = x_mass.as<double>();
+    eb = x_base.as<uint32_t>();
+    ep = x_pat.as<uint32_t>();
+    hb = r.hit_off.as<uint64_t>();
+    eo = 0;
+  }
   r.pep_off.alloc((nq + 1) * 8, h->arena);
   uint64_t NP = 0, SB = 0, PI = 0;
   if (H) {
@@ -1573,8 +1709,8 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     stmp3.alloc(full_scan_tmp_bytes(NS), h->arena);
     r.pat.alloc(H * 4, h->arena);
     launch_hits_seg_fill(seg_off.as<uint64_t>(), nq, seg_q.as<uint32_t>(), s);
-    launch_hits_count_runs(h->entry_mass(), h->entry_base(), seg_q.as<uint32_t>(), seg_off.as<uint64_t>(), d_b,
-                           r.hit_off.as<uint64_t>(), NS, nruns32.as<uint32_t>(), s);
+    launch_hits_count_runs(em, eb, seg_q.as<uint32_t>(), seg_off.as<uint64_t>(), hb, r.hit_off.as<uint64_t>(), NS,
+                           nruns32.as<uint32_t>(), s);
     launch_full_scan_u32_to_u64(nruns32.as<uint32_t>(), NS, seg_run_off.as<uint64_t>(), stmp3.p, s);
     launch_hits_pep_off(seg_off.as<uint64_t>(), seg_run_off.as<uint64_t>(), nq, r.pep_off.as<uint64_t>(), s);
     NP = read_u64(h, seg_run_off.as<uint64_t>() + NS);
@@ -1586,8 +1722,8 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     len32.alloc(NP * 4, h->arena);
     np32.alloc(NP * 4, h->arena);
     stmp2.alloc(full_scan_tmp_bytes(NP), h->arena);
-    launch_hits_runs(h->entry_mass(), h->entry_base(), h->ent_base_off, h->entry_pat(), uv, seg_q.as<uint32_t>(),
-                     seg_off.as<uint64_t>(), d_b, r.hit_off.as<uint64_t>(), seg_run_off.as<uint64_t>(), NS,
+    launch_hits_runs(em, eb, eo, ep, uv, seg_q.as<uint32_t>(), seg_off.as<uint64_t>(), hb, r.hit_off.as<uint64_t>(),
+                     seg_run_off.as<uint64_t>(), NS,
                      r.pat.as<uint32_t>(), r.pep_hit_off.as<uint64_t>(), r.mass.as<double>(), pep_entry.as<uint32_t>(),
                      len32.as<uint32_t>(), np32.as<uint32_t>(), s);
     DBI_CUDA(cudaMemcpyAsync(r.pep_hit_off.as<uint64_t>() + NP, r.hit_off.as<uint64_t>() + nq, 8, cudaMemcpyDeviceToDevice, s));
@@ -1602,7 +1738,7 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     r.flanks.alloc(NP * 6, h->arena);
     r.seq.alloc(std::max<uint64_t>(SB, 1), h->arena);
     r.ids.alloc(std::max<uint64_t>(PI, 1) * 4, h->arena);
-    launch_peps_gather(h->d_res.as<uint8_t>(), h->d_pstart.as<uint32_t>(), h->entry_base(), h->ent_base_off, uv,
+    launch_peps_gather(h->d_res.as<uint8_t>(), h->d_pstart.as<uint32_t>(), eb, eo, uv,
                        pep_entry.as<uint32_t>(), r.seq_off.as<uint64_t>(), r.plo.as<uint64_t>(), NP,
                        r.prot.as<uint32_t>(), r.off.as<uint32_t>(), r.len.as<uint16_t>(), r.flanks.as<uint8_t>(),
                        r.seq.as<uint8_t>(), r.ids.as<uint32_t>(), s);
@@ -1870,13 +2006,13 @@ void spectra_probe(dbi_handle* h, SpectraBatch& b, const uint64_t* d_stop = null
   Stage sg(h, DBI_STAGE_QUERY);
   const double* w_lo = b.win.as<double>();
   const double* w_hi = w_lo + b.n;
-  launch_spec_probe_count(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
+  launch_spec_probe_count(h->key_mass(), h->n_keys(), b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
                           b.cnt.as<uint32_t>(), s);
   spectra_offsets(h, b);
-  launch_spec_probe_emit(h->entry_mass(), h->n_entries, b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
+  launch_spec_probe_emit(h->key_mass(), h->n_keys(), b.mass(), b.tol(), w_lo, w_hi, b.n, b.factor, d_stop,
                          b.ioff.as<uint64_t>(), b.iv.as<double>(), b.iv.as<double>() + b.n_iv, s);
   // both passes: (mass, ppm, window) read, one lower bound (or one stop) per spectrum; count, offsets, interval
-  const uint64_t probe = d_stop ? 8 : 32 + 8ull * (uint64_t)bit_length(h->n_entries);
+  const uint64_t probe = d_stop ? 8 : 32 + 8ull * (uint64_t)bit_length(h->n_keys());
   h->st.algo_bytes[DBI_STAGE_QUERY] += 2 * b.n * (32 + probe) + b.n * (4 + 8) + b.n_iv * 16;
 }
 
@@ -1888,9 +2024,9 @@ void spectra_stops(dbi_handle* h, SpectraBatch& b, const SliceCuts& cuts, uint64
   d_stop.alloc(b.n * 8, h->arena);
   {
     Stage sg(h, DBI_STAGE_QUERY);
-    launch_spec_stops(h->entry_mass(), h->n_entries, b.mass(), b.tol(), b.win.as<double>() + b.n, b.n, b.factor, cuts,
+    launch_spec_stops(h->key_mass(), h->n_keys(), b.mass(), b.tol(), b.win.as<double>() + b.n, b.n, b.factor, cuts,
                       d_stop.as<uint64_t>(), s);
-    h->st.algo_bytes[DBI_STAGE_QUERY] += b.n * (24 + 32 + 8ull * (uint64_t)bit_length(h->n_entries) + 8);
+    h->st.algo_bytes[DBI_STAGE_QUERY] += b.n * (24 + 32 + 8ull * (uint64_t)bit_length(h->n_keys()) + 8);
   }
   DBI_CUDA(cudaMemcpyAsync(stop, d_stop.p, b.n * 8, cudaMemcpyDeviceToHost, s));
   DBI_CUDA(cudaStreamSynchronize(s));
@@ -2103,7 +2239,7 @@ int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* 
   }
   // input: residues | offsets | patterns | found counter
   const uint64_t res_bytes = (R + 7) & ~7ull, pat_bytes = modpat ? (n * 4 + 7) & ~7ull : 0;
-  DevBuf in, np32, stmp;
+  DevBuf in, np32, stmp, gid;
   in.alloc(res_bytes + (n + 1) * 8 + pat_bytes + 8, h->arena);
   uint8_t* d_q = in.as<uint8_t>();
   uint64_t* d_off = (uint64_t*)(d_q + res_bytes);
@@ -2118,12 +2254,15 @@ int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* 
   uint64_t n_found = 0, PI = 0;
   {
     Stage sg(h, DBI_STAGE_QUERY);
-    launch_lookup_match(h->d_res.as<uint8_t>(), h->entry_mass(), h->n_entries, h->entry_base(), h->ent_base_off,
+    // compact index: the search runs over the groups, and gid[row] = the peptide found (K11b's input)
+    const GroupView gv{h->g_pay.as<uint64_t>(), h->g_eoff.as<uint64_t>(), h->u_cmask.as<uint64_t>(), h->cfg.n_classes};
+    if (h->n_groups) gid.alloc(n * 8, h->arena);
+    launch_lookup_match(h->d_res.as<uint8_t>(), h->key_mass(), h->n_keys(), h->entry_base(), h->ent_base_off,
                         h->entry_pat(), uv, h->d_tables.as<DevTables>(), h->cfg.init_mass, h->cfg.max_mods, d_q, d_off,
                         d_pat, n, L.status.as<uint8_t>(), L.mass.as<double>(), L.entry.as<uint64_t>(),
-                        np32.as<uint32_t>(), d_found, s);
+                        np32.as<uint32_t>(), d_found, h->n_groups ? &gv : nullptr, gid.as<uint64_t>(), s);
     int rounds = 1;  // the last one probes <= 32 consecutive entries
-    for (uint64_t w = h->n_entries; w > 32; w = w / 33 + 1) ++rounds;
+    for (uint64_t w = h->n_keys(); w > 32; w = w / 33 + 1) ++rounds;
     // rows read (residues, offset, pattern), 32 eight-byte probes per search round, the row's residues compared
     // once with its candidate, status + mass + entry + list length written
     h->st.algo_bytes[DBI_STAGE_QUERY] += 2 * R + n * (12 + 256ull * rounds + 21);
@@ -2135,9 +2274,13 @@ int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* 
     DBI_CUDA(cudaMemcpyAsync(&n_found, d_found, 8, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
     L.ids.alloc(std::max<uint64_t>(PI, 1) * 4, h->arena);
-    launch_lookup_gather(L.status.as<uint8_t>(), L.entry.as<uint64_t>(), h->entry_base(), h->ent_base_off, uv,
-                         h->d_pstart.as<uint32_t>(), L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(),
-                         L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
+    if (h->n_groups)
+      launch_lookup_gather(L.status.as<uint8_t>(), gid.as<uint64_t>(), nullptr, 0, uv, h->d_pstart.as<uint32_t>(),
+                           L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(), L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
+    else
+      launch_lookup_gather(L.status.as<uint8_t>(), L.entry.as<uint64_t>(), h->entry_base(), h->ent_base_off, uv,
+                           h->d_pstart.as<uint32_t>(), L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(),
+                           L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
     // list lengths scanned (4 read, 8 written); per row status + list offset read, first occurrence written;
     // per found row entry, base id, peptide tables (4 + 4 + 16) and protein start read; ids copied
     h->st.algo_bytes[DBI_STAGE_FETCH] += n * (12 + 9 + 8) + n_found * (8 + 4 + 24 + 4) + 8 * PI;
@@ -2257,7 +2400,7 @@ int dbi_entry_keys(dbi_handle* h, int32_t* keys, uint64_t capacity, uint64_t* n_
     return DBI_EINVAL;
   }
   *n_keys = 0;
-  const uint64_t n = h->n_entries;
+  const uint64_t n = h->n_keys();  // equal masses are adjacent: the groups give the same keys as the entries
   if (n == 0) return DBI_OK;
   cudaStream_t s = h->stream;
   const uint64_t tiles = (n + kScanTile - 1) / kScanTile;
@@ -2266,7 +2409,7 @@ int dbi_entry_keys(dbi_handle* h, int32_t* keys, uint64_t capacity, uint64_t* n_
   tcnt.alloc(tiles * 4, h->arena);
   toff.alloc((tiles + 1) * 8, h->arena);
   Stage sg(h, DBI_STAGE_OTHER);
-  launch_key_flags(h->entry_mass(), n, (double)h->p.mass_group_factor, flags.as<uint8_t>(), tcnt.as<uint32_t>(), s);
+  launch_key_flags(h->key_mass(), n, (double)h->p.mass_group_factor, flags.as<uint8_t>(), tcnt.as<uint32_t>(), s);
   launch_scan_u32_to_u64(tcnt.as<uint32_t>(), tiles, toff.as<uint64_t>(), s);
   const uint64_t nk = read_u64(h, toff.as<uint64_t>() + tiles);
   *n_keys = nk;
@@ -2276,7 +2419,7 @@ int dbi_entry_keys(dbi_handle* h, int32_t* keys, uint64_t capacity, uint64_t* n_
     return DBI_ERANGE;
   }
   out.alloc(nk * 4, h->arena);
-  launch_key_emit(h->entry_mass(), n, (double)h->p.mass_group_factor, flags.as<uint8_t>(), toff.as<uint64_t>(),
+  launch_key_emit(h->key_mass(), n, (double)h->p.mass_group_factor, flags.as<uint8_t>(), toff.as<uint64_t>(),
                   out.as<int32_t>(), s);
   DBI_CUDA(cudaMemcpyAsync(keys, out.p, nk * 4, cudaMemcpyDeviceToHost, s));
   DBI_CUDA(cudaStreamSynchronize(s));

@@ -233,6 +233,42 @@ void launch_grp_expand(const uint8_t* d_res, const DevTables* d_tb, const Digest
                        uint32_t* e_pat, uint32_t* long_list, uint32_t* long_count, uint32_t long_cap, uint32_t* d_err,
                        cudaStream_t s);
 
+// Compact index (group arrays kept, entries never written): K6q expands entry ranges.  Range q = entries
+// [begin[q], begin[q] + c_q) to output positions [out_off[q], out_off[q + 1]); tiles of kExpTile entries,
+// tile_q[t] = the range of tile t, tile_off = exclusive scan of the tiles per range.
+struct ExpRanges {
+  const uint32_t* tile_q;
+  const uint64_t* tile_off;
+  const uint64_t* begin;
+  const uint64_t* out_off;
+};
+// A compact index's groups for the lookup (K11a over the groups): payloads, entry offsets, site masks.
+struct GroupView {
+  const uint64_t* pay;
+  const uint64_t* eoff;
+  const uint64_t* cmask;
+  int n_classes;
+};
+// K6q: (mass, peptide, pattern) of every entry of the ranges, in the order of K6x.  Groups of peptides longer
+// than 64 residues are counted into *long_count and listed as (group, tile) pairs while there is room
+// (long_cap pairs); the caller runs the kernel again with a larger list when the count exceeds it.
+void launch_grp_expand_ranges(const DigestCfg& cfg, const uint64_t* cmask, const double* g_mass, const uint64_t* g_pay,
+                              const uint64_t* g_eoff, uint64_t n_groups, const ExpRanges& rg, uint64_t n_tiles,
+                              double* o_mass, uint32_t* o_base, uint32_t* o_pat, uint32_t* long_list,
+                              uint32_t* long_count, uint32_t long_cap, uint32_t* d_err, cudaStream_t s);
+// the windowed K6l over the n_listed pairs K6q listed
+void launch_grp_expand_ranges_long(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg,
+                                   const uint32_t* u_gpos, const uint16_t* u_len, const double* g_mass,
+                                   const uint64_t* g_pay, const uint64_t* g_eoff, const ExpRanges& rg,
+                                   const uint32_t* long_list, const uint32_t* long_count, uint32_t n_listed,
+                                   double* o_mass, uint32_t* o_base, uint32_t* o_pat, cudaStream_t s);
+// key[i] += base_bits: sorted group keys -> group mass bits
+void launch_grp_key_mass(uint64_t* key, uint64_t n, uint64_t base_bits, cudaStream_t s);
+// group ranges (K9 over the group masses) -> entry ranges through eoff, in place.  cnt32 (optional) = the
+// counts as u32, and *over = 1 if one is >= 2^32; ntile32 (optional) = K6q tiles of every range.
+void launch_grp_entry_ranges(const uint64_t* eoff, uint64_t nq, uint64_t* begin, uint64_t* count, uint32_t* cnt32,
+                             uint32_t* ntile32, uint32_t* over, cudaStream_t s);
+
 // ---- K9/K10 query ----------------------------------------------------------------
 // cnt32 (optional): the hit counts again as u32, the input of the hit-offset scan
 void launch_query(const double* e_mass, uint64_t n_entries, const double* lo, const double* hi, uint64_t nq,
@@ -316,7 +352,8 @@ void launch_lookup_match(const uint8_t* d_res, const double* e_mass, uint64_t n_
                          uint64_t ent_off, const uint32_t* e_pat, const UniqView& uv, const DevTables* d_tb,
                          double init_mass, int max_mods, const uint8_t* q_res, const uint64_t* q_off,
                          const uint32_t* q_pat, uint64_t n, uint8_t* o_status, double* o_mass, uint64_t* o_entry,
-                         uint32_t* o_np, unsigned long long* n_found, cudaStream_t s);
+                         uint32_t* o_np, unsigned long long* n_found, const GroupView* gv, uint64_t* o_gid,
+                         cudaStream_t s);
 // K11b: first occurrence + protein ids of the found rows (plo = scan of o_np); 0xffffffff for the others
 void launch_lookup_gather(const uint8_t* status, const uint64_t* entry, const uint32_t* e_base, uint64_t ent_off,
                           const UniqView& uv, const uint32_t* pstart, const uint64_t* plo, uint64_t n,

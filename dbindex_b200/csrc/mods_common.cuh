@@ -107,6 +107,48 @@ __device__ __forceinline__ uint32_t low_bytes_mask(int n_bytes) {
 }
 // bits strictly above position i
 __device__ __forceinline__ uint64_t above(int i) { return (~1ull) << i; }
+__device__ __forceinline__ uint64_t below(int i) { return ~(~0ull << i); }  // bits strictly below position i
+
+
+// pairs i2 < i3 above position i (third and fourth class)
+__device__ __forceinline__ uint32_t pairs_above(int i, uint64_t c2, uint64_t c3) {
+  uint32_t w = 0;
+  for (uint64_t m = c2 & above(i); m; m &= m - 1) w += (uint32_t)__popcll(c3 & above(__ffsll((long long)m) - 1));
+  return w;
+}
+
+// mask of the block sites of a group and the size of the block at site p
+__device__ __forceinline__ uint64_t block_sites(int k, uint64_t c0, uint64_t c1) { return k == 2 ? c0 : c1; }
+__device__ __forceinline__ uint32_t block_size(int k, int p, uint64_t c0, uint64_t c1, uint64_t c2, uint64_t c3) {
+  if (k == 2) return (uint32_t)__popcll(c1 & above(p));
+  const uint32_t nl = (uint32_t)__popcll(c0 & below(p));
+  if (k == 3) return nl * (uint32_t)__popcll(c2 & above(p));
+  return nl ? nl * pairs_above(p, c2, c3) : 0u;
+}
+
+// Inverse of the block order of K6x (mods_grp.cu group_entry_slow): the rank inside its group of the variant
+// whose level-j site is pos[j] (0-based, ascending), for a peptide of up to 64 residues.  c0..c3 = the site
+// masks of the classes of the sequence's levels.
+__device__ __forceinline__ uint32_t group_entry_rank(int k, const int* pos, uint64_t c0, uint64_t c1, uint64_t c2,
+                                                     uint64_t c3) {
+  if (k == 0) return 0u;
+  if (k == 1) return (uint32_t)__popcll(c0 & below(pos[0]));
+  const int pb = k == 2 ? pos[0] : pos[1];  // the block site
+  uint32_t r = 0;                           // entries of the blocks before
+  for (uint64_t m = block_sites(k, c0, c1) & below(pb); m; m &= m - 1)
+    r += block_size(k, __ffsll((long long)m) - 1, c0, c1, c2, c3);
+  if (k == 2) return r + (uint32_t)__popcll(c1 & above(pos[0]) & below(pos[1]));
+  const uint32_t a = (uint32_t)__popcll(c0 & below(pos[0]));
+  if (k == 3) {
+    const uint64_t R = c2 & above(pb);
+    return r + a * (uint32_t)__popcll(R) + (uint32_t)__popcll(R & below(pos[2]));
+  }
+  uint32_t b = (uint32_t)__popcll(c3 & above(pos[2]) & below(pos[3]));  // pairs (i2, i3) before (pos[2], pos[3])
+  for (uint64_t m = c2 & above(pb) & below(pos[2]); m; m &= m - 1)
+    b += (uint32_t)__popcll(c3 & above(__ffsll((long long)m) - 1));
+  return r + a * pairs_above(pb, c2, c3) + b;
+}
+
 
 }  // namespace
 }  // namespace dbi

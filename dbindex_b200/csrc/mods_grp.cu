@@ -17,6 +17,8 @@
 //                    time (product-set blocks, per-group block tables in shared memory) and write
 //                    (mass, peptide, pattern) -- coalesced stores, no divergent per-group enumeration
 //   K6l grp_expand_long : groups of peptides longer than 64 residues (no masks): one warp each
+//   K6q grp_expand_ranges : compact index (the sorted groups kept, no entry arrays): K6x's tile body over
+//                    tiles cut from arbitrary entry ranges, at query time; the windowed K6l for long groups
 //
 // HBM-bound byte/integer work; no tensor cores.  Algorithmic bytes: K5m 14 + len per peptide read,
 // 8 C written; K5g/K6g 25 + 8 C per peptide, 16 per group written; K6x 24 per group + 8 C per
@@ -382,8 +384,6 @@ struct ExpSmem {
   uint32_t scratch[ET_THREADS / 32 + 1];
 };
 
-__device__ __forceinline__ uint64_t below(int i) { return ~(~0ull << i); }  // bits strictly below position i
-
 // appends (position + 1) of every set bit of c, ascending, to the byte pool; the two 32-bit halves are walked
 // separately (most peptides have fewer than 33 residues: half the instructions of a 64-bit walk)
 __device__ __forceinline__ uint32_t fill_sites(uint64_t c, uint8_t* pool, uint32_t x) {
@@ -391,22 +391,6 @@ __device__ __forceinline__ uint32_t fill_sites(uint64_t c, uint8_t* pool, uint32
   for (; lo; lo &= lo - 1) pool[x++] = (uint8_t)__ffs((int)lo);
   for (; hi; hi &= hi - 1) pool[x++] = (uint8_t)(32 + __ffs((int)hi));
   return x;
-}
-
-// pairs i2 < i3 above position i (third and fourth class)
-__device__ __forceinline__ uint32_t pairs_above(int i, uint64_t c2, uint64_t c3) {
-  uint32_t w = 0;
-  for (uint64_t m = c2 & above(i); m; m &= m - 1) w += (uint32_t)__popcll(c3 & above(__ffsll((long long)m) - 1));
-  return w;
-}
-
-// mask of the block sites of a group and the size of the block at site p
-__device__ __forceinline__ uint64_t block_sites(int k, uint64_t c0, uint64_t c1) { return k == 2 ? c0 : c1; }
-__device__ __forceinline__ uint32_t block_size(int k, int p, uint64_t c0, uint64_t c1, uint64_t c2, uint64_t c3) {
-  if (k == 2) return (uint32_t)__popcll(c1 & above(p));
-  const uint32_t nl = (uint32_t)__popcll(c0 & below(p));
-  if (k == 3) return nl * (uint32_t)__popcll(c2 & above(p));
-  return nl ? nl * pairs_above(p, c2, c3) : 0u;
 }
 
 // pattern of entry q of the block at site p, from the masks (slow path)
@@ -450,25 +434,23 @@ __device__ __forceinline__ uint32_t group_entry_slow(int k, uint32_t q, uint64_t
   return block_entry(k, p, q, c0, c1, c2, c3);
 }
 
+// One tile of K6x / K6q: the entries [e0, e0 + tile_n) of the sorted groups, which are the groups g0 ..
+// g0 + ngrp - 1, written to positions o0 + 0 .. o0 + tile_n - 1 of the outputs.
 // cmask[row * C + c]: the site masks; row = the payload's peptide field.  gid_tab (sharded build: the
 // rows are arrival slots of the group exchange) maps a row to the peptide's global id, else row = id.
-__global__ void __launch_bounds__(ET_THREADS, 4)
-    grp_expand_tab_kernel(DigestCfg cfg, const uint64_t* __restrict__ cmask, const uint32_t* __restrict__ gid_tab,
-                          const uint64_t* __restrict__ skey, const uint64_t* __restrict__ spay,
-                          const uint64_t* __restrict__ eoff, const uint32_t* __restrict__ tile_first,
-                          uint64_t n_entries, uint64_t base_bits, double* __restrict__ e_mass,
-                          uint32_t* __restrict__ e_base, uint32_t* __restrict__ e_pat,
-                          uint32_t* __restrict__ long_list, uint32_t* __restrict__ long_count, uint32_t long_cap,
-                          uint32_t* err) {
-  __shared__ __align__(16) ExpSmem s;
+// Groups of long peptides go to long_list: K6x lists a group once, in the tile where it starts (K6l writes it
+// whole); K6q (kWindow) lists every (group, tile) pair, and the windowed K6l writes the tile's share.
+template <bool kWindow>
+__device__ __forceinline__ void expand_tile(ExpSmem& s, const DigestCfg& cfg, const uint64_t* __restrict__ cmask,
+                                            const uint32_t* __restrict__ gid_tab, const uint64_t* __restrict__ skey,
+                                            const uint64_t* __restrict__ spay, const uint64_t* __restrict__ eoff,
+                                            uint64_t base_bits, uint64_t tile, uint64_t e0, uint32_t tile_n,
+                                            uint32_t g0, uint32_t ngrp, uint64_t o0, double* __restrict__ e_mass,
+                                            uint32_t* __restrict__ e_base, uint32_t* __restrict__ e_pat,
+                                            uint32_t* __restrict__ long_list, uint32_t* __restrict__ long_count,
+                                            uint32_t long_cap, uint32_t* err) {
   const int C = cfg.n_classes;
   const int t = threadIdx.x;
-  const uint64_t tile = blockIdx.x;
-  const uint64_t e0 = tile * (uint64_t)kExpTile;
-  const uint32_t tile_n = (uint32_t)min((uint64_t)kExpTile, n_entries - e0);
-  const uint32_t g0 = tile_first[tile];
-  const uint32_t ngrp = tile_first[tile + 1] - g0 + 1;
-
   for (int i = t; i < kExpTile; i += ET_THREADS) s.head[i] = 0;
   if (t <= 64) s.recip[t] = t ? ((1u << 20) + (uint32_t)t - 1u) / (uint32_t)t : 0u;
   if (t == 0) {
@@ -511,7 +493,13 @@ __global__ void __launch_bounds__(ET_THREADS, 4)
     if (c0 == 0) {  // a peptide longer than 64 residues: K6l writes this group
       b.k = kLongGroup;
       append(b);
-      if (rel >= 0 && rel < (int32_t)kExpTile) {
+      if constexpr (kWindow) {  // the caller grows the list and runs the tile again when it overflows
+        const uint32_t slot = atomicAdd(long_count, 1u);
+        if (slot < long_cap) {
+          long_list[2 * slot] = (uint32_t)g;
+          long_list[2 * slot + 1] = (uint32_t)tile;
+        }
+      } else if (rel >= 0 && rel < (int32_t)kExpTile) {
         const uint32_t slot = atomicAdd(long_count, 1u);
         if (slot < long_cap) long_list[slot] = (uint32_t)g; else atomicOr(err, kErrModPos);
       }
@@ -616,17 +604,104 @@ __global__ void __launch_bounds__(ET_THREADS, 4)
     } else {
       continue;  // long group: K6l
     }
-    const uint64_t e = e0 + i;
+    const uint64_t e = o0 + i;
     e_mass[e] = s.mass[j];
     e_base[e] = s.base[j];
     e_pat[e] = pat;
   }
 }
 
+__global__ void __launch_bounds__(ET_THREADS, 4)
+    grp_expand_tab_kernel(DigestCfg cfg, const uint64_t* __restrict__ cmask, const uint32_t* __restrict__ gid_tab,
+                          const uint64_t* __restrict__ skey, const uint64_t* __restrict__ spay,
+                          const uint64_t* __restrict__ eoff, const uint32_t* __restrict__ tile_first,
+                          uint64_t n_entries, uint64_t base_bits, double* __restrict__ e_mass,
+                          uint32_t* __restrict__ e_base, uint32_t* __restrict__ e_pat,
+                          uint32_t* __restrict__ long_list, uint32_t* __restrict__ long_count, uint32_t long_cap,
+                          uint32_t* err) {
+  __shared__ __align__(16) ExpSmem s;
+  const uint64_t tile = blockIdx.x;
+  const uint64_t e0 = tile * (uint64_t)kExpTile;
+  const uint32_t tile_n = (uint32_t)min((uint64_t)kExpTile, n_entries - e0);
+  const uint32_t g0 = tile_first[tile];
+  const uint32_t ngrp = tile_first[tile + 1] - g0 + 1;
+  expand_tile<false>(s, cfg, cmask, gid_tab, skey, spay, eoff, base_bits, tile, e0, tile_n, g0, ngrp, e0, e_mass,
+                     e_base, e_pat, long_list, long_count, long_cap, err);
+}
+
+// ---- K6q ------------------------------------------------------------------------------
+// Entry ranges of a compact index: range q = entries [begin[q], begin[q] + c_q) goes to output positions
+// [out_off[q], out_off[q + 1]).  Every range is cut into tiles of kExpTile entries; tile_q[t] = its range and
+// tile_off = the exclusive scan of the tiles per range.
+__device__ __forceinline__ void range_tile(const ExpRanges& rg, uint64_t tile, uint64_t* e0, uint32_t* tile_n,
+                                           uint64_t* o0) {
+  const uint32_t q = rg.tile_q[tile];
+  const uint64_t k = (tile - rg.tile_off[q]) * (uint64_t)kExpTile;
+  const uint64_t lo = rg.out_off[q];
+  *e0 = rg.begin[q] + k;
+  *tile_n = (uint32_t)min((uint64_t)kExpTile, rg.out_off[q + 1] - lo - k);
+  *o0 = lo + k;
+}
+
+// the group that holds entry e: last g with eoff[g] <= e (eoff[0] = 0, eoff[n_groups] > e)
+__device__ __forceinline__ uint32_t group_of(const uint64_t* __restrict__ eoff, uint64_t n_groups, uint64_t e) {
+  uint64_t lo = 0, hi = n_groups;
+  while (hi - lo > 1) {
+    const uint64_t mid = (lo + hi) >> 1;
+    if (__ldg(eoff + mid) <= e) lo = mid; else hi = mid;
+  }
+  return (uint32_t)lo;
+}
+
+// compact index: the sorted keys become the group masses in place (key = mass bits - base_bits)
+__global__ void __launch_bounds__(MD_THREADS)
+    grp_key_mass_kernel(uint64_t* __restrict__ key, uint64_t n, uint64_t base_bits) {
+  const uint64_t i = (uint64_t)blockIdx.x * MD_THREADS + threadIdx.x;
+  if (i < n) key[i] += base_bits;
+}
+
+__global__ void __launch_bounds__(MD_THREADS)
+    grp_entry_ranges_kernel(const uint64_t* __restrict__ eoff, uint64_t nq, uint64_t* __restrict__ begin,
+                            uint64_t* __restrict__ count, uint32_t* __restrict__ cnt32, uint32_t* __restrict__ ntile32,
+                            uint32_t* __restrict__ over) {
+  const uint64_t q = (uint64_t)blockIdx.x * MD_THREADS + threadIdx.x;
+  if (q >= nq) return;
+  const uint64_t g = begin[q];
+  const uint64_t b = eoff[g], c = eoff[g + count[q]] - b;
+  begin[q] = b;
+  count[q] = c;
+  if (cnt32) {
+    cnt32[q] = (uint32_t)c;
+    if (c >> 32) *over = 1u;
+  }
+  if (ntile32) ntile32[q] = (uint32_t)min((c + kExpTile - 1) / kExpTile, (uint64_t)UINT32_MAX);
+}
+
+// g_mass (the groups' masses, as bits) stands where K6x reads key + base_bits
+__global__ void __launch_bounds__(ET_THREADS, 4)
+    grp_expand_ranges_kernel(DigestCfg cfg, const uint64_t* __restrict__ cmask, const uint64_t* __restrict__ g_mass,
+                             const uint64_t* __restrict__ g_pay, const uint64_t* __restrict__ g_eoff, uint64_t n_groups,
+                             const ExpRanges rg, double* __restrict__ o_mass, uint32_t* __restrict__ o_base,
+                             uint32_t* __restrict__ o_pat, uint32_t* __restrict__ long_list,
+                             uint32_t* __restrict__ long_count, uint32_t long_cap, uint32_t* err) {
+  __shared__ __align__(16) ExpSmem s;
+  const uint64_t tile = blockIdx.x;
+  uint64_t e0, o0;
+  uint32_t tile_n;
+  range_tile(rg, tile, &e0, &tile_n, &o0);
+  const uint32_t g0 = group_of(g_eoff, n_groups, e0);
+  const uint32_t g1 = group_of(g_eoff, n_groups, e0 + tile_n - 1);
+  expand_tile<true>(s, cfg, cmask, nullptr, g_mass, g_pay, g_eoff, 0, tile, e0, tile_n, g0, g1 - g0 + 1, o0, o_mass,
+                    o_base, o_pat, long_list, long_count, long_cap, err);
+}
+
 // ---- K6l ------------------------------------------------------------------------------
 // Groups of peptides longer than 64 residues (rare): one warp per listed group enumerates the
 // occurrences from the site list in shared memory; the last matched site is searched by all lanes
-// in parallel, the prefix sites by a warp-uniform odometer.
+// in parallel, the prefix sites by a warp-uniform odometer.  The order is lexicographic in the site
+// tuple.  kWindow (after K6q): the list holds (group, tile) pairs, and only the group's entries inside
+// the tile are written, at the tile's output positions.
+template <bool kWindow>
 __global__ void __launch_bounds__(MD_THREADS)
     grp_expand_long_kernel(const uint8_t* __restrict__ res, const DevTables* __restrict__ tb, DigestCfg cfg,
                            const uint32_t* __restrict__ u_gpos, const uint16_t* __restrict__ u_len,
@@ -635,7 +710,7 @@ __global__ void __launch_bounds__(MD_THREADS)
                            const uint64_t* __restrict__ spay, const uint64_t* __restrict__ eoff,
                            const uint32_t* __restrict__ long_list,
                            const uint32_t* __restrict__ long_count, uint64_t base_bits, double* __restrict__ e_mass,
-                           uint32_t* __restrict__ e_base, uint32_t* __restrict__ e_pat) {
+                           uint32_t* __restrict__ e_base, uint32_t* __restrict__ e_pat, const ExpRanges rg) {
   __shared__ ModTables mt;
   __shared__ WarpSites wsites[MD_WARPS];
   load_mod_tables(mt, tb);
@@ -646,7 +721,13 @@ __global__ void __launch_bounds__(MD_THREADS)
   const int C = cfg.n_classes;
   const uint32_t n_list = *long_count;
   for (uint32_t li = blockIdx.x * MD_WARPS + w; li < n_list; li += gridDim.x * MD_WARPS) {
-    const uint64_t g = long_list[li];
+    const uint64_t g = long_list[kWindow ? 2 * li : li];
+    uint64_t w0 = 0, o0 = 0, w1 = UINT64_MAX;  // entries [w0, w1) go to o0 ..
+    if constexpr (kWindow) {
+      uint32_t tile_n;
+      range_tile(rg, long_list[2 * li + 1], &w0, &tile_n, &o0);
+      w1 = w0 + tile_n;
+    }
     const uint64_t pay = spay[g];
     const uint32_t bb = (uint32_t)(pay >> 32);
     const uint32_t bseq = ((uint32_t)pay >> kGrpCntBits) & 31u;
@@ -681,14 +762,21 @@ __global__ void __launch_bounds__(MD_THREADS)
           const int j = j0 + (int)l;
           const bool ok = j < n && (int)mt.cls[ws.res[j]] == want;
           const unsigned om = __ballot_sync(0xffffffffu, ok);
-          if (ok) {
-            const uint64_t slot = bo + __popc(om & lanemask_lt());
+          uint64_t slot = bo + __popc(om & lanemask_lt());
+          bool put = ok;
+          if (kWindow) {
+            put = put && slot >= w0 && slot < w1;
+            slot = o0 + (slot - w0);
+          }
+          if (put) {
             e_mass[slot] = bmass;
             e_base[slot] = gid_tab ? gid_tab[bb] : bb;
             e_pat[slot] = prefix | (((uint32_t)ws.pos[j] + 1u) << (8 * level));
           }
           bo += __popc(om);
+          if (kWindow && bo >= w1) break;
         }
+        if (kWindow && bo >= w1) break;  // the rest of the group lies after the window
         --level;
         continue;
       }
@@ -779,10 +867,45 @@ void launch_grp_expand(const uint8_t* d_res, const DevTables* d_tb, const Digest
     if (grid > (unsigned)kNumSMsB200 * 4) grid = (unsigned)kNumSMsB200 * 4;
     UniqView none;
     std::memset(&none, 0, sizeof(none));
-    DBI_LAUNCH(grp_expand_long_kernel, grid, MD_THREADS, 0, s, d_res, d_tb, cfg, u_gpos, u_len, gid_tab,
+    DBI_LAUNCH(grp_expand_long_kernel<false>, grid, MD_THREADS, 0, s, d_res, d_tb, cfg, u_gpos, u_len, gid_tab,
                (uv && gid_tab) ? 1 : 0, uv ? *uv : none, skey, spay, eoff, long_list, long_count, base_bits, e_mass,
-               e_base, e_pat);
+               e_base, e_pat, ExpRanges{});
   }
+}
+
+void launch_grp_key_mass(uint64_t* key, uint64_t n, uint64_t base_bits, cudaStream_t s) {
+  if (n == 0) return;
+  DBI_LAUNCH(grp_key_mass_kernel, (unsigned)((n + MD_THREADS - 1) / MD_THREADS), MD_THREADS, 0, s, key, n, base_bits);
+}
+
+void launch_grp_entry_ranges(const uint64_t* eoff, uint64_t nq, uint64_t* begin, uint64_t* count, uint32_t* cnt32,
+                             uint32_t* ntile32, uint32_t* over, cudaStream_t s) {
+  if (nq == 0) return;
+  DBI_LAUNCH(grp_entry_ranges_kernel, (unsigned)((nq + MD_THREADS - 1) / MD_THREADS), MD_THREADS, 0, s, eoff, nq, begin,
+             count, cnt32, ntile32, over);
+}
+
+void launch_grp_expand_ranges(const DigestCfg& cfg, const uint64_t* cmask, const double* g_mass, const uint64_t* g_pay,
+                              const uint64_t* g_eoff, uint64_t n_groups, const ExpRanges& rg, uint64_t n_tiles,
+                              double* o_mass, uint32_t* o_base, uint32_t* o_pat, uint32_t* long_list,
+                              uint32_t* long_count, uint32_t long_cap, uint32_t* d_err, cudaStream_t s) {
+  if (n_groups == 0 || n_tiles == 0) return;
+  DBI_LAUNCH(grp_expand_ranges_kernel, (unsigned)n_tiles, ET_THREADS, 0, s, cfg, cmask, (const uint64_t*)g_mass, g_pay,
+             g_eoff, n_groups, rg, o_mass, o_base, o_pat, long_list, long_count, long_cap, d_err);
+}
+
+void launch_grp_expand_ranges_long(const uint8_t* d_res, const DevTables* d_tb, const DigestCfg& cfg,
+                                   const uint32_t* u_gpos, const uint16_t* u_len, const double* g_mass,
+                                   const uint64_t* g_pay, const uint64_t* g_eoff, const ExpRanges& rg,
+                                   const uint32_t* long_list, const uint32_t* long_count, uint32_t n_listed,
+                                   double* o_mass, uint32_t* o_base, uint32_t* o_pat, cudaStream_t s) {
+  if (n_listed == 0) return;
+  unsigned grid = (n_listed + MD_WARPS - 1) / MD_WARPS;
+  if (grid > (unsigned)kNumSMsB200 * 4) grid = (unsigned)kNumSMsB200 * 4;
+  UniqView none;
+  std::memset(&none, 0, sizeof(none));
+  DBI_LAUNCH(grp_expand_long_kernel<true>, grid, MD_THREADS, 0, s, d_res, d_tb, cfg, u_gpos, u_len, nullptr, 0, none,
+             (const uint64_t*)g_mass, g_pay, g_eoff, long_list, long_count, 0, o_mass, o_base, o_pat, rg);
 }
 
 }  // namespace dbi

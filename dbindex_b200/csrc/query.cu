@@ -7,6 +7,7 @@
 #include <cassert>
 
 #include "kernels.cuh"
+#include "mods_common.cuh"
 
 namespace dbi {
 namespace {
@@ -379,6 +380,35 @@ __global__ void __launch_bounds__(Q_THREADS)
 constexpr uint8_t kLookupAbsent = 0, kLookupFound = 1, kLookupMalformed = 2;
 constexpr unsigned kFull = 0xffffffffu;
 
+// lookup_match_kernel<true>: the rank of the variant (sites pos[], of classes cls[]) in its group of
+// peptide gid, whose residues are q[0 .. len): K6x's block order over the site masks for peptides of up to 64
+// residues, K6l's lexicographic order of the site tuples for longer ones.
+__device__ __noinline__ uint64_t group_rank(const GroupView& gv, const DevTables* __restrict__ tb,
+                                            const uint8_t* __restrict__ q, uint32_t len, uint64_t gid, int k,
+                                            const int* pos, const int* cls) {
+  if (len <= 64) {
+    const uint64_t* cm = gv.cmask + gid * (uint64_t)gv.n_classes;
+    return group_entry_rank(k, pos, k > 0 ? cm[cls[0]] : 0ull, k > 1 ? cm[cls[1]] : 0ull, k > 2 ? cm[cls[2]] : 0ull,
+                            k > 3 ? cm[cls[3]] : 0ull);
+  }
+  // right to left over the sites; S[j] = chains of levels j .. k-1 on the sites seen so far.  A site x of
+  // level j's class between the row's sites of levels j-1 and j starts S[j + 1] tuples that precede the row's.
+  uint64_t S[DBI_MAX_MODS_PER_PEP + 1] = {};
+  S[k] = 1;
+  uint64_t rank = 0;
+  for (int x = (int)len - 1; x >= 0; --x) {
+    const uint8_t c = q[x];
+    if (!(__ldg(&tb->flags[c]) & kFlagDiffMod)) continue;
+    const int cl = __ldg(&tb->cls[c]);
+    for (int j = 0; j < k; ++j) {
+      if (cls[j] != cl) continue;
+      if (x < pos[j] && (j == 0 || x > pos[j - 1])) rank += S[j + 1];
+      S[j] += S[j + 1];
+    }
+  }
+  return rank;
+}
+
 // K11a: one warp per row.
 //  1. The row's mass in the index's own summation order: init_mass, the residues left to right (digest.cu), then
 //     the shift of every pattern position left to right (mods.cu, mods_grp.cu), so that it equals the indexed
@@ -391,6 +421,9 @@ constexpr unsigned kFull = 0xffffffffu;
 //     length; the warp compares its residues with the row's (lane j: positions j, j + 32, ...).  Unique
 //     peptides are distinct strings and a (peptide, pattern) pair is indexed once, so the first full match is
 //     the answer (a build with -DDBI_DEBUG walks the rest of the run and asserts that no second one exists).
+// kGroups (compact index): steps 2 and 3 run over the groups; a candidate group has the class sequence of the
+// row's pattern, and the entry is the group's first entry + the rank of the pattern in the group's order.
+template <bool kGroups>
 __global__ void __launch_bounds__(Q_THREADS)
     lookup_match_kernel(const uint8_t* __restrict__ res, const double* __restrict__ e_mass, uint64_t n_entries,
                         const uint32_t* __restrict__ e_base, uint64_t ent_off, const uint32_t* __restrict__ e_pat,
@@ -398,7 +431,7 @@ __global__ void __launch_bounds__(Q_THREADS)
                         int max_mods, const uint8_t* __restrict__ q_res, const uint64_t* __restrict__ q_off,
                         const uint32_t* __restrict__ q_pat, uint64_t n, uint8_t* __restrict__ o_status,
                         double* __restrict__ o_mass, uint64_t* __restrict__ o_entry, uint32_t* __restrict__ o_np,
-                        unsigned long long* __restrict__ n_found) {
+                        unsigned long long* __restrict__ n_found, const GroupView gv, uint64_t* __restrict__ o_gid) {
   const uint64_t i = (uint64_t)blockIdx.x * HX_WARPS + (threadIdx.x >> 5);
   if (i >= n) return;  // warp-uniform
   const unsigned lane = lane_id();
@@ -406,6 +439,8 @@ __global__ void __launch_bounds__(Q_THREADS)
   const uint64_t len = q_off[i + 1] - q_off[i];
   const uint32_t pat = q_pat ? q_pat[i] : 0u;
   bool ok = len >= 1 && len <= DBI_MAX_PEP_LEN;
+  uint32_t row_seq = 0;  // kGroups: the class sequence of the pattern, its sites and their classes
+  int row_k = 0, row_pos[DBI_MAX_MODS_PER_PEP] = {}, row_cls[DBI_MAX_MODS_PER_PEP] = {};
   double m = init_mass;
   if (ok) {
     for (uint32_t c = 0; c < len; c += 32) {
@@ -416,6 +451,7 @@ __global__ void __launch_bounds__(Q_THREADS)
     }
     // mod pattern: byte k = position + 1 of the k-th modified residue, strictly ascending, zeros only at the end
     uint32_t prev = 0, n_mods = 0;
+    if constexpr (kGroups) row_seq = 0;
     bool ended = false;
     for (int k = 0; k < DBI_MAX_MODS_PER_PEP && ok; ++k) {
       const uint32_t b = (pat >> (8 * k)) & 0xFFu;
@@ -430,7 +466,13 @@ __global__ void __launch_bounds__(Q_THREADS)
       ok = (__ldg(&tb->flags[c]) & kFlagDiffMod) != 0;
       m = __dadd_rn(m, __ldg(&tb->diff[c]));
       prev = b;
+      if constexpr (kGroups) {  // heap numbering of class sequences: children of v are v * C + c + 1
+        row_cls[n_mods - 1] = __ldg(&tb->cls[c]);
+        row_pos[n_mods - 1] = (int)pos;
+        row_seq = row_seq * (uint32_t)gv.n_classes + row_cls[n_mods - 1] + 1u;
+      }
     }
+    if constexpr (kGroups) row_k = (int)n_mods;
   }
   if (!ok) {
     if (lane == 0) {
@@ -438,6 +480,7 @@ __global__ void __launch_bounds__(Q_THREADS)
       o_mass[i] = 0.0;
       o_entry[i] = UINT64_MAX;
       o_np[i] = 0;
+      if constexpr (kGroups) o_gid[i] = 0;
     }
     return;
   }
@@ -456,16 +499,25 @@ __global__ void __launch_bounds__(Q_THREADS)
 
   const unsigned long long mb = (unsigned long long)__double_as_longlong(m);
   const unsigned long long* e_bits = reinterpret_cast<const unsigned long long*>(e_mass);
-  uint64_t hit = UINT64_MAX;
+  uint64_t hit = UINT64_MAX, hit_gid = 0;
   uint32_t hit_np = 0;
   for (uint64_t e0 = first; e0 < n_entries; e0 += 32) {
     const uint64_t e = e0 + lane;
     const bool eq = e < n_entries && __ldg(e_bits + e) == mb;
-    bool cand = eq && (e_pat ? __ldg(e_pat + e) : 0u) == pat;
+    bool cand;
+    uint64_t gid = 0;
+    if constexpr (kGroups) {
+      const uint64_t pay = eq ? __ldg(gv.pay + e) : 0ull;
+      cand = eq && (((uint32_t)pay >> 27) & 31u) == row_seq;
+      gid = pay >> 32;
+    } else {
+      cand = eq && (e_pat ? __ldg(e_pat + e) : 0u) == pat;
+      if (cand) gid = e_base ? (uint64_t)__ldg(e_base + e) : ent_off + e;
+    }
     int r = 0;
     uint64_t row = 0;
     if (cand) {
-      r = uniq_owner(uv, e_base ? (uint64_t)__ldg(e_base + e) : ent_off + e, &row);
+      r = uniq_owner(uv, gid, &row);
       cand = uv.len[r][row] == len;
     }
     for (unsigned cm = __ballot_sync(kFull, cand); cm; cm &= cm - 1) {
@@ -480,6 +532,7 @@ __global__ void __launch_bounds__(Q_THREADS)
         assert(hit == UINT64_MAX);
 #endif
         hit = e0 + src;
+        hit_gid = __shfl_sync(kFull, gid, src);
         hit_np = (uint32_t)(uv.plo[cr][crow + 1] - uv.plo[cr][crow]);
 #ifndef DBI_DEBUG
         break;
@@ -491,7 +544,11 @@ __global__ void __launch_bounds__(Q_THREADS)
 #endif
     if (__ballot_sync(kFull, eq) != kFull) break;  // the run of equal mass bits ends in this step
   }
+  if constexpr (kGroups)
+    if (hit != UINT64_MAX) hit = __ldg(gv.eoff + hit) + group_rank(gv, tb, q, (uint32_t)len, hit_gid, row_k, row_pos,
+                                                                   row_cls);
   if (lane == 0) {
+    if constexpr (kGroups) o_gid[i] = hit_gid;
     o_status[i] = hit != UINT64_MAX ? kLookupFound : kLookupAbsent;
     o_mass[i] = m;
     o_entry[i] = hit;
@@ -634,11 +691,17 @@ void launch_lookup_match(const uint8_t* d_res, const double* e_mass, uint64_t n_
                          uint64_t ent_off, const uint32_t* e_pat, const UniqView& uv, const DevTables* d_tb,
                          double init_mass, int max_mods, const uint8_t* q_res, const uint64_t* q_off,
                          const uint32_t* q_pat, uint64_t n, uint8_t* o_status, double* o_mass, uint64_t* o_entry,
-                         uint32_t* o_np, unsigned long long* n_found, cudaStream_t s) {
+                         uint32_t* o_np, unsigned long long* n_found, const GroupView* gv, uint64_t* o_gid,
+                         cudaStream_t s) {
   if (n == 0) return;
   const unsigned grid = (unsigned)((n + HX_WARPS - 1) / HX_WARPS);
-  DBI_LAUNCH(lookup_match_kernel, grid, Q_THREADS, 0, s, d_res, e_mass, n_entries, e_base, ent_off, e_pat, uv, d_tb,
-             init_mass, max_mods, q_res, q_off, q_pat, n, o_status, o_mass, o_entry, o_np, n_found);
+  if (gv)
+    DBI_LAUNCH(lookup_match_kernel<true>, grid, Q_THREADS, 0, s, d_res, e_mass, n_entries, e_base, ent_off, e_pat, uv,
+               d_tb, init_mass, max_mods, q_res, q_off, q_pat, n, o_status, o_mass, o_entry, o_np, n_found, *gv, o_gid);
+  else
+    DBI_LAUNCH(lookup_match_kernel<false>, grid, Q_THREADS, 0, s, d_res, e_mass, n_entries, e_base, ent_off, e_pat, uv,
+               d_tb, init_mass, max_mods, q_res, q_off, q_pat, n, o_status, o_mass, o_entry, o_np, n_found,
+               GroupView{}, nullptr);
 }
 
 void launch_lookup_gather(const uint8_t* status, const uint64_t* entry, const uint32_t* e_base, uint64_t ent_off,

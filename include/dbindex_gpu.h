@@ -132,7 +132,7 @@ typedef struct dbi_stats {
    * same way; bench.py reports whichever of the two takes more of the build. */
   uint32_t exp_launches;
   float exp_ms;
-  uint32_t _pad;
+  uint32_t n_groups;       /* variant groups a compact index holds; 0 = entries expanded (DESIGN.md 2) */
   uint64_t exp_bytes_per_launch;
 } dbi_stats;
 
