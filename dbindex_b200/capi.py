@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import threading
 from typing import Optional
 
 import numpy as np
@@ -234,6 +235,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "dbi_params_add_diff_mod": (C.c_int, [pp, C.c_char_p, C.c_double]),
         "dbi_create": (C.c_int, [pp, C.POINTER(vp)]),
         "dbi_set_stream": (C.c_int, [vp, vp]),
+        "dbi_view_open": (C.c_int, [vp, C.POINTER(vp)]),
         "dbi_add_proteins": (C.c_int, [vp, vp, vp, C.c_uint32]),
         "dbi_upload": (C.c_int, [vp]),
         "dbi_reset_index": (C.c_int, [vp]),
@@ -292,7 +294,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
 
 ABI_SYMBOLS = [
     "dbi_default_params", "dbi_params_add_static_mod", "dbi_params_set_enzyme", "dbi_params_add_diff_mod",
-    "dbi_create", "dbi_set_stream", "dbi_add_proteins", "dbi_upload", "dbi_reset_index", "dbi_build",
+    "dbi_create", "dbi_set_stream", "dbi_view_open", "dbi_add_proteins", "dbi_upload", "dbi_reset_index", "dbi_build",
     "dbi_stats_get", "dbi_save", "dbi_load", "dbi_query", "dbi_query_device", "dbi_fetch", "dbi_query_hits", "dbi_query_hits_device", "dbi_query_hits_read",
     "dbi_search_unindexed", "dbi_query_spectra", "dbi_search_unindexed_spectra",
     "dbi_lookup_peptides", "dbi_lookup_peptides_read", "dbi_host_alloc", "dbi_host_free", "dbi_get_protein", "dbi_calculate_mass",
@@ -389,15 +391,26 @@ def pack_peptides(seqs):
 
 
 class GpuIndex:
-    """One dbi_handle: a peptide index in the HBM of one GPU."""
+    """One dbi_handle: a peptide index in the HBM of one GPU.
+
+    Safe to share between threads: a per-object lock spans every call pair that leaves a pending result on the handle
+    and reads it back (query_hits, query_spectra, lookup_peptides, the unindexed searches), so those calls of
+    different threads run one after the other.  Threads that should query in parallel each open a view()."""
 
     def __init__(self, params: DbiParams):
         self.lib = load_library()
         self.params = params.copy()
+        self.lock = threading.RLock()
         h = C.c_void_p()
         rc = self.lib.dbi_create(C.byref(self.params), C.byref(h))
         self._h = h if rc == 0 else None
         self._check(rc)
+
+    def view(self) -> "GpuView":
+        """dbi_view_open: a GpuIndex over this built index with its own stream, scratch and pending results, for one
+        more thread that queries in parallel with this object and its other views.  A context manager; close()
+        destroys the view.  While views are open this index refuses to change (DBI_EINVAL)."""
+        return GpuView(self)
 
     def _check(self, rc: int):
         if rc != 0:
@@ -524,8 +537,9 @@ class GpuIndex:
         lo = np.ascontiguousarray(lo, dtype=np.float64)
         hi = np.ascontiguousarray(hi, dtype=np.float64)
         cnt = DbiHitCounts()
-        self._check(self.lib.dbi_query_hits(self._h, _ptr(lo), _ptr(hi), len(lo), C.byref(cnt)))
-        return self._read_hits(cnt, fields, alloc, per_hit)
+        with self.lock:
+            self._check(self.lib.dbi_query_hits(self._h, _ptr(lo), _ptr(hi), len(lo), C.byref(cnt)))
+            return self._read_hits(cnt, fields, alloc, per_hit)
 
     def search_unindexed_begin(self, lo: np.ndarray, hi: np.ndarray, max_candidates: int = 0) -> DbiHitCounts:
         """dbi_search_unindexed alone: the hits stay in HBM until query_hits_read / the next call.  Raises DbiError
@@ -535,9 +549,10 @@ class GpuIndex:
         if len(lo) != len(hi):
             raise ValueError(f"{len(lo)} lower and {len(hi)} upper bounds")
         cnt, n_cand = DbiHitCounts(), C.c_uint64(0)
-        rc = self.lib.dbi_search_unindexed(self._h, _ptr(lo), _ptr(hi), len(lo), int(max_candidates), C.byref(cnt),
-                                           C.byref(n_cand))
-        self.last_candidates = n_cand.value
+        with self.lock:
+            rc = self.lib.dbi_search_unindexed(self._h, _ptr(lo), _ptr(hi), len(lo), int(max_candidates),
+                                               C.byref(cnt), C.byref(n_cand))
+            self.last_candidates = n_cand.value
         if rc != 0:
             raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
         return cnt
@@ -547,7 +562,8 @@ class GpuIndex:
         """dbi_search_unindexed + dbi_query_hits_read: what query_hits returns for these ranges, answered from the
         proteins added so far without a built index (the handle stays unbuilt).  The candidate records of the
         call are in self.last_candidates."""
-        return self._read_hits(self.search_unindexed_begin(lo, hi, max_candidates), fields, alloc, per_hit)
+        with self.lock:
+            return self._read_hits(self.search_unindexed_begin(lo, hi, max_candidates), fields, alloc, per_hit)
 
     def query_spectra(self, mass, tol, range_off=None, tol_mode: int = DBI_TOL_DA, index_factor: int = 0,
                       fields=None, alloc=None, per_hit: bool = True) -> dict:
@@ -557,9 +573,10 @@ class GpuIndex:
         getSequencesUsingPPMTolerance.  index_factor: the bucket rule of the reference (0 = off)."""
         mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
         cnt = DbiHitCounts()
-        self._check(self.lib.dbi_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
-                                               int(index_factor), C.byref(cnt)))
-        return self._read_hits(cnt, fields, alloc, per_hit)
+        with self.lock:
+            self._check(self.lib.dbi_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
+                                                   int(index_factor), C.byref(cnt)))
+            return self._read_hits(cnt, fields, alloc, per_hit)
 
     def search_unindexed_spectra(self, mass, tol, range_off=None, tol_mode: int = DBI_TOL_DA, index_factor: int = 0,
                                  max_candidates: int = 0, fields=None, alloc=None, per_hit: bool = True) -> dict:
@@ -568,13 +585,14 @@ class GpuIndex:
         candidate records of the call are in self.last_candidates."""
         mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
         cnt, n_cand = DbiHitCounts(), C.c_uint64(0)
-        rc = self.lib.dbi_search_unindexed_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
-                                                   int(index_factor), int(max_candidates), C.byref(cnt),
-                                                   C.byref(n_cand))
-        self.last_candidates = n_cand.value
-        if rc != 0:
-            raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
-        return self._read_hits(cnt, fields, alloc, per_hit)
+        with self.lock:
+            rc = self.lib.dbi_search_unindexed_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n,
+                                                       int(tol_mode), int(index_factor), int(max_candidates),
+                                                       C.byref(cnt), C.byref(n_cand))
+            self.last_candidates = n_cand.value
+            if rc != 0:
+                raise DbiError(rc, (self.lib.dbi_last_error() or b"").decode(errors="replace"), n_cand.value)
+            return self._read_hits(cnt, fields, alloc, per_hit)
 
     def mg_spectra_stops(self, mass, ppm, split_mass, rank: int, world: int, index_factor: int = 0) -> np.ndarray:
         """dbi_mg_spectra_stops: K_r of every PPM spectrum (mass[s] at ppm[s]) on this built handle as rank `rank` of
@@ -594,9 +612,10 @@ class GpuIndex:
         mass, tol, range_off, n = spectra_arrays(mass, tol, range_off, tol_mode)
         stop = None if stop is None else np.ascontiguousarray(stop, dtype=np.uint64)
         cnt = DbiHitCounts()
-        self._check(self.lib.dbi_mg_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n, int(tol_mode),
-                                                  int(index_factor), _ptr(stop), C.byref(cnt)))
-        return self._read_hits(cnt, fields, alloc, per_hit)
+        with self.lock:
+            self._check(self.lib.dbi_mg_query_spectra(self._h, _ptr(mass), _ptr(tol), _ptr(range_off), n,
+                                                      int(tol_mode), int(index_factor), _ptr(stop), C.byref(cnt)))
+            return self._read_hits(cnt, fields, alloc, per_hit)
 
     def _read_hits(self, cnt: DbiHitCounts, fields, alloc, per_hit: bool) -> dict:
         out, bufs = {"counts": cnt}, DbiHitBuffers()
@@ -638,7 +657,8 @@ class GpuIndex:
         (residues, offsets) pair) and mod pattern (byte k = position + 1 of the k-th modified residue; None = all
         unmodified) whether the index holds it (status: LOOKUP_ABSENT / _FOUND / _MALFORMED), its mass, index entry,
         first occurrence and protein ids (CSR prot_list_off / prot_ids), as numpy arrays."""
-        return self.lookup_peptides_read(self.lookup_peptides_begin(seqs, modpat))
+        with self.lock:
+            return self.lookup_peptides_read(self.lookup_peptides_begin(seqs, modpat))
 
     def entry_keys(self) -> np.ndarray:
         n = C.c_uint64(0)
@@ -676,3 +696,19 @@ class GpuIndex:
 
     def kernel_launches(self) -> int:
         return int(self.lib.dbi_kernel_launches())
+
+
+class GpuView(GpuIndex):
+    """A query view of a built GpuIndex (dbi_view_open): the same index, no copy, with its own CUDA stream, scratch
+    and pending results.  Answers every query exactly as the owner does and refuses the calls that would change the
+    index.  The owner's index memory lives until the last view is closed, even when the owner is closed first."""
+
+    def __init__(self, owner: GpuIndex):
+        self.lib = owner.lib
+        self.params = owner.params
+        self.lock = threading.RLock()
+        self.owner = owner
+        h = C.c_void_p()
+        rc = self.lib.dbi_view_open(owner._h, C.byref(h))
+        self._h = h if rc == 0 else None
+        self._check(rc)

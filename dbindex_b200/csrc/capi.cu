@@ -19,6 +19,7 @@
 namespace dbi {
 
 std::atomic<uint64_t> g_kernel_launches{0};
+thread_local uint64_t t_kernel_launches = 0;
 static thread_local char t_err[512] = "";
 
 void set_error(const char* fmt, ...) {
@@ -277,6 +278,13 @@ struct dbi_handle {
     return ev_pool[ev_used++];
   }
 
+  // query views (dbi_view_open): a view names its owner; an owner counts its open views and, when destroyed while
+  // some are open, lives on (orphaned) until the last of them is destroyed
+  dbi_handle* owner = nullptr;
+  std::atomic<int> n_views{0};
+  std::mutex view_mu;  // guards the last-view / orphaned hand-over
+  bool orphaned = false;
+
   const double* entry_mass() const { return e_mass.p ? e_mass.as<double>() : u_mass.as<double>(); }
   const uint32_t* entry_base() const { return e_base.as<uint32_t>(); }
   const uint32_t* entry_pat() const { return e_pat.as<uint32_t>(); }
@@ -332,6 +340,23 @@ struct ArenaFlush {
   try {                                       \
     DBI_CUDA(cudaSetDevice((h)->device));
 
+// A call that only an owner may make: one that changes the proteins or the index, or joins several handles.
+#define DBI_OWNER_ONLY(h)                                                        \
+  if ((h)->owner) {                                                              \
+    set_error("%s is not available on a query view (dbi_view_open)", __func__); \
+    return DBI_EINVAL;                                                           \
+  }
+
+// A call that changes the residues, the candidate index or the index tables: refused on a view, and on an owner
+// while views of it are open (they read the same memory).  After DBI_API_BEGIN, so under the owner's mutex,
+// which dbi_view_open holds too.
+#define DBI_MUTATES(h)                                           \
+  DBI_OWNER_ONLY(h)                                              \
+  if (const int nv_ = (h)->n_views.load()) {                     \
+    set_error("%s: %d views open on this handle", __func__, nv_); \
+    return DBI_EINVAL;                                           \
+  }
+
 #define DBI_API_END                              \
   }                                              \
   catch (const CudaError& e) { return fail_cuda(e); } \
@@ -356,14 +381,14 @@ struct Stage {
   uint64_t l0;
   cudaEvent_t a = nullptr;
   Stage(dbi_handle* h_, int id_) : h(h_), id(id_) {
-    l0 = g_kernel_launches.load();
+    l0 = t_kernel_launches;
     if (h->p.profile) {
       a = h->get_event();
       cudaEventRecord(a, h->stream);
     }
   }
   ~Stage() {  // never throws: a failed event creation only loses this stage's timing
-    h->st.stage_launches[id] += (uint32_t)(g_kernel_launches.load() - l0);
+    h->st.stage_launches[id] += (uint32_t)(t_kernel_launches - l0);
     if (h->p.profile && a) {
       try {
         cudaEvent_t b = h->get_event();
@@ -1209,6 +1234,53 @@ void expand_ranges(dbi_handle* h, const ExpRanges& rg, uint64_t n_tiles, uint64_
 
 void mg_release(dbi_handle* h);  // capi_mg.inl
 
+// A view runs the query helpers unchanged: it borrows every index buffer of its owner and copies the scalars that
+// describe the index, next to its own stream, arena, d_err, pending results and stats.  The owner is pinned while
+// views are open (DBI_MUTATES), so none of this can go stale.  The windows keep only their peer mappings: a view
+// reads the other ranks' tables as its owner does, and never hands a window back (mg_release).
+void view_share_index(dbi_handle* v, const dbi_handle* o) {
+  using Buf = DevBuf dbi_handle::*;
+  const Buf bufs[] = {
+      &dbi_handle::d_tables, &dbi_handle::d_res,   &dbi_handle::d_pstart, &dbi_handle::u_mass, &dbi_handle::u_gpos,
+      &dbi_handle::u_prot,   &dbi_handle::u_len,   &dbi_handle::u_plo,    &dbi_handle::plist,  &dbi_handle::e_mass,
+      &dbi_handle::e_base,   &dbi_handle::e_pat,   &dbi_handle::u_cmask,  &dbi_handle::d_nlong, &dbi_handle::g_mass,
+      &dbi_handle::g_pay,    &dbi_handle::g_eoff};
+  for (auto b : bufs) (v->*b).borrow((o->*b).p, (o->*b).bytes);
+  v->built = o->built;
+  v->packed_prot = o->packed_prot;
+  v->res_end = o->res_end;
+  v->res_alloc = o->res_alloc;
+  v->n_emitted = o->n_emitted;
+  v->n_unique = o->n_unique;
+  v->n_entries = o->n_entries;
+  v->cmask_n = o->cmask_n;
+  v->n_groups = o->n_groups;
+  v->n_long = o->n_long;
+  v->mg_rank = o->mg_rank;
+  v->mg_world = o->mg_world;
+  for (int w = 0; w < 3; ++w) {
+    std::memcpy(v->win[w].peer, o->win[w].peer, sizeof(o->win[w].peer));
+    std::memcpy(v->win[w].peer_cap, o->win[w].peer_cap, sizeof(o->win[w].peer_cap));
+  }
+  std::memcpy(v->prot_off, o->prot_off, sizeof(o->prot_off));
+  std::memcpy(v->pos_off, o->pos_off, sizeof(o->pos_off));
+  v->mg_layout = o->mg_layout;
+  v->ent_base_off = o->ent_base_off;
+  std::memcpy(v->uoff, o->uoff, sizeof(o->uoff));
+  std::memcpy(v->uniq_cap, o->uniq_cap, sizeof(o->uniq_cap));
+  std::memcpy(v->mg_thr, o->mg_thr, sizeof(o->mg_thr));
+  std::memcpy(v->mg_nthr, o->mg_nthr, sizeof(o->mg_nthr));
+  v->cfg = o->cfg;
+  v->shifts = o->shifts;
+  // the owner's index counters; the launches, bytes and times are the view's own
+  v->st = o->st;
+  std::memset(v->st.algo_bytes, 0, sizeof(v->st.algo_bytes));
+  std::memset(v->st.stage_ms, 0, sizeof(v->st.stage_ms));
+  std::memset(v->st.stage_launches, 0, sizeof(v->st.stage_launches));
+  v->st.dom_ms = v->st.exp_ms = 0;
+  v->st.dom_launches = v->st.exp_launches = 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1273,6 +1345,46 @@ int dbi_create(const dbi_params* params, dbi_handle** out) {
   }
 }
 
+int dbi_view_open(dbi_handle* h, dbi_handle** view) {
+  if (!view) {
+    set_error("null argument");
+    return DBI_EINVAL;
+  }
+  *view = nullptr;
+  DBI_API_BEGIN(h)
+  if (h->owner) {
+    set_error("a view of a view: open views on the owner");
+    return DBI_EINVAL;
+  }
+  if (!h->built) {
+    set_error("Indexer is not initialized: a view needs a built index");
+    return DBI_ENOTINIT;
+  }
+  dbi_handle* v = new dbi_handle();
+  try {
+    v->p = h->p;
+    v->device = h->device;
+    DBI_CUDA(cudaStreamCreateWithFlags(&v->own_stream, cudaStreamNonBlocking));
+    v->stream = v->own_stream;
+    v->arena.device = v->device;
+    v->d_err.alloc(4, v->arena);
+    DBI_CUDA(cudaMemsetAsync(v->d_err.p, 0, 4, v->stream));
+    DBI_CUDA(cudaStreamSynchronize(v->stream));
+  } catch (...) {
+    dbi_destroy(v);  // nothing borrowed yet: torn down like a fresh handle
+    throw;
+  }
+  view_share_index(v, h);
+  v->owner = h;
+  {
+    std::lock_guard<std::mutex> lk(h->view_mu);
+    h->n_views.fetch_add(1);
+  }
+  *view = v;
+  return DBI_OK;
+  DBI_API_END
+}
+
 int dbi_set_stream(dbi_handle* h, void* cuda_stream) {
   DBI_API_BEGIN(h)
   DBI_CUDA(cudaStreamSynchronize(h->stream));
@@ -1283,6 +1395,7 @@ int dbi_set_stream(dbi_handle* h, void* cuda_stream) {
 
 int dbi_add_proteins(dbi_handle* h, const uint8_t* residues, const uint64_t* offsets, uint32_t n) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   if (h->built) {
     set_error("index already built");  // "Already intialized", DBIndexStoreSQLiteMult.java:97-99
     return DBI_EALREADY;
@@ -1330,6 +1443,7 @@ int dbi_add_proteins(dbi_handle* h, const uint8_t* residues, const uint64_t* off
 
 int dbi_upload(dbi_handle* h) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   ensure_uploaded(h);
   DBI_CUDA(cudaStreamSynchronize(h->stream));
   return DBI_OK;
@@ -1338,6 +1452,7 @@ int dbi_upload(dbi_handle* h) {
 
 int dbi_reset_index(dbi_handle* h) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   free_index(h);
   DBI_CUDA(cudaStreamSynchronize(h->stream));
   return DBI_OK;
@@ -1346,6 +1461,7 @@ int dbi_reset_index(dbi_handle* h) {
 
 int dbi_build(dbi_handle* h) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   if (h->built) {
     set_error("index already built");
     return DBI_EALREADY;
@@ -1419,6 +1535,7 @@ int dbi_build(dbi_handle* h) {
 int dbi_build_from_records(dbi_handle* h, const double* mass, const uint32_t* prot, const uint32_t* off,
                            const uint16_t* len, uint64_t n) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   if (h->built) {
     set_error("index already built");
     return DBI_EALREADY;
@@ -2137,6 +2254,7 @@ int dbi_query_hits_read(dbi_handle* h, const dbi_hit_buffers* out) {
 int dbi_search_unindexed(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, uint64_t max_candidates,
                          dbi_hit_counts* counts, uint64_t* n_candidates) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   if (int rc = check_unindexed(h)) return rc;
   if (!counts || (nq && (!lo || !hi))) {
     set_error("null argument");
@@ -2171,6 +2289,7 @@ int dbi_search_unindexed_spectra(dbi_handle* h, const double* mass, const double
                                  uint64_t n_spectra, int tol_mode, int index_factor, uint64_t max_candidates,
                                  dbi_hit_counts* counts, uint64_t* n_candidates) {
   DBI_API_BEGIN(h)
+  DBI_MUTATES(h)
   if (int rc = check_unindexed(h)) return rc;
   if (int rc = check_spectra(mass, tol, range_off, n_spectra, tol_mode, index_factor, counts)) return rc;
   drop_results(h);
@@ -2353,6 +2472,7 @@ int dbi_get_protein(dbi_handle* h, uint32_t id, const uint8_t** residues, uint64
     set_error("null argument");
     return DBI_EINVAL;
   }
+  if (h->owner) h = h->owner;  // the host copy is built lazily, once, by the owner under its mutex
   std::lock_guard<std::mutex> lk(h->mu);
   if ((uint64_t)id + 1 >= h->h_off.size()) {
     set_error("protein id %u out of range", id);
@@ -2430,6 +2550,7 @@ int dbi_entry_keys(dbi_handle* h, int32_t* keys, uint64_t capacity, uint64_t* n_
 int dbi_debug_emitted(dbi_handle* h, uint64_t capacity, double* mass, uint32_t* prot, uint32_t* off, uint16_t* len,
                       uint64_t* n) {
   DBI_API_BEGIN(h)
+  DBI_OWNER_ONLY(h)
   if (!h->built || !h->p.keep_emitted) {
     set_error("emitted records were not kept (params.keep_emitted) or the index is not built");
     return DBI_ENOTINIT;
@@ -2460,6 +2581,7 @@ int dbi_debug_emitted(dbi_handle* h, uint64_t capacity, double* mass, uint32_t* 
 
 int dbi_debug_radix_sort(dbi_handle* h, uint64_t* keys, uint64_t* vals, uint64_t n, int begin_bit, int end_bit) {
   DBI_API_BEGIN(h)
+  DBI_OWNER_ONLY(h)
   if (n == 0) return DBI_OK;
   if (!keys || !vals || begin_bit < 0 || end_bit > 64 || end_bit < begin_bit) {
     set_error("bad argument");
@@ -2486,10 +2608,18 @@ int dbi_debug_radix_sort(dbi_handle* h, uint64_t* keys, uint64_t* vals, uint64_t
 
 void dbi_destroy(dbi_handle* h) {
   if (!h) return;
+  dbi_handle* owner = h->owner;
+  if (!owner) {  // the index memory lives until the last view is destroyed
+    std::lock_guard<std::mutex> lk(h->view_mu);
+    if (h->n_views.load()) {
+      h->orphaned = true;
+      return;
+    }
+  }
   cudaSetDevice(h->device);
   cudaStreamSynchronize(h->stream);
-  free_index(h);
-  mg_release(h);
+  free_index(h);  // on a view: forgets the borrowed buffers
+  if (!owner) mg_release(h);
   h->d_raw.release();
   h->d_off.release();
   h->mg_wtab.release();
@@ -2505,6 +2635,14 @@ void dbi_destroy(dbi_handle* h) {
   }
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   delete h;
+  if (owner) {
+    bool last = false;
+    {
+      std::lock_guard<std::mutex> lk(owner->view_mu);
+      last = owner->n_views.fetch_sub(1) == 1 && owner->orphaned;
+    }
+    if (last) dbi_destroy(owner);
+  }
 }
 
 int dbi_release_cached_memory(int device) {

@@ -15,6 +15,9 @@ namespace dbi {
 // ---- error plumbing --------------------------------------------------------
 void set_error(const char* fmt, ...);
 extern std::atomic<uint64_t> g_kernel_launches;
+// the same count for the calling thread only: a handle's stage counters stay exact while other handles or
+// views launch from other threads
+extern thread_local uint64_t t_kernel_launches;
 
 struct CudaError {
   cudaError_t e;
@@ -34,6 +37,7 @@ struct CudaError {
   do {                                                                      \
     kernel<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__);             \
     ::dbi::g_kernel_launches.fetch_add(1, std::memory_order_relaxed);       \
+    ++::dbi::t_kernel_launches;                                             \
     DBI_CUDA(cudaGetLastError());                                           \
   } while (0)
 

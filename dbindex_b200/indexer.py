@@ -16,6 +16,7 @@ under ``java/`` is the same logic in the reference's own language (INTEGRATION.m
 from __future__ import annotations
 
 import os
+import threading
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Set, Tuple
 
@@ -380,6 +381,12 @@ class DBIndexer:
         self.index: Optional[GpuIndex] = None
         self.deflines: List[str] = []   # ProteinCache.defs
         self._seq_cache: dict = {}
+        # Search-engine threads query a built index through one view each (dbi_view_open), so their calls run in
+        # parallel; the unindexed and sharded searches go through the owner handles, one thread at a time.
+        self._tls = threading.local()
+        self._views: List[GpuIndex] = []
+        self._views_lock = threading.Lock()
+        self._owner_lock = threading.Lock()
 
     # -- lifecycle: init() (DBIndexer.java:412) -> run() (:508) --------------------------
     def init(self):
@@ -474,6 +481,10 @@ class DBIndexer:
             raise DBIndexerException(str(e)) from e
 
     def close(self):
+        with self._views_lock:
+            for v in self._views:
+                v.close()
+            self._views = []
         for g in self.shards or ([self.index] if self.index is not None else []):
             g.close()
         self.index = None
@@ -500,13 +511,24 @@ class DBIndexer:
         nb = self.index_factor
         return int(lo) // bucket_range > nb - 1 or int(hi) // bucket_range > nb - 1
 
+    def _view(self) -> GpuIndex:
+        """The calling thread's view of the built index, opened on its first query."""
+        t = self._tls
+        if getattr(t, "owner", None) is not self.index:
+            v = self.index.view()
+            with self._views_lock:
+                self._views.append(v)
+            t.owner, t.view = self.index, v
+        return t.view
+
     def _hits(self, lo: np.ndarray, hi: np.ndarray) -> dict:
         """The hit source of every getSequences*: one record per hit of every [lo[i], hi[i]] (query_hits), from
         the index, or in unindexed mode from the proteins (chunked dbi_search_unindexed)."""
         try:
             if self.use_index:
-                return self.index.query_hits(lo, hi)
-            return search_unindexed_chunked(self._searcher, lo, hi, self.max_candidates)
+                return self._view().query_hits(lo, hi)
+            with self._owner_lock:
+                return search_unindexed_chunked(self._searcher, lo, hi, self.max_candidates)
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
 
@@ -515,9 +537,10 @@ class DBIndexer:
         the chunked dbi_search_unindexed_spectra), the bucket rule of this index_factor applied on the device."""
         try:
             if self.use_index:
-                return self.index.query_spectra(mass, tol, range_off, tol_mode, self.index_factor)
-            return search_unindexed_spectra_chunked(self._searcher, mass, tol, range_off, tol_mode, self.index_factor,
-                                                    self.max_candidates)
+                return self._view().query_spectra(mass, tol, range_off, tol_mode, self.index_factor)
+            with self._owner_lock:
+                return search_unindexed_spectra_chunked(self._searcher, mass, tol, range_off, tol_mode,
+                                                        self.index_factor, self.max_candidates)
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
 
@@ -640,7 +663,7 @@ class DBIndexer:
         if not self.use_index:
             return self._proteins_unindexed(seqs)
         try:
-            r = self.index.lookup_peptides(list(seqs))
+            r = self._view().lookup_peptides(list(seqs))
         except DbiError as e:
             raise DBIndexStoreException(str(e)) from e
         plo = r["prot_list_off"].astype(np.int64)

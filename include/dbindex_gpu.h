@@ -178,6 +178,45 @@ int dbi_create(const dbi_params* params, dbi_handle** out);
  * and copy of this handle; NULL = the handle's own stream. */
 int dbi_set_stream(dbi_handle* h, void* cuda_stream);
 
+/* ---- threads and query views ----------------------------------------------
+ * Calls on one handle are serialised by the handle's mutex; calls on different
+ * handles or views may run at the same time from different threads.  A pending
+ * result (dbi_query_hits, dbi_lookup_peptides) belongs to the handle or view
+ * that made it, so a begin / read pair on a handle shared between threads needs
+ * a lock of the caller's around both calls.
+ *
+ * A VIEW of a built handle is a dbi_handle that shares the handle's index (no
+ * copy) but has its own CUDA stream (non-blocking), scratch arena, mutex,
+ * pending hit result, pending lookup result, error flag and query stats.  The
+ * search-engine threads of the reference (DBIndexer.java:468-469) each open one
+ * and then query in parallel.  Closed with dbi_destroy(view).
+ *
+ * - Views accept dbi_query, dbi_query_device, dbi_fetch, dbi_query_hits,
+ *   dbi_query_hits_device, dbi_query_hits_read, dbi_query_spectra,
+ *   dbi_lookup_peptides, dbi_lookup_peptides_read, dbi_entry_keys,
+ *   dbi_stats_get, dbi_set_stream, dbi_calculate_mass, dbi_get_protein,
+ *   dbi_mg_slices and dbi_mg_split_masses.  Every answer is byte-identical to
+ *   the owner's answer to the same call: on a single-GPU index, a compact
+ *   index and one rank of a sharded index (the view reads the other ranks'
+ *   window 2 as the owner does).  dbi_get_protein is answered by the owner
+ *   under the owner's mutex.
+ * - Views refuse (DBI_EINVAL) every call that changes the proteins or the
+ *   index or runs across several handles: dbi_add_proteins, dbi_upload,
+ *   dbi_reset_index, dbi_build, dbi_build_from_records, dbi_save, dbi_load,
+ *   dbi_search_unindexed, dbi_search_unindexed_spectra, every dbi_mg_* staging
+ *   and rank-level call, the dbi_mg_*_local calls and dbi_debug_*.  A view of a
+ *   view is DBI_EINVAL; a view of an unbuilt handle is DBI_ENOTINIT.
+ * - The owner keeps answering queries while views are open, but is pinned:
+ *   the calls of that list that change its residues, candidate index or index
+ *   tables return DBI_EINVAL ("n views open") until the last view is closed.
+ * - dbi_destroy(owner) does not wait for its views: the index memory lives
+ *   until the last view is destroyed, and the views keep answering until then.
+ * - dbi_stats_get on a view reports the owner's index counters (n_*,
+ *   device_bytes, n_groups, sort bits) with the view's own launches,
+ *   algorithmic bytes and (params.profile) times; calls on a view leave the
+ *   owner's stats alone. */
+int dbi_view_open(dbi_handle* h, dbi_handle** view);
+
 /* The per-protein body of DBIndexer.run() (DBIndexer.java:600-616):
  * ProteinCache.addProtein (ProteinCache.java:84-95) for n proteins whose
  * residues are concatenated in `residues`, protein i occupying

@@ -83,6 +83,8 @@ public final class DbiNative {
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_DOUBLE));
 	static final MethodHandle dbi_abi_sizes = h("dbi_abi_sizes", FunctionDescriptor.ofVoid(ADDRESS, ADDRESS));
 	static final MethodHandle dbi_create = h("dbi_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
+	// a query view of a built handle: same index, own stream, scratch and pending results (one per thread)
+	static final MethodHandle dbi_view_open = h("dbi_view_open", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
 	static final MethodHandle dbi_add_proteins = h("dbi_add_proteins",
 			FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT));
 	static final MethodHandle dbi_build = h("dbi_build", FunctionDescriptor.of(JAVA_INT, ADDRESS));

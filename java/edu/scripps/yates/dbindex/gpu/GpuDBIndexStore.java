@@ -54,6 +54,13 @@ public class GpuDBIndexStore implements DBIndexStore {
 	// proteins gathered by addProteinDef until stopAddSeq() (subsystem 1: packed residue buffer)
 	private final java.io.ByteArrayOutputStream residues = new java.io.ByteArrayOutputStream();
 	private final List<Long> offsets = new ArrayList<>(List.of(0L));
+	// Search-engine threads (DBIndexer.java:468-469) query the built index through views (dbi_view_open): one per
+	// thread and GPU, opened on the thread's first query, each with its own stream and pending results, so their
+	// calls run in parallel.  The paths that need the owner handles (the unindexed searches, the sharded spectrum
+	// batches) take ownerLock around every call pair, so no thread reads another one's pending result.
+	private final ThreadLocal<MemorySegment[]> views = new ThreadLocal<>();
+	private final java.util.concurrent.ConcurrentLinkedQueue<MemorySegment> openViews = new java.util.concurrent.ConcurrentLinkedQueue<>();
+	private final Object ownerLock = new Object();
 
 	public GpuDBIndexStore(DBIndexSearchParams sparam, boolean unindexed) {
 		this.sparam = sparam;
@@ -63,6 +70,32 @@ public class GpuDBIndexStore implements DBIndexStore {
 	private static void check(int rc) throws DBIndexStoreException {
 		if (rc != DbiNative.DBI_OK)
 			throw new DBIndexStoreException(DbiNative.lastError());
+	}
+
+	/** this thread's views of the built index, one per GPU (handles[d] -> views()[d]) */
+	private MemorySegment[] views() throws Throwable {
+		MemorySegment[] v = views.get();
+		if (v == null) {
+			v = new MemorySegment[handles.length];
+			try (Arena a = Arena.ofConfined()) {
+				final MemorySegment out = a.allocate(ADDRESS);
+				for (int d = 0; d < handles.length; ++d) {
+					final int rc = (int) DbiNative.dbi_view_open.invoke(handles[d], out);
+					if (rc != DbiNative.DBI_OK) {
+						final DBIndexStoreException e = new DBIndexStoreException(DbiNative.lastError());
+						for (int k = 0; k < d; ++k) {
+							openViews.remove(v[k]);
+							DbiNative.dbi_destroy.invoke(v[k]);
+						}
+						throw e;
+					}
+					v[d] = out.get(ADDRESS, 0);
+					openViews.add(v[d]);
+				}
+			}
+			views.set(v);
+		}
+		return v;
 	}
 
 	/** dbi_params from the live AssignMass / Enzyme / search parameters (SURVEY.md 5.1). */
@@ -323,19 +356,19 @@ public class GpuDBIndexStore implements DBIndexStore {
 					}
 				}
 				if (!l.isEmpty())
-					queryOn(handles[d], l.stream().mapToDouble(Double::doubleValue).toArray(),
+					queryOn(d, l.stream().mapToDouble(Double::doubleValue).toArray(),
 							h.stream().mapToDouble(Double::doubleValue).toArray(), ret);
 			}
 			return ret;
 		}
-		queryOn(handle, lo, hi, ret);
+		queryOn(0, lo, hi, ret);
 		return ret;
 	}
 
-	/** one dbi_query_hits + dbi_query_hits_read on one GPU; the hits are appended to ret */
-	private void queryOn(MemorySegment handle, double[] lo, double[] hi, List<IndexedSequence> ret)
-			throws DBIndexStoreException {
+	/** one dbi_query_hits + dbi_query_hits_read on this thread's view of GPU d; the hits are appended to ret */
+	private void queryOn(int d, double[] lo, double[] hi, List<IndexedSequence> ret) throws DBIndexStoreException {
 		try (Arena a = Arena.ofConfined()) {
+			final MemorySegment handle = views()[d];
 			final int nq = lo.length;
 			final MemorySegment dlo = a.allocate(JAVA_DOUBLE, nq), dhi = a.allocate(JAVA_DOUBLE, nq);
 			MemorySegment.copy(lo, 0, dlo, JAVA_DOUBLE, 0, nq);
@@ -391,6 +424,16 @@ public class GpuDBIndexStore implements DBIndexStore {
 
 	private void spectraChunk(double[] mass, double[] tol, long[] rangeOff, int tolMode, int[] ids, RunSink sink)
 			throws DBIndexStoreException {
+		if (unindexed || nDevices > 1)
+			synchronized (ownerLock) {
+				spectraChunkOn(mass, tol, rangeOff, tolMode, ids, sink);
+			}
+		else
+			spectraChunkOn(mass, tol, rangeOff, tolMode, ids, sink);
+	}
+
+	private void spectraChunkOn(double[] mass, double[] tol, long[] rangeOff, int tolMode, int[] ids, RunSink sink)
+			throws DBIndexStoreException {
 		try (Arena a = Arena.ofConfined()) {
 			final int n = ids.length;
 			long nr = 0;
@@ -416,9 +459,10 @@ public class GpuDBIndexStore implements DBIndexStore {
 			for (int d = 0; d < nDevices; ++d)
 				hs.setAtIndex(ADDRESS, d, handles[d]);
 			final int factor = sparam.getIndexFactor();
+			final MemorySegment[] readFrom = !unindexed && nDevices == 1 ? views() : handles;
 			if (!unindexed) {
 				if (nDevices == 1)
-					check((int) DbiNative.dbi_query_spectra.invoke(handle, dm, dt, dro, (long) n, tolMode, factor, cnt));
+					check((int) DbiNative.dbi_query_spectra.invoke(readFrom[0], dm, dt, dro, (long) n, tolMode, factor, cnt));
 				else
 					check((int) DbiNative.dbi_mg_query_spectra_local.invoke(hs, nDevices, dm, dt, dro, (long) n, tolMode,
 							factor, cnt));
@@ -444,7 +488,7 @@ public class GpuDBIndexStore implements DBIndexStore {
 			}
 			final long cb = DbiNative.HIT_COUNTS.byteSize();
 			for (int d = 0; d < nDevices; ++d) // every GPU answers for the mass slices it owns
-				readHits(handles[d], a, cnt.asSlice(d * cb, cb), ids, sink);
+				readHits(readFrom[d], a, cnt.asSlice(d * cb, cb), ids, sink);
 		} catch (final DBIndexStoreException e) {
 			throw e;
 		} catch (final Throwable t) {
@@ -483,7 +527,9 @@ public class GpuDBIndexStore implements DBIndexStore {
 		final int[] ids = new int[order.length];
 		for (int i = 0; i < ids.length; ++i)
 			ids[i] = order[i];
-		searchChunk(lo, hi, ids, sink);
+		synchronized (ownerLock) {
+			searchChunk(lo, hi, ids, sink);
+		}
 	}
 
 	private void searchChunk(double[] lo, double[] hi, int[] ids, RunSink sink) throws DBIndexStoreException {
@@ -612,7 +658,7 @@ public class GpuDBIndexStore implements DBIndexStore {
 			final MemorySegment r = a.allocate(Math.max(1, res.length));
 			MemorySegment.copy(res, 0, r, JAVA_BYTE, 0, res.length);
 			final boolean[] found = new boolean[n];
-			for (final MemorySegment h : handles) {
+			for (final MemorySegment h : views()) {
 				final MemorySegment cnt = a.allocate(DbiNative.LOOKUP_COUNTS);
 				check((int) DbiNative.dbi_lookup_peptides.invoke(h, r, off, MemorySegment.NULL, (long) n, cnt));
 				final long nIds = cnt.get(JAVA_LONG, 16);
@@ -763,6 +809,11 @@ public class GpuDBIndexStore implements DBIndexStore {
 	}
 
 	public void close() {
+		for (MemorySegment v; (v = openViews.poll()) != null;)
+			try {
+				DbiNative.dbi_destroy.invoke(v);
+			} catch (final Throwable ignored) {
+			}
 		for (final MemorySegment h : handles)
 			try {
 				if (h != null && !h.equals(MemorySegment.NULL))
