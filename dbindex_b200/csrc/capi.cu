@@ -149,6 +149,28 @@ struct DevBuf {
   T* as() const { return (T*)p; }
 };
 
+// Emitted records as they leave K4 (or arrive from the other GPUs).
+struct RecView {
+  const uint64_t* mass;  // IEEE bits
+  const uint32_t* gpos;
+  const uint32_t* prot;
+  const uint16_t* len;
+};
+
+// The device buffers of a set of emitted records.
+struct RecSet {
+  DevBuf mass, gpos, prot, len;  // mass as IEEE bits
+  void alloc(uint64_t n, DevArena& arena) {
+    mass.alloc(n * 8, arena);
+    gpos.alloc(n * 4, arena);
+    prot.alloc(n * 4, arena);
+    len.alloc(n * 2, arena);
+  }
+  void release() { mass.release(); gpos.release(); prot.release(); len.release(); }
+  void swap(RecSet& o) { mass.swap(o.mass); gpos.swap(o.gpos); prot.swap(o.prot); len.swap(o.len); }
+  RecView view() const { return {mass.as<uint64_t>(), gpos.as<uint32_t>(), prot.as<uint32_t>(), len.as<uint16_t>()}; }
+};
+
 inline uint64_t dbits(double d) {
   uint64_t u;
   std::memcpy(&u, &d, 8);
@@ -199,8 +221,7 @@ struct dbi_handle {
   // (n_groups + 1); n_groups = 0 when the entries are expanded.  n_long = peptides longer than 64 residues.
   DevBuf g_mass, g_pay, g_eoff;
   uint64_t n_groups = 0, n_long = 0;
-  // kept raw records (params.keep_emitted)
-  DevBuf k_mass, k_gpos, k_prot, k_len;
+  RecSet kept;  // kept raw records (params.keep_emitted)
 
   // ---- sharded build (dbi_mg_*, capi_mg.inl) ----
   // Three WINDOWS per rank are visible to the other ranks (mapped peer memory over NVLink):
@@ -228,7 +249,7 @@ struct dbi_handle {
   uint64_t ent_base_off = 0;  // global id of this rank's first unique peptide (0 on a single GPU)
   uint64_t uoff[kMaxRanks + 1] = {};      // global id of every rank's first unique peptide
   uint64_t uniq_cap[kMaxRanks] = {};      // layout capacity of every rank's window 2
-  DevBuf mg_mass, mg_gpos, mg_prot, mg_len;  // local records between digest and exchange
+  RecSet mg_rec;                             // local records between digest and exchange
   DevBuf mg_nmod, mg_wtab;                   // their mod-site counts, and variants of a peptide with n sites
   uint64_t mg_n = 0;
   DevBuf mg_vkey, mg_vpay;                   // local groups / variants between listing and exchange
@@ -443,6 +464,11 @@ uint32_t read_err(dbi_handle* h) {
   return e;
 }
 
+void clear_err(dbi_handle* h) {
+  const uint32_t zero = 0;
+  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, h->stream));
+}
+
 uint64_t read_u64(dbi_handle* h, const uint64_t* d) {
   uint64_t v = 0;
   DBI_CUDA(cudaMemcpyAsync(&v, d, 8, cudaMemcpyDeviceToHost, h->stream));
@@ -459,7 +485,7 @@ void free_tables(dbi_handle* h) {
   h->g_mass.release(); h->g_pay.release(); h->g_eoff.release();
   h->n_groups = h->n_long = 0;
   h->cmask_n = UINT64_MAX;
-  h->k_mass.release(); h->k_gpos.release(); h->k_prot.release(); h->k_len.release();
+  h->kept.release();
   h->n_emitted = h->n_unique = h->n_entries = 0;
 }
 
@@ -473,7 +499,7 @@ void drop_results(dbi_handle* h) {
 void free_sharded_tables(dbi_handle* h) {
   h->built = false;
   free_tables(h);
-  h->mg_mass.release(); h->mg_gpos.release(); h->mg_prot.release(); h->mg_len.release();
+  h->mg_rec.release();
   h->mg_nmod.release();
   h->mg_vkey.release(); h->mg_vpay.release();
   h->mg_n = h->mg_v = 0;
@@ -604,13 +630,63 @@ void pack_residues(dbi_handle* h) {
   h->st.algo_bytes[DBI_STAGE_PACK] += 2 * n_res + (uint64_t)n_prot * 12;
 }
 
-// Emitted records as they leave K4 (or arrive from the other GPUs).
-struct RecView {
-  const uint64_t* mass;  // IEEE bits
-  const uint32_t* gpos;
-  const uint32_t* prot;
-  const uint16_t* len;
+// The start of a single-GPU build: protein offsets on the device, error bits cleared, K1.
+void build_begin(dbi_handle* h) {
+  ensure_uploaded(h);
+  clear_err(h);
+  pack_residues(h);
+}
+
+// K2 (count) and K4 (emit) over the start positions of rg in tiles [t0, t0 + nt); with windows only the records
+// that can land in one of them (K2u / K4u).  Each kernel is charged 2 * span residue bytes.  The caller checks the
+// error bits and the record count between count() and emit().
+struct Digest {
+  dbi_handle* h;
+  DigestRange rg;
+  uint32_t t0, nt;
+  uint64_t span;
+  const MassWindows* windows;
+  DevBuf tile_counts, tile_offs, start_cnt;  // what K2 leaves for K4
+  uint64_t n = 0;
+
+  // K2 and the scan of its tile counts: the number of records K4 emits
+  uint64_t count() {
+    tile_counts.alloc((uint64_t)nt * 4, h->arena);
+    tile_offs.alloc(((uint64_t)nt + 1) * 8, h->arena);
+    start_cnt.alloc((uint64_t)nt * kDigestTile, h->arena);
+    if (!nt) return n = 0;
+    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
+    launch_digest_count(h->d_res.as<uint8_t>(), rg, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
+                        start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), h->stream, windows);
+    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), nt, tile_offs.as<uint64_t>(), h->stream);
+    n = read_u64(h, tile_offs.as<uint64_t>() + nt);
+    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2 * span + (uint64_t)nt * 16;
+    return n;
+  }
+  // K4 into out, allocated for the counted records; nmod (optional): their mod-site counts
+  void emit(RecSet& out, DevBuf* nmod) {
+    out.alloc(n, h->arena);
+    if (nmod) nmod->alloc(std::max<uint64_t>(n, 1), h->arena);
+    {
+      Stage sg(h, DBI_STAGE_DIGEST_EMIT);
+      launch_digest_emit(h->d_res.as<uint8_t>(), rg, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
+                         start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
+                         out.mass.as<uint64_t>(), out.gpos.as<uint32_t>(), out.prot.as<uint32_t>(),
+                         out.len.as<uint16_t>(), nmod ? nmod->as<uint8_t>() : nullptr, h->d_err.as<uint32_t>(),
+                         h->stream, windows);
+      h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2 * span + n * 18;
+    }
+    tile_counts.release();
+    tile_offs.release();
+    start_cnt.release();
+  }
 };
+
+// The digest of a single-GPU build or unindexed search: every start position, none when there are no windows.
+Digest whole_digest(dbi_handle* h, const MassWindows* windows) {
+  const uint32_t nt = windows && !windows->n ? 0u : (uint32_t)(((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile);
+  return {h, DigestRange{0u, h->res_end, 0u, (uint32_t)(h->h_off.size() - 1)}, 0u, nt, h->res_end, windows};
+}
 
 // Radix key of a mass: bits(mass) - bits(lo); every mass of a build lies in [lo, hi].
 struct KeySpace {
@@ -1147,6 +1223,23 @@ void finish_stats(dbi_handle* h) {
     h->st.device_bytes += h->g_mass.bytes + h->g_pay.bytes + h->g_eoff.bytes + h->u_cmask.bytes;
 }
 
+// The end of a single-GPU build: the index of the N records in recs, whose masses lie in [lo_mass, hi_mass].  A
+// failure leaves the handle unbuilt with its proteins; params.keep_emitted keeps the records.
+int build_end(dbi_handle* h, RecSet& recs, uint64_t N, double lo_mass, double hi_mass) {
+  int rc = index_records(h, recs.view(), N, lo_mass, hi_mass);
+  TR("index_records");
+  if (rc == DBI_OK) rc = check_err_bits(read_err(h));
+  if (rc != DBI_OK) {
+    free_index(h);
+    return rc;
+  }
+  if (h->p.keep_emitted) h->kept.swap(recs);
+  DBI_CUDA(cudaStreamSynchronize(h->stream));
+  finish_stats(h);
+  TR("final_sync");
+  return DBI_OK;
+}
+
 // The unique-peptide tables a fetch resolves base peptides through: this GPU's own, and in a
 // sharded build the mapped tables of every connected rank.
 UniqView uniq_view(dbi_handle* h) {
@@ -1466,67 +1559,20 @@ int dbi_build(dbi_handle* h) {
     set_error("index already built");
     return DBI_EALREADY;
   }
-  cudaStream_t s = h->stream;
   TR("begin");
-  ensure_uploaded(h);
-  const uint32_t zero = 0;
-  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, s));
-  pack_residues(h);
+  build_begin(h);
   TR("pack");
-
-  const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
-  const uint64_t tiles = ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile;
-  DevBuf tile_counts, tile_offs, start_cnt;
-  tile_counts.alloc(tiles * 4, h->arena);
-  tile_offs.alloc((tiles + 1) * 8, h->arena);
-  start_cnt.alloc(tiles * kDigestTile, h->arena);
-  uint64_t N = 0;
-  const DigestRange whole{0u, h->res_end, 0u, n_prot};
-  {
-    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
-    launch_digest_count(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                        (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), s);
-    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
-    N = read_u64(h, tile_offs.as<uint64_t>() + tiles);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2ull * h->res_end + tiles * 16;
-  }
+  Digest dg = whole_digest(h, nullptr);
+  const uint64_t N = dg.count();
   if (int rc = check_err_bits(read_err(h))) {
     free_index(h);
     return rc;
   }
   TR("count+sync");
-  DevBuf r_mass, r_gpos, r_prot, r_len;
-  r_mass.alloc(N * 8, h->arena);
-  r_gpos.alloc(N * 4, h->arena);
-  r_prot.alloc(N * 4, h->arena);
-  r_len.alloc(N * 2, h->arena);
-  {
-    Stage sg(h, DBI_STAGE_DIGEST_EMIT);
-    launch_digest_emit(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                       (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
-                       r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(),
-                       r_len.as<uint16_t>(), nullptr, h->d_err.as<uint32_t>(), s);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2ull * h->res_end + N * 18;
-  }
-  tile_counts.release();
-  tile_offs.release();
-  start_cnt.release();
+  RecSet recs;
+  dg.emit(recs, nullptr);
   TR("emit");
-  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
-  int rc = index_records(h, rv, N, h->p.min_mass, h->p.max_mass);
-  TR("index_records");
-  if (rc == DBI_OK)
-    if (int rc2 = check_err_bits(read_err(h))) rc = rc2;
-  if (rc != DBI_OK) {
-    free_index(h);
-    return rc;
-  }
-  if (h->p.keep_emitted) {
-    h->k_mass.swap(r_mass); h->k_gpos.swap(r_gpos); h->k_prot.swap(r_prot); h->k_len.swap(r_len);
-  }
-  DBI_CUDA(cudaStreamSynchronize(s));
-  finish_stats(h);
-  TR("final_sync");
+  if (int rc = build_end(h, recs, N, h->p.min_mass, h->p.max_mass)) return rc;
   g_trace.dump();
   return DBI_OK;
   DBI_API_END
@@ -1557,20 +1603,14 @@ int dbi_build_from_records(dbi_handle* h, const double* mass, const uint32_t* pr
     lo = i ? std::min(lo, mass[i]) : mass[i];
     hi = i ? std::max(hi, mass[i]) : mass[i];
   }
-  ensure_uploaded(h);
-  const uint32_t zero = 0;
-  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, s));
-  pack_residues(h);
-  DevBuf r_mass, r_gpos, r_prot, r_len;
-  r_mass.alloc(n * 8, h->arena);
-  r_gpos.alloc(n * 4, h->arena);
-  r_prot.alloc(n * 4, h->arena);
-  r_len.alloc(n * 2, h->arena);
+  build_begin(h);
+  RecSet recs;
+  recs.alloc(n, h->arena);
   if (n) {
-    DBI_CUDA(cudaMemcpyAsync(r_mass.p, mass, n * 8, cudaMemcpyHostToDevice, s));
-    DBI_CUDA(cudaMemcpyAsync(r_gpos.p, gpos.data(), n * 4, cudaMemcpyHostToDevice, s));
-    DBI_CUDA(cudaMemcpyAsync(r_prot.p, prot, n * 4, cudaMemcpyHostToDevice, s));
-    DBI_CUDA(cudaMemcpyAsync(r_len.p, len, n * 2, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(recs.mass.p, mass, n * 8, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(recs.gpos.p, gpos.data(), n * 4, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(recs.prot.p, prot, n * 4, cudaMemcpyHostToDevice, s));
+    DBI_CUDA(cudaMemcpyAsync(recs.len.p, len, n * 2, cudaMemcpyHostToDevice, s));
     DBI_CUDA(cudaStreamSynchronize(s));
   }
   // mod variants may move masses outside [lo, hi]: widen by the gate
@@ -1578,20 +1618,7 @@ int dbi_build_from_records(dbi_handle* h, const double* mass, const uint32_t* pr
     lo = std::min(lo, h->p.min_mass);
     hi = std::max(hi, h->p.max_mass);
   }
-  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
-  int rc = index_records(h, rv, n, lo, hi);
-  if (rc == DBI_OK)
-    if (int rc2 = check_err_bits(read_err(h))) rc = rc2;
-  if (rc != DBI_OK) {
-    free_index(h);
-    return rc;
-  }
-  if (h->p.keep_emitted) {
-    h->k_mass.swap(r_mass); h->k_gpos.swap(r_gpos); h->k_prot.swap(r_prot); h->k_len.swap(r_len);
-  }
-  DBI_CUDA(cudaStreamSynchronize(s));
-  finish_stats(h);
-  return DBI_OK;
+  return build_end(h, recs, n, lo, hi);
   DBI_API_END
 }
 
@@ -1891,8 +1918,7 @@ void search_begin(dbi_handle* h) {
   h->st.n_proteins = np;
   h->st.n_residues = nr;
   ensure_uploaded(h);
-  const uint32_t zero = 0;
-  DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &zero, 4, cudaMemcpyHostToDevice, h->stream));
+  clear_err(h);
 }
 
 // K12: a batch's windows on the handle's GPU, sorted by lo, with the prefix maximum of hi.  io = lo | hi (the
@@ -1958,7 +1984,6 @@ struct DropCandidates {
 // 2 nq doubles are lo | hi on the device.  N_c over max_candidates (or at 2^32): DBI_ERANGE with *n_candidates set.
 int index_candidates(dbi_handle* h, const double* lo, const double* hi, uint64_t nq, cudaMemcpyKind kind,
                      uint64_t max_candidates, uint64_t* n_candidates, DevBuf& io) {
-  cudaStream_t s = h->stream;
   if (nq >= (1ull << 32)) {
     set_error("%llu windows in one batch (< 2^32)", (unsigned long long)nq);
     return DBI_ERANGE;
@@ -1970,22 +1995,8 @@ int index_candidates(dbi_handle* h, const double* lo, const double* hi, uint64_t
   MassWindows win;
   upload_windows(h, lo, hi, nq, io, &win, kind);
   // K2u: the records that can land in a window, counted before anything is allocated
-  const uint64_t tiles = nq ? ((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile : 0;
-  DevBuf tile_counts, tile_offs, start_cnt;
-  tile_counts.alloc(std::max<uint64_t>(tiles, 1) * 4, h->arena);
-  tile_offs.alloc((tiles + 1) * 8, h->arena);
-  start_cnt.alloc(std::max<uint64_t>(tiles, 1) * kDigestTile, h->arena);
-  const DigestRange whole{0u, h->res_end, 0u, n_prot};
-  uint64_t N = 0;
-  if (tiles) {
-    Stage sg(h, DBI_STAGE_DIGEST_COUNT);
-    launch_digest_count(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                        (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), s,
-                        &win);
-    launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
-    N = read_u64(h, tile_offs.as<uint64_t>() + tiles);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_COUNT] += 2ull * h->res_end + tiles * 16;
-  }
+  Digest dg = whole_digest(h, &win);
+  const uint64_t N = dg.count();
   if (int rc = check_err_bits(read_err(h))) return rc;
   if (n_candidates) *n_candidates = N;
   h->st.n_emitted = N;
@@ -1995,28 +2006,11 @@ int index_candidates(dbi_handle* h, const double* lo, const double* hi, uint64_t
     resolve_spans(h);
     return DBI_ERANGE;
   }
-  DevBuf r_mass, r_gpos, r_prot, r_len;
-  r_mass.alloc(std::max<uint64_t>(N, 1) * 8, h->arena);
-  r_gpos.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
-  r_prot.alloc(std::max<uint64_t>(N, 1) * 4, h->arena);
-  r_len.alloc(std::max<uint64_t>(N, 1) * 2, h->arena);
-  if (N) {  // K4u
-    Stage sg(h, DBI_STAGE_DIGEST_EMIT);
-    launch_digest_emit(h->d_res.as<uint8_t>(), whole, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, 0,
-                       (uint32_t)tiles, start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
-                       r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>(),
-                       nullptr, h->d_err.as<uint32_t>(), s, &win);
-    h->st.algo_bytes[DBI_STAGE_DIGEST_EMIT] += 2ull * h->res_end + N * 18;
-  }
-  tile_counts.release();
-  tile_offs.release();
-  start_cnt.release();
-
+  RecSet cand;
+  if (N) dg.emit(cand, nullptr);  // K4u
   DropCandidates drop_candidates{h};
-  const RecView rv{r_mass.as<uint64_t>(), r_gpos.as<uint32_t>(), r_prot.as<uint32_t>(), r_len.as<uint16_t>()};
-  if (int rc = index_records(h, rv, N, h->p.min_mass, h->p.max_mass)) return rc;
+  if (int rc = index_records(h, cand.view(), N, h->p.min_mass, h->p.max_mass)) return rc;
   if (int rc = check_err_bits(read_err(h))) return rc;
-  r_mass.release(); r_gpos.release(); r_prot.release(); r_len.release();
   drop_candidates.armed = false;
   return DBI_OK;
 }
@@ -2565,10 +2559,10 @@ int dbi_debug_emitted(dbi_handle* h, uint64_t capacity, double* mass, uint32_t* 
   cudaStream_t s = h->stream;
   std::vector<uint32_t> gpos(N), pr(N);
   if (N) {
-    DBI_CUDA(cudaMemcpyAsync(gpos.data(), h->k_gpos.p, N * 4, cudaMemcpyDeviceToHost, s));
-    DBI_CUDA(cudaMemcpyAsync(pr.data(), h->k_prot.p, N * 4, cudaMemcpyDeviceToHost, s));
-    if (mass) DBI_CUDA(cudaMemcpyAsync(mass, h->k_mass.p, N * 8, cudaMemcpyDeviceToHost, s));
-    if (len) DBI_CUDA(cudaMemcpyAsync(len, h->k_len.p, N * 2, cudaMemcpyDeviceToHost, s));
+    DBI_CUDA(cudaMemcpyAsync(gpos.data(), h->kept.gpos.p, N * 4, cudaMemcpyDeviceToHost, s));
+    DBI_CUDA(cudaMemcpyAsync(pr.data(), h->kept.prot.p, N * 4, cudaMemcpyDeviceToHost, s));
+    if (mass) DBI_CUDA(cudaMemcpyAsync(mass, h->kept.mass.p, N * 8, cudaMemcpyDeviceToHost, s));
+    if (len) DBI_CUDA(cudaMemcpyAsync(len, h->kept.len.p, N * 2, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
   }
   for (uint64_t i = 0; i < N; ++i) {
