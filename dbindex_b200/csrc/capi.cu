@@ -205,22 +205,31 @@ struct dbi_handle {
   // index
   bool built = false;
   DevBuf d_tables, d_err;
-  DevBuf d_res, d_pstart;
-  uint64_t packed_prot = UINT64_MAX;  // proteins d_res / d_pstart hold (K1 ran on them)
-  uint32_t res_end = 0;
-  uint64_t res_alloc = 0;  // bytes readable at d_res (multiple of 16: tiles are staged with bulk copies)
-  uint64_t n_emitted = 0, n_unique = 0, n_entries = 0;
-  DevBuf u_mass, u_gpos, u_prot, u_len, u_plo, plist;
-  DevBuf e_mass, e_base, e_pat;  // empty when there are no differential mods (entries == unique peptides)
-  // group path: site masks of the unique peptides (u_cmask[u * C + c]), valid for cmask_n peptides;
-  // d_nlong = how many peptides are longer than 64 residues (they have no masks)
-  DevBuf u_cmask, d_nlong;
-  uint64_t cmask_n = UINT64_MAX;
-  // compact layout (single GPU, group path): the sorted groups instead of the entry arrays.  g_mass = group
-  // mass, g_pay = peptide << 32 | class sequence << 27 | variant count, g_eoff = entries before each group
-  // (n_groups + 1); n_groups = 0 when the entries are expanded.  n_long = peptides longer than 64 residues.
-  DevBuf g_mass, g_pay, g_eoff;
-  uint64_t n_groups = 0, n_long = 0;
+  // The device arrays of a built index (kIndexBufs below lists them for release, borrow and device_bytes).
+  struct IndexBufs {
+    DevBuf d_res, d_pstart;  // packed residues + protein starts: outlive the tables (free_tables keeps them)
+    DevBuf u_mass, u_gpos, u_prot, u_len, u_plo, plist;
+    DevBuf e_mass, e_base, e_pat;  // empty when there are no differential mods (entries == unique peptides)
+    // group path: site masks of the unique peptides (u_cmask[u * C + c]), valid for cmask_n peptides;
+    // d_nlong = how many peptides are longer than 64 residues (they have no masks)
+    DevBuf u_cmask, d_nlong;
+    // compact layout (single GPU, group path): the sorted groups instead of the entry arrays.  g_mass = group
+    // mass, g_pay = peptide << 32 | class sequence << 27 | variant count, g_eoff = entries before each group
+    // (n_groups + 1).
+    DevBuf g_mass, g_pay, g_eoff;
+  } ix;
+  struct TableCounts {  // the sizes of the tables; free_tables resets them
+    uint64_t n_emitted = 0, n_unique = 0, n_entries = 0;
+    uint64_t n_groups = 0;  // 0 when the entries are expanded
+    uint64_t n_long = 0;    // peptides longer than 64 residues
+    uint64_t cmask_n = UINT64_MAX;
+  } cnt;
+  struct ResLayout {  // what d_res / d_pstart hold; free_index resets it
+    uint64_t packed_prot = UINT64_MAX;  // proteins d_res / d_pstart hold (K1 ran on them)
+    uint32_t res_end = 0;
+    uint64_t res_alloc = 0;  // bytes readable at d_res (multiple of 16: tiles are staged with bulk copies)
+    bool mg_layout = false;  // dbi_mg_set_shards done (d_res / d_pstart are views of window 0)
+  } lay;
   RecSet kept;  // kept raw records (params.keep_emitted)
 
   // ---- sharded build (dbi_mg_*, capi_mg.inl) ----
@@ -228,35 +237,49 @@ struct dbi_handle {
   //   0 proteome: the packed residues of ALL ranks + their protein starts (every rank packs its own
   //     shard in place and pulls the others);  1 arena: what the exchanges deliver to this rank;
   //   2 unique tables: first occurrence + protein lists of the peptides this rank owns.
-  struct MgWindow {
-    void* p = nullptr;                 // local allocation (exportable)
+  struct MgWindow {  // the block this rank owns (exportable)
+    void* p = nullptr;
     uint64_t cap = 0;
-    void* peer[kMaxRanks] = {};        // mapped base of every rank's window (own rank: p)
+  };
+  struct MgPeers {  // mapped base of every rank's window (own rank: MgWindow::p)
+    void* peer[kMaxRanks] = {};
     uint64_t peer_cap[kMaxRanks] = {};
   };
-  int mg_rank = 0, mg_world = 1;
   bool mg_begun = false;  // dbi_mg_begin was called
   MgWindow win[3];
-  uint64_t prot_off[kMaxRanks + 1] = {};  // global id of every rank's first protein
-  uint64_t pos_off[kMaxRanks + 1] = {};   // buffer position of every rank's first separator
-  bool mg_layout = false;                 // dbi_mg_set_shards done (d_res / d_pstart are views of window 0)
-  cudaStream_t side_stream = nullptr;     // carries the peer pulls of the proteome next to the digest
+  // Where a query finds the other ranks' proteins, peptides and mass slices.  Set by the stages that lay them
+  // out; free_sharded_tables resets ent_base_off and uoff.
+  struct MgRoute {
+    int mg_rank = 0, mg_world = 1;
+    MgPeers win[3];
+    uint64_t prot_off[kMaxRanks + 1] = {};  // global id of every rank's first protein
+    uint64_t pos_off[kMaxRanks + 1] = {};   // buffer position of every rank's first separator
+    uint64_t ent_base_off = 0;              // global id of this rank's first unique peptide (0 on a single GPU)
+    uint64_t uoff[kMaxRanks + 1] = {};      // global id of every rank's first unique peptide
+    uint64_t uniq_cap[kMaxRanks] = {};      // layout capacity of every rank's window 2
+    uint64_t mg_thr[2][kMaxSlices] = {};    // key thresholds of the two exchanges
+    int mg_nthr[2] = {};                    // how many: slices - 1
+  } rt;
+  cudaStream_t side_stream = nullptr;  // carries the peer pulls of the proteome next to the digest
   cudaEvent_t pull_done = nullptr;
   bool pull_pending = false;
   // world of the sharded unindexed search whose layout window 0 still holds (0 = none): the next search of the
   // same handles with the same shards reuses it (dbi_mg_search_unindexed_local)
   int mg_search_world = 0;
-  uint64_t ent_base_off = 0;  // global id of this rank's first unique peptide (0 on a single GPU)
-  uint64_t uoff[kMaxRanks + 1] = {};      // global id of every rank's first unique peptide
-  uint64_t uniq_cap[kMaxRanks] = {};      // layout capacity of every rank's window 2
-  RecSet mg_rec;                             // local records between digest and exchange
-  DevBuf mg_nmod, mg_wtab;                   // their mod-site counts, and variants of a peptide with n sites
-  uint64_t mg_n = 0;
-  DevBuf mg_vkey, mg_vpay;                   // local groups / variants between listing and exchange
-  uint64_t mg_v = 0;
-  uint64_t mg_recv[2] = {};                  // items delivered to this rank by exchange 0 / 1
-  uint64_t mg_thr[2][kMaxSlices] = {};       // key thresholds of the two exchanges (query routing)
-  int mg_nthr[2] = {};                       // how many: slices - 1
+  struct MgStaged {            // the local items between the stages of a sharded build
+    RecSet mg_rec;             // local records between digest and exchange
+    DevBuf mg_nmod;            // their mod-site counts
+    uint64_t mg_n = 0;
+    DevBuf mg_vkey, mg_vpay;   // local groups / variants between listing and exchange
+    uint64_t mg_v = 0;
+    uint64_t mg_recv[2] = {};  // items delivered to this rank by exchange 0 / 1
+    void release() {
+      mg_rec.release(); mg_nmod.release(); mg_vkey.release(); mg_vpay.release();
+      mg_n = mg_v = 0;
+      mg_recv[0] = mg_recv[1] = 0;
+    }
+  } mgs;
+  DevBuf mg_wtab;  // variants of a peptide with n sites
 
   // pending result of dbi_query_hits (device side), read by dbi_query_hits_read
   struct HitResult {
@@ -306,12 +329,25 @@ struct dbi_handle {
   std::mutex view_mu;  // guards the last-view / orphaned hand-over
   bool orphaned = false;
 
-  const double* entry_mass() const { return e_mass.p ? e_mass.as<double>() : u_mass.as<double>(); }
-  const uint32_t* entry_base() const { return e_base.as<uint32_t>(); }
-  const uint32_t* entry_pat() const { return e_pat.as<uint32_t>(); }
+  const double* entry_mass() const { return ix.e_mass.p ? ix.e_mass.as<double>() : ix.u_mass.as<double>(); }
+  const uint32_t* entry_base() const { return ix.e_base.as<uint32_t>(); }
+  const uint32_t* entry_pat() const { return ix.e_pat.as<uint32_t>(); }
   // what K9 / K14 / the key listing search: the groups of a compact index, else the entries
-  const double* key_mass() const { return n_groups ? g_mass.as<double>() : entry_mass(); }
-  uint64_t n_keys() const { return n_groups ? n_groups : n_entries; }
+  const double* key_mass() const { return cnt.n_groups ? ix.g_mass.as<double>() : entry_mass(); }
+  uint64_t n_keys() const { return cnt.n_groups ? cnt.n_groups : cnt.n_entries; }
+};
+
+// Every array of an index, once.  kResidues: only free_index releases it (the tables of a rebuild reuse the
+// packed residues).  kCompact: device_bytes counts it only in a compact index, which needs the site masks to
+// expand its groups.  kUncounted: device_bytes never counts it.
+enum BufUse { kResidues, kCounted, kCompact, kUncounted };
+using IB = dbi_handle::IndexBufs;
+using IndexBuf = DevBuf IB::*;
+constexpr struct { IndexBuf buf; BufUse use; } kIndexBufs[] = {
+    {&IB::d_res, kResidues}, {&IB::d_pstart, kResidues}, {&IB::u_mass, kCounted},    {&IB::u_gpos, kCounted},
+    {&IB::u_prot, kCounted}, {&IB::u_len, kCounted},     {&IB::u_plo, kCounted},     {&IB::plist, kCounted},
+    {&IB::e_mass, kCounted}, {&IB::e_base, kCounted},    {&IB::e_pat, kCounted},     {&IB::u_cmask, kCompact},
+    {&IB::d_nlong, kUncounted}, {&IB::g_mass, kCompact}, {&IB::g_pay, kCompact},     {&IB::g_eoff, kCompact},
 };
 
 namespace {
@@ -478,15 +514,10 @@ uint64_t read_u64(dbi_handle* h, const uint64_t* d) {
 
 // The tables an index build derives from the packed residues: unique peptides, protein lists, entries.
 void free_tables(dbi_handle* h) {
-  h->u_mass.release(); h->u_gpos.release(); h->u_prot.release(); h->u_len.release();
-  h->u_plo.release(); h->plist.release();
-  h->e_mass.release(); h->e_base.release(); h->e_pat.release();
-  h->u_cmask.release(); h->d_nlong.release();
-  h->g_mass.release(); h->g_pay.release(); h->g_eoff.release();
-  h->n_groups = h->n_long = 0;
-  h->cmask_n = UINT64_MAX;
+  for (const auto& b : kIndexBufs)
+    if (b.use != kResidues) (h->ix.*b.buf).release();
+  h->cnt = {};
   h->kept.release();
-  h->n_emitted = h->n_unique = h->n_entries = 0;
 }
 
 // The pending results of dbi_query_hits / dbi_search_unindexed and dbi_lookup_peptides.
@@ -499,13 +530,9 @@ void drop_results(dbi_handle* h) {
 void free_sharded_tables(dbi_handle* h) {
   h->built = false;
   free_tables(h);
-  h->mg_rec.release();
-  h->mg_nmod.release();
-  h->mg_vkey.release(); h->mg_vpay.release();
-  h->mg_n = h->mg_v = 0;
-  h->mg_recv[0] = h->mg_recv[1] = 0;
-  h->ent_base_off = 0;
-  std::memset(h->uoff, 0, sizeof(h->uoff));
+  h->mgs.release();
+  h->rt.ent_base_off = 0;
+  std::memset(h->rt.uoff, 0, sizeof(h->rt.uoff));
 }
 
 void free_index(dbi_handle* h) {
@@ -514,11 +541,10 @@ void free_index(dbi_handle* h) {
     h->pull_pending = false;
   }
   drop_results(h);
-  h->d_res.release();
-  h->d_pstart.release();
-  h->packed_prot = UINT64_MAX;
+  for (const auto& b : kIndexBufs)
+    if (b.use == kResidues) (h->ix.*b.buf).release();
+  h->lay = {};
   free_sharded_tables(h);
-  h->mg_layout = false;
   h->mg_search_world = 0;
   h->spans.clear();
   h->ev_used = 0;
@@ -619,14 +645,14 @@ void pack_residues(dbi_handle* h) {
   const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
   const uint64_t res_end = n_res + n_prot + 1;
   const uint64_t padded = (res_end + 64 + 15) & ~15ull;
-  h->res_end = (uint32_t)res_end;
-  h->res_alloc = padded;
-  h->d_res.alloc(padded, h->arena);
-  h->d_pstart.alloc(((uint64_t)n_prot + 1) * 4, h->arena);
-  DBI_CUDA(cudaMemsetAsync((uint8_t*)h->d_res.p + res_end, 0, padded - res_end, h->stream));
-  launch_pack(h->d_raw.as<uint8_t>(), h->d_off.as<uint64_t>(), n_prot, n_res, h->d_res.as<uint8_t>(),
-              h->d_pstart.as<uint32_t>(), 0u, h->d_err.as<uint32_t>(), h->stream);
-  h->packed_prot = n_prot;
+  h->lay.res_end = (uint32_t)res_end;
+  h->lay.res_alloc = padded;
+  h->ix.d_res.alloc(padded, h->arena);
+  h->ix.d_pstart.alloc(((uint64_t)n_prot + 1) * 4, h->arena);
+  DBI_CUDA(cudaMemsetAsync((uint8_t*)h->ix.d_res.p + res_end, 0, padded - res_end, h->stream));
+  launch_pack(h->d_raw.as<uint8_t>(), h->d_off.as<uint64_t>(), n_prot, n_res, h->ix.d_res.as<uint8_t>(),
+              h->ix.d_pstart.as<uint32_t>(), 0u, h->d_err.as<uint32_t>(), h->stream);
+  h->lay.packed_prot = n_prot;
   h->st.algo_bytes[DBI_STAGE_PACK] += 2 * n_res + (uint64_t)n_prot * 12;
 }
 
@@ -656,7 +682,7 @@ struct Digest {
     start_cnt.alloc((uint64_t)nt * kDigestTile, h->arena);
     if (!nt) return n = 0;
     Stage sg(h, DBI_STAGE_DIGEST_COUNT);
-    launch_digest_count(h->d_res.as<uint8_t>(), rg, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
+    launch_digest_count(h->ix.d_res.as<uint8_t>(), rg, h->lay.res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
                         start_cnt.as<uint8_t>(), tile_counts.as<uint32_t>(), h->d_err.as<uint32_t>(), h->stream, windows);
     launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), nt, tile_offs.as<uint64_t>(), h->stream);
     n = read_u64(h, tile_offs.as<uint64_t>() + nt);
@@ -669,8 +695,8 @@ struct Digest {
     if (nmod) nmod->alloc(std::max<uint64_t>(n, 1), h->arena);
     {
       Stage sg(h, DBI_STAGE_DIGEST_EMIT);
-      launch_digest_emit(h->d_res.as<uint8_t>(), rg, h->res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
-                         start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->d_pstart.as<uint32_t>(),
+      launch_digest_emit(h->ix.d_res.as<uint8_t>(), rg, h->lay.res_alloc, h->d_tables.as<DevTables>(), h->cfg, t0, nt,
+                         start_cnt.as<uint8_t>(), tile_offs.as<uint64_t>(), h->ix.d_pstart.as<uint32_t>(),
                          out.mass.as<uint64_t>(), out.gpos.as<uint32_t>(), out.prot.as<uint32_t>(),
                          out.len.as<uint16_t>(), nmod ? nmod->as<uint8_t>() : nullptr, h->d_err.as<uint32_t>(),
                          h->stream, windows);
@@ -684,8 +710,9 @@ struct Digest {
 
 // The digest of a single-GPU build or unindexed search: every start position, none when there are no windows.
 Digest whole_digest(dbi_handle* h, const MassWindows* windows) {
-  const uint32_t nt = windows && !windows->n ? 0u : (uint32_t)(((uint64_t)h->res_end + kDigestTile - 1) / kDigestTile);
-  return {h, DigestRange{0u, h->res_end, 0u, (uint32_t)(h->h_off.size() - 1)}, 0u, nt, h->res_end, windows};
+  const uint32_t nt =
+      windows && !windows->n ? 0u : (uint32_t)(((uint64_t)h->lay.res_end + kDigestTile - 1) / kDigestTile);
+  return {h, DigestRange{0u, h->lay.res_end, 0u, (uint32_t)(h->h_off.size() - 1)}, 0u, nt, h->lay.res_end, windows};
 }
 
 // Radix key of a mass: bits(mass) - bits(lo); every mass of a build lies in [lo, hi].
@@ -726,12 +753,12 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
     set_error("more than 2^32 emitted records on one GPU (%llu)", (unsigned long long)N);
     return DBI_ERANGE;
   }
-  h->n_unique = 0;
+  h->cnt.n_unique = 0;
   h->st.n_unique = 0;
   if (N == 0) {
-    if (h->mg_world > 1 && h->win[2].p) h->u_plo.borrow((uint8_t*)h->win[2].p + UniqLayout(h->uniq_cap[h->mg_rank]).plo, 8);
-    else h->u_plo.alloc(8, h->arena);
-    DBI_CUDA(cudaMemsetAsync(h->u_plo.p, 0, 8, s));
+    if (h->rt.mg_world > 1 && h->win[2].p) h->ix.u_plo.borrow((uint8_t*)h->win[2].p + UniqLayout(h->rt.uniq_cap[h->rt.mg_rank]).plo, 8);
+    else h->ix.u_plo.alloc(8, h->arena);
+    DBI_CUDA(cudaMemsetAsync(h->ix.u_plo.p, 0, 8, s));
     return DBI_OK;
   }
   const uint64_t base_bits = ks.base_bits;
@@ -769,7 +796,7 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
       hash.alloc(N * (wide ? 8 : 4), h->arena);
       hkey[0].alloc(N * (wide ? 8 : 4), h->arena);
       hkey[1].alloc(N * (wide ? 8 : 4), h->arena);
-      launch_hash_records(h->d_res.as<uint8_t>(), r.gpos, r.len, N, seed, wide, hash.p, idx[0].as<uint32_t>(), s);
+      launch_hash_records(h->ix.d_res.as<uint8_t>(), r.gpos, r.len, N, seed, wide, hash.p, idx[0].as<uint32_t>(), s);
       DBI_CUDA(cudaMemcpyAsync(hkey[0].p, hash.p, N * (wide ? 8 : 4), cudaMemcpyDeviceToDevice, s));
       // less significant key first: sequence hash ...
       uint32_t* ix[2] = {idx[0].as<uint32_t>(), idx[1].as<uint32_t>()};
@@ -784,7 +811,7 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
       DomProbe base_probe(h);
       // the largest K7 sort of the build: the base sort, unless the variant groups go through K7 too
       const bool base_is_dominant =
-          h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->mg_world <= 1 && !group_radix(h)));
+          h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->rt.mg_world <= 1 && !group_radix(h)));
       if (base_is_dominant) {  // a retry re-runs the sort: count only the final attempt
         h->spans.erase(std::remove_if(h->spans.begin(), h->spans.end(),
                                       [](const dbi_handle::Span& sp) { return sp.kind == kSpanDominant; }),
@@ -808,7 +835,7 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
     }
     {
       Stage sg(h, DBI_STAGE_DEDUP);
-      launch_dedup_flags(h->d_res.as<uint8_t>(), mkey[sorted].as<uint64_t>(), idx[0].as<uint32_t>(), hash.p,
+      launch_dedup_flags(h->ix.d_res.as<uint8_t>(), mkey[sorted].as<uint64_t>(), idx[0].as<uint32_t>(), hash.p,
                          hash_bits, r.gpos, r.len, N, flags.as<uint8_t>(), tile_counts.as<uint32_t>(),
                          h->d_err.as<uint32_t>(), s);
       launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
@@ -833,32 +860,32 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
   }
   {
     Stage sg(h, DBI_STAGE_DEDUP);
-    h->n_unique = n_unique;
+    h->cnt.n_unique = n_unique;
     h->st.n_unique = n_unique;
-    h->u_mass.alloc(n_unique * 8, h->arena);
-    if (h->mg_world > 1) {  // the other ranks read these through their mapping of window 2
-      const UniqLayout L(h->uniq_cap[h->mg_rank]);
+    h->ix.u_mass.alloc(n_unique * 8, h->arena);
+    if (h->rt.mg_world > 1) {  // the other ranks read these through their mapping of window 2
+      const UniqLayout L(h->rt.uniq_cap[h->rt.mg_rank]);
       uint8_t* base = (uint8_t*)h->win[2].p;
-      if (!base || h->win[2].cap < L.total || h->uniq_cap[h->mg_rank] < N) {
+      if (!base || h->win[2].cap < L.total || h->rt.uniq_cap[h->rt.mg_rank] < N) {
         set_error("window 2 (unique tables) is smaller than the %llu records delivered", (unsigned long long)N);
         return DBI_EINVAL;
       }
-      h->u_gpos.borrow(base + L.gpos, n_unique * 4);
-      h->u_prot.borrow(base + L.prot, n_unique * 4);
-      h->u_len.borrow(base + L.len, n_unique * 2);
-      h->u_plo.borrow(base + L.plo, (n_unique + 1) * 8);
-      h->plist.borrow(base + L.plist, N * 4);
+      h->ix.u_gpos.borrow(base + L.gpos, n_unique * 4);
+      h->ix.u_prot.borrow(base + L.prot, n_unique * 4);
+      h->ix.u_len.borrow(base + L.len, n_unique * 2);
+      h->ix.u_plo.borrow(base + L.plo, (n_unique + 1) * 8);
+      h->ix.plist.borrow(base + L.plist, N * 4);
     } else {
-      h->u_gpos.alloc(n_unique * 4, h->arena);
-      h->u_prot.alloc(n_unique * 4, h->arena);
-      h->u_len.alloc(n_unique * 2, h->arena);
-      h->u_plo.alloc((n_unique + 1) * 8, h->arena);
-      h->plist.alloc(N * 4, h->arena);
+      h->ix.u_gpos.alloc(n_unique * 4, h->arena);
+      h->ix.u_prot.alloc(n_unique * 4, h->arena);
+      h->ix.u_len.alloc(n_unique * 2, h->arena);
+      h->ix.u_plo.alloc((n_unique + 1) * 8, h->arena);
+      h->ix.plist.alloc(N * 4, h->arena);
     }
     launch_dedup_emit(mkey[sorted].as<uint64_t>(), idx[0].as<uint32_t>(), flags.as<uint8_t>(),
-                      tile_offs.as<uint64_t>(), r.gpos, r.prot, r.len, N, base_bits, n_unique, h->u_mass.as<double>(),
-                      h->u_gpos.as<uint32_t>(), h->u_prot.as<uint32_t>(), h->u_len.as<uint16_t>(),
-                      h->u_plo.as<uint64_t>(), h->plist.as<uint32_t>(), s);
+                      tile_offs.as<uint64_t>(), r.gpos, r.prot, r.len, N, base_bits, n_unique,
+                      h->ix.u_mass.as<double>(), h->ix.u_gpos.as<uint32_t>(), h->ix.u_prot.as<uint32_t>(),
+                      h->ix.u_len.as<uint16_t>(), h->ix.u_plo.as<uint64_t>(), h->ix.plist.as<uint32_t>(), s);
     h->st.algo_bytes[DBI_STAGE_DEDUP] += N * (8 + 4 + 1) + N * (1 + 4 + 4 + 4) + n_unique * (8 + 4 + 4 + 2 + 8 + 10);
   }
   TR("ir_dedup_emit");
@@ -870,7 +897,7 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
 int emit_variants(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& ks, DevBuf& vkey, DevBuf& vpay,
                   uint64_t* V_out) {
   cudaStream_t s = h->stream;
-  const uint64_t n_unique = h->n_unique;
+  const uint64_t n_unique = h->cnt.n_unique;
   *V_out = 0;
   if (ntiles == 0 || n_unique == 0) {
     vkey.alloc(8, h->arena);
@@ -885,8 +912,8 @@ int emit_variants(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace
   uint64_t V = 0;
   {
     Stage sg(h, DBI_STAGE_MOD_COUNT);
-    launch_mod_count(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
-                     h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), n_unique, tile0, ntiles,
+    launch_mod_count(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_mass.as<double>(),
+                     h->ix.u_gpos.as<uint32_t>(), h->ix.u_len.as<uint16_t>(), n_unique, tile0, ntiles,
                      counts.as<uint32_t>(), ucounts.as<uint32_t>(), h->d_err.as<uint32_t>(), s);
     launch_scan_u32_to_u64(ucounts.as<uint32_t>(), ntiles, uoffs.as<uint64_t>(), s);
     V = read_u64(h, uoffs.as<uint64_t>() + ntiles);
@@ -899,9 +926,9 @@ int emit_variants(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace
   TR("ir_valloc");
   {
     Stage sg(h, DBI_STAGE_MOD_EMIT);
-    launch_mod_emit(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
-                    h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), n_unique, tile0, ntiles,
-                    counts.as<uint32_t>(), uoffs.as<uint64_t>(), ks.base_bits, h->ent_base_off, vkey.as<uint64_t>(),
+    launch_mod_emit(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_mass.as<double>(),
+                    h->ix.u_gpos.as<uint32_t>(), h->ix.u_len.as<uint16_t>(), n_unique, tile0, ntiles,
+                    counts.as<uint32_t>(), uoffs.as<uint64_t>(), ks.base_bits, h->rt.ent_base_off, vkey.as<uint64_t>(),
                     vpay.as<uint64_t>(), s);
     h->st.algo_bytes[DBI_STAGE_MOD_EMIT] += n_in_tiles * (8 + 4 + 2 + 4 + 20) + V * 16;
   }
@@ -921,9 +948,9 @@ int sort_variants(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64_t V,
   key2.alloc(V * 8, h->arena);
   pay2.alloc(V * 8, h->arena);
   vtmp.alloc(radix_sort_tmp_bytes(V), h->arena);
-  h->e_mass.alloc(V * 8, h->arena);
-  h->e_base.alloc(V * 4, h->arena);
-  h->e_pat.alloc(V * 4, h->arena);
+  h->ix.e_mass.alloc(V * 8, h->arena);
+  h->ix.e_base.alloc(V * 4, h->arena);
+  h->ix.e_pat.alloc(V * 4, h->arena);
   TR("ir_ealloc");
   {
     // the last pass of the sort writes the final entry arrays (mass, base id, mod pattern)
@@ -935,19 +962,20 @@ int sort_variants(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64_t V,
       h->st.dom_kernel = 1;
       h->st.dom_bytes_per_launch = V * 32ull;
     }
-    SplitOut<uint64_t> split{h->e_mass.as<uint64_t>(), ks.base_bits, h->e_base.as<uint32_t>(), h->e_pat.as<uint32_t>()};
+    SplitOut<uint64_t> split{h->ix.e_mass.as<uint64_t>(), ks.base_bits, h->ix.e_base.as<uint32_t>(),
+                             h->ix.e_pat.as<uint32_t>()};
     const int passes = (ks.nbits + 7) / 8;
     if (V > 1 && passes > 0) {
       radix_sort_pairs<uint64_t, uint64_t>(vk, vp, V, 0, ks.nbits, vtmp.p, s, h->p.profile ? &var_probe : nullptr, &split);
     } else {  // nothing to sort: plain split
-      launch_split_entries(vk[0], vp[0], V, ks.base_bits, h->e_mass.as<double>(), h->e_base.as<uint32_t>(),
-                           h->e_pat.as<uint32_t>(), s);
+      launch_split_entries(vk[0], vp[0], V, ks.base_bits, h->ix.e_mass.as<double>(), h->ix.e_base.as<uint32_t>(),
+                           h->ix.e_pat.as<uint32_t>(), s);
     }
     h->st.sort_bits_var = (uint32_t)ks.nbits;
     h->st.algo_bytes[DBI_STAGE_SORT_VAR] += V * 8 + V * 32ull * passes;
   }
   TR("ir_sortvar");
-  h->n_entries = V;
+  h->cnt.n_entries = V;
   h->st.n_entries = V;
   return DBI_OK;
 }
@@ -958,16 +986,16 @@ constexpr uint64_t kGrpCntMask = (1ull << 27) - 1;
 
 // K5m over the whole unique table (once per table: the multi-GPU build replaces the table).
 void ensure_site_masks(dbi_handle* h) {
-  if (h->cmask_n == h->n_unique && h->u_cmask.p) return;
+  if (h->cnt.cmask_n == h->cnt.n_unique && h->ix.u_cmask.p) return;
   Stage sg(h, DBI_STAGE_MOD_COUNT);
-  h->u_cmask.alloc(std::max<uint64_t>(1, h->n_unique) * (uint64_t)h->cfg.n_classes * 8, h->arena);
-  h->d_nlong.alloc(16, h->arena);
-  DBI_CUDA(cudaMemsetAsync(h->d_nlong.p, 0, 16, h->stream));
-  launch_site_masks(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_gpos.as<uint32_t>(),
-                    h->u_len.as<uint16_t>(), h->n_unique, h->u_cmask.as<uint64_t>(),
-                    (unsigned long long*)h->d_nlong.p, h->stream);
-  h->cmask_n = h->n_unique;
-  h->st.algo_bytes[DBI_STAGE_MOD_COUNT] += h->n_unique * (4 + 2 + 12 + 8ull * h->cfg.n_classes);
+  h->ix.u_cmask.alloc(std::max<uint64_t>(1, h->cnt.n_unique) * (uint64_t)h->cfg.n_classes * 8, h->arena);
+  h->ix.d_nlong.alloc(16, h->arena);
+  DBI_CUDA(cudaMemsetAsync(h->ix.d_nlong.p, 0, 16, h->stream));
+  launch_site_masks(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_gpos.as<uint32_t>(),
+                    h->ix.u_len.as<uint16_t>(), h->cnt.n_unique, h->ix.u_cmask.as<uint64_t>(),
+                    (unsigned long long*)h->ix.d_nlong.p, h->stream);
+  h->cnt.cmask_n = h->cnt.n_unique;
+  h->st.algo_bytes[DBI_STAGE_MOD_COUNT] += h->cnt.n_unique * (4 + 2 + 12 + 8ull * h->cfg.n_classes);
 }
 
 // lists != nullptr (single GPU): K6g writes one sorted list per class sequence, described in *lists (the
@@ -975,7 +1003,7 @@ void ensure_site_masks(dbi_handle* h) {
 int emit_groups(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& ks, DevBuf& gkey, DevBuf& gpay,
                 uint64_t* NG_out, uint64_t* V_out, GroupLists* lists = nullptr) {
   cudaStream_t s = h->stream;
-  const uint64_t n_unique = h->n_unique;
+  const uint64_t n_unique = h->cnt.n_unique;
   const int S = h->cfg.n_seq;
   *NG_out = 0;
   *V_out = 0;
@@ -1007,9 +1035,9 @@ int emit_groups(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& 
   uint64_t NG = 0, V = 0;
   {
     Stage sg(h, DBI_STAGE_MOD_COUNT);
-    launch_grp_count(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
-                     h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->u_cmask.as<uint64_t>(), n_unique, tile0,
-                     ntiles, mask.as<uint32_t>(), tg.as<uint32_t>(), tv.as<uint32_t>(),
+    launch_grp_count(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_mass.as<double>(),
+                     h->ix.u_gpos.as<uint32_t>(), h->ix.u_len.as<uint16_t>(), h->ix.u_cmask.as<uint64_t>(), n_unique,
+                     tile0, ntiles, mask.as<uint32_t>(), tg.as<uint32_t>(), tv.as<uint32_t>(),
                      lists ? vt.as<uint32_t>() : nullptr, h->d_err.as<uint32_t>(), s);
     if (lists) launch_full_scan_u32_to_u64(vt.as<uint32_t>(), n_vt, goffs.as<uint64_t>(), vtmp.p, s);
     else launch_scan_u32_to_u64(tg.as<uint32_t>(), ntiles, goffs.as<uint64_t>(), s);
@@ -1036,10 +1064,10 @@ int emit_groups(dbi_handle* h, uint32_t tile0, uint32_t ntiles, const KeySpace& 
   TR("ir_valloc");
   {
     Stage sg(h, DBI_STAGE_MOD_EMIT);
-    launch_grp_emit(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_mass.as<double>(),
-                    h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->u_cmask.as<uint64_t>(), n_unique, tile0,
-                    ntiles, mask.as<uint32_t>(), goffs.as<uint64_t>(), lists != nullptr, ks.base_bits,
-                    h->ent_base_off, gkey.as<uint64_t>(), gpay.as<uint64_t>(), h->d_err.as<uint32_t>(), s);
+    launch_grp_emit(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_mass.as<double>(),
+                    h->ix.u_gpos.as<uint32_t>(), h->ix.u_len.as<uint16_t>(), h->ix.u_cmask.as<uint64_t>(), n_unique,
+                    tile0, ntiles, mask.as<uint32_t>(), goffs.as<uint64_t>(), lists != nullptr, ks.base_bits,
+                    h->rt.ent_base_off, gkey.as<uint64_t>(), gpay.as<uint64_t>(), h->d_err.as<uint32_t>(), s);
     h->st.algo_bytes[DBI_STAGE_MOD_EMIT] += n_in_tiles * per_pep + NG * 16;
   }
   TR("ir_modemit");
@@ -1067,8 +1095,8 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
     return DBI_ERANGE;
   }
   if (NG == 0) {
-    h->e_mass.alloc(8, h->arena); h->e_base.alloc(8, h->arena); h->e_pat.alloc(8, h->arena);
-    h->n_entries = 0;
+    h->ix.e_mass.alloc(8, h->arena); h->ix.e_base.alloc(8, h->arena); h->ix.e_pat.alloc(8, h->arena);
+    h->cnt.n_entries = 0;
     h->st.n_entries = 0;
     return DBI_OK;
   }
@@ -1114,7 +1142,7 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
     launch_full_scan_u32_to_u64(cnt.as<uint32_t>(), NG, eoff.as<uint64_t>(), stmp.p, s);
     DBI_CUDA(cudaMemsetAsync(lcount.p, 0, 16, s));
     DBI_CUDA(cudaMemcpyAsync(&V, eoff.as<uint64_t>() + NG, 8, cudaMemcpyDeviceToHost, s));
-    if (!sharded) DBI_CUDA(cudaMemcpyAsync(&n_long, h->d_nlong.p, 8, cudaMemcpyDeviceToHost, s));
+    if (!sharded) DBI_CUDA(cudaMemcpyAsync(&n_long, h->ix.d_nlong.p, 8, cudaMemcpyDeviceToHost, s));
     uint32_t e = 0;
     DBI_CUDA(cudaMemcpyAsync(&e, h->d_err.p, 4, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
@@ -1127,15 +1155,15 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
     if (!sharded && in_bufs && (V >= (1ull << 32) || compact_variants(h))) {
       // compact layout: keep the sorted groups, their masses and entry offsets; queries expand what they return
       launch_grp_key_mass(vk[r], NG, ks.base_bits, s);
-      h->g_mass.swap(r ? key2 : *in_bufs[0]);
-      h->g_pay.swap(r ? pay2 : *in_bufs[1]);
-      h->g_eoff.swap(eoff);
-      h->e_mass.release(); h->e_base.release(); h->e_pat.release();
-      h->n_groups = NG;
-      h->n_long = n_long;
+      h->ix.g_mass.swap(r ? key2 : *in_bufs[0]);
+      h->ix.g_pay.swap(r ? pay2 : *in_bufs[1]);
+      h->ix.g_eoff.swap(eoff);
+      h->ix.e_mass.release(); h->ix.e_base.release(); h->ix.e_pat.release();
+      h->cnt.n_groups = NG;
+      h->cnt.n_long = n_long;
       h->st.n_groups = (uint32_t)NG;
       h->st.algo_bytes[DBI_STAGE_GATHER_VAR] += NG * ((lists ? 0 : 8 + 4) + 16);
-      h->n_entries = V;
+      h->cnt.n_entries = V;
       h->st.n_entries = V;
       return DBI_OK;
     }
@@ -1147,9 +1175,9 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
     const uint64_t long_cap = std::min<uint64_t>(sharded ? std::min<uint64_t>(NG, 1u << 22) : NG,
                                                  n_long * (uint64_t)(h->cfg.n_seq - 1));
     const uint64_t tiles = (V + kExpTile - 1) / kExpTile;
-    h->e_mass.alloc(V * 8, h->arena);
-    h->e_base.alloc(V * 4, h->arena);
-    h->e_pat.alloc(V * 4, h->arena);
+    h->ix.e_mass.alloc(V * 8, h->arena);
+    h->ix.e_base.alloc(V * 4, h->arena);
+    h->ix.e_pat.alloc(V * 4, h->arena);
     tfirst.alloc((tiles + 1) * 4, h->arena);
     llist.alloc(std::max<uint64_t>(1, long_cap) * 4, h->arena);
     TR("ir_ealloc");
@@ -1159,12 +1187,12 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
       xa = h->get_event();
       cudaEventRecord(xa, s);
     }
-    launch_grp_expand(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->u_gpos.as<uint32_t>(),
-                      h->u_len.as<uint16_t>(), sharded ? side->cmask : h->u_cmask.as<uint64_t>(),
+    launch_grp_expand(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg, h->ix.u_gpos.as<uint32_t>(),
+                      h->ix.u_len.as<uint16_t>(), sharded ? side->cmask : h->ix.u_cmask.as<uint64_t>(),
                       sharded ? side->gid : nullptr, sharded ? side->uv : nullptr, vk[r], vp[r], eoff.as<uint64_t>(),
-                      tfirst.as<uint32_t>(), NG, V, ks.base_bits, h->e_mass.as<double>(), h->e_base.as<uint32_t>(),
-                      h->e_pat.as<uint32_t>(), llist.as<uint32_t>(), lcount.as<uint32_t>(), (uint32_t)long_cap,
-                      h->d_err.as<uint32_t>(), s);
+                      tfirst.as<uint32_t>(), NG, V, ks.base_bits, h->ix.e_mass.as<double>(),
+                      h->ix.e_base.as<uint32_t>(), h->ix.e_pat.as<uint32_t>(), llist.as<uint32_t>(),
+                      lcount.as<uint32_t>(), (uint32_t)long_cap, h->d_err.as<uint32_t>(), s);
     if (h->p.profile) {
       cudaEvent_t xb = h->get_event();
       cudaEventRecord(xb, s);
@@ -1177,7 +1205,7 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
         NG * ((lists ? 0 : 8 + 4) + 8 + 8 + 8 + 8ull * h->cfg.max_mods) + V * 16;
   }
   TR("ir_expand");
-  h->n_entries = V;
+  h->cnt.n_entries = V;
   h->st.n_entries = V;
   return DBI_OK;
 }
@@ -1185,19 +1213,19 @@ int sort_expand_groups(dbi_handle* h, uint64_t* key_in, uint64_t* pay_in, uint64
 // Single-GPU: sort + merge + (mods) expand + sort on N emitted records already on the device.
 // lo_mass / hi_mass bound every record mass (they fix the radix key width).
 int index_records(dbi_handle* h, const RecView& r, uint64_t N, double lo_mass, double hi_mass) {
-  h->n_emitted = N;
+  h->cnt.n_emitted = N;
   h->st.n_emitted = N;
   const KeySpace ks(lo_mass, hi_mass);
   h->st.n_groups = 0;  // set again if the build keeps the compact layout
   if (int rc = sort_dedup(h, r, N, ks)) return rc;
-  h->ent_base_off = 0;
-  if (h->cfg.max_mods == 0 || h->n_unique == 0) {
-    h->n_entries = h->n_unique;
-    h->st.n_entries = h->n_unique;
+  h->rt.ent_base_off = 0;
+  if (h->cfg.max_mods == 0 || h->cnt.n_unique == 0) {
+    h->cnt.n_entries = h->cnt.n_unique;
+    h->st.n_entries = h->cnt.n_unique;
     h->built = true;
     return DBI_OK;
   }
-  const uint32_t utiles = (uint32_t)((h->n_unique + kModTile - 1) / kModTile);
+  const uint32_t utiles = (uint32_t)((h->cnt.n_unique + kModTile - 1) / kModTile);
   DevBuf vkey, vpay;
   uint64_t V = 0, NG = 0;
   if (h->cfg.n_seq > 0) {  // group path: one record per (peptide, class sequence), merged from sorted lists
@@ -1216,11 +1244,10 @@ int index_records(dbi_handle* h, const RecView& r, uint64_t N, double lo_mass, d
 
 void finish_stats(dbi_handle* h) {
   resolve_spans(h);
-  h->st.device_bytes = h->d_res.bytes + h->d_pstart.bytes + h->u_mass.bytes + h->u_gpos.bytes + h->u_prot.bytes +
-                       h->u_len.bytes + h->u_plo.bytes + h->plist.bytes + h->e_mass.bytes + h->e_base.bytes +
-                       h->e_pat.bytes;
-  if (h->n_groups)  // a compact index needs the site masks to expand its groups
-    h->st.device_bytes += h->g_mass.bytes + h->g_pay.bytes + h->g_eoff.bytes + h->u_cmask.bytes;
+  h->st.device_bytes = 0;
+  for (const auto& b : kIndexBufs)
+    if (b.use != kUncounted && (b.use != kCompact || h->cnt.n_groups))
+      h->st.device_bytes += (h->ix.*b.buf).bytes;
 }
 
 // The end of a single-GPU build: the index of the N records in recs, whose masses lie in [lo_mass, hi_mass].  A
@@ -1245,30 +1272,30 @@ int build_end(dbi_handle* h, RecSet& recs, uint64_t N, double lo_mass, double hi
 UniqView uniq_view(dbi_handle* h) {
   UniqView uv;
   std::memset(&uv, 0, sizeof(uv));
-  if (h->mg_world <= 1) {
+  if (h->rt.mg_world <= 1) {
     uv.world = 1;
-    uv.gpos[0] = h->u_gpos.as<uint32_t>();
-    uv.prot[0] = h->u_prot.as<uint32_t>();
-    uv.len[0] = h->u_len.as<uint16_t>();
-    uv.plo[0] = h->u_plo.as<uint64_t>();
-    uv.plist[0] = h->plist.as<uint32_t>();
+    uv.gpos[0] = h->ix.u_gpos.as<uint32_t>();
+    uv.prot[0] = h->ix.u_prot.as<uint32_t>();
+    uv.len[0] = h->ix.u_len.as<uint16_t>();
+    uv.plo[0] = h->ix.u_plo.as<uint64_t>();
+    uv.plist[0] = h->ix.plist.as<uint32_t>();
     uv.uoff[0] = 0;
-    uv.uoff[1] = h->n_unique;
+    uv.uoff[1] = h->cnt.n_unique;
     return uv;
   }
-  uv.world = h->mg_world;
-  for (int r = 0; r < h->mg_world; ++r) {
-    uv.uoff[r] = h->uoff[r];
-    uint8_t* base = (uint8_t*)h->win[2].peer[r];
+  uv.world = h->rt.mg_world;
+  for (int r = 0; r < h->rt.mg_world; ++r) {
+    uv.uoff[r] = h->rt.uoff[r];
+    uint8_t* base = (uint8_t*)h->rt.win[2].peer[r];
     if (!base) continue;  // not connected: its peptides come back as DBI_REMOTE_BASE
-    const UniqLayout L(h->uniq_cap[r]);
+    const UniqLayout L(h->rt.uniq_cap[r]);
     uv.gpos[r] = (const uint32_t*)(base + L.gpos);
     uv.prot[r] = (const uint32_t*)(base + L.prot);
     uv.len[r] = (const uint16_t*)(base + L.len);
     uv.plo[r] = (const uint64_t*)(base + L.plo);
     uv.plist[r] = (const uint32_t*)(base + L.plist);
   }
-  uv.uoff[h->mg_world] = h->uoff[h->mg_world];
+  uv.uoff[h->rt.mg_world] = h->rt.uoff[h->rt.mg_world];
   return uv;
 }
 
@@ -1276,10 +1303,10 @@ UniqView uniq_view(dbi_handle* h) {
 // which become entry ranges through g_eoff; cnt32 / ntile32 / over as in launch_grp_entry_ranges.
 void query_ranges(dbi_handle* h, const double* d_lo, const double* d_hi, uint64_t nq, uint64_t* d_b, uint64_t* d_c,
                   uint32_t* cnt32, uint32_t* ntile32 = nullptr, uint32_t* over = nullptr) {
-  launch_query(h->key_mass(), h->n_keys(), d_lo, d_hi, nq, d_b, d_c, h->n_groups ? nullptr : cnt32, h->stream);
+  launch_query(h->key_mass(), h->n_keys(), d_lo, d_hi, nq, d_b, d_c, h->cnt.n_groups ? nullptr : cnt32, h->stream);
   h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (32 + 2ull * 32 * (uint64_t)bit_length(h->n_keys()));
-  if (h->n_groups) {
-    launch_grp_entry_ranges(h->g_eoff.as<uint64_t>(), nq, d_b, d_c, cnt32, ntile32, over, h->stream);
+  if (h->cnt.n_groups) {
+    launch_grp_entry_ranges(h->ix.g_eoff.as<uint64_t>(), nq, d_b, d_c, cnt32, ntile32, over, h->stream);
     h->st.algo_bytes[DBI_STAGE_QUERY] += nq * (16 + 2 * 32 + 16 + (cnt32 ? 4 : 0) + (ntile32 ? 4 : 0));
   }
 }
@@ -1298,22 +1325,22 @@ void expand_ranges(dbi_handle* h, const ExpRanges& rg, uint64_t n_tiles, uint64_
   lcount.alloc(16, h->arena);
   // one (group, tile) pair per tile is the common case; a tile can hold up to kExpTile + 1 long groups (peptides
   // over 64 residues with few sites), and then the list overflows and the tiles run again with room for all
-  uint64_t cap = h->n_long ? n_tiles + 1024 : 0;
+  uint64_t cap = h->cnt.n_long ? n_tiles + 1024 : 0;
   for (;;) {
     llist.alloc(std::max<uint64_t>(cap, 1) * 8, h->arena);
     DBI_CUDA(cudaMemsetAsync(lcount.p, 0, 4, s));
-    launch_grp_expand_ranges(h->cfg, h->u_cmask.as<uint64_t>(), h->g_mass.as<double>(), h->g_pay.as<uint64_t>(),
-                             h->g_eoff.as<uint64_t>(), h->n_groups, rg, n_tiles, x_mass.as<double>(),
-                             x_base.as<uint32_t>(), x_pat.as<uint32_t>(), llist.as<uint32_t>(), lcount.as<uint32_t>(),
-                             (uint32_t)cap, h->d_err.as<uint32_t>(), s);
-    if (!h->n_long) break;
+    launch_grp_expand_ranges(h->cfg, h->ix.u_cmask.as<uint64_t>(), h->ix.g_mass.as<double>(),
+                             h->ix.g_pay.as<uint64_t>(), h->ix.g_eoff.as<uint64_t>(), h->cnt.n_groups, rg, n_tiles,
+                             x_mass.as<double>(), x_base.as<uint32_t>(), x_pat.as<uint32_t>(), llist.as<uint32_t>(),
+                             lcount.as<uint32_t>(), (uint32_t)cap, h->d_err.as<uint32_t>(), s);
+    if (!h->cnt.n_long) break;
     uint32_t n_listed = 0;
     DBI_CUDA(cudaMemcpyAsync(&n_listed, lcount.p, 4, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
     if (n_listed <= cap) {
-      launch_grp_expand_ranges_long(h->d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg,
-                                    h->u_gpos.as<uint32_t>(), h->u_len.as<uint16_t>(), h->g_mass.as<double>(),
-                                    h->g_pay.as<uint64_t>(), h->g_eoff.as<uint64_t>(), rg, llist.as<uint32_t>(),
+      launch_grp_expand_ranges_long(h->ix.d_res.as<uint8_t>(), h->d_tables.as<DevTables>(), h->cfg,
+                                    h->ix.u_gpos.as<uint32_t>(), h->ix.u_len.as<uint16_t>(), h->ix.g_mass.as<double>(),
+                                    h->ix.g_pay.as<uint64_t>(), h->ix.g_eoff.as<uint64_t>(), rg, llist.as<uint32_t>(),
                                     lcount.as<uint32_t>(), n_listed, x_mass.as<double>(), x_base.as<uint32_t>(),
                                     x_pat.as<uint32_t>(), s);
       break;
@@ -1322,7 +1349,7 @@ void expand_ranges(dbi_handle* h, const ExpRanges& rg, uint64_t n_tiles, uint64_
   }
   // per tile: the range and two searches of g_eoff; per entry 16 written.  The group records a tile reads (offset,
   // mass, payload, site masks; between 1 and kExpTile + 1 of them) are not counted.
-  h->st.algo_bytes[DBI_STAGE_FETCH] += n_tiles * (28 + 16ull * (uint64_t)bit_length(h->n_groups)) + n_out * 16;
+  h->st.algo_bytes[DBI_STAGE_FETCH] += n_tiles * (28 + 16ull * (uint64_t)bit_length(h->cnt.n_groups)) + n_out * 16;
 }
 
 void mg_release(dbi_handle* h);  // capi_mg.inl
@@ -1332,37 +1359,12 @@ void mg_release(dbi_handle* h);  // capi_mg.inl
 // views are open (DBI_MUTATES), so none of this can go stale.  The windows keep only their peer mappings: a view
 // reads the other ranks' tables as its owner does, and never hands a window back (mg_release).
 void view_share_index(dbi_handle* v, const dbi_handle* o) {
-  using Buf = DevBuf dbi_handle::*;
-  const Buf bufs[] = {
-      &dbi_handle::d_tables, &dbi_handle::d_res,   &dbi_handle::d_pstart, &dbi_handle::u_mass, &dbi_handle::u_gpos,
-      &dbi_handle::u_prot,   &dbi_handle::u_len,   &dbi_handle::u_plo,    &dbi_handle::plist,  &dbi_handle::e_mass,
-      &dbi_handle::e_base,   &dbi_handle::e_pat,   &dbi_handle::u_cmask,  &dbi_handle::d_nlong, &dbi_handle::g_mass,
-      &dbi_handle::g_pay,    &dbi_handle::g_eoff};
-  for (auto b : bufs) (v->*b).borrow((o->*b).p, (o->*b).bytes);
+  v->d_tables.borrow(o->d_tables.p, o->d_tables.bytes);
+  for (const auto& b : kIndexBufs) (v->ix.*b.buf).borrow((o->ix.*b.buf).p, (o->ix.*b.buf).bytes);
   v->built = o->built;
-  v->packed_prot = o->packed_prot;
-  v->res_end = o->res_end;
-  v->res_alloc = o->res_alloc;
-  v->n_emitted = o->n_emitted;
-  v->n_unique = o->n_unique;
-  v->n_entries = o->n_entries;
-  v->cmask_n = o->cmask_n;
-  v->n_groups = o->n_groups;
-  v->n_long = o->n_long;
-  v->mg_rank = o->mg_rank;
-  v->mg_world = o->mg_world;
-  for (int w = 0; w < 3; ++w) {
-    std::memcpy(v->win[w].peer, o->win[w].peer, sizeof(o->win[w].peer));
-    std::memcpy(v->win[w].peer_cap, o->win[w].peer_cap, sizeof(o->win[w].peer_cap));
-  }
-  std::memcpy(v->prot_off, o->prot_off, sizeof(o->prot_off));
-  std::memcpy(v->pos_off, o->pos_off, sizeof(o->pos_off));
-  v->mg_layout = o->mg_layout;
-  v->ent_base_off = o->ent_base_off;
-  std::memcpy(v->uoff, o->uoff, sizeof(o->uoff));
-  std::memcpy(v->uniq_cap, o->uniq_cap, sizeof(o->uniq_cap));
-  std::memcpy(v->mg_thr, o->mg_thr, sizeof(o->mg_thr));
-  std::memcpy(v->mg_nthr, o->mg_nthr, sizeof(o->mg_nthr));
+  v->cnt = o->cnt;
+  v->lay = o->lay;
+  v->rt = o->rt;
   v->cfg = o->cfg;
   v->shifts = o->shifts;
   // the owner's index counters; the launches, bytes and times are the view's own
@@ -1686,9 +1688,9 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
     set_error("Indexer is not initialized");
     return DBI_ENOTINIT;
   }
-  if (begin > h->n_entries || count > h->n_entries - begin) {
+  if (begin > h->cnt.n_entries || count > h->cnt.n_entries - begin) {
     set_error("entry range [%llu, +%llu) outside the index (%llu entries)", (unsigned long long)begin,
-              (unsigned long long)count, (unsigned long long)h->n_entries);
+              (unsigned long long)count, (unsigned long long)h->cnt.n_entries);
     return DBI_EINVAL;
   }
   if (n_prot_ids) *n_prot_ids = 0;
@@ -1704,7 +1706,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   const uint32_t* ep = h->entry_pat();
   uint64_t fb = begin;
   DevBuf x_mass, x_base, x_pat, rng;
-  if (h->n_groups) {  // compact index: K6q expands the range first
+  if (h->cnt.n_groups) {  // compact index: K6q expands the range first
     const uint64_t NT = (count + kExpTile - 1) / kExpTile;
     const uint64_t hr[5] = {begin, 0, count, 0, NT};  // begin | out_off | tile_off
     rng.alloc(40 + NT * 4, h->arena);
@@ -1726,7 +1728,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   uint64_t total_ids = 0;
   {
     Stage sg(h, DBI_STAGE_FETCH);
-    launch_fetch_sizes(eb, h->ent_base_off, uv, fb, count, sizes.as<uint32_t>(), tcnt.as<uint32_t>(), s);
+    launch_fetch_sizes(eb, h->rt.ent_base_off, uv, fb, count, sizes.as<uint32_t>(), tcnt.as<uint32_t>(), s);
     launch_scan_u32_to_u64(tcnt.as<uint32_t>(), tiles, toff.as<uint64_t>(), s);
     total_ids = read_u64(h, toff.as<uint64_t>() + tiles);
   }
@@ -1746,7 +1748,7 @@ int dbi_fetch(dbi_handle* h, uint64_t begin, uint64_t count, double* mass, uint3
   if (want_ids) o_ids.alloc(total_ids * 4, h->arena);
   {
     Stage sg(h, DBI_STAGE_FETCH);
-    launch_fetch_gather(em, eb, h->ent_base_off, uv, ep, h->d_pstart.as<uint32_t>(), fb, count, sizes.as<uint32_t>(), toff.as<uint64_t>(),
+    launch_fetch_gather(em, eb, h->rt.ent_base_off, uv, ep, h->ix.d_pstart.as<uint32_t>(), fb, count, sizes.as<uint32_t>(), toff.as<uint64_t>(),
                         o_mass.as<double>(), o_prot.as<uint32_t>(), o_off.as<uint32_t>(), o_len.as<uint16_t>(),
                         o_pat.as<uint32_t>(), o_lo.as<uint64_t>(), o_ids.as<uint32_t>(), s);
     h->st.algo_bytes[DBI_STAGE_FETCH] += count * (20 + 8 + 26) + total_ids * 8;
@@ -1790,7 +1792,7 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
   uint32_t* d_over = (uint32_t*)(d_c + nq);
   cnt32.alloc(nq * 4, h->arena);
   stmp.alloc(full_scan_tmp_bytes(nq), h->arena);
-  const bool compact = h->n_groups > 0;
+  const bool compact = h->cnt.n_groups > 0;
   uint64_t H = 0, NS = 0, NT = 0;
   uint32_t over = 0;
   {
@@ -1829,7 +1831,7 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
   const uint32_t* eb = h->entry_base();
   const uint32_t* ep = h->entry_pat();
   const uint64_t* hb = d_b;
-  uint64_t eo = h->ent_base_off;
+  uint64_t eo = h->rt.ent_base_off;
   DevBuf x_mass, x_base, x_pat, tile_q;
   if (compact && H) {
     tile_q.alloc(NT * 4, h->arena);
@@ -1882,7 +1884,7 @@ int query_hits_impl(dbi_handle* h, const double* d_lo, const double* d_hi, uint6
     r.flanks.alloc(NP * 6, h->arena);
     r.seq.alloc(std::max<uint64_t>(SB, 1), h->arena);
     r.ids.alloc(std::max<uint64_t>(PI, 1) * 4, h->arena);
-    launch_peps_gather(h->d_res.as<uint8_t>(), h->d_pstart.as<uint32_t>(), eb, eo, uv,
+    launch_peps_gather(h->ix.d_res.as<uint8_t>(), h->ix.d_pstart.as<uint32_t>(), eb, eo, uv,
                        pep_entry.as<uint32_t>(), r.seq_off.as<uint64_t>(), r.plo.as<uint64_t>(), NP,
                        r.prot.as<uint32_t>(), r.off.as<uint32_t>(), r.len.as<uint16_t>(), r.flanks.as<uint8_t>(),
                        r.seq.as<uint8_t>(), r.ids.as<uint32_t>(), s);
@@ -1990,7 +1992,7 @@ int index_candidates(dbi_handle* h, const double* lo, const double* hi, uint64_t
   }
   search_begin(h);
   const uint32_t n_prot = (uint32_t)(h->h_off.size() - 1);
-  if (h->packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
+  if (h->lay.packed_prot != n_prot) pack_residues(h);  // K1 only when proteins were added since the last pack
 
   MassWindows win;
   upload_windows(h, lo, hi, nq, io, &win, kind);
@@ -2368,12 +2370,13 @@ int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* 
   {
     Stage sg(h, DBI_STAGE_QUERY);
     // compact index: the search runs over the groups, and gid[row] = the peptide found (K11b's input)
-    const GroupView gv{h->g_pay.as<uint64_t>(), h->g_eoff.as<uint64_t>(), h->u_cmask.as<uint64_t>(), h->cfg.n_classes};
-    if (h->n_groups) gid.alloc(n * 8, h->arena);
-    launch_lookup_match(h->d_res.as<uint8_t>(), h->key_mass(), h->n_keys(), h->entry_base(), h->ent_base_off,
+    const GroupView gv{h->ix.g_pay.as<uint64_t>(), h->ix.g_eoff.as<uint64_t>(), h->ix.u_cmask.as<uint64_t>(),
+                       h->cfg.n_classes};
+    if (h->cnt.n_groups) gid.alloc(n * 8, h->arena);
+    launch_lookup_match(h->ix.d_res.as<uint8_t>(), h->key_mass(), h->n_keys(), h->entry_base(), h->rt.ent_base_off,
                         h->entry_pat(), uv, h->d_tables.as<DevTables>(), h->cfg.init_mass, h->cfg.max_mods, d_q, d_off,
                         d_pat, n, L.status.as<uint8_t>(), L.mass.as<double>(), L.entry.as<uint64_t>(),
-                        np32.as<uint32_t>(), d_found, h->n_groups ? &gv : nullptr, gid.as<uint64_t>(), s);
+                        np32.as<uint32_t>(), d_found, h->cnt.n_groups ? &gv : nullptr, gid.as<uint64_t>(), s);
     int rounds = 1;  // the last one probes <= 32 consecutive entries
     for (uint64_t w = h->n_keys(); w > 32; w = w / 33 + 1) ++rounds;
     // rows read (residues, offset, pattern), 32 eight-byte probes per search round, the row's residues compared
@@ -2387,12 +2390,12 @@ int dbi_lookup_peptides(dbi_handle* h, const uint8_t* residues, const uint64_t* 
     DBI_CUDA(cudaMemcpyAsync(&n_found, d_found, 8, cudaMemcpyDeviceToHost, s));
     DBI_CUDA(cudaStreamSynchronize(s));
     L.ids.alloc(std::max<uint64_t>(PI, 1) * 4, h->arena);
-    if (h->n_groups)
-      launch_lookup_gather(L.status.as<uint8_t>(), gid.as<uint64_t>(), nullptr, 0, uv, h->d_pstart.as<uint32_t>(),
+    if (h->cnt.n_groups)
+      launch_lookup_gather(L.status.as<uint8_t>(), gid.as<uint64_t>(), nullptr, 0, uv, h->ix.d_pstart.as<uint32_t>(),
                            L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(), L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
     else
-      launch_lookup_gather(L.status.as<uint8_t>(), L.entry.as<uint64_t>(), h->entry_base(), h->ent_base_off, uv,
-                           h->d_pstart.as<uint32_t>(), L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(),
+      launch_lookup_gather(L.status.as<uint8_t>(), L.entry.as<uint64_t>(), h->entry_base(), h->rt.ent_base_off, uv,
+                           h->ix.d_pstart.as<uint32_t>(), L.plo.as<uint64_t>(), n, L.prot.as<uint32_t>(),
                            L.off.as<uint32_t>(), L.ids.as<uint32_t>(), s);
     // list lengths scanned (4 read, 8 written); per row status + list offset read, first occurrence written;
     // per found row entry, base id, peptide tables (4 + 4 + 16) and protein start read; ids copied
@@ -2549,13 +2552,13 @@ int dbi_debug_emitted(dbi_handle* h, uint64_t capacity, double* mass, uint32_t* 
     set_error("emitted records were not kept (params.keep_emitted) or the index is not built");
     return DBI_ENOTINIT;
   }
-  if (n) *n = h->n_emitted;
-  if (capacity < h->n_emitted) {
+  if (n) *n = h->cnt.n_emitted;
+  if (capacity < h->cnt.n_emitted) {
     if (!mass && !prot && !off && !len) return DBI_OK;  // sizing call
-    set_error("capacity %llu < %llu", (unsigned long long)capacity, (unsigned long long)h->n_emitted);
+    set_error("capacity %llu < %llu", (unsigned long long)capacity, (unsigned long long)h->cnt.n_emitted);
     return DBI_ERANGE;
   }
-  const uint64_t N = h->n_emitted;
+  const uint64_t N = h->cnt.n_emitted;
   cudaStream_t s = h->stream;
   std::vector<uint32_t> gpos(N), pr(N);
   if (N) {
