@@ -745,8 +745,66 @@ bool group_radix(const dbi_handle*) { return std::getenv("DBI_GROUP_RADIX") != n
 // tests and benchmarks can compare the two layouts on small proteomes
 bool compact_variants(const dbi_handle*) { return std::getenv("DBI_COMPACT_VARIANTS") != nullptr; }
 
-// K7 + K8: sort N records by (mass, sequence hash, arrival order), merge equal peptides into
-// the handle's unique tables (u_*, plist).
+// The hash pre-sort of large builds (K7 twice): idx[0] <- the records in (mass, hash & mask(hash_bits),
+// arrival order), hash <- every record's hash; returns the buffer index of the sorted mass keys.
+int hash_presort(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks, uint32_t seed, int hash_bits,
+                 DevBuf& hash, DevBuf* idx, DevBuf* hkey, DevBuf* mkey, DevBuf& tmp) {
+  cudaStream_t s = h->stream;
+  const bool wide = hash_bits > 32;
+  const int nbits = ks.nbits;
+  Stage sg(h, DBI_STAGE_SORT_BASE);
+  hash.alloc(N * (wide ? 8 : 4), h->arena);
+  hkey[0].alloc(N * (wide ? 8 : 4), h->arena);
+  hkey[1].alloc(N * (wide ? 8 : 4), h->arena);
+  launch_hash_records(h->ix.d_res.as<uint8_t>(), r.gpos, r.len, N, seed, wide, hash.p, idx[0].as<uint32_t>(), s);
+  DBI_CUDA(cudaMemcpyAsync(hkey[0].p, hash.p, N * (wide ? 8 : 4), cudaMemcpyDeviceToDevice, s));
+  // less significant key first: sequence hash ...
+  uint32_t* ix[2] = {idx[0].as<uint32_t>(), idx[1].as<uint32_t>()};
+  int r1;
+  if (wide) {
+    uint64_t* hk[2] = {hkey[0].as<uint64_t>(), hkey[1].as<uint64_t>()};
+    r1 = radix_sort_pairs<uint64_t, uint32_t>(hk, ix, N, 0, hash_bits, tmp.p, s, nullptr);
+  } else {
+    uint32_t* hk[2] = {hkey[0].as<uint32_t>(), hkey[1].as<uint32_t>()};
+    r1 = radix_sort_pairs<uint32_t, uint32_t>(hk, ix, N, 0, 32, tmp.p, s, nullptr);
+  }
+  DomProbe base_probe(h);
+  // the largest K7 sort of the build: the base sort, unless the variant groups go through K7 too
+  const bool base_is_dominant =
+      h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->rt.mg_world <= 1 && !group_radix(h)));
+  if (base_is_dominant) {  // a retry re-runs the sort: count only the final attempt
+    h->spans.erase(std::remove_if(h->spans.begin(), h->spans.end(),
+                                  [](const dbi_handle::Span& sp) { return sp.kind == kSpanDominant; }),
+                   h->spans.end());
+    h->st.dom_kernel = 0;
+    h->st.dom_bytes_per_launch = N * 24ull;
+  }
+  // ... then the exact mass bits (stable), so order = (mass, hash, arrival order)
+  launch_gather_mass_key(r.mass, ix[r1], N, ks.base_bits, mkey[0].as<uint64_t>(), s);
+  uint64_t* mk[2] = {mkey[0].as<uint64_t>(), mkey[1].as<uint64_t>()};
+  uint32_t* ix2[2] = {ix[r1], ix[r1 ^ 1]};
+  const int r2 = radix_sort_pairs<uint64_t, uint32_t>(mk, ix2, N, 0, nbits, tmp.p, s,
+                                                      base_is_dominant ? &base_probe : nullptr);
+  // normalise: sorted idx in idx[0]
+  if (ix2[r2] != idx[0].as<uint32_t>()) idx[0].swap(idx[1]);
+  const int hpasses = (hash_bits + 7) / 8, mpasses = (nbits + 7) / 8;
+  const uint64_t hw = wide ? 8 : 4;
+  h->st.algo_bytes[DBI_STAGE_SORT_BASE] += N * (16 /*hash: len + gpos*/ + 3 * hw + 4 + 8 + 8 + 4) +
+                                           N * 2 * (hw + 4) * hpasses + N * 24ull * mpasses + N * 20;
+  return r2;
+}
+
+// Builds of fewer records than this order the base records with the mass-only K7 + K8r; larger ones keep
+// the hash pre-sort.  Records with bit-equal masses (isomers and repeats) grow with N: at cfg1 / cfg2
+// size (2.7 M records) the longest equal-mass run has 244 records and K8r costs less than the four hash
+// passes it replaces, while at 514 M (cfg3) runs are long enough that one CTA per run loses to K7.
+constexpr uint64_t kRunOrderMaxRecords = 1ull << 23;
+
+// K7 (+ K8r) + K8: sort N records by (mass, sequence hash, arrival order), merge equal peptides into
+// the handle's unique tables (u_*, plist).  Below kRunOrderMaxRecords K7 sorts by mass alone (stable,
+// so every run of equal mass sits in arrival order) and K8r then orders each such run by (hash, arrival
+// order), hashing only records that share their mass bits with another one.  Above it K7 sorts by the
+// hash of every record and then, stably, by mass.  Both give the same order.
 int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) {
   cudaStream_t s = h->stream;
   if (N >= (1ull << 32)) {
@@ -765,7 +823,8 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
   const int nbits = ks.nbits;
   h->st.sort_bits_base = (uint32_t)nbits + 32;
 
-  DevBuf hash, idx[2], hkey[2], mkey[2], tmp, flags, tile_counts, tile_offs;
+  DevBuf hash, idx[2], hkey[2], mkey[2], tmp, flags, tile_counts, tile_offs, rlist;
+  const bool run_order = N < kRunOrderMaxRecords;
   const uint64_t tiles = (N + kScanTile - 1) / kScanTile;
   TR("ir_begin");
   // Width of the sequence hash: the number of distinct-string pairs with bit-equal mass grows with
@@ -783,68 +842,60 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
   flags.alloc(N, h->arena);
   tile_counts.alloc(tiles * 4, h->arena);
   tile_offs.alloc((tiles + 1) * 8, h->arena);
+  if (run_order) rlist.alloc((run_order_list_cap(N) + 1) * 4, h->arena);  // [0]: count, then the listed run heads
 
   TR("ir_alloc");
   int sorted = 0;
+  if (run_order) {
+    Stage sg(h, DBI_STAGE_SORT_BASE);
+    launch_mass_key(r.mass, N, base_bits, mkey[0].as<uint64_t>(), idx[0].as<uint32_t>(), s);
+    DomProbe base_probe(h);
+    // the largest K7 sort of the build: the base sort, unless the variant groups go through K7 too
+    const bool base_is_dominant =
+        h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->rt.mg_world <= 1 && !group_radix(h)));
+    if (base_is_dominant) {  // count only this sort's passes
+      h->spans.erase(std::remove_if(h->spans.begin(), h->spans.end(),
+                                    [](const dbi_handle::Span& sp) { return sp.kind == kSpanDominant; }),
+                     h->spans.end());
+      h->st.dom_kernel = 0;
+      h->st.dom_bytes_per_launch = N * 24ull;
+    }
+    uint64_t* mk[2] = {mkey[0].as<uint64_t>(), mkey[1].as<uint64_t>()};
+    uint32_t* ix[2] = {idx[0].as<uint32_t>(), idx[1].as<uint32_t>()};
+    sorted = radix_sort_pairs<uint64_t, uint32_t>(mk, ix, N, 0, nbits, tmp.p, s, base_is_dominant ? &base_probe : nullptr);
+    // normalise: sorted keys in mkey[sorted], sorted idx in idx[0]
+    if (sorted) idx[0].swap(idx[1]);
+    const int mpasses = (nbits + 7) / 8;
+    h->st.algo_bytes[DBI_STAGE_SORT_BASE] += N * (8 + 8 + 4) /*keys*/ + N * 8 /*histogram*/ + N * 24ull * mpasses;
+  }
   uint64_t n_unique = 0;
   for (uint32_t attempt = 0;; ++attempt) {
     const bool wide = hash_bits > 32;
     h->st.sort_bits_base = (uint32_t)(nbits + hash_bits);
-    {
-      Stage sg(h, DBI_STAGE_SORT_BASE);
-      const uint32_t seed = 0x9e3779b9u * attempt;
-      hash.alloc(N * (wide ? 8 : 4), h->arena);
-      hkey[0].alloc(N * (wide ? 8 : 4), h->arena);
-      hkey[1].alloc(N * (wide ? 8 : 4), h->arena);
-      launch_hash_records(h->ix.d_res.as<uint8_t>(), r.gpos, r.len, N, seed, wide, hash.p, idx[0].as<uint32_t>(), s);
-      DBI_CUDA(cudaMemcpyAsync(hkey[0].p, hash.p, N * (wide ? 8 : 4), cudaMemcpyDeviceToDevice, s));
-      // less significant key first: sequence hash ...
-      uint32_t* ix[2] = {idx[0].as<uint32_t>(), idx[1].as<uint32_t>()};
-      int r1;
-      if (wide) {
-        uint64_t* hk[2] = {hkey[0].as<uint64_t>(), hkey[1].as<uint64_t>()};
-        r1 = radix_sort_pairs<uint64_t, uint32_t>(hk, ix, N, 0, hash_bits, tmp.p, s, nullptr);
-      } else {
-        uint32_t* hk[2] = {hkey[0].as<uint32_t>(), hkey[1].as<uint32_t>()};
-        r1 = radix_sort_pairs<uint32_t, uint32_t>(hk, ix, N, 0, 32, tmp.p, s, nullptr);
-      }
-      DomProbe base_probe(h);
-      // the largest K7 sort of the build: the base sort, unless the variant groups go through K7 too
-      const bool base_is_dominant =
-          h->p.profile && (h->cfg.max_mods == 0 || (h->cfg.n_seq > 0 && h->rt.mg_world <= 1 && !group_radix(h)));
-      if (base_is_dominant) {  // a retry re-runs the sort: count only the final attempt
-        h->spans.erase(std::remove_if(h->spans.begin(), h->spans.end(),
-                                      [](const dbi_handle::Span& sp) { return sp.kind == kSpanDominant; }),
-                       h->spans.end());
-        h->st.dom_kernel = 0;
-        h->st.dom_bytes_per_launch = N * 24ull;
-      }
-      // ... then the exact mass bits (stable), so order = (mass, hash, arrival order)
-      launch_gather_mass_key(r.mass, ix[r1], N, base_bits, mkey[0].as<uint64_t>(), s);
-      uint64_t* mk[2] = {mkey[0].as<uint64_t>(), mkey[1].as<uint64_t>()};
-      uint32_t* ix2[2] = {ix[r1], ix[r1 ^ 1]};
-      const int r2 = radix_sort_pairs<uint64_t, uint32_t>(mk, ix2, N, 0, nbits, tmp.p, s,
-                                                          base_is_dominant ? &base_probe : nullptr);
-      sorted = r2;
-      // normalise: sorted keys in mkey[sorted], sorted idx in idx[0]
-      if (ix2[r2] != idx[0].as<uint32_t>()) idx[0].swap(idx[1]);
-      const int hpasses = (hash_bits + 7) / 8, mpasses = (nbits + 7) / 8;
-      const uint64_t hw = wide ? 8 : 4;
-      h->st.algo_bytes[DBI_STAGE_SORT_BASE] += N * (16 /*hash: len + gpos*/ + 3 * hw + 4 + 8 + 8 + 4) +
-                                               N * 2 * (hw + 4) * hpasses + N * 24ull * mpasses + N * 20;
-    }
+    const uint32_t seed = 0x9e3779b9u * attempt;
+    if (!run_order) sorted = hash_presort(h, r, N, ks, seed, hash_bits, hash, idx, hkey, mkey, tmp);
     {
       Stage sg(h, DBI_STAGE_DEDUP);
+      // K8r: equal-mass runs by (hash, arrival order); independent of the order a previous attempt left
+      if (run_order) {
+        hash.alloc(N * (wide ? 8 : 4), h->arena);
+        launch_run_order(h->ix.d_res.as<uint8_t>(), mkey[sorted].as<uint64_t>(), idx[0].as<uint32_t>(),
+                         idx[1].as<uint32_t>(), r.gpos, r.len, N, seed, hash_bits, hash.p, rlist.as<uint32_t>() + 1,
+                         rlist.as<uint32_t>(), s);
+      }
       launch_dedup_flags(h->ix.d_res.as<uint8_t>(), mkey[sorted].as<uint64_t>(), idx[0].as<uint32_t>(), hash.p,
                          hash_bits, r.gpos, r.len, N, flags.as<uint8_t>(), tile_counts.as<uint32_t>(),
                          h->d_err.as<uint32_t>(), s);
       launch_scan_u32_to_u64(tile_counts.as<uint32_t>(), tiles, tile_offs.as<uint64_t>(), s);
       n_unique = read_u64(h, tile_offs.as<uint64_t>() + tiles);
+      // K8r streams the keys and indices (the hashing of run members is not counted); K8 flags
+      h->st.algo_bytes[DBI_STAGE_DEDUP] += (run_order ? N * (8 + 4) : 0) + N * (8 + 4 + 1);
     }
     const uint32_t e = read_err(h);
     TR("ir_sort+flags+sync");
     if (e & kErrHashCollision) {
-      // two different sequences with equal mass bits and equal hash: re-sort with another seed
+      // two different sequences with equal mass bits and equal hash: re-order the runs with another
+      // seed and a wider hash (on the K8r path the mass sort stays valid)
       h->st.n_hash_retries++;
       const uint32_t cleared = e & ~kErrHashCollision;
       DBI_CUDA(cudaMemcpyAsync(h->d_err.p, &cleared, 4, cudaMemcpyHostToDevice, s));
@@ -886,7 +937,7 @@ int sort_dedup(dbi_handle* h, const RecView& r, uint64_t N, const KeySpace& ks) 
                       tile_offs.as<uint64_t>(), r.gpos, r.prot, r.len, N, base_bits, n_unique,
                       h->ix.u_mass.as<double>(), h->ix.u_gpos.as<uint32_t>(), h->ix.u_prot.as<uint32_t>(),
                       h->ix.u_len.as<uint16_t>(), h->ix.u_plo.as<uint64_t>(), h->ix.plist.as<uint32_t>(), s);
-    h->st.algo_bytes[DBI_STAGE_DEDUP] += N * (8 + 4 + 1) + N * (1 + 4 + 4 + 4) + n_unique * (8 + 4 + 4 + 2 + 8 + 10);
+    h->st.algo_bytes[DBI_STAGE_DEDUP] += N * (1 + 4 + 4 + 4) + n_unique * (8 + 4 + 4 + 2 + 8 + 10);
   }
   TR("ir_dedup_emit");
   return DBI_OK;

@@ -122,14 +122,25 @@ void launch_win_pmax(const uint64_t* key, const uint64_t* val, uint64_t n, doubl
                      double* w_lo, double* w_pmax, cudaStream_t s);
 
 // ---- sort helpers / K8 dedup -------------------------------------------------
-// hash[i] = seeded hash of the residues of record i (u32, or u64 when wide); idx[i] = i.
+// Hash pre-sort of large builds: hash[i] = seeded hash of the residues of record i (u32, or u64 when
+// wide), idx[i] = i; then key[i] = mass_bits[idx[i]] - base_bits
 void launch_hash_records(const uint8_t* d_res, const uint32_t* gpos, const uint16_t* len, uint64_t n, uint32_t seed,
                          bool wide, void* hash, uint32_t* idx, cudaStream_t s);
-// key[i] = mass_bits[idx[i]] - base_bits
 void launch_gather_mass_key(const uint64_t* mass_bits, const uint32_t* idx, uint64_t n, uint64_t base_bits,
                             uint64_t* key, cudaStream_t s);
+// key[i] = mass_bits[i] - base_bits, idx[i] = i: the input of the mass-only base sort
+void launch_mass_key(const uint64_t* mass_bits, uint64_t n, uint64_t base_bits, uint64_t* key, uint32_t* idx,
+                     cudaStream_t s);
+// K8r: after the mass sort (skey, sidx), orders every run of equal skey by (hash & mask(hash_bits),
+// record index), rewriting its sidx slots, and writes hash[r] (u32, or u64 when hash_bits > 32) of
+// every record r of such a run.  alt: n spare u32 slots; list: run_order_list_cap(n) u32; n_list: 1 u32.
+uint64_t run_order_list_cap(uint64_t n);
+void launch_run_order(const uint8_t* d_res, const uint64_t* skey, uint32_t* sidx, uint32_t* alt,
+                      const uint32_t* gpos, const uint16_t* len, uint64_t n, uint32_t seed, int hash_bits, void* hash,
+                      uint32_t* list, uint32_t* n_list, cudaStream_t s);
 // head flag of every sorted record + per-tile head counts (tile = kScanTile).
-// (hash: u32[n] when hash_bits <= 32, else u64[n] of which the low hash_bits were sorted)
+// (hash: u32[n] when hash_bits <= 32, else u64[n] of which the low hash_bits order a run; read only
+// for records whose sorted neighbour has the same key)
 void launch_dedup_flags(const uint8_t* d_res, const uint64_t* skey, const uint32_t* sidx, const void* hash,
                         int hash_bits, const uint32_t* gpos, const uint16_t* len, uint64_t n, uint8_t* flags,
                         uint32_t* tile_counts, uint32_t* d_err, cudaStream_t s);
