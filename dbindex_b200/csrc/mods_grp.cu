@@ -352,12 +352,16 @@ constexpr uint8_t kSlowGroup = 0xfe;   // k = 4, or the tile's list pool is full
 //   k = 3: block = MIDDLE site p;  entries = (sites of the first class below p) x (sites of the
 //          third class above p), the third site running fastest;
 //   k = 4: block = second site p;  entries = (first-class sites below p) x (pairs i2 < i3 above p).
-// (The order of the entries INSIDE a group is free: they all have the same mass and peptide.)
-// Phase 1 (thread per group) turns the site masks of a group into byte LISTS of site positions in a
-// shared pool and appends one record per block that overlaps the tile; phase 2 max-scans the block
+// (The order of the entries INSIDE a group is free for the index, but group_entry_rank, the compact
+// index's peptide lookup, inverts exactly this order: it is fixed.)
+// Phase 1 turns the site masks of a group into byte LISTS of site positions in a shared pool and
+// appends one record per block that overlaps the tile, with constant work per lane: a warp takes up to
+// 32 consecutive groups, sizes their lists and blocks by popcounts (lane per group), then fills the
+// lists (lane per list byte) and the block records (lane per block site); phase 2 max-scans the block
 // heads so that every entry knows its block; phase 3 (thread per entry) is then
 //   rank in block -> (a, b) by one multiplication -> two byte loads -> pattern -> three coalesced stores.
 constexpr int ET_THREADS = 128;
+constexpr int ET_WARPS = ET_THREADS / 32;
 constexpr int ET_PER = kExpTile / ET_THREADS;
 constexpr int EP_POOL = 3072;  // bytes of site lists shared by the groups of a tile; pool[0] = 0 = "no site"
 
@@ -371,26 +375,43 @@ struct ExpBlk {    // 16 bytes, read with one LDS.128
   uint32_t k;      // class-sequence length, or kLongGroup / kSlowGroup
 };
 
+// The groups' masses, peptides and sequences are not kept here: phase 3 reads them from skey / spay, whose lines
+// phase 1 has just brought into L1 (consecutive entries share a group).  The kernel is bound by the tiles in flight:
+// 13.7 KB and 32 registers (launch bound 15) let 15 CTAs share an SM, where 22.3 KB allowed 9.
 struct ExpSmem {
-  double mass[EX_GMAX];
-  uint32_t base[EX_GMAX];
-  uint32_t idx[EX_GMAX];      // row of the group's peptide in the mask table
   uint32_t head[kExpTile];    // (entry << 16 | block slot) at block starts, max-scanned
   ExpBlk blk[kExpTile];       // every listed block owns >= 1 entry of the tile
   uint8_t pool[EP_POOL];
-  uint8_t seq[EX_GMAX];
   uint32_t recip[65];         // ceil(2^20 / n): exact quotient for ranks < 4096
+  uint32_t seqtab[32];        // class sequence v: pack_seq's packed classes | length << 16
   uint32_t nblk, pool_used;
-  uint32_t scratch[ET_THREADS / 32 + 1];
+  uint32_t scratch[ET_WARPS];
 };
 
-// appends (position + 1) of every set bit of c, ascending, to the byte pool; the two 32-bit halves are walked
-// separately (most peptides have fewer than 33 residues: half the instructions of a 64-bit walk)
-__device__ __forceinline__ uint32_t fill_sites(uint64_t c, uint8_t* pool, uint32_t x) {
-  uint32_t lo = (uint32_t)c, hi = (uint32_t)(c >> 32);
-  for (; lo; lo &= lo - 1) pool[x++] = (uint8_t)__ffs((int)lo);
-  for (; hi; hi &= hi - 1) pool[x++] = (uint8_t)(32 + __ffs((int)hi));
-  return x;
+struct RecipTable {
+  uint32_t v[65];
+  constexpr RecipTable() : v() {
+    for (uint32_t n = 1; n <= 64; ++n) v[n] = ((1u << 20) + n - 1u) / n;
+  }
+};
+__device__ const RecipTable kRecip = RecipTable();
+
+// the lane that owns item x of a warp's items: the last lane whose exclusive prefix `beg` is <= x (beg does not
+// decrease over the lanes, and x < the warp's total)
+__device__ __forceinline__ uint32_t owner_lane(uint32_t beg, uint32_t x) {
+  uint32_t o = 0;
+#pragma unroll
+  for (uint32_t d = 16; d > 0; d >>= 1) {
+    const uint32_t v = __shfl_sync(0xffffffffu, beg, o + d);
+    if (v <= x) o += d;
+  }
+  return o;
+}
+
+__device__ __forceinline__ uint64_t shfl64(uint64_t v, uint32_t src) {
+  const uint32_t lo = __shfl_sync(0xffffffffu, (uint32_t)v, src);
+  const uint32_t hi = __shfl_sync(0xffffffffu, (uint32_t)(v >> 32), src);
+  return (uint64_t)hi << 32 | lo;
 }
 
 // pattern of entry q of the block at site p, from the masks (slow path)
@@ -451,109 +472,175 @@ __device__ __forceinline__ void expand_tile(ExpSmem& s, const DigestCfg& cfg, co
                                             uint32_t long_cap, uint32_t* err) {
   const int C = cfg.n_classes;
   const int t = threadIdx.x;
+  const uint32_t lane = lane_id();
   for (int i = t; i < kExpTile; i += ET_THREADS) s.head[i] = 0;
-  if (t <= 64) s.recip[t] = t ? ((1u << 20) + (uint32_t)t - 1u) / (uint32_t)t : 0u;
+  if (t <= 64) s.recip[t] = kRecip.v[t];
+  if (t < 32) {  // the divisions of pack_seq once per tile, not once per group
+    uint32_t pk;
+    const int k = pack_seq((uint32_t)t, C, &pk);
+    s.seqtab[t] = pk | (uint32_t)k << 16;
+  }
   if (t == 0) {
     s.nblk = 0;
     s.pool_used = 1;
     s.pool[0] = 0;
   }
   __syncthreads();
-  // (1) one thread per group: site lists + block records
-  for (uint32_t j = t; j < ngrp; j += ET_THREADS) {
-    const uint64_t g = (uint64_t)g0 + j;
-    const int64_t rel64 = (int64_t)eoff[g] - (int64_t)e0;
-    const int32_t rel = (int32_t)max(rel64, (int64_t)INT32_MIN / 2);
-    const uint64_t pay = spay[g];
-    const uint32_t row = (uint32_t)(pay >> 32);
-    const uint32_t seq = ((uint32_t)pay >> kGrpCntBits) & 31u;
-    uint32_t pk;
-    int k = pack_seq(seq, C, &pk);
-    s.mass[j] = __longlong_as_double((long long)(skey[g] + base_bits));
-    s.base[j] = gid_tab ? gid_tab[row] : row;
-    s.idx[j] = row;
-    s.seq[j] = (uint8_t)seq;
-    if (rel >= (int32_t)tile_n) continue;  // the group of the NEXT tile's first entry starts right after this tile
-    ExpBlk b;
-    b.start = rel; b.grp = (uint16_t)j; b.a0 = 0; b.b0 = 0; b.nb = 1; b.p = 0; b.k = (uint32_t)k;
-    auto append = [&](const ExpBlk& x) {
-      const uint32_t slot = atomicAdd(&s.nblk, 1u);  // < kExpTile: every listed block owns an entry of the tile
+  // appends the block x of every lane with `want`: one shared atomic per warp.  The slots are < kExpTile (every
+  // listed block owns an entry of the tile); their order does not matter, the heads find them.
+  auto append = [&](bool want, const ExpBlk& x) {
+    const unsigned bal = __ballot_sync(0xffffffffu, want);
+    uint32_t slot = 0;
+    if (lane == 0 && bal) slot = atomicAdd(&s.nblk, (uint32_t)__popc(bal));
+    slot = __shfl_sync(0xffffffffu, slot, 0) + (uint32_t)__popc(bal & lanemask_lt());
+    if (want) {
       s.blk[slot] = x;
-      s.head[x.start > 0 ? x.start : 0] = ((uint32_t)(x.start > 0 ? x.start : 0) << 16) | slot;
-    };
-    if (k == 0) {
-      append(b);
-      continue;
+      const int32_t h = x.start > 0 ? x.start : 0;
+      s.head[h] = ((uint32_t)h << 16) | slot;
     }
-    const uint64_t* cm = cmask + (uint64_t)row * (uint64_t)C;
-    const int q0 = seq_class_at(pk, 0), q1 = k > 1 ? seq_class_at(pk, 1) : q0, q2 = k > 2 ? seq_class_at(pk, 2) : q0;
-    const uint64_t c0 = cm[q0];
-    const uint64_t c1 = k > 1 ? cm[q1] : 0ull;
-    const uint64_t c2 = k > 2 ? cm[q2] : 0ull;
-    if (c0 == 0) {  // a peptide longer than 64 residues: K6l writes this group
-      b.k = kLongGroup;
-      append(b);
-      if constexpr (kWindow) {  // the caller grows the list and runs the tile again when it overflows
-        const uint32_t slot = atomicAdd(long_count, 1u);
-        if (slot < long_cap) {
-          long_list[2 * slot] = (uint32_t)g;
-          long_list[2 * slot + 1] = (uint32_t)tile;
+  };
+  // (1) the groups in chunks of up to 32, one chunk per warp at a time (chunks shrink when the tile has few groups,
+  // so that every warp gets some).  No lane loops over the sites or blocks of its own group.
+  const uint32_t chunk = min(32u, (ngrp + ET_WARPS - 1) / ET_WARPS);
+  const uint32_t n_chunks = (ngrp + chunk - 1) / chunk;
+  for (uint32_t ch = (uint32_t)t >> 5; ch < n_chunks; ch += ET_WARPS) {
+    // (1a) lane per group: loads, then list bytes and block sites by popcounts
+    const uint32_t jb = ch * chunk;
+    const uint32_t j = jb + lane;
+    ExpBlk b;
+    b.start = 0; b.grp = (uint16_t)j; b.a0 = 0; b.b0 = 0; b.nb = 1; b.p = 0; b.k = 0;
+    bool single = false;                  // the group is one block record: k <= 1, long or slow
+    uint64_t c0 = 0, c1 = 0, c2 = 0;
+    uint32_t n01 = 0, need = 0, bb = 0;  // n0 | n1 << 8; list bytes; last-level list end, relative to the first list
+    if (lane < chunk && j < ngrp) {
+      const uint64_t g = (uint64_t)g0 + j;
+      const int64_t rel64 = (int64_t)eoff[g] - (int64_t)e0;
+      b.start = (int32_t)max(rel64, (int64_t)INT32_MIN / 2);
+      const uint64_t pay = spay[g];
+      const uint32_t row = (uint32_t)(pay >> 32);
+      const uint32_t seq = ((uint32_t)pay >> kGrpCntBits) & 31u;
+      const uint32_t pk = s.seqtab[seq] & 0xffffu;
+      const int k = (int)(s.seqtab[seq] >> 16);
+      b.k = (uint32_t)k;
+      // a group that starts at or after tile_n is the group of the NEXT tile's first entry: nothing to list
+      single = b.start < (int32_t)tile_n && k == 0;
+      if (b.start < (int32_t)tile_n && k > 0) {
+        const uint64_t* cm = cmask + (uint64_t)row * (uint64_t)C;
+        const int q0 = seq_class_at(pk, 0), q1 = k > 1 ? seq_class_at(pk, 1) : q0;
+        const int q2 = k > 2 ? seq_class_at(pk, 2) : q0;
+        c0 = cm[q0];
+        c1 = k > 1 ? cm[q1] : 0ull;
+        c2 = k > 2 ? cm[q2] : 0ull;
+        if (c0 == 0) {  // a peptide longer than 64 residues: K6l writes this group
+          single = true;
+          b.k = kLongGroup;
+          if constexpr (kWindow) {  // the caller grows the list and runs the tile again when it overflows
+            const uint32_t slot = atomicAdd(long_count, 1u);
+            if (slot < long_cap) {
+              long_list[2 * slot] = (uint32_t)g;
+              long_list[2 * slot + 1] = (uint32_t)tile;
+            }
+          } else if (b.start >= 0 && b.start < (int32_t)kExpTile) {
+            const uint32_t slot = atomicAdd(long_count, 1u);
+            if (slot < long_cap) long_list[slot] = (uint32_t)g; else atomicOr(err, kErrModPos);
+          }
+        } else if (k == 4) {
+          single = true;
+          b.k = kSlowGroup;
+        } else {
+          // lists of the distinct classes of the sequence (a class used at two levels shares its list)
+          const uint32_t n0 = (uint32_t)__popcll(c0);
+          const uint32_t n1 = (k > 1 && q1 != q0) ? (uint32_t)__popcll(c1) : 0u;
+          const uint32_t n2 = (k > 2 && q2 != q0 && q2 != q1) ? (uint32_t)__popcll(c2) : 0u;
+          n01 = n0 | n1 << 8;
+          need = n0 + n1 + n2;
+          // k = 2: blocks over the first site, last level = list 1;  k = 3: blocks over the middle site,
+          // last level = the list of q2 (maybe shared)
+          const uint32_t l1 = n1 ? n0 : 0u;
+          const uint32_t lb = k == 2 ? l1 : (q2 == q0 ? 0u : (q2 == q1 ? l1 : n0 + n1));
+          bb = lb + (uint32_t)__popcll(k == 2 ? c1 : c2);
         }
-      } else if (rel >= 0 && rel < (int32_t)kExpTile) {
-        const uint32_t slot = atomicAdd(long_count, 1u);
-        if (slot < long_cap) long_list[slot] = (uint32_t)g; else atomicOr(err, kErrModPos);
       }
-      continue;
     }
-    // lists of the distinct classes of the sequence (a class used at two levels shares its list)
-    const uint32_t n0 = (uint32_t)__popcll(c0);
-    const uint32_t n1 = (k > 1 && q1 != q0) ? (uint32_t)__popcll(c1) : 0u;
-    const uint32_t n2 = (k > 2 && q2 != q0 && q2 != q1) ? (uint32_t)__popcll(c2) : 0u;
-    const uint32_t need = n0 + n1 + n2;
-    const uint32_t at = k == 4 ? (uint32_t)EP_POOL : atomicAdd(&s.pool_used, need);
-    if (at + need > (uint32_t)EP_POOL) {
+    // pool offsets: a warp-wide exclusive scan, one shared atomic per warp.  The groups that fit form a prefix of
+    // the lanes; the others un-rank their entries from the masks (the same entries).
+    const uint32_t pinc = warp_inclusive_sum(need);
+    const uint32_t pbeg = pinc - need;
+    uint32_t pool0 = 0;
+    if (lane == 31 && pinc) pool0 = atomicAdd(&s.pool_used, pinc);
+    pool0 = __shfl_sync(0xffffffffu, pool0, 31);
+    const bool fits = need && pool0 + pinc <= (uint32_t)EP_POOL;
+    if (need && !fits) {
+      single = true;
       b.k = kSlowGroup;
-      append(b);
-      continue;
     }
-    uint32_t x = fill_sites(c0, s.pool, at);
-    const uint32_t l0 = at;
-    uint32_t l1 = l0, l2 = l0;
-    if (n1) {
-      l1 = x;
-      x = fill_sites(c1, s.pool, x);
-    }
-    if (k > 2) {
-      l2 = q2 == q0 ? l0 : (q2 == q1 ? l1 : x);
-      if (n2) x = fill_sites(c2, s.pool, x);
-    }
-    if (k == 1) {
+    const uint32_t l0 = pool0 + pbeg;
+    if (fits && b.k == 1u) {
+      single = true;
       b.b0 = (uint16_t)l0;
-      b.nb = (uint8_t)n0;
-      append(b);
-      continue;
+      b.nb = (uint8_t)need;
     }
-    // k = 2: blocks over the first site;  k = 3: blocks over the middle site
-    const uint64_t sites = k == 2 ? c0 : c1;
-    const uint64_t cb = k == 2 ? c1 : c2;  // last-level class
-    const uint32_t lb = k == 2 ? l1 : l2;
-    const uint32_t nb_all = (uint32_t)__popcll(cb);
-    int32_t run = rel;
-    for (uint64_t m = sites; m && run < (int32_t)tile_n; m &= m - 1) {
-      const int p = __ffsll((long long)m) - 1;
-      const uint32_t nB = (uint32_t)__popcll(cb & above(p));
-      const uint32_t nA = k == 3 ? (uint32_t)__popcll(c0 & below(p)) : 1u;
-      const uint32_t sz = nA * nB;
-      if (sz == 0) continue;
-      if (run + (int32_t)sz > 0) {
-        b.start = run;
-        b.a0 = k == 3 ? (uint16_t)l0 : (uint16_t)0;
-        b.b0 = (uint16_t)(lb + nb_all - nB);  // the last nB sites of the list lie above p
-        b.nb = (uint8_t)nB;
-        b.p = (uint8_t)p;
-        append(b);
+    append(single, b);
+    // (1b) lane per list byte: (position + 1) of the r-th site of the owner's list
+    const uint32_t fill_n = __reduce_max_sync(0xffffffffu, fits ? pinc : 0u);
+    for (uint32_t x0 = 0; x0 < fill_n; x0 += 32) {
+      const uint32_t x = min(x0 + lane, fill_n - 1);
+      const uint32_t o = owner_lane(pbeg, x);
+      uint32_t r = x - __shfl_sync(0xffffffffu, pbeg, o);
+      const uint32_t on = __shfl_sync(0xffffffffu, n01, o);
+      const uint64_t m0 = shfl64(c0, o), m1 = shfl64(c1, o), m2 = shfl64(c2, o);
+      const uint32_t on0 = on & 0xffu, on1 = on >> 8;
+      uint64_t m = m0;
+      if (r >= on0 + on1) {
+        m = m2;
+        r -= on0 + on1;
+      } else if (r >= on0) {
+        m = m1;
+        r -= on0;
       }
-      run += (int32_t)sz;
+      if (x0 + lane < fill_n) s.pool[pool0 + x] = (uint8_t)(select_bit(m, r) + 1);
+    }
+    // (1c) lane per block site of the k = 2 and 3 groups in the pool.  A block's start is its group's start plus
+    // the sizes of the group's earlier blocks: a segmented scan over the lanes, carried from pass to pass.
+    const uint32_t nu = (fits && b.k >= 2u) ? (uint32_t)__popcll(b.k == 2u ? c0 : c1) : 0u;
+    const uint32_t uinc = warp_inclusive_sum(nu);
+    const uint32_t ubeg = uinc - nu;
+    const uint32_t meta = (b.k == 3u ? 1u : 0u) | l0 << 1 | (l0 + bb) << 13;  // pool indices < EP_POOL < 4096
+    const uint32_t u_n = __shfl_sync(0xffffffffu, uinc, 31);
+    uint32_t carry_o = 32, carry = 0;  // the last pass's last owner and its run so far
+    for (uint32_t x0 = 0; x0 < u_n; x0 += 32) {
+      const uint32_t x = min(x0 + lane, u_n - 1);
+      const uint32_t o = owner_lane(ubeg, x);
+      const uint32_t i = x - __shfl_sync(0xffffffffu, ubeg, o);
+      const uint64_t m0 = shfl64(c0, o), m1 = shfl64(c1, o), m2 = shfl64(c2, o);
+      const uint32_t om = __shfl_sync(0xffffffffu, meta, o);
+      const int32_t orel = __shfl_sync(0xffffffffu, b.start, o);
+      const bool k3 = om & 1u;
+      const uint64_t cb = k3 ? m2 : m1;  // last-level class
+      const int p = select_bit(k3 ? m1 : m0, i);
+      const uint32_t nB = (uint32_t)__popcll(cb & above(p));
+      const uint32_t nA = k3 ? (uint32_t)__popcll(m0 & below(p)) : 1u;
+      const uint32_t sz = x0 + lane < u_n ? nA * nB : 0u;
+      uint32_t inc = sz;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xffffffffu, inc, d);
+        const uint32_t vo = __shfl_up_sync(0xffffffffu, o, d);
+        if ((int)lane >= d && vo == o) inc += v;
+      }
+      const uint32_t run = (o == carry_o ? carry : 0u) + inc - sz;
+      carry_o = __shfl_sync(0xffffffffu, o, 31);
+      carry = __shfl_sync(0xffffffffu, run + sz, 31);
+      ExpBlk u;
+      u.start = orel + (int32_t)run;
+      u.grp = (uint16_t)(jb + o);
+      u.a0 = k3 ? (uint16_t)((om >> 1) & 0xfffu) : (uint16_t)0;
+      u.b0 = (uint16_t)((om >> 13) - nB);  // the last nB sites of the list lie above p
+      u.nb = (uint8_t)nB;
+      u.p = (uint8_t)p;
+      u.k = k3 ? 3u : 2u;
+      // blocks of size 0, wholly before the tile, or from tile_n on are not listed
+      append(sz && u.start + (int32_t)sz > 0 && u.start < (int32_t)tile_n, u);
     }
   }
   __syncthreads();
@@ -596,22 +683,26 @@ __device__ __forceinline__ void expand_tile(ExpSmem& s, const DigestCfg& cfg, co
       const uint32_t pb = s.pool[(br.z & 0xffffu) + (q - a * nb)];
       pat = k == 3u ? (pa | (p1 << 8) | (pb << 16)) : (k == 2u ? (p1 | (pb << 8)) : pb);
     } else if (k == kSlowGroup) {
-      uint32_t pk;
-      const int kk = pack_seq(s.seq[j], C, &pk);
-      const uint64_t* cm = cmask + (uint64_t)s.idx[j] * (uint64_t)C;
+      const uint64_t pay = spay[(uint64_t)g0 + j];
+      const uint32_t seq = ((uint32_t)pay >> kGrpCntBits) & 31u;
+      const uint32_t pk = s.seqtab[seq] & 0xffffu;
+      const int kk = (int)(s.seqtab[seq] >> 16);
+      const uint64_t* cm = cmask + (pay >> 32) * (uint64_t)C;
       pat = group_entry_slow(kk, q, cm[seq_class_at(pk, 0)], kk > 1 ? cm[seq_class_at(pk, 1)] : 0ull,
                              kk > 2 ? cm[seq_class_at(pk, 2)] : 0ull, kk > 3 ? cm[seq_class_at(pk, 3)] : 0ull);
     } else {
       continue;  // long group: K6l
     }
+    const uint64_t g = (uint64_t)g0 + j;
+    const uint32_t row = (uint32_t)(spay[g] >> 32);
     const uint64_t e = o0 + i;
-    e_mass[e] = s.mass[j];
-    e_base[e] = s.base[j];
+    e_mass[e] = __longlong_as_double((long long)(skey[g] + base_bits));
+    e_base[e] = gid_tab ? gid_tab[row] : row;
     e_pat[e] = pat;
   }
 }
 
-__global__ void __launch_bounds__(ET_THREADS, 4)
+__global__ void __launch_bounds__(ET_THREADS, 15)
     grp_expand_tab_kernel(DigestCfg cfg, const uint64_t* __restrict__ cmask, const uint32_t* __restrict__ gid_tab,
                           const uint64_t* __restrict__ skey, const uint64_t* __restrict__ spay,
                           const uint64_t* __restrict__ eoff, const uint32_t* __restrict__ tile_first,
@@ -678,7 +769,7 @@ __global__ void __launch_bounds__(MD_THREADS)
 }
 
 // g_mass (the groups' masses, as bits) stands where K6x reads key + base_bits
-__global__ void __launch_bounds__(ET_THREADS, 4)
+__global__ void __launch_bounds__(ET_THREADS, 15)
     grp_expand_ranges_kernel(DigestCfg cfg, const uint64_t* __restrict__ cmask, const uint64_t* __restrict__ g_mass,
                              const uint64_t* __restrict__ g_pay, const uint64_t* __restrict__ g_eoff, uint64_t n_groups,
                              const ExpRanges rg, double* __restrict__ o_mass, uint32_t* __restrict__ o_base,
